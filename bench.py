@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric: PnP solves/sec (device-timed) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[1] -- 1,048,576 problems x 68-point face
@@ -14,6 +14,8 @@ the only inter-GPU traffic).  The K timed steps are replays of a CUDA graph of u
 Inputs are resident in HBM for `value`; `e2e` runs the same solve through the host-buffer entry
 point (pinned host memory -> H2D -> solve -> D2H of all results) inside the timed region; `e2e_i16` the same
 for a caller that holds its detections as int16; `extra_configs` (one GPU) times the other BASELINE configs.
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs): the inputs are seeded, so two builds
+run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -426,6 +428,33 @@ def extra_configs(dev, sampler_index=0, min_ms=200.0):
 # ------------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------------
+DUMP_SAMPLE = 1 << 16
+
+
+def dump_outputs(path, out, stats):
+    """Write one step's results as float64 DIR/<name>.npy: every per-problem output of solve_report_batch (R, t, euler,
+    res_norm, iters, report, flags, max_idx) for a fixed sample of DUMP_SAMPLE problems of the batch (seeded: the same
+    problems in every run with the same --problems; all of them if the batch is smaller), their indices in
+    problem_index, and the error statistics [depth, roll, pitch, yaw] x classes x STAT_KEYS of the classes that hold
+    problems, listed in statistics_class (depth class 0..11, 12 = all problems; an empty class has no statistics, only
+    n = 0).  21 MB at the default sizes.  The per-problem outputs are bit-identical from run to run; the statistics
+    agree to rounding only (the kernels sum with FP64 atomics, whose order varies)."""
+    import torch
+    B = int(out["R"].shape[0])
+    idx = np.arange(B) if B <= DUMP_SAMPLE else np.sort(np.random.default_rng(0).choice(B, DUMP_SAMPLE, replace=False))
+    sel = torch.from_numpy(idx).to(out["R"].device)
+    arrays = {"problem_index": idx}
+    for k, v in out.items():
+        arrays[k] = v.index_select(0, sel).cpu().numpy()
+    st = np.stack([np.concatenate([stats[q]["by_depth"].numpy(), stats[q]["all"].numpy()[None]])
+                   for q in ("depth", "roll", "pitch", "yaw")])
+    held = st[0, :, 0] > 0                                  # the four quantities share the classes
+    arrays["statistics"], arrays["statistics_class"] = st[:, held], np.flatnonzero(held)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def _largest_divisor(k, cap):
     for d in range(min(k, cap), 0, -1):
         if k % d == 0:
@@ -469,7 +498,7 @@ def run_ours(args):
 
     def stats_of(out):
         last["stats"] = wl.error_statistics(out["report"], gt, lazy="device")   # two kernels, two exchange phases, nothing on the host
-        last["pass"] = out["flags"]
+        last["out"] = out
 
     def step():
         # solve (pattern constants, moments, 14 LM iterations + SO(3) projection + Euler) and the error report with the
@@ -549,6 +578,8 @@ def run_ours(args):
     t_end.record()
     barrier()
     sampler.mark_end()
+    if args.dump_outputs and rank == 0:                     # before anything below can run the step again
+        dump_outputs(args.dump_outputs, last["out"], last["stats"].result())
     kms = (C.c_float * 3)()
     ncall = C.c_int(0)
     kernel_times = "CUDA events around each kernel inside the timed region" + \
@@ -573,7 +604,7 @@ def run_ours(args):
     value = world * B * args.steps / (ms_total * 1e-3)
     params.flags = 0
     st = last["stats"].result()
-    pass_rate = float(last["pass"].all(dim=1).double().mean())
+    pass_rate = float(last["out"]["flags"].all(dim=1).double().mean())
 
     def timed_host(fn, k):
         """wall-clock seconds per call of fn over k calls, barrier on both sides, max over ranks"""
@@ -782,7 +813,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="time eager launches instead of CUDA-graph replays")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra_configs block (other BASELINE configs, FP32, mappings)")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the rank to its GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float64; a fixed sample of %d problems of "
+                         "rank 0's batch, and the error statistics)" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm keeps no outputs")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

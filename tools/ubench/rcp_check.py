@@ -1,5 +1,5 @@
-import sys, ctypes as C, numpy as np, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, ctypes as C, numpy as np, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 from pnp_solver_test_b200 import _lib
 rng = np.random.default_rng(5)
 a = np.concatenate([rng.uniform(0.5, 2.0, 2000000), 10.0 ** rng.uniform(-250, 250, 100000)])
