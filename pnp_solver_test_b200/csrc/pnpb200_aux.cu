@@ -317,30 +317,31 @@ PNP_DEV void fold_camera(const double* K, const double (&R)[9], const double (&t
     }
 }
 
-// o = (u, v); behind = the homogeneous coordinate z / |z| is -1 (the point is behind the camera)
-PNP_DEV void project_folded(const double (&M)[9], const double (&m)[3], double x, double y, double z, double (&o)[2], bool& behind)
+// The projection of one point before its division by |z|: o = (r0, r1), inv = 1 / r2 (:4548 divides by |z|; branch-free,
+// <= 0.5003 ulp); behind = the homogeneous coordinate z / |z| is -1 (the point is behind the camera)
+PNP_DEV void project_folded(const double (&M)[9], const double (&m)[3], double x, double y, double z, double (&o)[2], double& inv, bool& behind)
 {
-    const double r0 = fma(M[0], x, fma(M[1], y, fma(M[2], z, m[0])));
-    const double r1 = fma(M[3], x, fma(M[4], y, fma(M[5], z, m[1])));
+    o[0] = fma(M[0], x, fma(M[1], y, fma(M[2], z, m[0])));
+    o[1] = fma(M[3], x, fma(M[4], y, fma(M[5], z, m[1])));
     const double r2 = fma(M[6], x, fma(M[7], y, fma(M[8], z, m[2])));
-    const double inv = t_rcp<double>(r2);                 // :4548 divides by |z|; branch-free, <= 0.5003 ulp; the
-    o[0] = r0 * fabs(inv); o[1] = r1 * fabs(inv);         // absolute value rides on the multiplies as an operand modifier
+    inv = t_rcp<double>(r2);
     behind = __double2hiint(r2) < 0;
 }
 
 // The three error distances of one landmark (cal_LM_error_distances, TEST_TOOLBOX.py:252-286).  The
 // third component of every difference is a difference of homogeneous coordinates that are exactly +-1
-// (the measured one is +1), so its square is 0 or 4.
-PNP_DEV void landmark_errors(const double (&pe)[2], bool be, const double (&pg)[2], bool bg, double mu, double mv,
-                             double& e0, double& e1, double& e2)
+// (the measured one is +1), so its square is 0 or 4.  The division of each projection by |z| and its
+// difference to the measured pixel are one FMA per coordinate (the absolute value rides on it as an
+// operand modifier); the prediction-vs-GT difference is the difference of the other two.
+PNP_DEV void landmark_errors(const double (&re)[2], double inv_e, bool be, const double (&rg)[2], double inv_g, bool bg,
+                             double mu, double mv, double& e0, double& e1, double& e2)
 {
-    double d0, d1;
-    d0 = mu - pg[0]; d1 = mv - pg[1];                          // LM vs GT (:321)
-    e0 = sqrt_nonneg(fma(d0, d0, fma(d1, d1, bg ? 4.0 : 0.0)));
-    d0 = pe[0] - mu; d1 = pe[1] - mv;                          // prediction vs LM (:326)
-    e1 = sqrt_nonneg(fma(d0, d0, fma(d1, d1, be ? 4.0 : 0.0)));
-    d0 = pe[0] - pg[0]; d1 = pe[1] - pg[1];                    // prediction vs GT (:331)
-    e2 = sqrt_nonneg(fma(d0, d0, fma(d1, d1, (be != bg) ? 4.0 : 0.0)));
+    const double gx = fma(rg[0], fabs(inv_g), -mu), gy = fma(rg[1], fabs(inv_g), -mv);   // GT - LM (:321, squared)
+    const double ex = fma(re[0], fabs(inv_e), -mu), ey = fma(re[1], fabs(inv_e), -mv);   // prediction - LM (:326)
+    e0 = sqrt_nonneg(fma(gx, gx, fma(gy, gy, bg ? 4.0 : 0.0)));
+    e1 = sqrt_nonneg(fma(ex, ex, fma(ey, ey, be ? 4.0 : 0.0)));
+    const double dx = ex - gx, dy = ey - gy;                                                 // prediction - GT (:331)
+    e2 = sqrt_nonneg(fma(dx, dx, fma(dy, dy, (be != bg) ? 4.0 : 0.0)));
 }
 
 template <typename T>
@@ -396,12 +397,12 @@ __global__ void __launch_bounds__(32) k_report_thread(const __grid_constant__ Re
         int i0 = -1, i1 = -1, i2 = -1;
         for (int i = 0; i < a.n; ++i) {
             const double x = (double)sP[3 * i], y = (double)sP[3 * i + 1], z = (double)sP[3 * i + 2];
-            double pe[2], pg[2], e0, e1, e2;
+            double pe[2], pg[2], ie, ig, e0, e1, e2;
             bool be, bg;
-            project_folded(Me, me, x, y, z, pe, be);      // TEST_TOOLBOX.py:312
-            project_folded(Mg, mg, x, y, z, pg, bg);      // :314
+            project_folded(Me, me, x, y, z, pe, ie, be);  // TEST_TOOLBOX.py:312
+            project_folded(Mg, mg, x, y, z, pg, ig, bg);  // :314
             const V2 px = row[i];
-            landmark_errors(pe, be, pg, bg, (double)px.x, (double)px.y, e0, e1, e2);
+            landmark_errors(pe, ie, be, pg, ig, bg, (double)px.x, (double)px.y, e0, e1, e2);
             s0 += e0; if (e0 > m0) { m0 = e0; i0 = i; }
             s1 += e1; if (e1 > m1) { m1 = e1; i1 = i; }
             s2 += e2; if (e2 > m2) { m2 = e2; i2 = i; }
@@ -434,14 +435,16 @@ __global__ void __launch_bounds__(32) k_report_thread(const __grid_constant__ Re
 // RES != 0 fuses the last pass of the moment mapping into it (pnpb200_solve_report_batch): the rows are streamed ONCE
 // for the error report and for res_norm = ||z - hx|| at the state k_iterate stored (RES = 1: LM, PNP_SOLVER_LIB.py:2679-2681;
 // RES = 2: linear F2, :3368-3374) -- the same arithmetic, in the same order, as k_stream_chunk<T, METHOD, 1>.
+// SKEW = false: K^-1 has k01 = k10 = 0, the pixels are normalised with one FMA per coordinate (normalise_px).
 #ifndef PNP_REPORT_UNROLL
-#define PNP_REPORT_UNROLL 2       // landmarks in flight per thread
+#define PNP_REPORT_UNROLL 4       // landmarks in flight per thread
 #endif
 #ifndef PNP_REPORT_MINBLOCKS
-#define PNP_REPORT_MINBLOCKS 12   // one-warp CTAs per SM the register allocation must allow (12 -> <= 168 registers, 3 warps per sub-partition)
+#define PNP_REPORT_MINBLOCKS 11   // one-warp CTAs per SM the register allocation must allow (11 -> <= 184 registers): the two
+                                  // chunk buffers (~19 KB per CTA) admit 11 CTAs per SM, so a tighter cap buys no occupancy
 #endif
 constexpr int kReportUnroll = PNP_REPORT_UNROLL;
-template <typename T, int RES>
+template <typename T, int RES, bool SKEW>
 __global__ void __launch_bounds__(32, PNP_REPORT_MINBLOCKS) k_report_chunk(const __grid_constant__ ReportArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -459,10 +462,12 @@ __global__ void __launch_bounds__(32, PNP_REPORT_MINBLOCKS) k_report_chunk(const
     if (!ok) b = a.B - 1;
     double Re[9], te[3], eu[3], g4[4];
     T st[RES ? PNP_NTAIL : 1];
+    LmResidualState<T> lr;          // RES = 1: the state with gamma folded in, as soon as it is loaded
     load_report_pose(a, b, Re, te, eu, g4);
     if (RES) {
 #pragma unroll
         for (int k = 0; k < PNP_NTAIL; ++k) st[k] = __ldg(a.tail + (size_t)k * a.ld + b);
+        if constexpr (RES == 1) lr.load(st);
     }
     RowStream<T> rs;
     rs.init(sBuf, bars, a.uv, a.B, a.n, a.use_tma /* chunk */, a.row_pitch, lane, a.use_tmap ? &a.tmap : nullptr);
@@ -494,25 +499,20 @@ __global__ void __launch_bounds__(32, PNP_REPORT_MINBLOCKS) k_report_chunk(const
                 const int i = base + k;
                 const T th[3] = { sP[3 * i], sP[3 * i + 1], sP[3 * i + 2] };
                 const double x = (double)th[0], y = (double)th[1], z = (double)th[2];
-                double pe[2], pg[2], e0, e1, e2;
+                double pe[2], pg[2], ie, ig, e0, e1, e2;
                 bool be, bg;
-                project_folded(Me, me, x, y, z, pe, be);  // TEST_TOOLBOX.py:312
-                project_folded(Mg, mg, x, y, z, pg, bg);  // :314
+                project_folded(Me, me, x, y, z, pe, ie, be);  // TEST_TOOLBOX.py:312
+                project_folded(Mg, mg, x, y, z, pg, ig, bg);  // :314
                 const V2 px = row[k];
-                landmark_errors(pe, be, pg, bg, (double)px.x, (double)px.y, e0, e1, e2);
+                landmark_errors(pe, ie, be, pg, ig, bg, (double)px.x, (double)px.y, e0, e1, e2);
                 s0 += e0; if (e0 > m0) { m0 = e0; i0 = i; }
                 s1 += e1; if (e1 > m1) { m1 = e1; i1 = i; }
                 s2 += e2; if (e2 > m2) { m2 = e2; i2 = i; }
                 if (RES) {
                     T bx, by;                                     // nu = K^-1 [u, v, 1]^T (:3305)
-                    normalise_px<T>(px.x, px.y, k00, k01, k02, k10, k11, k12, bx, by);
+                    normalise_px<T, SKEW>(px.x, px.y, k00, k01, k02, k10, k11, k12, bx, by);
                     if (RES == 1) {
-                        const T aa = th[0] * st[0] + th[1] * st[1] + th[2] * st[2];
-                        const T bb = th[0] * st[3] + th[1] * st[4] + th[2] * st[5];
-                        const T cc = th[0] * st[6] + th[1] * st[7] + th[2] * st[8];
-                        const T rx = bx - (st[11] * (aa - bx * cc) + st[9]);    // z - hx (:3750, :2679)
-                        const T ry = by - (st[11] * (bb - by * cc) + st[10]);
-                        acc0 = t_fma(rx, rx, t_fma(ry, ry, acc0));
+                        lr.add(th, bx, by, acc0);                 // z - hx (:3750, :2679)
                     } else {
                         const T db = T(1) + (th[0] * st[0] + th[1] * st[1] + th[2] * st[2]);
                         const T dx = th[0] * st[3] + th[1] * st[4] + th[2] * st[5] + st[6];
@@ -555,6 +555,7 @@ __global__ void __launch_bounds__(32, PNP_REPORT_MINBLOCKS) k_report_chunk(const
             if (RES) {
 #pragma unroll
                 for (int k = 0; k < PNP_NTAIL; ++k) st[k] = __ldg(a.tail + (size_t)k * a.ld + b);
+                if constexpr (RES == 1) lr.load(st);
             }
         }
     }
@@ -1058,6 +1059,14 @@ using namespace pnpb200;
 
 namespace pnpb200 {
 
+template <typename T, int RES, bool SKEW>
+int launch_report_chunk(const ReportArgs<T>& a, unsigned grid, size_t smem, cudaStream_t st)
+{
+    PNP_CUDA_OK(set_dynamic_smem((const void*)k_report_chunk<T, RES, SKEW>, smem));
+    k_report_chunk<T, RES, SKEW><<<grid, 32, smem, st>>>(a);
+    return PNPB200_OK;
+}
+
 bool report_can_fuse(int dtype, int n)
 {
     const RowGeom g = (dtype == PNPB200_DTYPE_F64) ? row_geometry<double>(n) : row_geometry<float>(n);
@@ -1090,6 +1099,7 @@ int report_launch(int dtype, int64_t B, int n, const void* pattern, const void* 
         const unsigned grid = (unsigned)(n_tiles < 0x7fffffffLL ? n_tiles : 0x7fffffffLL);
         const size_t csmem = 2 * sg.buf_bytes + (size_t)n * 3 * esz + 32;
         const int res_mode = fuse ? fuse->res_mode : 0;
+        const bool skew = fuse && (fuse->kinv[1] != 0.0 || fuse->kinv[3] != 0.0);
 #define LAUNCH_REPORT_CHUNK(TT)                                                                                         \
         {                                                                                                               \
             ReportArgs<TT> a;                                                                                           \
@@ -1101,16 +1111,12 @@ int report_launch(int dtype, int64_t B, int n, const void* pattern, const void* 
             a.tail = fuse ? (const TT*)fuse->tail : nullptr; a.ld = fuse ? fuse->ld : 0; a.res = fuse ? (TT*)fuse->res : nullptr; \
             for (int e = 0; e < 6; ++e) a.kinv[e] = fuse ? fuse->kinv[e] : 0.0;                                         \
             a.use_tmap = (sg.pitch == sg.chunk * 2) ? make_row_tensor_map(&a.tmap, uv, (int)sizeof(TT), B, n, sg.chunk) : 0; \
-            if (res_mode == 1) {                                                                                        \
-                PNP_CUDA_OK(set_dynamic_smem((const void*)k_report_chunk<TT, 1>, csmem));                               \
-                k_report_chunk<TT, 1><<<grid, 32, csmem, st>>>(a);                                                      \
-            } else if (res_mode == 2) {                                                                                 \
-                PNP_CUDA_OK(set_dynamic_smem((const void*)k_report_chunk<TT, 2>, csmem));                               \
-                k_report_chunk<TT, 2><<<grid, 32, csmem, st>>>(a);                                                      \
-            } else {                                                                                                    \
-                PNP_CUDA_OK(set_dynamic_smem((const void*)k_report_chunk<TT, 0>, csmem));                               \
-                k_report_chunk<TT, 0><<<grid, 32, csmem, st>>>(a);                                                      \
-            }                                                                                                           \
+            const int rc = (res_mode == 1) ? (skew ? launch_report_chunk<TT, 1, true>(a, grid, csmem, st)               \
+                                                   : launch_report_chunk<TT, 1, false>(a, grid, csmem, st))             \
+                         : (res_mode == 2) ? (skew ? launch_report_chunk<TT, 2, true>(a, grid, csmem, st)               \
+                                                   : launch_report_chunk<TT, 2, false>(a, grid, csmem, st))             \
+                                           : launch_report_chunk<TT, 0, true>(a, grid, csmem, st);                      \
+            if (rc != PNPB200_OK) return rc;                                                                            \
             count_kernel_launches(1);                                                                                   \
         }
         DISPATCH_DTYPE(dtype, LAUNCH_REPORT_CHUNK(double), LAUNCH_REPORT_CHUNK(float));

@@ -399,7 +399,7 @@ __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ Mom
         const bool ok = b < a.B;
         if (!ok) b = a.B - 1;
         Moments<T> mom;
-        T x[12];
+        LmResidualState<T> lr;
         F2Tail<T> f;
         T acc0 = T(0), acc1 = T(0);
         if (PASS == 0) mom.zero();
@@ -408,8 +408,7 @@ __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ Mom
 #pragma unroll
             for (int k = 0; k < PNP_NTAIL; ++k) st[k] = a.tail[(size_t)k * a.ld + b];
             if (method_lm_residual(METHOD)) {
-#pragma unroll
-                for (int k = 0; k < 12; ++k) x[k] = st[k];
+                lr.load(st);
             } else {
 #pragma unroll
                 for (int k = 0; k < 3; ++k) f.phi3[k] = st[k];
@@ -429,12 +428,7 @@ __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ Mom
                 if (PASS == 0) {
                     mom.template add<method_with_w(METHOD), method_with_s(METHOD)>(th, bx, by);
                 } else if (method_lm_residual(METHOD)) {
-                    const T aa = th[0] * x[0] + th[1] * x[1] + th[2] * x[2];
-                    const T bb = th[0] * x[3] + th[1] * x[4] + th[2] * x[5];
-                    const T cc = th[0] * x[6] + th[1] * x[7] + th[2] * x[8];
-                    const T rx = bx - (x[11] * (aa - bx * cc) + x[9]);    // z - hx (:3750, :2679)
-                    const T ry = by - (x[11] * (bb - by * cc) + x[10]);
-                    acc0 = t_fma(rx, rx, t_fma(ry, ry, acc0));
+                    lr.add(th, bx, by, acc0);                 // z - hx (:3750, :2679)
                 } else {
                     const T db = T(1) + (th[0] * f.phi3[0] + th[1] * f.phi3[1] + th[2] * f.phi3[2]);
                     const T dx = th[0] * f.pxn[0] + th[1] * f.pxn[1] + th[2] * f.pxn[2] + f.pxn[3];
@@ -596,11 +590,13 @@ __global__ void __launch_bounds__(kRingWarps * 32) k_stream_warp_tma(const __gri
         const long long b = w0 + p * wstride;
         Moments<T> mom;
         T st[PNP_NTAIL];
+        LmResidualState<T> lr;
         T acc0 = T(0), acc1 = T(0);
         if (PASS == 0) mom.zero();
         else {
 #pragma unroll
             for (int k = 0; k < PNP_NTAIL; ++k) st[k] = a.tail[(size_t)k * a.ld + b];
+            if (method_lm_residual(METHOD)) lr.load(st);
         }
         for (int c = 0; c < cpp; ++c) {
             // refill the slot that was consumed one step ago, then wait for this one
@@ -624,12 +620,7 @@ __global__ void __launch_bounds__(kRingWarps * 32) k_stream_warp_tma(const __gri
                 if (PASS == 0) {
                     mom.template add<method_with_w(METHOD), method_with_s(METHOD)>(th, bx, by);
                 } else if (method_lm_residual(METHOD)) {
-                    const T aa = th[0] * st[0] + th[1] * st[1] + th[2] * st[2];
-                    const T bb = th[0] * st[3] + th[1] * st[4] + th[2] * st[5];
-                    const T cc = th[0] * st[6] + th[1] * st[7] + th[2] * st[8];
-                    const T rx = bx - (st[11] * (aa - bx * cc) + st[9]);      // z - hx (:3750, :2679)
-                    const T ry = by - (st[11] * (bb - by * cc) + st[10]);
-                    acc0 = t_fma(rx, rx, t_fma(ry, ry, acc0));
+                    lr.add(th, bx, by, acc0);                                 // z - hx (:3750, :2679)
                 } else {
                     const T db = T(1) + (th[0] * st[0] + th[1] * st[1] + th[2] * st[2]);
                     const T dx = th[0] * st[3] + th[1] * st[4] + th[2] * st[5] + st[6];

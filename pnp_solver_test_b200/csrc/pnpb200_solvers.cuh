@@ -792,19 +792,15 @@ PNP_DEV T lm_step_core(T (&x)[12], const M& m, const T* __restrict__ sC, T lambd
 template <typename T, int LPP, typename Pts>
 PNP_DEV T lm_residual_direct(const Pts& pts, const T* __restrict__ sP, int n, int sub, const T (&x)[12])
 {
-    const T gam = x[11], d1 = x[9], d2 = x[10];
+    LmResidualState<T> lr;
+    lr.load(x);
     T rr = T(0);
 #pragma unroll 4
     for (int i = sub; i < n; i += LPP) {
-        const T th0 = sP[3 * i], th1 = sP[3 * i + 1], th2 = sP[3 * i + 2];
+        const T th[3] = { sP[3 * i], sP[3 * i + 1], sP[3 * i + 2] };
         T bx, by;
         pts.get(i, bx, by);
-        const T a = th0 * x[0] + th1 * x[1] + th2 * x[2];
-        const T b = th0 * x[3] + th1 * x[4] + th2 * x[5];
-        const T c = th0 * x[6] + th1 * x[7] + th2 * x[8];
-        const T rx = bx - (gam * (a - bx * c) + d1);
-        const T ry = by - (gam * (b - by * c) + d2);
-        rr = t_fma(rx, rx, t_fma(ry, ry, rr));
+        lr.add(th, bx, by, rr);
     }
     return t_sqrt(group_sum<LPP>(rr));
 }
