@@ -221,6 +221,22 @@ int pnpb200_solve_batch_host_px(pnpb200_pipeline* p, int method, int64_t B, int 
                                 int32_t* iters, int32_t* best_pattern);
 
 /*
+ * pnpb200_solve_batch_host_px with the solution check (pnpb200_check_batch) of every chunk on the chunk's stream,
+ * right after its solve, on the pixels in the pipeline's dtype (after widening) and the solve's best_pattern: the
+ * per-problem loop of random_stress_test.py:322 with a verdict per pose, for callers without ground truth.
+ * status [B] int32 (required) and reproj [B, 2] (pipeline dtype, may be NULL) are host buffers filled like the others;
+ * res_norm enters the NONFINITE bit only where it is requested.  Every other output is that of
+ * pnpb200_solve_batch_host_px.  The pipeline allocates the device buffers of the two outputs on its first checked call.
+ */
+int pnpb200_solve_check_batch_host(pnpb200_pipeline* p, int method, int64_t B, int n, int pixel_type,
+                                   const void* uv_host, const void* pattern_host,
+                                   const int32_t* point_index, const double* K,
+                                   const pnpb200_params* params,
+                                   void* R, void* t, void* euler_deg, void* res_norm,
+                                   int32_t* iters, int32_t* best_pattern,
+                                   double reproj_limit_px, int32_t* status, void* reproj);
+
+/*
  * Page-locked host memory for the buffers of the two calls above (cudaHostAlloc): copies from / to pinned memory
  * run asynchronously at full PCIe rate, pageable buffers are staged by the driver and block the submitting thread.
  * write_combined = 1 for buffers the CPU only WRITES (the pixels): not snooped, faster for the device to read,
@@ -312,6 +328,43 @@ int pnpb200_report_batch_strided(int dtype, int64_t B, int n, const void* patter
                                  const double* gt, const double* bounds,
                                  double* report, int64_t report_stride_problem, int64_t report_stride_column,
                                  int32_t* flags, int32_t* max_idx, void* stream);
+
+/*
+ * Per-problem solution check WITHOUT ground truth.  Not a reference function: the reference returns a diverged pose
+ * without any signal (see the conventions above), and its res_norm, taken at the state before the last update, does not
+ * tell the failures apart.  This is the ground-truth-free counterpart of pnpb200_report_batch, for any pose (not only
+ * this library's), and it never changes R, t.  Like the report it uses ALL n_total landmarks of each row; there is no
+ * landmark subset.  Inputs and arithmetic as pnpb200_report_batch (FP32 inputs are widened and computed in FP64).
+ *   pattern      [device] [n_patterns, n_total, 3]; problem b is checked against pattern best_pattern[b]
+ *   best_pattern [device] [B] int32 (as pnpb200_solve_batch returns it), or NULL for pattern 0.  An entry outside
+ *                [0, n_patterns) gives reproj = NaN and PNPB200_CHECK_NONFINITE.
+ *   res_norm     [device] [B] dtype or NULL; only its finiteness is looked at
+ *   status       [device] [B] int32, a set of PNPB200_CHECK_* bits, 0 = nothing found
+ *   reproj       [device] [B, 2] dtype or NULL: (mean, max) over the landmarks of the prediction-vs-landmark distance of
+ *                cal_LM_error_distances (TEST_TOOLBOX.py:252-286), in pixels: report columns 6, 7 with distance_GT = 1
+ *                (bit for bit where the report runs its streaming kernel)
+ *   reproj_limit_px  PNPB200_CHECK_REPROJ is set where the mean exceeds it; <= 0 or NaN disables that bit
+ * What the bits find (C oracle, random_stress_test.py pose distribution, quantised noise-free pixels, seed 42, 8 192
+ * problems, against the 10 cm / 10 deg test of random_stress_test.py; "flagged" = BEHIND or REPROJ at 1 px):
+ *   LM, 68 landmarks: 30.6 % fail.  BEHIND is set on 12.5 % of the problems and every one of them fails; 36.4 % are
+ *   flagged, which catches 85 % of the failures, and 7.1 % of the unflagged problems fail.
+ *   LM, 15 landmarks (Alexander): 35.9 % fail; BEHIND 18.7 %, all failing; 32.6 % flagged, 80 % of the failures caught,
+ *   10.9 % of the unflagged fail.  LM+, 68: 1.05 % fail, all flagged, none of the unflagged fail.
+ *   EIF2, 15: 2.0 % fail and reproject well -- the check does NOT find the failures of EIF2.
+ *   (Multiplying the mean by the ground-truth distance, as report column 6 does, would separate LM-68 better -- 96 % of
+ *   the failures caught, 2.0 % of the unflagged failing -- but needs the ground truth this check does without.)
+ *   1 px assumes whole-pixel, noise-free detections: with pixel noise of sigma px scale the limit with sigma.
+ * Returns PNPB200_ETOOLARGE when the streaming kernel cannot hold every pattern in shared memory.
+ */
+#define PNPB200_CHECK_NONFINITE 1   /* R, t, res_norm (if given) or the reprojection is not finite                     */
+#define PNPB200_CHECK_DEPTH     2   /* t3 <= 0: the pattern is not in front of the camera                               */
+#define PNPB200_CHECK_BEHIND    4   /* a landmark projects with homogeneous coordinate -1 (behind the camera); the      */
+                                    /* reference's projection (perspective_projection :4548) turns it into plausible pixels */
+#define PNPB200_CHECK_REPROJ    8   /* mean reprojection distance > reproj_limit_px                                     */
+int pnpb200_check_batch(int dtype, int64_t B, int n_total, const void* pattern, int n_patterns, const void* uv,
+                        const double* K, const void* R, const void* t, const void* res_norm,
+                        const int32_t* best_pattern, double reproj_limit_px, int32_t* status, void* reproj,
+                        void* stream);
 
 /*
  * Error statistics, two passes so that shards can be combined with two small all-reduce phases

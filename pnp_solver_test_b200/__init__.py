@@ -20,6 +20,8 @@ _LAZY = {
     "PNP_SOLVER": (".solver", "PNP_SOLVER"), "HostPipeline": (".solver", "HostPipeline"), "host_buffer": (".solver", "host_buffer"),
     "solve_batch": (".solver", "solve_batch"), "R_from_euler_batch": (".solver", "R_from_euler_batch"),
     "euler_from_R_batch": (".solver", "euler_from_R_batch"), "project_batch": (".solver", "project_batch"),
+    "check_batch": (".solver", "check_batch"), "CHECK_NONFINITE": ("._lib", "CHECK_NONFINITE"),
+    "CHECK_DEPTH": ("._lib", "CHECK_DEPTH"), "CHECK_BEHIND": ("._lib", "CHECK_BEHIND"), "CHECK_REPROJ": ("._lib", "CHECK_REPROJ"),
 }
 
 

@@ -22,6 +22,8 @@ FLAG_QEIF_DIRECT = 2
 FLAG_LM_TRUE_JACOBIAN = 4
 MAX_PATTERNS = 8
 PIXEL_NATIVE, PIXEL_I16, PIXEL_U16, PIXEL_F32 = 0, 1, 2, 3
+# bits of the status word of the solution check (pnpb200_check_batch)
+CHECK_NONFINITE, CHECK_DEPTH, CHECK_BEHIND, CHECK_REPROJ = 1, 2, 4, 8
 
 EXPORTS = [
     "pnpb200_version", "pnpb200_launch_count", "pnpb200_last_error", "pnpb200_default_params", "pnpb200_default_synth",
@@ -31,6 +33,7 @@ EXPORTS = [
     "pnpb200_fma_peak", "pnpb200_selftest_math", "pnpb200_selftest_sincos", "pnpb200_pipeline_set_packing", "pnpb200_pipeline_last_packed", "pnpb200_pack_i16", "pnpb200_synth_face_variation", "pnpb200_topk_histogram",
     "pnpb200_fragility_accumulate", "pnpb200_write_result_csv", "pnpb200_format_repr", "pnpb200_classify", "pnpb200_classify_drpy", "pnpb200_profile_reset", "pnpb200_profile_read",
     "pnpb200_solve_batch_host_px", "pnpb200_host_alloc", "pnpb200_host_free", "pnpb200_solve_report_batch", "pnpb200_normalise_uvw",
+    "pnpb200_check_batch", "pnpb200_solve_check_batch_host",
 ]
 
 
@@ -67,6 +70,11 @@ for _name in EXPORTS:
     if _name not in ("pnpb200_last_error",):
         getattr(lib, _name).restype = C.c_int
 lib.pnpb200_workspace_bytes.restype = C.c_int64
+_VP, _PD, _PI = C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int32)
+lib.pnpb200_check_batch.argtypes = [C.c_int, C.c_int64, C.c_int, _VP, C.c_int, _VP, _PD, _VP, _VP, _VP, _PI, C.c_double, _PI, _VP,
+                                    _VP]
+lib.pnpb200_solve_check_batch_host.argtypes = [_VP, C.c_int, C.c_int64, C.c_int, C.c_int, _VP, _VP, _PI, _PD, _VP, _VP, _VP, _VP,
+                                               _VP, _PI, _PI, C.c_double, _PI, _VP]
 lib.pnpb200_launch_count.restype = C.c_int64
 
 _ERR = {-1: "EINVAL (bad argument)", -2: "ECUDA (CUDA runtime error)", -3: "ENODEVICE (no usable CUDA device)",

@@ -319,6 +319,8 @@ struct PipeSlot {
     int32_t *d_it = nullptr, *d_best = nullptr;
     int16_t *h_pack = nullptr, *d_pack = nullptr;        // pinned staging / device copy of the packed pixels
     void* d_narrow = nullptr;                             // device copy of a chunk of int16 / uint16 / float32 pixels (solve_batch_host_px)
+    int32_t* d_status = nullptr;                          // outputs of the solution check (solve_check_batch_host), from its first call
+    void* d_reproj = nullptr;
     cudaEvent_t pack_free = nullptr;                      // the H2D copy out of h_pack has finished
     cudaEvent_t h2d_done = nullptr;                       // the slot's last pixel copy has finished (back-pressure)
     cudaEvent_t piece_done[2] = { nullptr, nullptr };     // parts of a plain chunk's pixel copy, two in flight (submit_chunk)
@@ -368,7 +370,7 @@ static void free_slot(PipeSlot& sl)
 {
     if (sl.stream) { cudaStreamSynchronize(sl.stream); cudaStreamDestroy(sl.stream); }
     cudaFree(sl.d_uv); cudaFree(sl.d_R); cudaFree(sl.d_t); cudaFree(sl.d_e); cudaFree(sl.d_res); cudaFree(sl.d_ws);
-    cudaFree(sl.d_it); cudaFree(sl.d_best); cudaFree(sl.d_pack); cudaFree(sl.d_narrow);
+    cudaFree(sl.d_it); cudaFree(sl.d_best); cudaFree(sl.d_pack); cudaFree(sl.d_narrow); cudaFree(sl.d_status); cudaFree(sl.d_reproj);
     if (sl.h_pack) cudaFreeHost(sl.h_pack);
     if (sl.pack_free) cudaEventDestroy(sl.pack_free);
     if (sl.h2d_done) cudaEventDestroy(sl.h2d_done);
@@ -458,6 +460,9 @@ struct HostCall {
     const pnpb200_params* params;
     void *R, *t, *euler_deg, *res_norm;
     int32_t *iters, *best_pattern;
+    int32_t* status;                                      // non-NULL: the solution check runs after each chunk's solve
+    void* reproj;
+    double reproj_limit_px;
 };
 
 // queue one chunk on a slot: pixels host -> device (packed if `packed`), solve, results device -> host.
@@ -500,11 +505,22 @@ int submit_chunk(const HostCall& c, PipeSlot& sl, int64_t done, int64_t nb, bool
     if (c.params) prm = *c.params; else fill_default_params(&prm);
     // always the slot's own scratch: chunks run concurrently on several streams, one caller workspace would be shared by them
     prm.workspace = sl.d_ws; prm.workspace_bytes = (int64_t)p->ws_bytes;
-    const int rc = pnpb200_solve_batch(c.method, p->dtype, nb, p->n_total, c.n, sl.d_uv, p->d_pattern, p->n_patterns,
-                                       c.point_index, c.K, &prm, c.R ? sl.d_R : nullptr, c.t ? sl.d_t : nullptr,
-                                       c.euler_deg ? sl.d_e : nullptr, c.res_norm ? sl.d_res : nullptr,
-                                       c.iters ? sl.d_it : nullptr, c.best_pattern ? sl.d_best : nullptr, st);
+    // the check reads the pose and the winning pattern whether or not the caller asked for them
+    const bool chk = c.status != nullptr, want_best = c.best_pattern || (chk && p->n_patterns > 1);
+    int rc = pnpb200_solve_batch(c.method, p->dtype, nb, p->n_total, c.n, sl.d_uv, p->d_pattern, p->n_patterns,
+                                 c.point_index, c.K, &prm, (c.R || chk) ? sl.d_R : nullptr, (c.t || chk) ? sl.d_t : nullptr,
+                                 c.euler_deg ? sl.d_e : nullptr, c.res_norm ? sl.d_res : nullptr,
+                                 c.iters ? sl.d_it : nullptr, want_best ? sl.d_best : nullptr, st);
     if (rc != PNPB200_OK) return rc;
+    if (chk) {
+        rc = check_launch(p->dtype, nb, p->n_total, p->d_pattern, p->n_patterns, sl.d_uv, c.K, sl.d_R, sl.d_t,
+                          c.res_norm ? sl.d_res : nullptr, p->n_patterns > 1 ? sl.d_best : nullptr, c.reproj_limit_px,
+                          sl.d_status, c.reproj ? sl.d_reproj : nullptr, st);
+        if (rc != PNPB200_OK) return rc;
+        PNP_CUDA_OK(cudaMemcpyAsync(c.status + done, sl.d_status, sizeof(int32_t) * (size_t)nb, cudaMemcpyDeviceToHost, st));
+        if (c.reproj)
+            PNP_CUDA_OK(cudaMemcpyAsync((char*)c.reproj + esz * (size_t)done * 2, sl.d_reproj, esz * (size_t)nb * 2, cudaMemcpyDeviceToHost, st));
+    }
     if (c.R) PNP_CUDA_OK(cudaMemcpyAsync((char*)c.R + esz * (size_t)done * 9, sl.d_R, esz * (size_t)nb * 9, cudaMemcpyDeviceToHost, st));
     if (c.t) PNP_CUDA_OK(cudaMemcpyAsync((char*)c.t + esz * (size_t)done * 3, sl.d_t, esz * (size_t)nb * 3, cudaMemcpyDeviceToHost, st));
     if (c.euler_deg) PNP_CUDA_OK(cudaMemcpyAsync((char*)c.euler_deg + esz * (size_t)done * 3, sl.d_e, esz * (size_t)nb * 3, cudaMemcpyDeviceToHost, st));
@@ -524,10 +540,10 @@ int pnpb200_solve_batch_host(pnpb200_pipeline* p, int method, int64_t B, int n, 
                                        euler_deg, res_norm, iters, best_pattern);
 }
 
-int pnpb200_solve_batch_host_px(pnpb200_pipeline* p, int method, int64_t B, int n, int pixel_type, const void* uv_host,
-                                const void* pattern_host, const int32_t* point_index, const double* K,
-                                const pnpb200_params* params, void* R, void* t, void* euler_deg, void* res_norm,
-                                int32_t* iters, int32_t* best_pattern)
+namespace {
+int solve_host(pnpb200_pipeline* p, int method, int64_t B, int n, int pixel_type, const void* uv_host, const void* pattern_host,
+               const int32_t* point_index, const double* K, const pnpb200_params* params, void* R, void* t, void* euler_deg,
+               void* res_norm, int32_t* iters, int32_t* best_pattern, int32_t* status, void* reproj, double reproj_limit_px)
 {
     if (!p || !uv_host || !pattern_host || !K || B < 0) return PNPB200_EINVAL;
     if (n < 1 || n > p->n_total || (!point_index && n != p->n_total)) return PNPB200_EINVAL;
@@ -543,10 +559,17 @@ int pnpb200_solve_batch_host_px(pnpb200_pipeline* p, int method, int64_t B, int 
             if (!sl.d_narrow) PNP_CUDA_OK(cudaMalloc(&sl.d_narrow, 4 * ((size_t)p->chunk * p->n_total * 2 + 8)));
         }
     }
+    if (status) {                                             // first checked call: the per-slot check outputs
+        for (PipeSlot& sl : p->slots) {
+            if (!sl.d_status) PNP_CUDA_OK(cudaMalloc((void**)&sl.d_status, sizeof(int32_t) * (size_t)p->chunk));
+            if (!sl.d_reproj) PNP_CUDA_OK(cudaMalloc(&sl.d_reproj, esz * (size_t)p->chunk * 2));
+        }
+    }
     PNP_CUDA_OK(cudaMemcpyAsync(p->d_pattern, pattern_host, esz * (size_t)p->n_patterns * p->n_total * 3,
                                 cudaMemcpyHostToDevice, p->slots[0].stream));
     PNP_CUDA_OK(cudaStreamSynchronize(p->slots[0].stream));
-    const HostCall call = { p, method, n, pixel_type, B, uv_host, point_index, K, params, R, t, euler_deg, res_norm, iters, best_pattern };
+    const HostCall call = { p, method, n, pixel_type, B, uv_host, point_index, K, params, R, t, euler_deg, res_norm, iters, best_pattern,
+                            status, reproj, reproj_limit_px };
     const int64_t n_chunks = (B + p->chunk - 1) / p->chunk;
     p->last_chunks = n_chunks; p->last_packed = 0;
     // Chunks are handed out from both ends of the batch: this thread sends chunks as they are from the front
@@ -610,6 +633,26 @@ int pnpb200_solve_batch_host_px(pnpb200_pipeline* p, int method, int64_t B, int 
     if (rc_main != PNPB200_OK) return rc_main;
     if (rc_pack.load() != PNPB200_OK) memcpy(g_last_error, packer_error, sizeof(g_last_error));
     return rc_pack.load();
+}
+}  // namespace
+
+int pnpb200_solve_batch_host_px(pnpb200_pipeline* p, int method, int64_t B, int n, int pixel_type, const void* uv_host,
+                                const void* pattern_host, const int32_t* point_index, const double* K,
+                                const pnpb200_params* params, void* R, void* t, void* euler_deg, void* res_norm,
+                                int32_t* iters, int32_t* best_pattern)
+{
+    return solve_host(p, method, B, n, pixel_type, uv_host, pattern_host, point_index, K, params, R, t, euler_deg, res_norm, iters,
+                      best_pattern, nullptr, nullptr, 0.0);
+}
+
+int pnpb200_solve_check_batch_host(pnpb200_pipeline* p, int method, int64_t B, int n, int pixel_type, const void* uv_host,
+                                   const void* pattern_host, const int32_t* point_index, const double* K,
+                                   const pnpb200_params* params, void* R, void* t, void* euler_deg, void* res_norm,
+                                   int32_t* iters, int32_t* best_pattern, double reproj_limit_px, int32_t* status, void* reproj)
+{
+    if (!status) return PNPB200_EINVAL;
+    return solve_host(p, method, B, n, pixel_type, uv_host, pattern_host, point_index, K, params, R, t, euler_deg, res_norm, iters,
+                      best_pattern, status, reproj, reproj_limit_px);
 }
 
 }  // extern "C"

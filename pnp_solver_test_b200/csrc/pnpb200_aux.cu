@@ -333,15 +333,23 @@ PNP_DEV void project_folded(const double (&M)[9], const double (&m)[3], double x
 // (the measured one is +1), so its square is 0 or 4.  The division of each projection by |z| and its
 // difference to the measured pixel are one FMA per coordinate (the absolute value rides on it as an
 // operand modifier); the prediction-vs-GT difference is the difference of the other two.
+PNP_DEV void px_difference(const double (&r)[2], double inv, double mu, double mv, double& dx, double& dy)
+{
+    dx = fma(r[0], fabs(inv), -mu); dy = fma(r[1], fabs(inv), -mv);
+}
+PNP_DEV double homogeneous_distance(double dx, double dy, bool flipped)
+{
+    return sqrt_nonneg(fma(dx, dx, fma(dy, dy, flipped ? 4.0 : 0.0)));
+}
 PNP_DEV void landmark_errors(const double (&re)[2], double inv_e, bool be, const double (&rg)[2], double inv_g, bool bg,
                              double mu, double mv, double& e0, double& e1, double& e2)
 {
-    const double gx = fma(rg[0], fabs(inv_g), -mu), gy = fma(rg[1], fabs(inv_g), -mv);   // GT - LM (:321, squared)
-    const double ex = fma(re[0], fabs(inv_e), -mu), ey = fma(re[1], fabs(inv_e), -mv);   // prediction - LM (:326)
-    e0 = sqrt_nonneg(fma(gx, gx, fma(gy, gy, bg ? 4.0 : 0.0)));
-    e1 = sqrt_nonneg(fma(ex, ex, fma(ey, ey, be ? 4.0 : 0.0)));
-    const double dx = ex - gx, dy = ey - gy;                                                 // prediction - GT (:331)
-    e2 = sqrt_nonneg(fma(dx, dx, fma(dy, dy, (be != bg) ? 4.0 : 0.0)));
+    double gx, gy, ex, ey;
+    px_difference(rg, inv_g, mu, mv, gx, gy);             // GT - LM (:321, squared)
+    px_difference(re, inv_e, mu, mv, ex, ey);             // prediction - LM (:326)
+    e0 = homogeneous_distance(gx, gy, bg);
+    e1 = homogeneous_distance(ex, ey, be);
+    e2 = homogeneous_distance(ex - gx, ey - gy, be != bg);   // prediction - GT (:331)
 }
 
 template <typename T>
@@ -559,6 +567,161 @@ __global__ void __launch_bounds__(32, PNP_REPORT_MINBLOCKS) k_report_chunk(const
             }
         }
     }
+}
+
+// ------------------------------------------------------------------------------------------
+// solution check without ground truth (SURVEY.md 5, failure detection): per problem, over all n landmarks, the
+// prediction-vs-landmark distance of cal_LM_error_distances (TEST_TOOLBOX.py:252-286) -- report columns 6, 7 with
+// distance_GT = 1, computed as e1 of landmark_errors -- and a status word (PNPB200_CHECK_*).  Problem b is checked
+// against pattern best[b] (pattern 0 without best).
+// ------------------------------------------------------------------------------------------
+template <typename T>
+struct CheckArgs {
+    const T* pattern; const T* uv; const T* R; const T* t; const T* res; const int32_t* best;
+    long long B;
+    int n, n_patterns, row_pitch, chunk;
+    double K[9], limit;             // limit > 0: the REPROJ bit is on
+    int32_t* status; T* reproj;
+    int use_tmap;
+    alignas(64) CUtensorMap tmap;   // uv as a 2-D tensor (RowStream), valid when use_tmap
+};
+
+template <typename T>
+PNP_DEV void load_check_pose(const CheckArgs<T>& a, long long b, double (&R)[9], double (&t)[3], double& res, int& pat)
+{
+#pragma unroll
+    for (int k = 0; k < 3; ++k) t[k] = (double)__ldg(a.t + b * 3 + k);
+#pragma unroll
+    for (int k = 0; k < 9; ++k) R[k] = (double)__ldg(a.R + b * 9 + k);
+    res = a.res ? (double)__ldg(a.res + b) : 0.0;
+    pat = a.best ? __ldg(a.best + b) : 0;
+}
+
+// mean = NaN marks a best_pattern entry outside [0, n_patterns): the problem was checked against nothing
+PNP_DEV int32_t check_status(const double (&R)[9], const double (&t)[3], double res, double mean, double mx, bool behind, double limit)
+{
+    double z = (res - res) + (mean - mean) + (mx - mx);   // x - x is 0 for finite x and NaN for NaN and +-Inf
+#pragma unroll
+    for (int k = 0; k < 9; ++k) z += R[k] - R[k];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) z += t[k] - t[k];
+    int32_t s = 0;
+    if (!(z == 0.0)) s |= PNPB200_CHECK_NONFINITE;
+    if (t[2] <= 0.0) s |= PNPB200_CHECK_DEPTH;
+    if (behind) s |= PNPB200_CHECK_BEHIND;
+    if (limit > 0.0 && mean > limit) s |= PNPB200_CHECK_REPROJ;
+    return s;
+}
+
+template <typename T>
+PNP_DEV void store_check(const CheckArgs<T>& a, long long b, const double (&R)[9], const double (&t)[3], double res, bool bad,
+                         double sum, double mx, bool behind)
+{
+    double mean = sum / a.n;                              // (s1 / n) * distance_GT of the report, distance_GT = 1
+    if (bad) mean = mx = __longlong_as_double(0x7ff8000000000000LL);
+    if (a.reproj) { a.reproj[b * 2] = (T)mean; a.reproj[b * 2 + 1] = (T)mx; }
+    a.status[b] = check_status(R, t, res, mean, mx, behind, a.limit);
+}
+
+// The streaming shape of k_report_chunk: one-warp CTAs, lane <-> problem, the rows through RowStream, every pattern in
+// shared memory.  The landmark loop is the report's e1 in the same order, so mean and max are the report's bits.
+#ifndef PNP_CHECK_MINBLOCKS
+#define PNP_CHECK_MINBLOCKS 16
+#endif
+template <typename T>
+__global__ void __launch_bounds__(32, PNP_CHECK_MINBLOCKS) k_check_chunk(const __grid_constant__ CheckArgs<T> a)
+{
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    typedef typename Vec2<T>::type V2;
+    T* sBuf = reinterpret_cast<T*>(smem_raw);
+    T* sP = sBuf + (size_t)2 * kTileProblems * a.row_pitch;
+    uint64_t* bars = carve_bar<T>(smem_raw, sP + (size_t)a.n_patterns * a.n * 3);
+    const int lane = threadIdx.x;
+    const long long n_tiles = (a.B + kTileProblems - 1) / kTileProblems;
+    long long tile = blockIdx.x;
+    long long b = tile * kTileProblems + lane;
+    bool ok = b < a.B;
+    if (!ok) b = a.B - 1;
+    double R[9], t[3], res;
+    int pat;
+    load_check_pose(a, b, R, t, res, pat);
+    RowStream<T> rs;
+    rs.init(sBuf, bars, a.uv, a.B, a.n, a.chunk, a.row_pitch, lane, a.use_tmap ? &a.tmap : nullptr);
+    if (tile < n_tiles) rs.begin_tile(tile, lane);
+    for (int e = lane; e < a.n_patterns * a.n * 3; e += 32) sP[e] = a.pattern[e];
+    __syncwarp();
+    while (tile < n_tiles) {
+        const bool bad = (unsigned)pat >= (unsigned)a.n_patterns;
+        const T* P = sP + (size_t)(bad ? 0 : pat) * a.n * 3;
+        double M[9], m[3];
+        fold_camera(a.K, R, t, M, m);
+        double s = 0, mx = 0;
+        bool behind = false;
+        for (int c = 0; c < rs.n_chunks; ++c) {
+            const V2* row = rs.wait(c, lane);
+            const int cnt = rs.count(c), base = c * rs.chunk;
+#pragma unroll kReportUnroll
+            for (int k = 0; k < cnt; ++k) {
+                const int i = base + k;
+                double pe[2], ie, ex, ey;
+                bool be;
+                project_folded(M, m, (double)P[3 * i], (double)P[3 * i + 1], (double)P[3 * i + 2], pe, ie, be);   // TEST_TOOLBOX.py:312
+                const V2 px = row[k];
+                px_difference(pe, ie, (double)px.x, (double)px.y, ex, ey);                                           // :326
+                const double e = homogeneous_distance(ex, ey, be);
+                s += e; if (e > mx) mx = e;
+                behind |= be;
+            }
+            rs.done(c, lane);
+        }
+        if (ok) store_check(a, b, R, t, res, bad, s, mx, behind);
+        tile += gridDim.x;
+        if (tile < n_tiles) {
+            fence_proxy_async();
+            rs.begin_tile(tile, lane);
+            b = tile * kTileProblems + lane;
+            ok = b < a.B;
+            if (!ok) b = a.B - 1;
+            load_check_pose(a, b, R, t, res, pat);
+        }
+    }
+}
+
+// Rows the streaming shape cannot take (large n, FP32 rows that are not 16-byte granular): one warp per problem, the
+// lanes stride over the landmarks, the patterns are read from global memory.
+template <typename T>
+__global__ void __launch_bounds__(256) k_check_warp(const __grid_constant__ CheckArgs<T> a)
+{
+    const long long b = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (b >= a.B) return;                                 // whole warps
+    double R[9], t[3], res;
+    int pat;
+    load_check_pose(a, b, R, t, res, pat);
+    const bool bad = (unsigned)pat >= (unsigned)a.n_patterns;
+    const T* P = a.pattern + (size_t)(bad ? 0 : pat) * a.n * 3;
+    double M[9], m[3];
+    fold_camera(a.K, R, t, M, m);
+    double s = 0, mx = 0;
+    bool behind = false;
+    for (int i = lane; i < a.n; i += 32) {
+        double pe[2], ie, ex, ey;
+        bool be;
+        project_folded(M, m, (double)__ldg(P + 3 * i), (double)__ldg(P + 3 * i + 1), (double)__ldg(P + 3 * i + 2), pe, ie, be);
+        const T* px = a.uv + ((size_t)b * a.n + i) * 2;
+        px_difference(pe, ie, (double)__ldg(px), (double)__ldg(px + 1), ex, ey);
+        const double e = homogeneous_distance(ex, ey, be);
+        s += e; if (e > mx) mx = e;
+        behind |= be;
+    }
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) {
+        s += __shfl_xor_sync(0xffffffffu, s, off);
+        const double o = __shfl_xor_sync(0xffffffffu, mx, off);
+        if (o > mx) mx = o;
+    }
+    behind = __any_sync(0xffffffffu, behind);
+    if (lane == 0) store_check(a, b, R, t, res, bad, s, mx, behind);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1148,9 +1311,59 @@ int report_launch(int dtype, int64_t B, int n, const void* pattern, const void* 
     return PNPB200_OK;
 }
 
+// the execution shape of report_launch: the streaming kernel where report_can_fuse, one warp per problem otherwise
+int check_launch(int dtype, int64_t B, int n, const void* pattern, int n_patterns, const void* uv, const double* K,
+                 const void* R, const void* t, const void* res_norm, const int32_t* best_pattern, double limit,
+                 int32_t* status, void* reproj, cudaStream_t st)
+{
+    if (B < 0 || n < 1 || !pattern || !uv || !K || !R || !t || !status) return PNPB200_EINVAL;
+    if (n_patterns < 1 || n_patterns > PNPB200_MAX_PATTERNS) return PNPB200_EINVAL;
+    if (dtype != PNPB200_DTYPE_F64 && dtype != PNPB200_DTYPE_F32) return PNPB200_EINVAL;
+    if (((uintptr_t)uv & 15u) != 0) return PNPB200_EINVAL;   // rows are staged with 16-byte bulk copies
+    if (B == 0) return PNPB200_OK;
+#define LAUNCH_CHECK(TT)                                                                                                \
+    {                                                                                                                   \
+        CheckArgs<TT> a;                                                                                                \
+        a.pattern = (const TT*)pattern; a.uv = (const TT*)uv; a.R = (const TT*)R; a.t = (const TT*)t;                  \
+        a.res = (const TT*)res_norm; a.best = best_pattern; a.B = B; a.n = n; a.n_patterns = n_patterns;              \
+        for (int e = 0; e < 9; ++e) a.K[e] = K[e];                                                                      \
+        a.limit = (limit > 0.0) ? limit : 0.0;                                                                          \
+        a.status = status; a.reproj = (TT*)reproj; a.use_tmap = 0;                                                      \
+        const StreamGeom sg = stream_geometry<TT>(n);                                                                   \
+        if (report_can_fuse(dtype, n)) {                                                                                \
+            DeviceProps dp;                                                                                             \
+            const int rc = get_device_props(&dp);                                                                       \
+            if (rc != PNPB200_OK) return rc;                                                                            \
+            const size_t smem = 2 * sg.buf_bytes + sizeof(TT) * (size_t)n_patterns * n * 3 + 32;                        \
+            if (smem > (size_t)dp.max_smem_optin) return PNPB200_ETOOLARGE;   /* every pattern stays in shared memory */ \
+            a.row_pitch = sg.pitch; a.chunk = sg.chunk;                                                                 \
+            a.use_tmap = (sg.pitch == sg.chunk * 2) ? make_row_tensor_map(&a.tmap, uv, (int)sizeof(TT), B, n, sg.chunk) : 0; \
+            const long long n_tiles = (B + kTileProblems - 1) / kTileProblems;                                          \
+            PNP_CUDA_OK(set_dynamic_smem((const void*)k_check_chunk<TT>, smem));                                        \
+            k_check_chunk<TT><<<(unsigned)(n_tiles < 0x7fffffffLL ? n_tiles : 0x7fffffffLL), 32, smem, st>>>(a);        \
+        } else {                                                                                                        \
+            a.row_pitch = 0; a.chunk = 0;                                                                               \
+            k_check_warp<TT><<<grid_for(B * 32, 256), 256, 0, st>>>(a);                                                 \
+        }                                                                                                               \
+        count_kernel_launches(1);                                                                                       \
+    }
+    DISPATCH_DTYPE(dtype, LAUNCH_CHECK(double), LAUNCH_CHECK(float));
+#undef LAUNCH_CHECK
+    PNP_CUDA_OK(cudaGetLastError());
+    return PNPB200_OK;
+}
+
 }  // namespace pnpb200
 
 extern "C" {
+
+int pnpb200_check_batch(int dtype, int64_t B, int n_total, const void* pattern, int n_patterns, const void* uv, const double* K,
+                        const void* R, const void* t, const void* res_norm, const int32_t* best_pattern, double reproj_limit_px,
+                        int32_t* status, void* reproj, void* stream)
+{
+    return check_launch(dtype, B, n_total, pattern, n_patterns, uv, K, R, t, res_norm, best_pattern, reproj_limit_px, status,
+                        reproj, (cudaStream_t)stream);
+}
 
 int pnpb200_default_synth(pnpb200_synth* s)
 {

@@ -65,6 +65,10 @@ bool report_can_fuse(int dtype, int n);
 int report_launch(int dtype, int64_t B, int n, const void* pattern, const void* uv, const double* K, const void* R, const void* t,
                   const void* euler_deg, const double* gt, const double* bounds, double* report, int64_t report_stride_problem,
                   int64_t report_stride_column, int32_t* flags, int32_t* max_idx, const ReportFuse* fuse, cudaStream_t st);
+// solution check (pnpb200_check_batch), pnpb200_aux.cu
+int check_launch(int dtype, int64_t B, int n, const void* pattern, int n_patterns, const void* uv, const double* K,
+                 const void* R, const void* t, const void* res_norm, const int32_t* best_pattern, double limit,
+                 int32_t* status, void* reproj, cudaStream_t st);
 cudaError_t set_dynamic_smem(const void* kernel, size_t bytes);                                   // defined in pnpb200_api.cu
 cudaError_t blocks_per_sm(int* out, const void* kernel, int block_threads, size_t smem_bytes);   // defined in pnpb200_api.cu
 

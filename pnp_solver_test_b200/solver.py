@@ -16,6 +16,7 @@ import torch
 
 from . import _lib
 from ._lib import lib, check, ptr
+_check_rc = check        # HostPipeline.solve's keyword `check` shadows the name there
 from .patterns import LM_KEY_LIST_6
 
 _TORCH_DTYPE = {_lib.DTYPE_F64: torch.float64, _lib.DTYPE_F32: torch.float32}
@@ -102,6 +103,46 @@ def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R
     return o
 
 
+def check_batch(uv, patterns, K, R, t, res_norm=None, best_pattern=None, reproj_limit_px=1.0):
+    """pnpb200_check_batch on device tensors: the solution check of any pose, without ground truth.
+
+    uv [B, n_total, 2], patterns [P, n_total, 3] (or [n_total, 3]), R [B,3,3], t [B,3] and res_norm [B] are CUDA
+    tensors of one float dtype; best_pattern [B] int32 picks each problem's pattern (None: pattern 0); K is a host
+    3x3.  Returns dict(status [B] int32 of CHECK_* bits, reproj [B,2] = (mean, max) prediction-vs-landmark distance in
+    pixels over all n_total landmarks).  REPROJ is set where the mean exceeds reproj_limit_px (<= 0 turns it off).
+    What the bits find, and what they miss (EIF2), is in include/pnpb200.h."""
+    if not all(x.is_cuda for x in (uv, patterns, R, t)):
+        raise ValueError("uv, patterns, R and t must be CUDA tensors (no CPU fallback)")
+    if len({x.dtype for x in (uv, patterns, R, t) + (() if res_norm is None else (res_norm,))}) != 1:
+        raise ValueError("uv, patterns, R, t and res_norm must share one dtype")
+    if patterns.dim() == 2:
+        patterns = patterns.unsqueeze(0)
+    B, n_total = int(uv.shape[0]), int(uv.shape[1])
+    if uv.dim() != 3 or uv.shape[2] != 2 or patterns.dim() != 3 or tuple(patterns.shape[1:]) != (n_total, 3):
+        raise ValueError("shape mismatch: uv [B,n,2], patterns [P,n,3]")
+    if R.numel() != 9 * B or t.numel() != 3 * B or (res_norm is not None and res_norm.numel() != B):
+        raise ValueError("R [B,3,3], t [B,3] and res_norm [B] must hold B = %d problems" % B)
+    if best_pattern is not None and (best_pattern.dtype != torch.int32 or best_pattern.numel() != B or not best_pattern.is_cuda):
+        raise ValueError("best_pattern must be a CUDA int32 tensor of B = %d entries" % B)
+    dev = uv.device
+    uv, patterns, R, t = uv.contiguous(), patterns.contiguous(), R.contiguous(), t.contiguous()
+    res_norm = None if res_norm is None else res_norm.contiguous()
+    best_pattern = None if best_pattern is None else best_pattern.contiguous()
+    status = torch.empty((B,), dtype=torch.int32, device=dev)
+    reproj = torch.empty((B, 2), dtype=uv.dtype, device=dev)
+    if B == 0:
+        return dict(status=status, reproj=reproj)
+    Kh, Kp = _k_host(K)
+    PI = C.POINTER(C.c_int32)
+    with torch.cuda.device(dev):
+        rc = lib.pnpb200_check_batch(_dtype_code(uv.dtype), B, n_total, ptr(patterns), int(patterns.shape[0]), ptr(uv), Kp, ptr(R),
+                                     ptr(t), ptr(res_norm), None if best_pattern is None else C.cast(ptr(best_pattern), PI),
+                                     float(reproj_limit_px), C.cast(ptr(status), PI), ptr(reproj), _stream_ptr(dev))
+    check(rc, "pnpb200_check_batch")
+    _lib.count_launch()
+    return dict(status=status, reproj=reproj)
+
+
 class HostPipeline(object):
     """Chunked H2D -> solve -> D2H pipeline over host (ideally pinned) buffers:
     pnpb200_pipeline_* / pnpb200_solve_batch_host.  This is the end-to-end call."""
@@ -145,14 +186,16 @@ class HostPipeline(object):
 
     _PIXEL_TYPES = {torch.int16: _lib.PIXEL_I16, torch.uint16: _lib.PIXEL_U16, torch.float32: _lib.PIXEL_F32}
     _OUT_SHAPES = {"R": (9, None), "t": (3, None), "euler": (3, None), "res_norm": (1, None), "iters": (1, torch.int32),
-                   "best_pattern": (1, torch.int32)}
+                   "best_pattern": (1, torch.int32), "status": (1, torch.int32), "reproj": (2, None)}
 
-    def solve(self, method, uv_host, patterns_host, K, out, point_index=None, params=None):
+    def solve(self, method, uv_host, patterns_host, K, out, point_index=None, params=None, check=None):
         """uv_host [B,n_total,2], patterns_host [P,n_total,3]: contiguous CPU torch tensors (pinned for overlap).
         uv_host may also be int16, uint16 or float32 whatever the pipeline's dtype (detections as a detector
         delivers them: pnpb200_solve_batch_host_px ships them as they are and widens them on the device).
         out: dict of contiguous CPU tensors to fill among R [B,3,3] / [B,9], t [B,3], euler [B,3], res_norm [B]
-        (pipeline dtype), iters [B], best_pattern [B] (int32).  Everything is checked here: the C side reads and
+        (pipeline dtype), iters [B], best_pattern [B] (int32).  check = a limit in px: each chunk's solve is followed
+        by the solution check (pnpb200_solve_check_batch_host), whose status [B] (int32, required then) and
+        reproj [B,2] (pipeline dtype) go to out as well.  Everything is checked here: the C side reads and
         writes B * (row size) elements through the raw pointers."""
         m = _lib.METHODS[method] if isinstance(method, str) else int(method)
         tdt = _TORCH_DTYPE[self.dt]
@@ -178,6 +221,10 @@ class HostPipeline(object):
             if not torch.is_tensor(v) or v.is_cuda or not v.is_contiguous() or v.dtype != (dt_k or tdt) or v.numel() != B * width \
                     or (B and int(v.shape[0]) != B):
                 raise ValueError("out[%r] must be a contiguous CPU %s tensor of %d x %d elements" % (k, dt_k or tdt, B, width))
+        if check is None and ("status" in out or "reproj" in out):
+            raise ValueError("out['status'] / out['reproj'] are the outputs of check=")
+        if check is not None and "status" not in out:
+            raise ValueError("check= needs out['status']")
         if params is not None and params.workspace:
             raise ValueError("params.workspace is not used by the host pipeline (it owns one scratch per stream)")
         if point_index is None:
@@ -187,12 +234,21 @@ class HostPipeline(object):
             n, idx_p = int(idx.shape[0]), idx.ctypes.data_as(C.POINTER(C.c_int32))
         Kh, Kp = _k_host(K)
         with torch.cuda.device(self.device):
-            rc = lib.pnpb200_solve_batch_host_px(
-                self._h, C.c_int(m), C.c_int64(B), C.c_int(n), C.c_int(px), ptr(uv_host), ptr(patterns_host), idx_p, Kp,
-                C.byref(params) if params is not None else None,
-                ptr(out.get("R")), ptr(out.get("t")), ptr(out.get("euler")), ptr(out.get("res_norm")),
-                ptr(out.get("iters")), ptr(out.get("best_pattern")))
-        check(rc, "pnpb200_solve_batch_host_px")
+            if check is None:
+                rc = lib.pnpb200_solve_batch_host_px(
+                    self._h, C.c_int(m), C.c_int64(B), C.c_int(n), C.c_int(px), ptr(uv_host), ptr(patterns_host), idx_p, Kp,
+                    C.byref(params) if params is not None else None,
+                    ptr(out.get("R")), ptr(out.get("t")), ptr(out.get("euler")), ptr(out.get("res_norm")),
+                    ptr(out.get("iters")), ptr(out.get("best_pattern")))
+            else:
+                PI = C.POINTER(C.c_int32)
+                pi = (lambda k: None if out.get(k) is None else C.cast(ptr(out[k]), PI))
+                rc = lib.pnpb200_solve_check_batch_host(
+                    self._h, m, B, n, px, ptr(uv_host), ptr(patterns_host), idx_p, Kp,
+                    C.byref(params) if params is not None else None,
+                    ptr(out.get("R")), ptr(out.get("t")), ptr(out.get("euler")), ptr(out.get("res_norm")),
+                    pi("iters"), pi("best_pattern"), float(check), pi("status"), ptr(out.get("reproj")))
+        _check_rc(rc, "pnpb200_solve_batch_host_px" if check is None else "pnpb200_solve_check_batch_host")
         _lib.count_launch((B + self.chunk - 1) // self.chunk)
         return out
 
@@ -427,14 +483,16 @@ class PNP_SOLVER(object):
         """PNP_SOLVER_LIB.py:205-430 (rows follow the image dict's key order, :3069)"""
         return self._solve_single("linear_f1", np_point_image_dict, np_point_3d_pretransfer_dict, list(np_point_image_dict.keys()))
 
-    def solve_pnp_batch(self, uv, method=None, key_list="default", params=None):
+    def solve_pnp_batch(self, uv, method=None, key_list="default", params=None, check=None):
         """The per-problem script loop as one launch.
 
         uv: [B, n_total, 2] pixels (or [B, n_total, 3] homogeneous image points, third entry as the reference's
         dicts carry it) in the key order of the stored patterns -- a CUDA tensor, or a NumPy array / CPU tensor
         (copied to the device).  key_list: landmark subset; "default" =
         the 6 keys of solve_pnp() for 'qeif', all points otherwise.  Returns a dict of CUDA
-        tensors (see solve_batch) and, like solve_pnp, works over every stored pattern."""
+        tensors (see solve_batch) and, like solve_pnp, works over every stored pattern.
+        check: a limit in px -> the dict also holds status [B] int32 and reproj [B,2] of check_batch on the
+        returned poses, over all n_total landmarks and each problem's winning pattern (0: no REPROJ bit)."""
         method = method or self.method
         all_keys = list(self.np_point_3d_pretransfer_dict_list[0].keys())
         if isinstance(key_list, str) and key_list == "default":
@@ -446,17 +504,24 @@ class PNP_SOLVER(object):
         ck = ("all", self.dtype_code)
         if ck not in self._dev_cache:
             self._dev_cache[ck] = self._pack_patterns(self.np_point_3d_pretransfer_dict_list, all_keys)
-        return solve_batch(method, uv, self._dev_cache[ck], K, point_index=idx,
-                           params=params if params is not None else self.params)
+        out = solve_batch(method, uv, self._dev_cache[ck], K, point_index=idx,
+                          params=params if params is not None else self.params)
+        if check is not None:
+            out.update(check_batch(uv, self._dev_cache[ck], K, out["R"], out["t"], res_norm=out["res_norm"],
+                                   best_pattern=out["best_pattern"], reproj_limit_px=check))
+        return out
 
-    def solve_pnp_batch_host(self, uv, method=None, key_list="default", params=None, chunk_problems=1 << 16, pack_threads=None):
+    def solve_pnp_batch_host(self, uv, method=None, key_list="default", params=None, chunk_problems=1 << 16, pack_threads=None,
+                             check=None):
         """solve_pnp_batch for data that lives on the HOST (what a script that loops over NumPy samples
         has): uv [B, n_total, 2] NumPy array or CPU tensor in; dict of NumPy arrays R [B,3,3], t [B,3],
         euler [B,3] (roll, yaw, pitch, deg.), res_norm [B], iters [B], best_pattern [B] out.  uv may be int16,
         uint16 or float32 (a detector's own output type): it then crosses PCIe as it is.  Runs the
         chunked host pipeline (pnpb200_solve_batch_host: H2D, solve and D2H overlap on three streams);
         pack_threads host threads (default: half the visible cores, at most 8) let chunks of whole-pixel
-        landmarks cross PCIe as int16 (lossless, checked per chunk; other chunks travel as they are)."""
+        landmarks cross PCIe as int16 (lossless, checked per chunk; other chunks travel as they are).
+        check: a limit in px -> each chunk's solve is followed by the solution check on the device, and the dict also
+        holds status [B] int32 and reproj [B,2] (see solve_pnp_batch); every other output is unchanged."""
         method = method or self.method
         all_keys = list(self.np_point_3d_pretransfer_dict_list[0].keys())
         if isinstance(key_list, str) and key_list == "default":
@@ -498,10 +563,16 @@ class PNP_SOLVER(object):
                     "euler": pin(torch.empty((B, 3), dtype=tdt)), "res_norm": pin(torch.empty((B,), dtype=tdt)),
                     "iters": pin(torch.empty((B,), dtype=torch.int32)), "best_pattern": pin(torch.empty((B,), dtype=torch.int32))}
             self._dev_cache[okey] = outs
+        sel = {k: v for k, v in outs.items() if k not in ("status", "reproj")}
+        if check is not None:
+            if "status" not in outs:
+                pin = (lambda t_: t_.pin_memory()) if B > 0 else (lambda t_: t_)
+                outs["status"], outs["reproj"] = pin(torch.empty((B,), dtype=torch.int32)), pin(torch.empty((B, 2), dtype=tdt))
+            sel["status"], sel["reproj"] = outs["status"], outs["reproj"]
         if B > 0:
-            pipe.solve(method, uv_h, pat_h, self.np_K_camera_est, outs, point_index=idx,
-                       params=params if params is not None else self.params)
-        return {k: v.numpy().copy() for k, v in outs.items()}
+            pipe.solve(method, uv_h, pat_h, self.np_K_camera_est, sel, point_index=idx,
+                       params=params if params is not None else self.params, check=check)
+        return {k: v.numpy().copy() for k, v in sel.items()}
 
     # ---------------------------------------------------------------- Euler <-> R (:4442-4517)
     def get_rotation_matrix_from_Euler(self, roll, yaw, pitch, is_degree=False):
