@@ -367,6 +367,79 @@ int pnpb200_check_batch(int dtype, int64_t B, int n_total, const void* pattern, 
                         void* stream);
 
 /*
+ * Per-problem landmark visibility.  A detector does not find every landmark: self-occlusion, leaving the image or a
+ * confidence threshold hide a different set in every frame.  The _masked entries below are the entries above plus
+ *   visible  [device] (host for pnpb200_solve_batch_host_masked) [B, W] uint32, W = ceil(n_total / 32), row-major,
+ *            4-byte aligned: bit i % 32 of word i / 32 (least significant bit first) = landmark i is visible; bits at and
+ *            beyond n_total are ignored.  NULL or a misaligned pointer is PNPB200_EINVAL (the unmasked entries are the
+ *            call without a mask).
+ * The rule, for every output: problem b is solved, reported and checked as the problem made of its visible landmarks
+ * alone -- with point_index, the visible landmarks of point_index in point_index order -- which is the reference's
+ * result with the pattern dict and the image-point dict both restricted to those keys (f2_get_P :3260, f2_get_B_xy
+ * :3291, LM_key_list :156).
+ *  - The pixels of a hidden landmark are never used in arithmetic: NaN, +-Inf or any other value there changes no
+ *    output bit, so "missing = NaN" works as is.
+ *  - Fewer than 4 visible selected landmarks: the problem is not solved.  R, t, euler_deg, res_norm are NaN, iters 0,
+ *    best_pattern 0; the check reports PNPB200_CHECK_NONFINITE with reproj NaN; report columns 4-9 are NaN and max_idx
+ *    is -1 (with the unsolved NaN pose every column but 11 and 15 is NaN and every pass flag false).  Its neighbours in
+ *    the batch are unaffected.
+ *  - Linear F1 / F2 (and so the start of LM+) need visible landmarks that are not coplanar.  On a coplanar set (e.g. 6 of
+ *    the 15 golden landmarks, 10 of which lie in z = 0) the reference's pinv solves a rank-deficient system; the device's
+ *    LDL^T / SPD solves have no rank-deficient branch and return NaN there.  LM, QEIF and EIF2 are not affected.
+ *  - Report: means and maxima of columns 4-9 run over the visible landmarks; max_idx is in the 0..n_total-1 numbering.
+ *    Check: reproj (mean, max) and the BEHIND bit run over the visible landmarks.  Several patterns: the arg-min is
+ *    taken on the masked res_norm.
+ * A masked solve takes the mapping the same call without a mask takes, every method and flag included (LM+ and
+ * PNPB200_FLAG_LM_TRUE_JACOBIAN too); its kernels keep the pattern constants (M0, m0, n, G) per problem: the moment
+ * mapping's moments pass stores sum theta theta^T, sum theta and the count of each problem beside its moments, and
+ * k_iterate builds the constants per thread.  Rows of 256 landmarks and more take the per-warp streaming shape (there is
+ * no masked TMA ring).  pnpb200_solve_report_batch_masked is the masked solve followed by the masked report (never the
+ * fused pass).  pnpb200_workspace_bytes_masked is the scratch of a masked solve: that of pnpb200_workspace_bytes plus
+ * 10 values per problem where that is not 0.
+ * pnpb200_solve_batch_host_masked is pnpb200_solve_batch_host_px with the chunk's mask words copied beside its pixels;
+ * with non-NULL status it also runs the check of pnpb200_solve_check_batch_host (reproj may then be NULL).
+ * How much visibility the methods tolerate (C oracle, random_stress_test.py pose distribution, quantised noise-free pixels,
+ * seed 42, 8 192 problems, 68 landmarks of which a uniformly drawn 100 / 75 / 50 % per problem are visible; share passing
+ * the 10 cm / 10 deg test of random_stress_test.py; tests/visibility_accuracy.py):
+ *            100 %    75 %    50 %
+ *   LM       69.4 %  68.3 %  67.0 %
+ *   LM+      99.0 %  98.8 %  98.7 %
+ *   EIF2     99.2 %  98.9 %  98.6 %
+ *   QEIF    100.0 % 100.0 % 100.0 %   (all 68 landmarks, not solve_pnp's 6)
+ * Half the landmarks cost the filters well under a point of pass rate on noise-free pixels.
+ */
+int pnpb200_solve_batch_masked(int method, int dtype, int64_t B, int n_total, int n,
+                               const void* uv, const void* pattern, int n_patterns,
+                               const int32_t* point_index, const double* K,
+                               const pnpb200_params* params,
+                               void* R, void* t, void* euler_deg, void* res_norm,
+                               int32_t* iters, int32_t* best_pattern, const uint32_t* visible, void* stream);
+int pnpb200_solve_report_batch_masked(int method, int dtype, int64_t B, int n_total, int n,
+                                      const void* uv, const void* pattern, const int32_t* point_index, const double* K,
+                                      const pnpb200_params* params,
+                                      void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters,
+                                      const double* gt, const double* bounds,
+                                      double* report, int64_t report_stride_problem, int64_t report_stride_column,
+                                      int32_t* flags, int32_t* max_idx, const uint32_t* visible, void* stream);
+int pnpb200_report_batch_strided_masked(int dtype, int64_t B, int n, const void* pattern, const void* uv,
+                                        const double* K, const void* R, const void* t, const void* euler_deg,
+                                        const double* gt, const double* bounds,
+                                        double* report, int64_t report_stride_problem, int64_t report_stride_column,
+                                        int32_t* flags, int32_t* max_idx, const uint32_t* visible, void* stream);
+int pnpb200_check_batch_masked(int dtype, int64_t B, int n_total, const void* pattern, int n_patterns, const void* uv,
+                               const double* K, const void* R, const void* t, const void* res_norm,
+                               const int32_t* best_pattern, double reproj_limit_px, int32_t* status, void* reproj,
+                               const uint32_t* visible, void* stream);
+int64_t pnpb200_workspace_bytes_masked(int method, int dtype, int64_t B, int n_patterns, int mapping);
+int pnpb200_solve_batch_host_masked(pnpb200_pipeline* p, int method, int64_t B, int n, int pixel_type,
+                                    const void* uv_host, const void* pattern_host,
+                                    const int32_t* point_index, const double* K,
+                                    const pnpb200_params* params,
+                                    void* R, void* t, void* euler_deg, void* res_norm,
+                                    int32_t* iters, int32_t* best_pattern, const uint32_t* visible,
+                                    double reproj_limit_px, int32_t* status, void* reproj);
+
+/*
  * Error statistics, two passes so that shards can be combined with two small all-reduce phases
  * (TEST_TOOLBOX.get_statistic_of_result, TEST_TOOLBOX.py:892-937), for nq <= 4 quantities at once
  * (depth, roll, pitch, yaw in TEST_TOOLBOX.data_analysis_and_saving, :1070-1112), per class and,

@@ -34,6 +34,8 @@ EXPORTS = [
     "pnpb200_fragility_accumulate", "pnpb200_write_result_csv", "pnpb200_format_repr", "pnpb200_classify", "pnpb200_classify_drpy", "pnpb200_profile_reset", "pnpb200_profile_read",
     "pnpb200_solve_batch_host_px", "pnpb200_host_alloc", "pnpb200_host_free", "pnpb200_solve_report_batch", "pnpb200_normalise_uvw",
     "pnpb200_check_batch", "pnpb200_solve_check_batch_host",
+    "pnpb200_solve_batch_masked", "pnpb200_solve_report_batch_masked", "pnpb200_report_batch_strided_masked",
+    "pnpb200_check_batch_masked", "pnpb200_workspace_bytes_masked", "pnpb200_solve_batch_host_masked",
 ]
 
 
@@ -76,6 +78,21 @@ lib.pnpb200_check_batch.argtypes = [C.c_int, C.c_int64, C.c_int, _VP, C.c_int, _
 lib.pnpb200_solve_check_batch_host.argtypes = [_VP, C.c_int, C.c_int64, C.c_int, C.c_int, _VP, _VP, _PI, _PD, _VP, _VP, _VP, _VP,
                                                _VP, _PI, _PI, C.c_double, _PI, _VP]
 lib.pnpb200_launch_count.restype = C.c_int64
+# the masked entries: the unmasked ones plus `const uint32_t* visible` (before the stream)
+_U32P = C.POINTER(C.c_uint32)
+lib.pnpb200_workspace_bytes_masked.restype = C.c_int64
+lib.pnpb200_workspace_bytes_masked.argtypes = [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int]
+lib.pnpb200_solve_batch_masked.argtypes = [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, _VP, _VP, C.c_int, _PI, _PD, _VP,
+                                           _VP, _VP, _VP, _VP, _PI, _PI, _U32P, _VP]
+lib.pnpb200_solve_report_batch_masked.argtypes = [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, _VP, _VP, _PI, _PD, _VP,
+                                                  _VP, _VP, _VP, _VP, _PI, _PD, _PD, _PD, C.c_int64, C.c_int64, _PI, _PI,
+                                                  _U32P, _VP]
+lib.pnpb200_report_batch_strided_masked.argtypes = [C.c_int, C.c_int64, C.c_int, _VP, _VP, _PD, _VP, _VP, _VP, _PD, _PD,
+                                                    _PD, C.c_int64, C.c_int64, _PI, _PI, _U32P, _VP]
+lib.pnpb200_check_batch_masked.argtypes = [C.c_int, C.c_int64, C.c_int, _VP, C.c_int, _VP, _PD, _VP, _VP, _VP, _PI, C.c_double,
+                                           _PI, _VP, _U32P, _VP]
+lib.pnpb200_solve_batch_host_masked.argtypes = [_VP, C.c_int, C.c_int64, C.c_int, C.c_int, _VP, _VP, _PI, _PD, _VP, _VP, _VP,
+                                                _VP, _VP, _PI, _PI, _U32P, C.c_double, _PI, _VP]
 
 _ERR = {-1: "EINVAL (bad argument)", -2: "ECUDA (CUDA runtime error)", -3: "ENODEVICE (no usable CUDA device)",
         -4: "ETOOLARGE (n too large for the selected mapping)"}

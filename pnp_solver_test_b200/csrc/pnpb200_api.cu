@@ -210,12 +210,21 @@ int64_t pnpb200_workspace_bytes(int method, int dtype, int64_t B, int n_patterns
     return ((int64_t)(PNP_NMOM + PNP_NTAIL) * B + PNP_PATC) * esz;
 }
 
+int64_t pnpb200_workspace_bytes_masked(int method, int dtype, int64_t B, int n_patterns, int mapping)
+{
+    // the moment mapping keeps 10 pattern moments (sum theta theta^T, sum theta, count) per problem beside the moments
+    const int64_t plain = pnpb200_workspace_bytes(method, dtype, B, n_patterns, mapping);
+    return plain > 0 ? plain + (int64_t)PNP_NPMOM * B * ((dtype == PNPB200_DTYPE_F32) ? 4 : 8) : 0;
+}
+
+// vis: [B, ceil(n_total / 32)] per-problem visibility bits (device), or nullptr for every landmark
 static int solve_batch_impl(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
                             int n_patterns, const int32_t* point_index, const double* K, const pnpb200_params& prm,
                             void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters, int32_t* best_pattern,
-                            cudaStream_t st)
+                            cudaStream_t st, const uint32_t* vis = nullptr)
 {
     if (B < 0 || n_total < 1 || n < 1 || (!point_index && n != n_total) || !uv || !pattern || !K) return PNPB200_EINVAL;
+    if (vis && !vis_aligned(vis)) return PNPB200_EINVAL;
     if (((uintptr_t)uv & 15u) != 0) return PNPB200_EINVAL;   // rows are staged with 16-byte bulk copies / vector loads
     if (n_patterns < 1 || n_patterns > PNPB200_MAX_PATTERNS) return PNPB200_EINVAL;
     if (method < 0 || method > 5 || (dtype != PNPB200_DTYPE_F64 && dtype != PNPB200_DTYPE_F32)) return PNPB200_EINVAL;
@@ -236,7 +245,7 @@ static int solve_batch_impl(int method, int dtype, int64_t B, int n_total, int n
                                          { solve_part_f32_g0, solve_part_f32_g1, solve_part_f32_g2, solve_part_f32_g3 } };
     const int rc = parts[dtype == PNPB200_DTYPE_F64 ? 0 : 1][group](method, B, n_total, n, uv, pattern, n_patterns, point_index,
                                                                    idx_dev, K, prm, R, t, euler_deg, res_norm, iters,
-                                                                   best_pattern, st);
+                                                                   best_pattern, st, vis);
     if (idx_dev) cudaFreeAsync(idx_dev, st);
     return rc;
 }
@@ -253,11 +262,24 @@ int pnpb200_solve_batch(int method, int dtype, int64_t B, int n_total, int n, co
                             iters, best_pattern, (cudaStream_t)stream);
 }
 
-int pnpb200_solve_report_batch(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
-                               const int32_t* point_index, const double* K, const pnpb200_params* params,
-                               void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters,
-                               const double* gt, const double* bounds, double* report, int64_t report_stride_problem,
-                               int64_t report_stride_column, int32_t* flags, int32_t* max_idx, void* stream)
+int pnpb200_solve_batch_masked(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
+                               int n_patterns, const int32_t* point_index, const double* K, const pnpb200_params* params,
+                               void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters, int32_t* best_pattern,
+                               const uint32_t* visible, void* stream)
+{
+    if (!visible) return PNPB200_EINVAL;
+    pnpb200_params prm;
+    if (params) prm = *params; else fill_default_params(&prm);
+    prm.flags &= ~PNP_FLAG_INTERNAL_NO_RESIDUAL;
+    return solve_batch_impl(method, dtype, B, n_total, n, uv, pattern, n_patterns, point_index, K, prm, R, t, euler_deg, res_norm,
+                            iters, best_pattern, (cudaStream_t)stream, visible);
+}
+
+static int solve_report_impl(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
+                             const int32_t* point_index, const double* K, const pnpb200_params* params,
+                             void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters,
+                             const double* gt, const double* bounds, double* report, int64_t report_stride_problem,
+                             int64_t report_stride_column, int32_t* flags, int32_t* max_idx, void* stream, const uint32_t* vis)
 {
     if (!R || !t || !euler_deg || !gt || !report) return PNPB200_EINVAL;          // the report reads the pose
     pnpb200_params prm;
@@ -270,14 +292,14 @@ int pnpb200_solve_report_batch(int method, int dtype, int64_t B, int n_total, in
                          (dtype == PNPB200_DTYPE_F64 && (method == PNPB200_METHOD_EIF2 ||
                           (method == PNPB200_METHOD_QEIF && n >= PNP_QEIF_HYBRID_MIN_N && !(prm.flags & PNPB200_FLAG_QEIF_DIRECT))))) &&
                         (prm.mapping == PNPB200_MAP_AUTO || prm.mapping == PNPB200_MAP_MOMENT);
-    const bool fuse = moment && !point_index && n == n_total && res_norm && B > 0 && ((prm.flags >> 8) & 0xff) != 9 &&
+    const bool fuse = !vis && moment && !point_index && n == n_total && res_norm && B > 0 && ((prm.flags >> 8) & 0xff) != 9 &&
                       (dtype == PNPB200_DTYPE_F64 || dtype == PNPB200_DTYPE_F32) && report_can_fuse(dtype, n_total);
     if (!fuse) {
         const int rc = solve_batch_impl(method, dtype, B, n_total, n, uv, pattern, 1, point_index, K, prm, R, t, euler_deg, res_norm,
-                                        iters, nullptr, st);
+                                        iters, nullptr, st, vis);
         if (rc != PNPB200_OK) return rc;
         return report_launch(dtype, B, n_total, pattern, uv, K, R, t, euler_deg, gt, bounds, report, report_stride_problem,
-                             report_stride_column, flags, max_idx, nullptr, st);
+                             report_stride_column, flags, max_idx, nullptr, st, vis);
     }
     const size_t esz = (dtype == PNPB200_DTYPE_F64) ? 8 : 4;
     const size_t ws_bytes = (size_t)pnpb200_workspace_bytes(method, dtype, B, 1, PNPB200_MAP_MOMENT);
@@ -308,6 +330,28 @@ int pnpb200_solve_report_batch(int method, int dtype, int64_t B, int n_total, in
     return rc;
 }
 
+int pnpb200_solve_report_batch(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
+                               const int32_t* point_index, const double* K, const pnpb200_params* params,
+                               void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters,
+                               const double* gt, const double* bounds, double* report, int64_t report_stride_problem,
+                               int64_t report_stride_column, int32_t* flags, int32_t* max_idx, void* stream)
+{
+    return solve_report_impl(method, dtype, B, n_total, n, uv, pattern, point_index, K, params, R, t, euler_deg, res_norm, iters, gt,
+                             bounds, report, report_stride_problem, report_stride_column, flags, max_idx, stream, nullptr);
+}
+
+int pnpb200_solve_report_batch_masked(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
+                                      const int32_t* point_index, const double* K, const pnpb200_params* params,
+                                      void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters,
+                                      const double* gt, const double* bounds, double* report, int64_t report_stride_problem,
+                                      int64_t report_stride_column, int32_t* flags, int32_t* max_idx, const uint32_t* visible,
+                                      void* stream)
+{
+    if (!visible) return PNPB200_EINVAL;
+    return solve_report_impl(method, dtype, B, n_total, n, uv, pattern, point_index, K, params, R, t, euler_deg, res_norm, iters, gt,
+                             bounds, report, report_stride_problem, report_stride_column, flags, max_idx, stream, visible);
+}
+
 // ------------------------------------------------------------------------------------------
 // host-buffer entry point: chunked, multi-stream H2D -> solve -> D2H pipeline
 // ------------------------------------------------------------------------------------------
@@ -321,6 +365,9 @@ struct PipeSlot {
     void* d_narrow = nullptr;                             // device copy of a chunk of int16 / uint16 / float32 pixels (solve_batch_host_px)
     int32_t* d_status = nullptr;                          // outputs of the solution check (solve_check_batch_host), from its first call
     void* d_reproj = nullptr;
+    uint32_t* d_vis = nullptr;                            // visibility words of a chunk (solve_batch_host_masked), from its first call
+    uint32_t* h_vis = nullptr;                            // ... staged in pinned memory so that their copy is asynchronous
+    cudaEvent_t vis_free = nullptr;                       // the H2D copy out of h_vis has finished
     cudaEvent_t pack_free = nullptr;                      // the H2D copy out of h_pack has finished
     cudaEvent_t h2d_done = nullptr;                       // the slot's last pixel copy has finished (back-pressure)
     cudaEvent_t piece_done[2] = { nullptr, nullptr };     // parts of a plain chunk's pixel copy, two in flight (submit_chunk)
@@ -370,8 +417,10 @@ static void free_slot(PipeSlot& sl)
 {
     if (sl.stream) { cudaStreamSynchronize(sl.stream); cudaStreamDestroy(sl.stream); }
     cudaFree(sl.d_uv); cudaFree(sl.d_R); cudaFree(sl.d_t); cudaFree(sl.d_e); cudaFree(sl.d_res); cudaFree(sl.d_ws);
-    cudaFree(sl.d_it); cudaFree(sl.d_best); cudaFree(sl.d_pack); cudaFree(sl.d_narrow); cudaFree(sl.d_status); cudaFree(sl.d_reproj);
+    cudaFree(sl.d_it); cudaFree(sl.d_best); cudaFree(sl.d_pack); cudaFree(sl.d_narrow); cudaFree(sl.d_status); cudaFree(sl.d_reproj); cudaFree(sl.d_vis);
     if (sl.h_pack) cudaFreeHost(sl.h_pack);
+    if (sl.h_vis) cudaFreeHost(sl.h_vis);
+    if (sl.vis_free) cudaEventDestroy(sl.vis_free);
     if (sl.pack_free) cudaEventDestroy(sl.pack_free);
     if (sl.h2d_done) cudaEventDestroy(sl.h2d_done);
     for (cudaEvent_t e : sl.piece_done) if (e) cudaEventDestroy(e);
@@ -463,6 +512,7 @@ struct HostCall {
     int32_t* status;                                      // non-NULL: the solution check runs after each chunk's solve
     void* reproj;
     double reproj_limit_px;
+    const uint32_t* vis;                                  // [B, ceil(n_total / 32)] host visibility words, or NULL
 };
 
 // queue one chunk on a slot: pixels host -> device (packed if `packed`), solve, results device -> host.
@@ -501,21 +551,31 @@ int submit_chunk(const HostCall& c, PipeSlot& sl, int64_t done, int64_t nb, bool
         }
         PNP_CUDA_OK(cudaEventRecord(sl.h2d_done, st));
     }
+    const uint32_t* vis = nullptr;
+    if (c.vis) {                                          // the chunk's mask travels with its pixels, on the same stream
+        const size_t W = ((size_t)p->n_total + 31) / 32;
+        PNP_CUDA_OK(cudaEventSynchronize(sl.vis_free));     // the slot's previous mask copy has left the staging buffer
+        memcpy(sl.h_vis, c.vis + (size_t)done * W, sizeof(uint32_t) * W * (size_t)nb);
+        PNP_CUDA_OK(cudaMemcpyAsync(sl.d_vis, sl.h_vis, sizeof(uint32_t) * W * (size_t)nb, cudaMemcpyHostToDevice, st));
+        PNP_CUDA_OK(cudaEventRecord(sl.vis_free, st));
+        vis = sl.d_vis;
+    }
     pnpb200_params prm;
     if (c.params) prm = *c.params; else fill_default_params(&prm);
+    prm.flags &= ~PNP_FLAG_INTERNAL_NO_RESIDUAL;
     // always the slot's own scratch: chunks run concurrently on several streams, one caller workspace would be shared by them
     prm.workspace = sl.d_ws; prm.workspace_bytes = (int64_t)p->ws_bytes;
     // the check reads the pose and the winning pattern whether or not the caller asked for them
     const bool chk = c.status != nullptr, want_best = c.best_pattern || (chk && p->n_patterns > 1);
-    int rc = pnpb200_solve_batch(c.method, p->dtype, nb, p->n_total, c.n, sl.d_uv, p->d_pattern, p->n_patterns,
-                                 c.point_index, c.K, &prm, (c.R || chk) ? sl.d_R : nullptr, (c.t || chk) ? sl.d_t : nullptr,
-                                 c.euler_deg ? sl.d_e : nullptr, c.res_norm ? sl.d_res : nullptr,
-                                 c.iters ? sl.d_it : nullptr, want_best ? sl.d_best : nullptr, st);
+    int rc = solve_batch_impl(c.method, p->dtype, nb, p->n_total, c.n, sl.d_uv, p->d_pattern, p->n_patterns,
+                              c.point_index, c.K, prm, (c.R || chk) ? sl.d_R : nullptr, (c.t || chk) ? sl.d_t : nullptr,
+                              c.euler_deg ? sl.d_e : nullptr, c.res_norm ? sl.d_res : nullptr,
+                              c.iters ? sl.d_it : nullptr, want_best ? sl.d_best : nullptr, st, vis);
     if (rc != PNPB200_OK) return rc;
     if (chk) {
         rc = check_launch(p->dtype, nb, p->n_total, p->d_pattern, p->n_patterns, sl.d_uv, c.K, sl.d_R, sl.d_t,
                           c.res_norm ? sl.d_res : nullptr, p->n_patterns > 1 ? sl.d_best : nullptr, c.reproj_limit_px,
-                          sl.d_status, c.reproj ? sl.d_reproj : nullptr, st);
+                          sl.d_status, c.reproj ? sl.d_reproj : nullptr, st, vis);
         if (rc != PNPB200_OK) return rc;
         PNP_CUDA_OK(cudaMemcpyAsync(c.status + done, sl.d_status, sizeof(int32_t) * (size_t)nb, cudaMemcpyDeviceToHost, st));
         if (c.reproj)
@@ -543,7 +603,8 @@ int pnpb200_solve_batch_host(pnpb200_pipeline* p, int method, int64_t B, int n, 
 namespace {
 int solve_host(pnpb200_pipeline* p, int method, int64_t B, int n, int pixel_type, const void* uv_host, const void* pattern_host,
                const int32_t* point_index, const double* K, const pnpb200_params* params, void* R, void* t, void* euler_deg,
-               void* res_norm, int32_t* iters, int32_t* best_pattern, int32_t* status, void* reproj, double reproj_limit_px)
+               void* res_norm, int32_t* iters, int32_t* best_pattern, int32_t* status, void* reproj, double reproj_limit_px,
+               const uint32_t* vis)
 {
     if (!p || !uv_host || !pattern_host || !K || B < 0) return PNPB200_EINVAL;
     if (n < 1 || n > p->n_total || (!point_index && n != p->n_total)) return PNPB200_EINVAL;
@@ -565,11 +626,30 @@ int solve_host(pnpb200_pipeline* p, int method, int64_t B, int n, int pixel_type
             if (!sl.d_reproj) PNP_CUDA_OK(cudaMalloc(&sl.d_reproj, esz * (size_t)p->chunk * 2));
         }
     }
+    if (vis) {                                                // first masked call: the per-slot mask buffers, the larger scratch
+        if (!vis_aligned(vis)) return PNPB200_EINVAL;
+        const size_t W = ((size_t)p->n_total + 31) / 32;
+        const size_t ws = (size_t)pnpb200_workspace_bytes_masked(PNPB200_METHOD_LM, p->dtype, p->chunk, 1, PNPB200_MAP_MOMENT);
+        for (PipeSlot& sl : p->slots) {
+            if (!sl.d_vis) {
+                PNP_CUDA_OK(cudaMalloc((void**)&sl.d_vis, sizeof(uint32_t) * (size_t)p->chunk * W));
+                PNP_CUDA_OK(cudaMallocHost((void**)&sl.h_vis, sizeof(uint32_t) * (size_t)p->chunk * W));
+                PNP_CUDA_OK(cudaEventCreateWithFlags(&sl.vis_free, cudaEventDisableTiming));
+            }
+            if (p->ws_bytes < ws) {
+                PNP_CUDA_OK(cudaStreamSynchronize(sl.stream));
+                PNP_CUDA_OK(cudaFree(sl.d_ws));
+                sl.d_ws = nullptr;
+                PNP_CUDA_OK(cudaMalloc(&sl.d_ws, ws));
+            }
+        }
+        if (p->ws_bytes < ws) p->ws_bytes = ws;
+    }
     PNP_CUDA_OK(cudaMemcpyAsync(p->d_pattern, pattern_host, esz * (size_t)p->n_patterns * p->n_total * 3,
                                 cudaMemcpyHostToDevice, p->slots[0].stream));
     PNP_CUDA_OK(cudaStreamSynchronize(p->slots[0].stream));
     const HostCall call = { p, method, n, pixel_type, B, uv_host, point_index, K, params, R, t, euler_deg, res_norm, iters, best_pattern,
-                            status, reproj, reproj_limit_px };
+                            status, reproj, reproj_limit_px, vis };
     const int64_t n_chunks = (B + p->chunk - 1) / p->chunk;
     p->last_chunks = n_chunks; p->last_packed = 0;
     // Chunks are handed out from both ends of the batch: this thread sends chunks as they are from the front
@@ -642,7 +722,7 @@ int pnpb200_solve_batch_host_px(pnpb200_pipeline* p, int method, int64_t B, int 
                                 int32_t* iters, int32_t* best_pattern)
 {
     return solve_host(p, method, B, n, pixel_type, uv_host, pattern_host, point_index, K, params, R, t, euler_deg, res_norm, iters,
-                      best_pattern, nullptr, nullptr, 0.0);
+                      best_pattern, nullptr, nullptr, 0.0, nullptr);
 }
 
 int pnpb200_solve_check_batch_host(pnpb200_pipeline* p, int method, int64_t B, int n, int pixel_type, const void* uv_host,
@@ -652,7 +732,18 @@ int pnpb200_solve_check_batch_host(pnpb200_pipeline* p, int method, int64_t B, i
 {
     if (!status) return PNPB200_EINVAL;
     return solve_host(p, method, B, n, pixel_type, uv_host, pattern_host, point_index, K, params, R, t, euler_deg, res_norm, iters,
-                      best_pattern, status, reproj, reproj_limit_px);
+                      best_pattern, status, reproj, reproj_limit_px, nullptr);
+}
+
+int pnpb200_solve_batch_host_masked(pnpb200_pipeline* p, int method, int64_t B, int n, int pixel_type, const void* uv_host,
+                                    const void* pattern_host, const int32_t* point_index, const double* K,
+                                    const pnpb200_params* params, void* R, void* t, void* euler_deg, void* res_norm,
+                                    int32_t* iters, int32_t* best_pattern, const uint32_t* visible, double reproj_limit_px,
+                                    int32_t* status, void* reproj)
+{
+    if (!visible || (reproj && !status)) return PNPB200_EINVAL;
+    return solve_host(p, method, B, n, pixel_type, uv_host, pattern_host, point_index, K, params, R, t, euler_deg, res_norm, iters,
+                      best_pattern, status, reproj, reproj_limit_px, visible);
 }
 
 }  // extern "C"

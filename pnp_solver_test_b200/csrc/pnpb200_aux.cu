@@ -222,6 +222,13 @@ __global__ void k_synth(long long b0, long long B, int n, const double* __restri
 // ------------------------------------------------------------------------------------------
 struct Bounds { double b[4]; };
 
+// a masked problem with fewer than kMinVisible visible landmarks: NaN statistics, no worst landmark
+PNP_DEV void too_few_for_report(double& s0, double& s1, double& s2, double& m0, double& m1, double& m2, int& i0, int& i1, int& i2)
+{
+    s0 = s1 = s2 = m0 = m1 = m2 = __longlong_as_double(0x7ff8000000000000LL);
+    i0 = i1 = i2 = -1;
+}
+
 PNP_DEV void warp_sum_max(double& s, double& m, int& im)
 {
 #pragma unroll
@@ -234,10 +241,12 @@ PNP_DEV void warp_sum_max(double& s, double& m, int& im)
     }
 }
 
-template <typename T>
+// MASKED: the statistics of columns 4-9 run over the landmarks whose bit is set in vis[b * vis_words ...]
+template <typename T, bool MASKED = false>
 __global__ void k_report(long long B, int n, const void* pattern, const void* uv, KMat K, const void* R, const void* t,
                          const void* euler, const double* __restrict__ gt, Bounds bounds, double* report,
-                         long long rs_b, long long rs_k, int32_t* flags, int32_t* max_idx)
+                         long long rs_b, long long rs_k, int32_t* flags, int32_t* max_idx,
+                         const uint32_t* vis = nullptr, int vis_words = 0)
 {
     const long long b = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
@@ -255,7 +264,10 @@ __global__ void k_report(long long B, int n, const void* pattern, const void* uv
     for (int k = 0; k < 3; ++k) tg[k] = (te[k] / t3) * dist;   // :367-368
     double s0 = 0, s1 = 0, s2 = 0, m0 = 0, m1 = 0, m2 = 0;
     int i0 = -1, i1 = -1, i2 = -1;
+    const uint32_t* vw = MASKED ? vis + (size_t)b * vis_words : nullptr;
+    const int nv = MASKED ? count_visible(vw, nullptr, n) : 0;
     for (int i = lane; i < n; i += 32) {
+        if constexpr (MASKED) { if (!mask_bit(vw, i)) continue; }
         const double x = ld<T>(pattern, 3 * i), y = ld<T>(pattern, 3 * i + 1), z = ld<T>(pattern, 3 * i + 2);
         double pe[3], pg[3];
         project_point_fast(K.k, Re, te, x, y, z, pe);          // TEST_TOOLBOX.py:312
@@ -270,13 +282,14 @@ __global__ void k_report(long long B, int n, const void* pattern, const void* uv
         e = sqrt(d0 * d0 + d1 * d1 + d2 * d2); s2 += e; if (e > m2) { m2 = e; i2 = i; }
     }
     warp_sum_max(s0, m0, i0); warp_sum_max(s1, m1, i1); warp_sum_max(s2, m2, i2);
+    if constexpr (MASKED) { if (nv < kMinVisible) too_few_for_report(s0, s1, s2, m0, m1, m2, i0, i1, i2); }
     if (lane == 0) {
         double* rp = report + b * rs_b;
         const long long sk = rs_k;
         rp[0] = t3 - dist; rp[sk] = roll_e - roll_g; rp[2 * sk] = pitch_e - pitch_g; rp[3 * sk] = yaw_e - yaw_g;
-        rp[4 * sk] = (s0 / n) * dist; rp[5 * sk] = m0 * dist;  // :452-453
-        rp[6 * sk] = (s1 / n) * dist; rp[7 * sk] = m1 * dist;
-        rp[8 * sk] = (s2 / n) * dist; rp[9 * sk] = m2 * dist;
+        rp[4 * sk] = (s0 / (MASKED ? nv : n)) * dist; rp[5 * sk] = m0 * dist;  // :452-453
+        rp[6 * sk] = (s1 / (MASKED ? nv : n)) * dist; rp[7 * sk] = m1 * dist;
+        rp[8 * sk] = (s2 / (MASKED ? nv : n)) * dist; rp[9 * sk] = m2 * dist;
         rp[10 * sk] = t3; rp[11 * sk] = dist; rp[12 * sk] = roll_e; rp[13 * sk] = pitch_e; rp[14 * sk] = yaw_e; rp[15 * sk] = 0.0;
         if (flags) {                                           // check_if_the_sample_passed (:55-62), depth in cm
             flags[b * 4] = fabs(t3 * 100.0 - dist * 100.0) < bounds.b[0];
@@ -305,6 +318,7 @@ struct ReportArgs {
     const T* tail; long long ld; T* res; double kinv[6];
     int use_tmap;
     alignas(64) CUtensorMap tmap;   // uv as a 2-D tensor (RowStream), valid when use_tmap
+    const uint32_t* vis; int vis_words;   // [B, vis_words] visibility bits (masked kernels only)
 };
 
 PNP_DEV void fold_camera(const double* K, const double (&R)[9], const double (&t)[3], double (&M)[9], double (&m)[3])
@@ -452,9 +466,11 @@ __global__ void __launch_bounds__(32) k_report_thread(const __grid_constant__ Re
                                   // chunk buffers (~19 KB per CTA) admit 11 CTAs per SM, so a tighter cap buys no occupancy
 #endif
 constexpr int kReportUnroll = PNP_REPORT_UNROLL;
-template <typename T, int RES, bool SKEW>
+// MASKED (RES = 0 only): columns 4-9 run over the landmarks whose bit is set in a.vis
+template <typename T, int RES, bool SKEW, bool MASKED = false>
 __global__ void __launch_bounds__(32, PNP_REPORT_MINBLOCKS) k_report_chunk(const __grid_constant__ ReportArgs<T> a)
 {
+    static_assert(!(MASKED && RES), "the fused residual has no masked form");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     typedef typename Vec2<T>::type V2;
     T* sBuf = reinterpret_cast<T*>(smem_raw);
@@ -499,12 +515,15 @@ __global__ void __launch_bounds__(32, PNP_REPORT_MINBLOCKS) k_report_chunk(const
         double s0 = 0, s1 = 0, s2 = 0, m0 = 0, m1 = 0, m2 = 0;
         int i0 = -1, i1 = -1, i2 = -1;
         T acc0 = T(0), acc1 = T(0);
+        const uint32_t* vw = MASKED ? a.vis + (size_t)b * a.vis_words : nullptr;
+        const int nv = MASKED ? count_visible(vw, nullptr, a.n) : 0;
         for (int c = 0; c < rs.n_chunks; ++c) {
             const V2* row = rs.wait(c, lane);
             const int cnt = rs.count(c), base = c * rs.chunk;
 #pragma unroll kReportUnroll
             for (int k = 0; k < cnt; ++k) {
                 const int i = base + k;
+                if constexpr (MASKED) { if (!mask_bit(vw, i)) continue; }
                 const T th[3] = { sP[3 * i], sP[3 * i + 1], sP[3 * i + 2] };
                 const double x = (double)th[0], y = (double)th[1], z = (double)th[2];
                 double pe[2], pg[2], ie, ig, e0, e1, e2;
@@ -532,13 +551,14 @@ __global__ void __launch_bounds__(32, PNP_REPORT_MINBLOCKS) k_report_chunk(const
             }
             rs.done(c, lane);
         }
+        if constexpr (MASKED) { if (nv < kMinVisible) too_few_for_report(s0, s1, s2, m0, m1, m2, i0, i1, i2); }
         if (ok) {
             double* rp = a.report + b * a.rs_b;
             const long long sk = a.rs_k;
             rp[0] = t3 - dist; rp[sk] = roll_e - roll_g; rp[2 * sk] = pitch_e - pitch_g; rp[3 * sk] = yaw_e - yaw_g;
-            rp[4 * sk] = (s0 / a.n) * dist; rp[5 * sk] = m0 * dist;
-            rp[6 * sk] = (s1 / a.n) * dist; rp[7 * sk] = m1 * dist;
-            rp[8 * sk] = (s2 / a.n) * dist; rp[9 * sk] = m2 * dist;
+            rp[4 * sk] = (s0 / (MASKED ? nv : a.n)) * dist; rp[5 * sk] = m0 * dist;
+            rp[6 * sk] = (s1 / (MASKED ? nv : a.n)) * dist; rp[7 * sk] = m1 * dist;
+            rp[8 * sk] = (s2 / (MASKED ? nv : a.n)) * dist; rp[9 * sk] = m2 * dist;
             rp[10 * sk] = t3; rp[11 * sk] = dist; rp[12 * sk] = roll_e; rp[13 * sk] = pitch_e; rp[14 * sk] = yaw_e; rp[15 * sk] = 0.0;
             if (a.flags) {
                 a.flags[b * 4] = fabs(t3 * 100.0 - dist * 100.0) < a.bounds[0];
@@ -584,6 +604,7 @@ struct CheckArgs {
     int32_t* status; T* reproj;
     int use_tmap;
     alignas(64) CUtensorMap tmap;   // uv as a 2-D tensor (RowStream), valid when use_tmap
+    const uint32_t* vis; int vis_words;   // [B, vis_words] visibility bits (masked kernels only)
 };
 
 template <typename T>
@@ -613,11 +634,12 @@ PNP_DEV int32_t check_status(const double (&R)[9], const double (&t)[3], double 
     return s;
 }
 
-template <typename T>
+// n_visible: the landmarks the sum ran over (MASKED), else a.n
+template <typename T, bool MASKED = false>
 PNP_DEV void store_check(const CheckArgs<T>& a, long long b, const double (&R)[9], const double (&t)[3], double res, bool bad,
-                         double sum, double mx, bool behind)
+                         double sum, double mx, bool behind, int n_visible = 0)
 {
-    double mean = sum / a.n;                              // (s1 / n) * distance_GT of the report, distance_GT = 1
+    double mean = sum / (MASKED ? n_visible : a.n);       // (s1 / n) * distance_GT of the report, distance_GT = 1
     if (bad) mean = mx = __longlong_as_double(0x7ff8000000000000LL);
     if (a.reproj) { a.reproj[b * 2] = (T)mean; a.reproj[b * 2 + 1] = (T)mx; }
     a.status[b] = check_status(R, t, res, mean, mx, behind, a.limit);
@@ -628,7 +650,8 @@ PNP_DEV void store_check(const CheckArgs<T>& a, long long b, const double (&R)[9
 #ifndef PNP_CHECK_MINBLOCKS
 #define PNP_CHECK_MINBLOCKS 16
 #endif
-template <typename T>
+// MASKED: mean, max and BEHIND over the landmarks whose bit is set in a.vis; fewer than kMinVisible of them: NaN, NONFINITE
+template <typename T, bool MASKED = false>
 __global__ void __launch_bounds__(32, PNP_CHECK_MINBLOCKS) k_check_chunk(const __grid_constant__ CheckArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -657,12 +680,15 @@ __global__ void __launch_bounds__(32, PNP_CHECK_MINBLOCKS) k_check_chunk(const _
         fold_camera(a.K, R, t, M, m);
         double s = 0, mx = 0;
         bool behind = false;
+        const uint32_t* vw = MASKED ? a.vis + (size_t)b * a.vis_words : nullptr;
+        const int nv = MASKED ? count_visible(vw, nullptr, a.n) : 0;
         for (int c = 0; c < rs.n_chunks; ++c) {
             const V2* row = rs.wait(c, lane);
             const int cnt = rs.count(c), base = c * rs.chunk;
 #pragma unroll kReportUnroll
             for (int k = 0; k < cnt; ++k) {
                 const int i = base + k;
+                if constexpr (MASKED) { if (!mask_bit(vw, i)) continue; }
                 double pe[2], ie, ex, ey;
                 bool be;
                 project_folded(M, m, (double)P[3 * i], (double)P[3 * i + 1], (double)P[3 * i + 2], pe, ie, be);   // TEST_TOOLBOX.py:312
@@ -674,7 +700,7 @@ __global__ void __launch_bounds__(32, PNP_CHECK_MINBLOCKS) k_check_chunk(const _
             }
             rs.done(c, lane);
         }
-        if (ok) store_check(a, b, R, t, res, bad, s, mx, behind);
+        if (ok) store_check<T, MASKED>(a, b, R, t, res, bad || (MASKED && nv < kMinVisible), s, mx, behind, nv);
         tile += gridDim.x;
         if (tile < n_tiles) {
             fence_proxy_async();
@@ -689,7 +715,7 @@ __global__ void __launch_bounds__(32, PNP_CHECK_MINBLOCKS) k_check_chunk(const _
 
 // Rows the streaming shape cannot take (large n, FP32 rows that are not 16-byte granular): one warp per problem, the
 // lanes stride over the landmarks, the patterns are read from global memory.
-template <typename T>
+template <typename T, bool MASKED = false>
 __global__ void __launch_bounds__(256) k_check_warp(const __grid_constant__ CheckArgs<T> a)
 {
     const long long b = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -704,7 +730,10 @@ __global__ void __launch_bounds__(256) k_check_warp(const __grid_constant__ Chec
     fold_camera(a.K, R, t, M, m);
     double s = 0, mx = 0;
     bool behind = false;
+    const uint32_t* vw = MASKED ? a.vis + (size_t)b * a.vis_words : nullptr;
+    const int nv = MASKED ? count_visible(vw, nullptr, a.n) : 0;
     for (int i = lane; i < a.n; i += 32) {
+        if constexpr (MASKED) { if (!mask_bit(vw, i)) continue; }
         double pe[2], ie, ex, ey;
         bool be;
         project_folded(M, m, (double)__ldg(P + 3 * i), (double)__ldg(P + 3 * i + 1), (double)__ldg(P + 3 * i + 2), pe, ie, be);
@@ -721,7 +750,7 @@ __global__ void __launch_bounds__(256) k_check_warp(const __grid_constant__ Chec
         if (o > mx) mx = o;
     }
     behind = __any_sync(0xffffffffu, behind);
-    if (lane == 0) store_check(a, b, R, t, res, bad, s, mx, behind);
+    if (lane == 0) store_check<T, MASKED>(a, b, R, t, res, bad || (MASKED && nv < kMinVisible), s, mx, behind, nv);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1222,11 +1251,11 @@ using namespace pnpb200;
 
 namespace pnpb200 {
 
-template <typename T, int RES, bool SKEW>
+template <typename T, int RES, bool SKEW, bool MASKED = false>
 int launch_report_chunk(const ReportArgs<T>& a, unsigned grid, size_t smem, cudaStream_t st)
 {
-    PNP_CUDA_OK(set_dynamic_smem((const void*)k_report_chunk<T, RES, SKEW>, smem));
-    k_report_chunk<T, RES, SKEW><<<grid, 32, smem, st>>>(a);
+    PNP_CUDA_OK(set_dynamic_smem((const void*)k_report_chunk<T, RES, SKEW, MASKED>, smem));
+    k_report_chunk<T, RES, SKEW, MASKED><<<grid, 32, smem, st>>>(a);
     return PNPB200_OK;
 }
 
@@ -1241,9 +1270,10 @@ bool report_can_fuse(int dtype, int n)
 int report_launch(int dtype, int64_t B, int n, const void* pattern, const void* uv, const double* K,
                   const void* R, const void* t, const void* euler_deg, const double* gt, const double* bounds,
                   double* report, int64_t report_stride_problem, int64_t report_stride_column,
-                  int32_t* flags, int32_t* max_idx, const ReportFuse* fuse, cudaStream_t st)
+                  int32_t* flags, int32_t* max_idx, const ReportFuse* fuse, cudaStream_t st, const uint32_t* vis)
 {
     if (B < 0 || n < 1 || !pattern || !uv || !K || !R || !t || !euler_deg || !gt || !report) return PNPB200_EINVAL;
+    if (vis && (fuse || !vis_aligned(vis))) return PNPB200_EINVAL;         // the fused residual has no masked form
     if (report_stride_problem < 1 || report_stride_column < 1) return PNPB200_EINVAL;
     const long long rs_b = report_stride_problem, rs_k = report_stride_column;
     if (((uintptr_t)uv & 15u) != 0) return PNPB200_EINVAL;   // rows are staged with 16-byte bulk copies
@@ -1274,7 +1304,8 @@ int report_launch(int dtype, int64_t B, int n, const void* pattern, const void* 
             a.tail = fuse ? (const TT*)fuse->tail : nullptr; a.ld = fuse ? fuse->ld : 0; a.res = fuse ? (TT*)fuse->res : nullptr; \
             for (int e = 0; e < 6; ++e) a.kinv[e] = fuse ? fuse->kinv[e] : 0.0;                                         \
             a.use_tmap = (sg.pitch == sg.chunk * 2) ? make_row_tensor_map(&a.tmap, uv, (int)sizeof(TT), B, n, sg.chunk) : 0; \
-            const int rc = (res_mode == 1) ? (skew ? launch_report_chunk<TT, 1, true>(a, grid, csmem, st)               \
+            a.vis = vis; a.vis_words = (n + 31) / 32;                                                                   \
+            const int rc = vis ? launch_report_chunk<TT, 0, true, true>(a, grid, csmem, st) : (res_mode == 1) ? (skew ? launch_report_chunk<TT, 1, true>(a, grid, csmem, st)               \
                                                    : launch_report_chunk<TT, 1, false>(a, grid, csmem, st))             \
                          : (res_mode == 2) ? (skew ? launch_report_chunk<TT, 2, true>(a, grid, csmem, st)               \
                                                    : launch_report_chunk<TT, 2, false>(a, grid, csmem, st))             \
@@ -1284,7 +1315,7 @@ int report_launch(int dtype, int64_t B, int n, const void* pattern, const void* 
         }
         DISPATCH_DTYPE(dtype, LAUNCH_REPORT_CHUNK(double), LAUNCH_REPORT_CHUNK(float));
 #undef LAUNCH_REPORT_CHUNK
-    } else if (g.tile_bytes <= 48 * 1024) {
+    } else if (g.tile_bytes <= 48 * 1024 && !vis) {
         const long long n_tiles = (B + kTileProblems - 1) / kTileProblems;
         const unsigned grid = (unsigned)(n_tiles < 0x7fffffffLL ? n_tiles : 0x7fffffffLL);
 #define LAUNCH_REPORT_THREAD(TT)                                                                                        \
@@ -1301,6 +1332,12 @@ int report_launch(int dtype, int64_t B, int n, const void* pattern, const void* 
         }
         DISPATCH_DTYPE(dtype, LAUNCH_REPORT_THREAD(double), LAUNCH_REPORT_THREAD(float));
 #undef LAUNCH_REPORT_THREAD
+    } else if (vis) {                                         // masked rows the streaming kernel cannot take: one warp per problem
+        const unsigned grid = grid_for(B * 32, 256);
+        const int W = (n + 31) / 32;
+        DISPATCH_DTYPE(dtype,
+                       (k_report<double, true><<<grid, 256, 0, st>>>(B, n, pattern, uv, km, R, t, euler_deg, gt, bd, report, rs_b, rs_k, flags, max_idx, vis, W)),
+                       (k_report<float, true><<<grid, 256, 0, st>>>(B, n, pattern, uv, km, R, t, euler_deg, gt, bd, report, rs_b, rs_k, flags, max_idx, vis, W))); count_kernel_launches(1);
     } else {
         const unsigned grid = grid_for(B * 32, 256);
         DISPATCH_DTYPE(dtype,
@@ -1314,9 +1351,10 @@ int report_launch(int dtype, int64_t B, int n, const void* pattern, const void* 
 // the execution shape of report_launch: the streaming kernel where report_can_fuse, one warp per problem otherwise
 int check_launch(int dtype, int64_t B, int n, const void* pattern, int n_patterns, const void* uv, const double* K,
                  const void* R, const void* t, const void* res_norm, const int32_t* best_pattern, double limit,
-                 int32_t* status, void* reproj, cudaStream_t st)
+                 int32_t* status, void* reproj, cudaStream_t st, const uint32_t* vis)
 {
     if (B < 0 || n < 1 || !pattern || !uv || !K || !R || !t || !status) return PNPB200_EINVAL;
+    if (vis && !vis_aligned(vis)) return PNPB200_EINVAL;
     if (n_patterns < 1 || n_patterns > PNPB200_MAX_PATTERNS) return PNPB200_EINVAL;
     if (dtype != PNPB200_DTYPE_F64 && dtype != PNPB200_DTYPE_F32) return PNPB200_EINVAL;
     if (((uintptr_t)uv & 15u) != 0) return PNPB200_EINVAL;   // rows are staged with 16-byte bulk copies
@@ -1329,6 +1367,7 @@ int check_launch(int dtype, int64_t B, int n, const void* pattern, int n_pattern
         for (int e = 0; e < 9; ++e) a.K[e] = K[e];                                                                      \
         a.limit = (limit > 0.0) ? limit : 0.0;                                                                          \
         a.status = status; a.reproj = (TT*)reproj; a.use_tmap = 0;                                                      \
+        a.vis = vis; a.vis_words = (n + 31) / 32;                                                                       \
         const StreamGeom sg = stream_geometry<TT>(n);                                                                   \
         if (report_can_fuse(dtype, n)) {                                                                                \
             DeviceProps dp;                                                                                             \
@@ -1339,11 +1378,18 @@ int check_launch(int dtype, int64_t B, int n, const void* pattern, int n_pattern
             a.row_pitch = sg.pitch; a.chunk = sg.chunk;                                                                 \
             a.use_tmap = (sg.pitch == sg.chunk * 2) ? make_row_tensor_map(&a.tmap, uv, (int)sizeof(TT), B, n, sg.chunk) : 0; \
             const long long n_tiles = (B + kTileProblems - 1) / kTileProblems;                                          \
-            PNP_CUDA_OK(set_dynamic_smem((const void*)k_check_chunk<TT>, smem));                                        \
-            k_check_chunk<TT><<<(unsigned)(n_tiles < 0x7fffffffLL ? n_tiles : 0x7fffffffLL), 32, smem, st>>>(a);        \
+            const unsigned grid = (unsigned)(n_tiles < 0x7fffffffLL ? n_tiles : 0x7fffffffLL);                          \
+            if (vis) {                                                                                                  \
+                PNP_CUDA_OK(set_dynamic_smem((const void*)k_check_chunk<TT, true>, smem));                              \
+                k_check_chunk<TT, true><<<grid, 32, smem, st>>>(a);                                                     \
+            } else {                                                                                                    \
+                PNP_CUDA_OK(set_dynamic_smem((const void*)k_check_chunk<TT>, smem));                                    \
+                k_check_chunk<TT><<<grid, 32, smem, st>>>(a);                                                           \
+            }                                                                                                           \
         } else {                                                                                                        \
             a.row_pitch = 0; a.chunk = 0;                                                                               \
-            k_check_warp<TT><<<grid_for(B * 32, 256), 256, 0, st>>>(a);                                                 \
+            if (vis) k_check_warp<TT, true><<<grid_for(B * 32, 256), 256, 0, st>>>(a);                                  \
+            else     k_check_warp<TT><<<grid_for(B * 32, 256), 256, 0, st>>>(a);                                        \
         }                                                                                                               \
         count_kernel_launches(1);                                                                                       \
     }
@@ -1363,6 +1409,15 @@ int pnpb200_check_batch(int dtype, int64_t B, int n_total, const void* pattern, 
 {
     return check_launch(dtype, B, n_total, pattern, n_patterns, uv, K, R, t, res_norm, best_pattern, reproj_limit_px, status,
                         reproj, (cudaStream_t)stream);
+}
+
+int pnpb200_check_batch_masked(int dtype, int64_t B, int n_total, const void* pattern, int n_patterns, const void* uv,
+                               const double* K, const void* R, const void* t, const void* res_norm, const int32_t* best_pattern,
+                               double reproj_limit_px, int32_t* status, void* reproj, const uint32_t* visible, void* stream)
+{
+    if (!visible) return PNPB200_EINVAL;
+    return check_launch(dtype, B, n_total, pattern, n_patterns, uv, K, R, t, res_norm, best_pattern, reproj_limit_px, status,
+                        reproj, (cudaStream_t)stream, visible);
 }
 
 int pnpb200_default_synth(pnpb200_synth* s)
@@ -1459,6 +1514,16 @@ int pnpb200_report_batch_strided(int dtype, int64_t B, int n, const void* patter
 {
     return report_launch(dtype, B, n, pattern, uv, K, R, t, euler_deg, gt, bounds, report, report_stride_problem,
                          report_stride_column, flags, max_idx, nullptr, (cudaStream_t)stream);
+}
+
+int pnpb200_report_batch_strided_masked(int dtype, int64_t B, int n, const void* pattern, const void* uv, const double* K,
+                                        const void* R, const void* t, const void* euler_deg, const double* gt, const double* bounds,
+                                        double* report, int64_t report_stride_problem, int64_t report_stride_column,
+                                        int32_t* flags, int32_t* max_idx, const uint32_t* visible, void* stream)
+{
+    if (!visible) return PNPB200_EINVAL;
+    return report_launch(dtype, B, n, pattern, uv, K, R, t, euler_deg, gt, bounds, report, report_stride_problem,
+                         report_stride_column, flags, max_idx, nullptr, (cudaStream_t)stream, visible);
 }
 
 }  // extern "C"

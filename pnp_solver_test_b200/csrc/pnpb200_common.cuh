@@ -13,6 +13,7 @@
 #define PNP_NCORE 33        // constants of the LM system kept next to the moments by k_iterate (S33 6, S13 9, S23 9, c 9)
 #define PNP_NTAIL 12
 #define PNP_PATC 20
+#define PNP_NPMOM 10       // masked moment mapping: per-problem pattern moments (sum theta theta^T 6, sum theta 3, count) behind the moments
 // landmark selections up to this size travel inside the kernel arguments; larger ones through device memory
 #define PNP_MAX_INLINE_IDX 96
 // QEIF takes H^T H, H^T v (and, in the moment mapping, the residual of its exit test) from the moments from this many landmarks on
@@ -64,11 +65,14 @@ struct ReportFuse { int res_mode; /* 1: LM, 2: linear F2 */ const void* tail; lo
 bool report_can_fuse(int dtype, int n);
 int report_launch(int dtype, int64_t B, int n, const void* pattern, const void* uv, const double* K, const void* R, const void* t,
                   const void* euler_deg, const double* gt, const double* bounds, double* report, int64_t report_stride_problem,
-                  int64_t report_stride_column, int32_t* flags, int32_t* max_idx, const ReportFuse* fuse, cudaStream_t st);
+                  int64_t report_stride_column, int32_t* flags, int32_t* max_idx, const ReportFuse* fuse, cudaStream_t st,
+                  const uint32_t* vis = nullptr);
+// a visibility mask [B, ceil(n_total / 32)] uint32 must be 4-byte aligned
+inline bool vis_aligned(const uint32_t* vis) { return ((uintptr_t)vis & 3u) == 0; }
 // solution check (pnpb200_check_batch), pnpb200_aux.cu
 int check_launch(int dtype, int64_t B, int n, const void* pattern, int n_patterns, const void* uv, const double* K,
                  const void* R, const void* t, const void* res_norm, const int32_t* best_pattern, double limit,
-                 int32_t* status, void* reproj, cudaStream_t st);
+                 int32_t* status, void* reproj, cudaStream_t st, const uint32_t* vis = nullptr);
 cudaError_t set_dynamic_smem(const void* kernel, size_t bytes);                                   // defined in pnpb200_api.cu
 cudaError_t blocks_per_sm(int* out, const void* kernel, int block_threads, size_t smem_bytes);   // defined in pnpb200_api.cu
 
@@ -118,7 +122,7 @@ extern thread_local ProfileRing g_prof;            // defined in pnpb200_api.cu
 #define PNP_SOLVE_PART_ARGS                                                                                          \
     int method, long long B, int n_total, int n, const void *uv, const void *pattern, int n_patterns,                 \
         const int32_t *idx_host, const int32_t *idx_dev, const double *K, const pnpb200_params &prm, void *R, void *t, \
-        void *euler, void *res, int32_t *iters, int32_t *best, cudaStream_t stream
+        void *euler, void *res, int32_t *iters, int32_t *best, cudaStream_t stream, const uint32_t *vis
 int solve_part_f64_g0(PNP_SOLVE_PART_ARGS);
 int solve_part_f64_g1(PNP_SOLVE_PART_ARGS);
 int solve_part_f64_g2(PNP_SOLVE_PART_ARGS);

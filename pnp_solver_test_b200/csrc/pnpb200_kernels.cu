@@ -67,6 +67,8 @@ struct SolveArgs {
     void* ws; size_t ws_bytes;   // optional caller scratch (moment mapping)
     int profile, tune;
     int skip_residual;           // moment mapping: leave res_norm to the caller's fused report pass (pnpb200_solve_report_batch)
+    const uint32_t* vis;         // [B, vis_words] per-problem visibility bits (masked kernels only)
+    int vis_words;
 };
 
 // raw pixels of one problem in global memory, normalised on the fly (warp mapping)
@@ -81,6 +83,8 @@ struct PtsGlobal {
         const typename Vec2<T>::type p = __ldg(reinterpret_cast<const typename Vec2<T>::type*>(row) + j);
         normalise_px<T>(p.x, p.y, k00, k01, k02, k10, k11, k12, bx, by);
     }
+    PNP_DEV bool vis(int) const { return true; }
+    PNP_DEV int count(int n) const { return n; }
 };
 
 // Pattern constants (PNP_PATC per pattern) by one warp: M0, m0, n and G = (D^T D)^-1.
@@ -118,6 +122,80 @@ PNP_DEV void pattern_constants(const T* __restrict__ sP, int n, T* __restrict__ 
 #pragma unroll
         for (int e = 0; e < 10; ++e) sC[10 + e] = (T)G[e];
     }
+}
+
+// Sum theta theta^T (6), sum theta (3) and the count (pm[9]) over the visible landmarks of ONE problem (masked kernels; LPP = 1:
+// one thread, 32: one warp, every lane ends with the sums).  The moment mapping keeps them per problem in the workspace.
+constexpr int kPatternMoments = PNP_NPMOM;
+template <typename T, int LPP, typename Pts>
+PNP_DEV void pattern_moments_masked(const Pts& pts, const T* __restrict__ sP, int n, int sub, double (&pm)[kPatternMoments])
+{
+#pragma unroll
+    for (int e = 0; e < 9; ++e) pm[e] = 0.0;
+    for (int i = sub; i < n; i += LPP) {
+        if (!pts.vis(i)) continue;
+        const double th[3] = { (double)sP[3 * i], (double)sP[3 * i + 1], (double)sP[3 * i + 2] };
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+#pragma unroll
+            for (int b = a; b < 3; ++b) pm[s3(a, b)] = fma(th[a], th[b], pm[s3(a, b)]);
+            pm[6 + a] += th[a];
+        }
+    }
+#pragma unroll
+    for (int e = 0; e < 9; ++e) pm[e] = group_sum<LPP, double>(pm[e]);
+    pm[9] = (double)pts.count(n);
+}
+
+// the PNP_PATC constants of one problem from its pattern moments: M0, m0, n and G = (D^T D)^-1 (pattern_constants, per problem).
+// n in sC[9] is the number of visible landmarks: it enters LM's and the filters' systems as well.
+template <typename T>
+PNP_DEV void constants_from_pattern_moments(const double (&pm)[kPatternMoments], T* __restrict__ sC)
+{
+    double G[10];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+#pragma unroll
+        for (int b = a; b < 3; ++b) G[sidx<4>(a, b)] = pm[s3(a, b)];
+        G[sidx<4>(a, 3)] = pm[6 + a];
+    }
+    G[sidx<4>(3, 3)] = pm[9];
+    spd_inverse<double, 4>(G);
+#pragma unroll
+    for (int e = 0; e < 10; ++e) sC[e] = (T)pm[e];
+#pragma unroll
+    for (int e = 0; e < 10; ++e) sC[10 + e] = (T)G[e];
+}
+
+template <typename T, int LPP, typename Pts>
+PNP_DEV void pattern_constants_masked(const Pts& pts, const T* __restrict__ sP, int n, T* __restrict__ sC, int sub)
+{
+    double pm[kPatternMoments];
+    pattern_moments_masked<T, LPP>(pts, sP, n, sub, pm);
+    if (sub == 0) constants_from_pattern_moments<T>(pm, sC);
+}
+
+// methods whose direct solvers read the pattern constants
+__host__ __device__ constexpr bool method_uses_patc(int m)
+{
+    return m == PNPB200_METHOD_LM || m == PNPB200_METHOD_LINEAR_F2 || m == PNP_METHOD_QEIF_HYBRID || m == PNPB200_METHOD_EIF2;
+}
+
+// fewer than 4 visible landmarks: no solve.  NaN pose and res_norm, 0 iterations, pattern 0.
+template <typename T>
+PNP_DEV T nan_of() { return (T)__longlong_as_double(0x7ff8000000000000LL); }
+
+template <typename T>
+PNP_DEV void too_few_landmarks(Result<T>& r, int& best_p)
+{
+    const T q = nan_of<T>();
+#pragma unroll
+    for (int e = 0; e < 9; ++e) r.R[e] = q;
+#pragma unroll
+    for (int e = 0; e < 3; ++e) r.t[e] = q;
+    r.res = q;
+    r.iters = 0;
+    best_p = 0;
 }
 
 template <typename T, int METHOD, int LPP, typename Pts>
@@ -198,15 +276,16 @@ PNP_DEV void load_pattern(const T* __restrict__ pattern, const int32_t* __restri
 // ------------------------------------------------------------------------------------------
 // direct mapping, one problem per thread; CTA = 1 warp = 32 consecutive problems
 // ------------------------------------------------------------------------------------------
-template <typename T, int METHOD>
+// MASKED: problem b sees only its visible landmarks (a.vis); every lane keeps its own constants, computed per tile
+template <typename T, int METHOD, bool MASKED = false>
 __global__ void __launch_bounds__(32) k_solve_thread(const __grid_constant__ SolveArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    // [tile rows | pattern | constants | index | mbarrier]
+    // [tile rows | pattern | constants (masked: per lane) | index | mbarrier]
     T* sRows = reinterpret_cast<T*>(smem_raw);
     T* sP = sRows + (size_t)kTileProblems * a.row_pitch;
     T* sC = sP + (size_t)a.n_patterns * a.n * 3;
-    int32_t* sIdx = reinterpret_cast<int32_t*>(sC + a.n_patterns * PNP_PATC);
+    int32_t* sIdx = reinterpret_cast<int32_t*>(sC + (MASKED ? kTileProblems : 1) * a.n_patterns * PNP_PATC);
     const int lane = threadIdx.x;
     const int32_t* sel = selection_of(a);
     RowTile<T> tile_buf;
@@ -217,18 +296,32 @@ __global__ void __launch_bounds__(32) k_solve_thread(const __grid_constant__ Sol
     // kick off the first tile's copies before touching the pattern so the two overlap
     int valid = (tile < n_tiles) ? tile_buf.issue(tile, lane) : 0;
     load_pattern<T>(a.pattern, sel, a.n_total, a.n, a.n_patterns, sP, sIdx, lane, 32);
-    if (METHOD == PNPB200_METHOD_LM || METHOD == PNPB200_METHOD_LINEAR_F2 || METHOD == PNP_METHOD_QEIF_HYBRID || METHOD == PNPB200_METHOD_EIF2) {
+    if (!MASKED && method_uses_patc(METHOD)) {
         for (int p = 0; p < a.n_patterns; ++p) pattern_constants<T>(sP + (size_t)p * a.n * 3, a.n, sC + p * PNP_PATC, lane);
         __syncwarp();
     }
     while (tile < n_tiles) {
         const long long b0 = tile * kTileProblems;
-        PtsRow<T> pts;
-        pts.row = tile_buf.acquire(lane, valid);
-        pts.idx = sel ? sIdx : nullptr;
         Result<T> best;
         int best_p;
-        solve_all_patterns<T, METHOD, 1, PtsRow<T> >(pts, sP, sC, a.n, a.n_patterns, 0, a.prm, best, best_p);
+        if constexpr (MASKED) {
+            // spare lanes of a ragged tile shadow the last problem, as their rows do (RowTile::acquire)
+            PtsMasked<PtsRow<T> > pts;
+            pts.row = tile_buf.acquire(lane, valid);
+            pts.idx = sel ? sIdx : nullptr;
+            pts.words = a.vis + (size_t)(b0 + (lane < valid ? lane : valid - 1)) * a.vis_words;
+            pts.nvis = count_visible(pts.words, pts.idx, a.n);
+            T* myC = sC + (size_t)lane * a.n_patterns * PNP_PATC;
+            if (method_uses_patc(METHOD))
+                for (int p = 0; p < a.n_patterns; ++p) pattern_constants_masked<T, 1>(pts, sP + (size_t)p * a.n * 3, a.n, myC + p * PNP_PATC, 0);
+            solve_all_patterns<T, METHOD, 1, PtsMasked<PtsRow<T> > >(pts, sP, myC, a.n, a.n_patterns, 0, a.prm, best, best_p);
+            if (pts.nvis < kMinVisible) too_few_landmarks<T>(best, best_p);
+        } else {
+            PtsRow<T> pts;
+            pts.row = tile_buf.acquire(lane, valid);
+            pts.idx = sel ? sIdx : nullptr;
+            solve_all_patterns<T, METHOD, 1, PtsRow<T> >(pts, sP, sC, a.n, a.n_patterns, 0, a.prm, best, best_p);
+        }
         const long long b = b0 + lane;
         if (b < a.B) write_result<T>(a, b, best, best_p);
         tile += gridDim.x;
@@ -265,6 +358,9 @@ struct MomArgs {
     int32_t* fix_list;      // filters: [0] = number of 32-problem tiles with a marked problem, [1..] = those tiles (k_iterate appends)
     int use_tmap;
     alignas(64) CUtensorMap tmap;   // uv of this launch as a 2-D tensor (RowStream), valid when use_tmap
+    // masked kernels: [B, vis_words] visibility bits, and the per-problem pattern moments [kPatternMoments][ld] in the workspace
+    const uint32_t* vis; int vis_words;
+    T* pmom;
 };
 
 template <typename T>
@@ -310,7 +406,8 @@ __global__ void __launch_bounds__(32) k_pattern_constants(const __grid_constant_
 }
 
 // PASS 0: moments.  PASS 1: residual at the stored state (LM: x before the last update; F2: tail).
-template <typename T, int METHOD, int PASS>
+// MASKED: over each problem's visible landmarks; PASS 0 also stores the problem's pattern moments (a.pmom).
+template <typename T, int METHOD, int PASS, bool MASKED = false>
 __global__ void __launch_bounds__(32) k_stream_thread(const __grid_constant__ MomArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -338,7 +435,41 @@ __global__ void __launch_bounds__(32) k_stream_thread(const __grid_constant__ Mo
         PtsRow<T> pts;
         pts.row = tile_buf.acquire(lane, valid);
         pts.idx = sel ? sIdx : nullptr;
-        if (PASS == 0) {
+        if constexpr (MASKED) {
+            PtsMasked<PtsRow<T> > pm;
+            static_cast<PtsRow<T>&>(pm) = pts;
+            pm.words = a.vis + (size_t)b * a.vis_words;
+            pm.nvis = count_visible(pm.words, pm.idx, a.n);
+            if (PASS == 0) {
+                Moments<T> mom;
+                accumulate_moments<T, 1, PtsMasked<PtsRow<T> >, method_with_w(METHOD), method_with_s(METHOD)>(pm, sP, a.n, 0, mom);
+                double pmo[kPatternMoments];
+                pattern_moments_masked<T, 1>(pm, sP, a.n, 0, pmo);
+                if (ok) {
+#pragma unroll
+                    for (int k = 0; k < method_nmom(METHOD); ++k) a.mom[(size_t)k * a.ld + b] = mom.at(k);
+#pragma unroll
+                    for (int k = 0; k < kPatternMoments; ++k) a.pmom[(size_t)k * a.ld + b] = (T)pmo[k];
+                }
+            } else {
+                T res;
+                if (method_lm_residual(METHOD)) {
+                    T x[12];
+#pragma unroll
+                    for (int k = 0; k < 12; ++k) x[k] = st[k];
+                    res = lm_residual_direct<T, 1, PtsMasked<PtsRow<T> > >(pm, sP, a.n, 0, x);
+                } else {
+                    F2Tail<T> f;
+#pragma unroll
+                    for (int k = 0; k < 3; ++k) f.phi3[k] = st[k];
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) { f.pxn[k] = st[3 + k]; f.pyn[k] = st[7 + k]; }
+                    res = f2_residual_direct<T, 1, PtsMasked<PtsRow<T> > >(pm, sP, a.n, 0, f);
+                }
+                if (pm.nvis < kMinVisible) res = nan_of<T>();     // not solved (a sum over no landmark would read 0)
+                if (ok && a.res) a.res[b] = res;
+            }
+        } else if (PASS == 0) {
             Moments<T> mom;
             accumulate_moments<T, 1, PtsRow<T>, method_with_w(METHOD), method_with_s(METHOD)>(pts, sP, a.n, 0, mom);
             if (ok) {
@@ -376,7 +507,8 @@ __global__ void __launch_bounds__(32) k_stream_thread(const __grid_constant__ Mo
 #define PNP_STREAM_UNROLL 2       // points in flight per thread in the chunk-streaming passes
 #endif
 constexpr int kStreamUnroll = PNP_STREAM_UNROLL;
-template <typename T, int METHOD, int PASS>
+// MASKED: over each problem's visible landmarks (a running mask word per chunk); PASS 0 also stores the pattern moments
+template <typename T, int METHOD, int PASS, bool MASKED = false>
 __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ MomArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -416,15 +548,38 @@ __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ Mom
                 for (int k = 0; k < 4; ++k) { f.pxn[k] = st[3 + k]; f.pyn[k] = st[7 + k]; }
             }
         }
+        const uint32_t* vw = MASKED ? a.vis + (size_t)b * a.vis_words : nullptr;
+        double pmo[kPatternMoments];
+        if constexpr (MASKED && PASS == 0) {
+#pragma unroll
+            for (int e = 0; e < kPatternMoments; ++e) pmo[e] = 0.0;
+        }
         for (int c = 0; c < rs.n_chunks; ++c) {
             const V2* row = rs.wait(c, lane);
             const int cnt = rs.count(c), i0 = c * rs.chunk;
+            uint32_t word = 0;                                // MASKED: bit 0 = landmark i0 + k
+            if constexpr (MASKED) word = __ldg(vw + (i0 >> 5)) >> (i0 & 31);
 #pragma unroll kStreamUnroll
             for (int k = 0; k < cnt; ++k) {
+                if constexpr (MASKED) {
+                    const int i = i0 + k;
+                    const bool v = word & 1u;
+                    word = ((i + 1) & 31) ? (word >> 1) : ((i + 1 < a.n) ? __ldg(vw + ((i + 1) >> 5)) : 0u);
+                    if (!v) continue;
+                }
                 const V2 px = row[k];
                 T bx, by;                                     // nu = K^-1 [u, v, 1]^T (:3305)
                 normalise_px<T>(px.x, px.y, k00, k01, k02, k10, k11, k12, bx, by);
                 const T th[3] = { sP[3 * (i0 + k)], sP[3 * (i0 + k) + 1], sP[3 * (i0 + k) + 2] };
+                if constexpr (MASKED && PASS == 0) {
+#pragma unroll
+                    for (int p = 0; p < 3; ++p) {
+#pragma unroll
+                        for (int q = p; q < 3; ++q) pmo[s3(p, q)] = fma((double)th[p], (double)th[q], pmo[s3(p, q)]);
+                        pmo[6 + p] += (double)th[p];
+                    }
+                    pmo[9] += 1.0;
+                }
                 if (PASS == 0) {
                     mom.template add<method_with_w(METHOD), method_with_s(METHOD)>(th, bx, by);
                 } else if (method_lm_residual(METHOD)) {
@@ -443,9 +598,16 @@ __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ Mom
             if (PASS == 0) {
 #pragma unroll
                 for (int k = 0; k < method_nmom(METHOD); ++k) a.mom[(size_t)k * a.ld + b] = mom.at(k);
+                if constexpr (MASKED) {
+#pragma unroll
+                    for (int k = 0; k < kPatternMoments; ++k) a.pmom[(size_t)k * a.ld + b] = (T)pmo[k];
+                }
             } else if (a.res) {
                 if (method_lm_residual(METHOD)) a.res[b] = t_sqrt(acc0);   // :2681
                 else { const T nx = t_sqrt(acc0), ny = t_sqrt(acc1); a.res[b] = t_sqrt(nx * nx + ny * ny); }   // :3374
+                if constexpr (MASKED) {
+                    if (count_visible(vw, nullptr, a.n) < kMinVisible) a.res[b] = nan_of<T>();   // not solved
+                }
             }
         }
         tile += gridDim.x;
@@ -456,7 +618,8 @@ __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ Mom
     }
 }
 
-template <typename T, int METHOD, int PASS>
+// MASKED: over each problem's visible landmarks; PASS 0 also stores the pattern moments
+template <typename T, int METHOD, int PASS, bool MASKED = false>
 __global__ void __launch_bounds__(256) k_stream_warp(const __grid_constant__ MomArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -471,6 +634,44 @@ __global__ void __launch_bounds__(256) k_stream_warp(const __grid_constant__ Mom
     pts.k10 = (T)a.kinv[3]; pts.k11 = (T)a.kinv[4]; pts.k12 = (T)a.kinv[5];
     for (long long b = (long long)blockIdx.x * nwarps + warp; b < a.B; b += (long long)gridDim.x * nwarps) {
         pts.row = a.uv + (size_t)b * a.n_total * 2;
+        if constexpr (MASKED) {
+            PtsMasked<PtsGlobal<T> > pm;
+            static_cast<PtsGlobal<T>&>(pm) = pts;
+            pm.words = a.vis + (size_t)b * a.vis_words;
+            pm.nvis = count_visible(pm.words, pm.idx, a.n);
+            if (PASS == 0) {
+                Moments<T> mom;
+                accumulate_moments<T, 32, PtsMasked<PtsGlobal<T> >, method_with_w(METHOD), method_with_s(METHOD)>(pm, sP, a.n, lane, mom);
+                double pmo[kPatternMoments];
+                pattern_moments_masked<T, 32>(pm, sP, a.n, lane, pmo);
+                T mine = T(0);
+#pragma unroll
+                for (int k = 0; k < method_nmom(METHOD); ++k) if (lane == k) mine = mom.at(k);
+                if (lane < method_nmom(METHOD)) a.mom[(size_t)lane * a.ld + b] = mine;
+                double pmine = 0.0;
+#pragma unroll
+                for (int k = 0; k < kPatternMoments; ++k) if (lane == k) pmine = pmo[k];
+                if (lane < kPatternMoments) a.pmom[(size_t)lane * a.ld + b] = (T)pmine;
+            } else {
+                T res;
+                if (method_lm_residual(METHOD)) {
+                    T x[12];
+#pragma unroll
+                    for (int k = 0; k < 12; ++k) x[k] = a.tail[(size_t)k * a.ld + b];
+                    res = lm_residual_direct<T, 32, PtsMasked<PtsGlobal<T> > >(pm, sP, a.n, lane, x);
+                } else {
+                    F2Tail<T> f;
+#pragma unroll
+                    for (int k = 0; k < 3; ++k) f.phi3[k] = a.tail[(size_t)k * a.ld + b];
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) { f.pxn[k] = a.tail[(size_t)(3 + k) * a.ld + b]; f.pyn[k] = a.tail[(size_t)(7 + k) * a.ld + b]; }
+                    res = f2_residual_direct<T, 32, PtsMasked<PtsGlobal<T> > >(pm, sP, a.n, lane, f);
+                }
+                if (pm.nvis < kMinVisible) res = nan_of<T>();     // not solved (a sum over no landmark would read 0)
+                if (lane == 0 && a.res) a.res[b] = res;
+            }
+            continue;
+        }
         if (PASS == 0) {
             Moments<T> mom;
             accumulate_moments<T, 32, PtsGlobal<T>, method_with_w(METHOD), method_with_s(METHOD)>(pts, sP, a.n, lane, mom);
@@ -662,6 +863,7 @@ __global__ void __launch_bounds__(kRingWarps * 32) k_stream_warp_tma(const __gri
 // problems are all unmarked reads 32 / 1 flags and leaves.
 // ------------------------------------------------------------------------------------------
 template <typename T> __device__ __forceinline__ void write_pose(const MomArgs<T>& a, long long b, const Result<T>& out);
+constexpr int kWarpsPerFixup = 8;                             // k_fixup_warp: 256 threads
 
 template <typename T, int METHOD, int LPP, typename Pts>
 PNP_DEV void run_filter_with_tail(const Pts& pts, const T* sP, const T* sC, int n, int sub, const SolverPrm<T>& prm, T (&xt)[12],
@@ -671,14 +873,15 @@ PNP_DEV void run_filter_with_tail(const Pts& pts, const T* sP, const T* sC, int 
     else                                  solve_eif2_with_tail<T, LPP, Pts>(pts, sP, sC, n, sub, prm, xt, out);
 }
 
-template <typename T, int METHOD>
+// MASKED: each lane solves on its problem's visible landmarks with its own constants
+template <typename T, int METHOD, bool MASKED = false>
 __global__ void __launch_bounds__(32) k_fixup_thread(const __grid_constant__ MomArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     T* sRows = reinterpret_cast<T*>(smem_raw);
     T* sP = sRows + (size_t)kTileProblems * a.row_pitch;
     T* sC = sP + (size_t)a.n * 3;
-    int32_t* sIdx = reinterpret_cast<int32_t*>(sC + PNP_PATC);
+    int32_t* sIdx = reinterpret_cast<int32_t*>(sC + (MASKED ? kTileProblems : 1) * PNP_PATC);
     const int lane = threadIdx.x;
     const int32_t* sel = selection_of(a);
     const int n_marked = a.fix_list[0];                       // (complete: k_iterate has finished)
@@ -692,7 +895,7 @@ __global__ void __launch_bounds__(32) k_fixup_thread(const __grid_constant__ Mom
         if (!staged) {                                        // first marked tile of this CTA: pattern, constants, barrier
             tile_buf.init(sRows, carve_bar<T>(smem_raw, sIdx + (sel ? a.n : 0)), a.uv, a.B, a.n_total, a.row_pitch, a.use_tma, a.kinv, lane);
             load_pattern<T>(a.pattern, sel, a.n_total, a.n, 1, sP, sIdx, lane, 32);
-            pattern_constants<T>(sP, a.n, sC, lane);
+            if (!MASKED) pattern_constants<T>(sP, a.n, sC, lane);
             __syncwarp();
             staged = true;
         } else {
@@ -704,7 +907,17 @@ __global__ void __launch_bounds__(32) k_fixup_thread(const __grid_constant__ Mom
         pts.idx = sel ? sIdx : nullptr;
         Result<T> out;
         T xt[12];
-        run_filter_with_tail<T, METHOD, 1, PtsRow<T> >(pts, sP, sC, a.n, 0, a.prm, xt, out);
+        if constexpr (MASKED) {
+            PtsMasked<PtsRow<T> > pm;
+            static_cast<PtsRow<T>&>(pm) = pts;
+            pm.words = a.vis + (size_t)(tile * kTileProblems + (lane < valid ? lane : valid - 1)) * a.vis_words;
+            pm.nvis = count_visible(pm.words, pm.idx, a.n);
+            T* myC = sC + (size_t)lane * PNP_PATC;
+            pattern_constants_masked<T, 1>(pm, sP, a.n, myC, 0);
+            run_filter_with_tail<T, METHOD, 1, PtsMasked<PtsRow<T> > >(pm, sP, myC, a.n, 0, a.prm, xt, out);
+        } else {
+            run_filter_with_tail<T, METHOD, 1, PtsRow<T> >(pts, sP, sC, a.n, 0, a.prm, xt, out);
+        }
         if (marked) {
 #pragma unroll
             for (int k = 0; k < PNP_NTAIL; ++k) a.tail[(size_t)k * a.ld + b] = xt[k];
@@ -713,19 +926,20 @@ __global__ void __launch_bounds__(32) k_fixup_thread(const __grid_constant__ Mom
     }
 }
 
-template <typename T, int METHOD>
+// MASKED: each warp solves on its problem's visible landmarks with the problem's constants
+template <typename T, int METHOD, bool MASKED = false>
 __global__ void __launch_bounds__(256) k_fixup_warp(const __grid_constant__ MomArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     T* sP = reinterpret_cast<T*>(smem_raw);
     T* sC = sP + (size_t)a.n * 3;
-    int32_t* sIdx = reinterpret_cast<int32_t*>(sC + PNP_PATC);
+    int32_t* sIdx = reinterpret_cast<int32_t*>(sC + (MASKED ? kWarpsPerFixup : 1) * PNP_PATC);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     const int32_t* sel = selection_of(a);
     const int n_marked = a.fix_list[0];                       // marked tiles (complete: k_iterate has finished)
     if ((int)blockIdx.x >= n_marked || n_marked > a.fix_warp_max) return;   // CTA i takes the marked tiles i, i + gridDim.x, ...; many: k_fixup_thread
     load_pattern<T>(a.pattern, sel, a.n_total, a.n, 1, sP, sIdx, threadIdx.x, blockDim.x);
-    if (warp == 0) pattern_constants<T>(sP, a.n, sC, lane);
+    if (!MASKED && warp == 0) pattern_constants<T>(sP, a.n, sC, lane);
     __syncthreads();
     PtsGlobal<T> pts;
     pts.idx = sel ? sIdx : nullptr;
@@ -739,7 +953,19 @@ __global__ void __launch_bounds__(256) k_fixup_warp(const __grid_constant__ MomA
         pts.row = a.uv + (size_t)b * a.n_total * 2;
         Result<T> out;
         T xt[12];
-        run_filter_with_tail<T, METHOD, 32, PtsGlobal<T> >(pts, sP, sC, a.n, lane, a.prm, xt, out);
+        if constexpr (MASKED) {
+            PtsMasked<PtsGlobal<T> > pm;
+            static_cast<PtsGlobal<T>&>(pm) = pts;
+            pm.words = a.vis + (size_t)b * a.vis_words;
+            pm.nvis = count_visible(pm.words, pm.idx, a.n);
+            T* myC = sC + (size_t)warp * PNP_PATC;
+            pattern_constants_masked<T, 32>(pm, sP, a.n, myC, lane);
+            __syncwarp();
+            run_filter_with_tail<T, METHOD, 32, PtsMasked<PtsGlobal<T> > >(pm, sP, myC, a.n, lane, a.prm, xt, out);
+            __syncwarp();                                     // the next problem's constants replace these
+        } else {
+            run_filter_with_tail<T, METHOD, 32, PtsGlobal<T> >(pts, sP, sC, a.n, lane, a.prm, xt, out);
+        }
         if (lane == 0) {
 #pragma unroll
             for (int k = 0; k < PNP_NTAIL; ++k) a.tail[(size_t)k * a.ld + b] = xt[k];
@@ -829,23 +1055,43 @@ __device__ __forceinline__ void write_pose(const MomArgs<T>& a, long long b, con
     if (a.best) a.best[b] = 0;
 }
 
-template <typename T, int METHOD, int BLOCK>
+// MASKED: every thread builds its problem's constants from the pattern moments of the workspace (a.pmom)
+template <typename T, int METHOD, int BLOCK, bool MASKED = false>
 __device__ __forceinline__ void iterate_body(const MomArgs<T>& a)
 {
     constexpr int kIterBlock = BLOCK;
     __shared__ T sC[PNP_PATC];
     constexpr int kRows = PNP_NMOM + (method_has_core(METHOD) ? PNP_NCORE : 0);
     __shared__ T sMom[kRows * kIterBlock];                // [moment | constant LM blocks][thread]: conflict-free columns
-    if (threadIdx.x < PNP_PATC) sC[threadIdx.x] = a.patc[threadIdx.x];
+    if (!MASKED && threadIdx.x < PNP_PATC) sC[threadIdx.x] = a.patc[threadIdx.x];
     long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const bool ok = b < a.B;
     if (!ok) b = a.B - 1;
 #pragma unroll
     for (int k = 0; k < method_nmom(METHOD); ++k) sMom[k * kIterBlock + threadIdx.x] = a.mom[(size_t)k * a.ld + b];
+    const T* myC = sC;
+    int nvis = 0;
+    if constexpr (MASKED) {
+        __shared__ T sCm[PNP_PATC * kIterBlock];          // [thread][constant]
+        double pm[kPatternMoments];
+#pragma unroll
+        for (int k = 0; k < kPatternMoments; ++k) pm[k] = (double)a.pmom[(size_t)k * a.ld + b];
+        constants_from_pattern_moments<T>(pm, sCm + threadIdx.x * PNP_PATC);
+        myC = sCm + threadIdx.x * PNP_PATC;
+        nvis = (int)pm[9];
+    }
     __syncthreads();
     Result<T> out;
     T st[PNP_NTAIL];
-    iterate_core<T, METHOD>(sMom + threadIdx.x, kIterBlock, sC, a.prm, st, out);
+    iterate_core<T, METHOD>(sMom + threadIdx.x, kIterBlock, myC, a.prm, st, out);
+    if constexpr (MASKED) {
+        if (nvis < kMinVisible) {                             // not solved: NaN pose, NaN state (so NaN res_norm), 0 iterations, unmarked
+            int unused;
+            too_few_landmarks<T>(out, unused);
+#pragma unroll
+            for (int k = 0; k < PNP_NTAIL; ++k) st[k] = out.res;
+        }
+    }
     if (method_with_s(METHOD) && BLOCK == 32 && a.fix_list) {    // a block is one 32-problem tile: list it if any of its problems is marked
         const bool marked = ok && out.iters < 0;
         if (__any_sync(0xffffffffu, marked) && threadIdx.x == 0) a.fix_list[1 + atomicAdd(a.fix_list, 1)] = (int32_t)blockIdx.x;
@@ -860,21 +1106,25 @@ __device__ __forceinline__ void iterate_body(const MomArgs<T>& a)
 // 16 Ki registers: 2 warps per sub-partition from 169 to 255 registers, 3 at <= 168 (FP64 LM wants ~214 and spills
 // ~26 doubles at 168).  Measured for 1 Mi x 68 LM FP64 on B200 (final step): 0.886 ms at 224, 0.904 at 255 (240 used),
 // 0.912 at 184, 0.905 at 168, 0.931 at 160 -- the third warp does not pay for its spills.
-template <typename T, int METHOD, int BLOCK, int MAXREG>
+template <typename T, int METHOD, int BLOCK, int MAXREG, bool MASKED = false>
 __global__ void __launch_bounds__(BLOCK) __maxnreg__(MAXREG) k_iterate(const __grid_constant__ MomArgs<T> a)
 {
-    iterate_body<T, METHOD, BLOCK>(a);
+    iterate_body<T, METHOD, BLOCK, MASKED>(a);
 }
 
-template <typename T, int METHOD, int BLOCK, int MAXREG>
+template <typename T, int METHOD, int BLOCK, int MAXREG, bool MASKED = false>
 static void launch_iterate_as(const MomArgs<T>& m, cudaStream_t stream)
 {
-    k_iterate<T, METHOD, BLOCK, MAXREG><<<(unsigned)((m.B + BLOCK - 1) / BLOCK), BLOCK, 0, stream>>>(m); count_kernel_launches(1);
+    k_iterate<T, METHOD, BLOCK, MAXREG, MASKED><<<(unsigned)((m.B + BLOCK - 1) / BLOCK), BLOCK, 0, stream>>>(m); count_kernel_launches(1);
 }
 
 template <typename T, int METHOD>
 static void launch_iterate(const MomArgs<T>& m, int tune, cudaStream_t stream)
 {
+    if (m.vis) {
+        launch_iterate_as<T, METHOD, 32, (METHOD == PNPB200_METHOD_EIF2 || METHOD == PNP_METHOD_QEIF_HYBRID) ? 255 : 224, true>(m, stream);
+        return;
+    }
     switch (tune) {
 #if PNP_TUNE_VARIANTS
     case 2:  launch_iterate_as<T, METHOD, 32, 255>(m, stream); break;    // no cap
@@ -896,18 +1146,19 @@ static void launch_iterate(const MomArgs<T>& m, int tune, cudaStream_t stream)
 // ------------------------------------------------------------------------------------------
 constexpr int kWarpsPerBlock = 8;
 
-template <typename T, int METHOD>
+// MASKED: problem b sees only its visible landmarks (a.vis); every warp computes its problem's constants
+template <typename T, int METHOD, bool MASKED = false>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32) k_solve_warp(const __grid_constant__ SolveArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     T* sP = reinterpret_cast<T*>(smem_raw);
     T* sC = sP + (size_t)a.n_patterns * a.n * 3;
-    int32_t* sIdx = reinterpret_cast<int32_t*>(sC + a.n_patterns * PNP_PATC);
+    int32_t* sIdx = reinterpret_cast<int32_t*>(sC + (MASKED ? kWarpsPerBlock : 1) * a.n_patterns * PNP_PATC);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 
     const int32_t* sel = selection_of(a);
     load_pattern<T>(a.pattern, sel, a.n_total, a.n, a.n_patterns, sP, sIdx, threadIdx.x, blockDim.x);
-    if (METHOD == PNPB200_METHOD_LM || METHOD == PNPB200_METHOD_LINEAR_F2 || METHOD == PNP_METHOD_QEIF_HYBRID || METHOD == PNPB200_METHOD_EIF2) {
+    if (!MASKED && method_uses_patc(METHOD)) {
         for (int p = warp; p < a.n_patterns; p += kWarpsPerBlock)
             pattern_constants<T>(sP + (size_t)p * a.n * 3, a.n, sC + p * PNP_PATC, lane);
         __syncthreads();
@@ -920,7 +1171,23 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) k_solve_warp(const __grid
         pts.row = a.uv + (size_t)b * a.n_total * 2;
         Result<T> best;
         int best_p;
-        solve_all_patterns<T, METHOD, 32, PtsGlobal<T> >(pts, sP, sC, a.n, a.n_patterns, lane, a.prm, best, best_p);
+        if constexpr (MASKED) {
+            PtsMasked<PtsGlobal<T> > pm;
+            static_cast<PtsGlobal<T>&>(pm) = pts;
+            pm.words = a.vis + (size_t)b * a.vis_words;
+            pm.nvis = count_visible(pm.words, pm.idx, a.n);
+            T* myC = sC + (size_t)warp * a.n_patterns * PNP_PATC;
+            if (method_uses_patc(METHOD)) {
+                for (int p = 0; p < a.n_patterns; ++p)
+                    pattern_constants_masked<T, 32>(pm, sP + (size_t)p * a.n * 3, a.n, myC + p * PNP_PATC, lane);
+                __syncwarp();
+            }
+            solve_all_patterns<T, METHOD, 32, PtsMasked<PtsGlobal<T> > >(pm, sP, myC, a.n, a.n_patterns, lane, a.prm, best, best_p);
+            if (pm.nvis < kMinVisible) too_few_landmarks<T>(best, best_p);
+            __syncwarp();                                     // the next problem's constants replace these
+        } else {
+            solve_all_patterns<T, METHOD, 32, PtsGlobal<T> >(pts, sP, sC, a.n, a.n_patterns, lane, a.prm, best, best_p);
+        }
         if (lane == 0) write_result<T>(a, b, best, best_p);
     }
 }
@@ -961,6 +1228,8 @@ static int launch_moment_pass(int pass, const MomArgs<T>& full, long long b0, lo
     m.B = nb;
     m.uv = full.uv + (size_t)b0 * full.n_total * 2;
     m.mom = full.mom + b0; m.tail = full.tail + b0;
+    if (full.pmom) m.pmom = full.pmom + b0;
+    if (full.vis) m.vis = full.vis + (size_t)b0 * full.vis_words;
     if (full.R) m.R = full.R + b0 * 9;
     if (full.t) m.t = full.t + b0 * 3;
     if (full.euler) m.euler = full.euler + b0 * 3;
@@ -970,15 +1239,22 @@ static int launch_moment_pass(int pass, const MomArgs<T>& full, long long b0, lo
     if (pass == 1) { launch_iterate<T, METHOD>(m, tune, stream); return PNPB200_OK; }
     const long long n_tiles = (nb + kTileProblems - 1) / kTileProblems;
     const unsigned tile_grid = (unsigned)(n_tiles < 0x7fffffffLL ? n_tiles : 0x7fffffffLL);
+    const bool masked = m.vis != nullptr;
     if (shape == 0) {                                         // chunked row streaming
         m.row_pitch = sg.pitch;
         m.use_tma = sg.chunk;                                 // RowStream: points per chunk
         m.use_tmap = (sg.pitch == sg.chunk * 2) ? make_row_tensor_map(&m.tmap, m.uv, (int)sizeof(T), nb, m.n_total, sg.chunk) : 0;
-        if (pass == 0) k_stream_chunk<T, METHOD, 0><<<tile_grid, 32, smem, stream>>>(m);
+        if (masked) {
+            if (pass == 0) k_stream_chunk<T, METHOD, 0, true><<<tile_grid, 32, smem, stream>>>(m);
+            else           k_stream_chunk<T, METHOD, 1, true><<<tile_grid, 32, smem, stream>>>(m);
+        } else if (pass == 0) k_stream_chunk<T, METHOD, 0><<<tile_grid, 32, smem, stream>>>(m);
         else           k_stream_chunk<T, METHOD, 1><<<tile_grid, 32, smem, stream>>>(m);
         count_kernel_launches(1);
     } else if (shape == 1) {                                  // whole-row tiles
-        if (pass == 0) k_stream_thread<T, METHOD, 0><<<tile_grid, 32, smem, stream>>>(m);
+        if (masked) {
+            if (pass == 0) k_stream_thread<T, METHOD, 0, true><<<tile_grid, 32, smem, stream>>>(m);
+            else           k_stream_thread<T, METHOD, 1, true><<<tile_grid, 32, smem, stream>>>(m);
+        } else if (pass == 0) k_stream_thread<T, METHOD, 0><<<tile_grid, 32, smem, stream>>>(m);
         else           k_stream_thread<T, METHOD, 1><<<tile_grid, 32, smem, stream>>>(m);
         count_kernel_launches(1);
     } else if (shape == 3) {                                  // one problem per warp, rows through a TMA ring
@@ -988,7 +1264,10 @@ static int launch_moment_pass(int pass, const MomArgs<T>& full, long long b0, lo
         count_kernel_launches(1);
     } else {                                                  // one problem per warp, coalesced loads
         const unsigned grid = (unsigned)persistent_grid((nb + 7) / 8, dp.sm_count, per_sm);
-        if (pass == 0) k_stream_warp<T, METHOD, 0><<<grid, 256, smem, stream>>>(m);
+        if (masked) {
+            if (pass == 0) k_stream_warp<T, METHOD, 0, true><<<grid, 256, smem, stream>>>(m);
+            else           k_stream_warp<T, METHOD, 1, true><<<grid, 256, smem, stream>>>(m);
+        } else if (pass == 0) k_stream_warp<T, METHOD, 0><<<grid, 256, smem, stream>>>(m);
         else           k_stream_warp<T, METHOD, 1><<<grid, 256, smem, stream>>>(m);
         count_kernel_launches(1);
     }
@@ -998,33 +1277,41 @@ static int launch_moment_pass(int pass, const MomArgs<T>& full, long long b0, lo
 // A handful of marked tiles (the normal case on detected pixels) is latency: one problem per warp finishes them in a few
 // microseconds; thousands of them (noise-free pixels) is throughput: one problem per thread.  Both kernels read the count and
 // exactly one of them acts (rows too long for a tile: always per warp).
-template <typename T, int METHOD>
-static int launch_filter_fixup(const MomArgs<T>& m, const RowGeom& g, bool by_thread, size_t thread_smem, size_t warp_smem,
-                               const DeviceProps& dp, cudaStream_t stream)
+template <typename T, int METHOD, bool MASKED>
+static int launch_filter_fixup_as(const MomArgs<T>& m, const RowGeom& g, bool by_thread, size_t thread_smem, size_t warp_smem,
+                                  const DeviceProps& dp, cudaStream_t stream)
 {
     MomArgs<T> f = m;
     const long long n_tiles = (m.B + kTileProblems - 1) / kTileProblems;
     f.fix_warp_max = by_thread ? dp.sm_count : 0x7fffffff;
     {
-        const size_t smem = warp_smem + PNP_PATC * sizeof(T);
-        PNP_CUDA_OK(set_dynamic_smem((const void*)k_fixup_warp<T, METHOD>, smem));
+        const size_t smem = warp_smem + (MASKED ? kWarpsPerFixup : 1) * PNP_PATC * sizeof(T);   // masked: constants per warp
+        PNP_CUDA_OK(set_dynamic_smem((const void*)k_fixup_warp<T, METHOD, MASKED>, smem));
         int per_sm = 1;
-        PNP_CUDA_OK(blocks_per_sm(&per_sm, (const void*)k_fixup_warp<T, METHOD>, 256, smem));
+        PNP_CUDA_OK(blocks_per_sm(&per_sm, (const void*)k_fixup_warp<T, METHOD, MASKED>, 256, smem));
         const unsigned grid = (unsigned)persistent_grid(n_tiles, dp.sm_count, per_sm);   // CTAs beyond the number of marked tiles leave at once
-        k_fixup_warp<T, METHOD><<<grid, 256, smem, stream>>>(f);
+        k_fixup_warp<T, METHOD, MASKED><<<grid, 256, smem, stream>>>(f);
         count_kernel_launches(1);
     }
     if (by_thread) {
         f.row_pitch = g.row_pitch; f.use_tma = g.use_tma;
-        const size_t smem = thread_smem + PNP_PATC * sizeof(T);
-        PNP_CUDA_OK(set_dynamic_smem((const void*)k_fixup_thread<T, METHOD>, smem));
+        const size_t smem = thread_smem + (MASKED ? kTileProblems : 1) * PNP_PATC * sizeof(T);   // masked: constants per lane
+        PNP_CUDA_OK(set_dynamic_smem((const void*)k_fixup_thread<T, METHOD, MASKED>, smem));
         int per_sm = 1;
-        PNP_CUDA_OK(blocks_per_sm(&per_sm, (const void*)k_fixup_thread<T, METHOD>, 32, smem));
+        PNP_CUDA_OK(blocks_per_sm(&per_sm, (const void*)k_fixup_thread<T, METHOD, MASKED>, 32, smem));
         const unsigned grid = (unsigned)persistent_grid(n_tiles, dp.sm_count, per_sm);
-        k_fixup_thread<T, METHOD><<<grid, 32, smem, stream>>>(f);
+        k_fixup_thread<T, METHOD, MASKED><<<grid, 32, smem, stream>>>(f);
         count_kernel_launches(1);
     }
     return PNPB200_OK;
+}
+
+template <typename T, int METHOD>
+static int launch_filter_fixup(const MomArgs<T>& m, const RowGeom& g, bool by_thread, size_t thread_smem, size_t warp_smem,
+                               const DeviceProps& dp, cudaStream_t stream)
+{
+    if (m.vis) return launch_filter_fixup_as<T, METHOD, true>(m, g, by_thread, thread_smem, warp_smem, dp, stream);
+    return launch_filter_fixup_as<T, METHOD, false>(m, g, by_thread, thread_smem, warp_smem, dp, stream);
 }
 
 // LM / linear F2 with one pattern: moments -> iterate -> residual (see the kernels' header).
@@ -1046,8 +1333,10 @@ static int launch_moment(const SolveArgs<T>& a, const DeviceProps& dp, cudaStrea
     const bool by_thread = g.tile_bytes <= 48 * 1024 && thread_smem <= (size_t)dp.max_smem_optin;
     if (!by_thread && warp_smem > (size_t)dp.max_smem_optin) return PNPB200_ETOOLARGE;
 
+    const bool masked = a.vis != nullptr;
     T* ws = nullptr;
-    const size_t ws_elems = (size_t)(PNP_NMOM + PNP_NTAIL) * (size_t)a.B + PNP_PATC;
+    // masked: the per-problem pattern moments ride behind the moments ([kPatternMoments][B])
+    const size_t ws_elems = (size_t)(PNP_NMOM + (masked ? kPatternMoments : 0) + PNP_NTAIL) * (size_t)a.B + PNP_PATC;
     const bool own_ws = !(a.ws && a.ws_bytes >= ws_elems * sizeof(T));
     if (own_ws) PNP_CUDA_OK(cudaMallocAsync((void**)&ws, ws_elems * sizeof(T), stream));
     else ws = (T*)a.ws;
@@ -1063,6 +1352,8 @@ static int launch_moment(const SolveArgs<T>& a, const DeviceProps& dp, cudaStrea
     for (int e = 0; e < 6; ++e) m.kinv[e] = a.kinv[e];
     m.prm = a.prm;
     m.mom = ws; m.tail = ws + (size_t)PNP_NMOM * a.B; m.patc = m.tail + (size_t)PNP_NTAIL * a.B;
+    m.vis = a.vis; m.vis_words = a.vis_words; m.pmom = nullptr;
+    if (masked) { m.pmom = ws + (size_t)PNP_NMOM * a.B; m.tail = m.pmom + (size_t)kPatternMoments * a.B; m.patc = m.tail + (size_t)PNP_NTAIL * a.B; }
     m.R = a.R; m.t = a.t; m.euler = a.euler; m.res = a.res; m.iters = a.iters; m.best = a.best;
     m.use_tmap = 0;
     struct ItersGuard { void* p; cudaStream_t st; ~ItersGuard() { if (p) cudaFreeAsync(p, st); } } iters_guard = { nullptr, stream }, list_guard = { nullptr, stream };
@@ -1084,14 +1375,14 @@ static int launch_moment(const SolveArgs<T>& a, const DeviceProps& dp, cudaStrea
     size_t smem;
     if (by_thread && !a.idx_mode && sg.use_stream && a.tune != 9) {
         shape = 0; smem = 2 * sg.buf_bytes + pat_bytes + 32;
-        PNP_CUDA_OK(set_dynamic_smem((const void*)k_stream_chunk<T, METHOD, 0>, smem));
-        PNP_CUDA_OK(set_dynamic_smem((const void*)k_stream_chunk<T, METHOD, 1>, smem));
+        PNP_CUDA_OK(set_dynamic_smem(masked ? (const void*)k_stream_chunk<T, METHOD, 0, true> : (const void*)k_stream_chunk<T, METHOD, 0>, smem));
+        PNP_CUDA_OK(set_dynamic_smem(masked ? (const void*)k_stream_chunk<T, METHOD, 1, true> : (const void*)k_stream_chunk<T, METHOD, 1>, smem));
     } else if (by_thread) {
         shape = 1; smem = thread_smem;
-        PNP_CUDA_OK(set_dynamic_smem((const void*)k_stream_thread<T, METHOD, 0>, smem));
-        PNP_CUDA_OK(set_dynamic_smem((const void*)k_stream_thread<T, METHOD, 1>, smem));
-    } else if (!a.idx_mode && ((size_t)a.n_total * 2 * sizeof(T)) % 16 == 0 && a.tune != 9 &&
-               a.n_total >= kRingPoints) {
+        PNP_CUDA_OK(set_dynamic_smem(masked ? (const void*)k_stream_thread<T, METHOD, 0, true> : (const void*)k_stream_thread<T, METHOD, 0>, smem));
+        PNP_CUDA_OK(set_dynamic_smem(masked ? (const void*)k_stream_thread<T, METHOD, 1, true> : (const void*)k_stream_thread<T, METHOD, 1>, smem));
+    } else if (!masked && !a.idx_mode && ((size_t)a.n_total * 2 * sizeof(T)) % 16 == 0 && a.tune != 9 &&
+               a.n_total >= kRingPoints) {                // (no masked ring kernel: masked rows take the per-warp shape below)
         shape = 3;
         smem = (size_t)kRingWarps * kRingSlots * (kRingPoints * 2 * sizeof(T) + 8);
         PNP_CUDA_OK(set_dynamic_smem((const void*)k_stream_warp_tma<T, METHOD, 0>, smem));
@@ -1099,9 +1390,10 @@ static int launch_moment(const SolveArgs<T>& a, const DeviceProps& dp, cudaStrea
         PNP_CUDA_OK(blocks_per_sm(&per_sm, (const void*)k_stream_warp_tma<T, METHOD, 0>, kRingWarps * 32, smem));
     } else {
         shape = 2; smem = warp_smem;
-        PNP_CUDA_OK(set_dynamic_smem((const void*)k_stream_warp<T, METHOD, 0>, smem));
-        PNP_CUDA_OK(set_dynamic_smem((const void*)k_stream_warp<T, METHOD, 1>, smem));
-        PNP_CUDA_OK(blocks_per_sm(&per_sm, (const void*)k_stream_warp<T, METHOD, 0>, 256, smem));
+        const void* k0 = masked ? (const void*)k_stream_warp<T, METHOD, 0, true> : (const void*)k_stream_warp<T, METHOD, 0>;
+        PNP_CUDA_OK(set_dynamic_smem(k0, smem));
+        PNP_CUDA_OK(set_dynamic_smem(masked ? (const void*)k_stream_warp<T, METHOD, 1, true> : (const void*)k_stream_warp<T, METHOD, 1>, smem));
+        PNP_CUDA_OK(blocks_per_sm(&per_sm, k0, 256, smem));
     }
 
     // -DPNP_DEBUG_SYNC (tools/build_variant.py): synchronise after every launch and name the kernel a fault belongs to
@@ -1111,8 +1403,10 @@ static int launch_moment(const SolveArgs<T>& a, const DeviceProps& dp, cudaStrea
 #else
 #define PNP_DEBUG_CHECK(what) do { } while (0)
 #endif
-    k_pattern_constants<T><<<1, 32, 0, stream>>>(m); count_kernel_launches(1);
-    PNP_DEBUG_CHECK("k_pattern_constants");
+    if (!masked) {                                            // (masked: per problem, from the moments pass)
+        k_pattern_constants<T><<<1, 32, 0, stream>>>(m); count_kernel_launches(1);
+        PNP_DEBUG_CHECK("k_pattern_constants");
+    }
     const int slot = a.profile ? g_prof.begin() : -1;
     g_prof.mark(slot, stream);
     launch_moment_pass<T, METHOD>(0, m, 0, a.B, shape, sg, smem, per_sm, dp, a.tune, stream);
@@ -1203,23 +1497,30 @@ static int launch_solve(const SolveArgs<T>& a, int mapping, cudaStream_t stream)
     constexpr bool has_moment_form = (METHOD == PNPB200_METHOD_LM || METHOD == PNPB200_METHOD_LINEAR_F2 || METHOD == PNPB200_METHOD_LM_PLUS ||
                                       METHOD == PNP_METHOD_LM_TRUEJAC ||
                                       ((METHOD == PNP_METHOD_QEIF_HYBRID || METHOD == PNPB200_METHOD_EIF2) && sizeof(T) == 8));
+    // a visibility mask (a.vis) takes the same mapping as the call without it; its kernels keep the pattern constants per
+    // problem.  (LM_TRUEJAC exists in the moment mapping only: no direct kernels, masked or not, are launched for it.)
+    constexpr bool can_mask = METHOD != PNP_METHOD_LM_TRUEJAC;
+    const bool masked = a.vis != nullptr;
     const RowGeom g = row_geometry<T>(a.n_total);
     const size_t pat_bytes = ((size_t)a.n_patterns * a.n * 3 + (size_t)a.n_patterns * PNP_PATC) * sizeof(T);
     const size_t idx_bytes = a.idx_mode ? (size_t)a.n * sizeof(int32_t) : 0;
-    const size_t thread_smem = g.tile_bytes + pat_bytes + idx_bytes + 16;
-    const size_t warp_smem = pat_bytes + idx_bytes;
-    if (mapping == PNPB200_MAP_AUTO) {
-        if (has_moment_form) mapping = PNPB200_MAP_MOMENT;
-        else mapping = (g.tile_bytes <= 48 * 1024 && thread_smem <= (size_t)dp.max_smem_optin) ? PNPB200_MAP_THREAD : PNPB200_MAP_WARP;
-    }
+    const size_t patc_bytes = (size_t)a.n_patterns * PNP_PATC * sizeof(T);
+    const size_t thread_smem = g.tile_bytes + pat_bytes + idx_bytes + 16 + (masked ? (kTileProblems - 1) * patc_bytes : 0);
+    const size_t warp_smem = pat_bytes + idx_bytes + (masked ? (kWarpsPerBlock - 1) * patc_bytes : 0);
+    const int direct = (g.tile_bytes <= 48 * 1024 && thread_smem <= (size_t)dp.max_smem_optin) ? PNPB200_MAP_THREAD : PNPB200_MAP_WARP;
+    if (mapping == PNPB200_MAP_AUTO) mapping = has_moment_form ? PNPB200_MAP_MOMENT : direct;
     if (mapping == PNPB200_MAP_MOMENT) {
         if (!has_moment_form) return PNPB200_EINVAL;
         if (a.n_patterns == 1) return launch_moment<T, has_moment_form ? METHOD : PNPB200_METHOD_LM>(a, dp, stream);
         return launch_moment_patterns<T, has_moment_form ? METHOD : PNPB200_METHOD_LM>(a, dp, stream);
     }
+    if ((mapping == PNPB200_MAP_THREAD || mapping == PNPB200_MAP_WARP) && masked && !can_mask) return PNPB200_EINVAL;
     if (mapping == PNPB200_MAP_THREAD) {
         if (thread_smem > (size_t)dp.max_smem_optin) return PNPB200_ETOOLARGE;
-        PNP_CUDA_OK(set_dynamic_smem((const void*)k_solve_thread<T, METHOD>, thread_smem));
+        if constexpr (can_mask) {
+            if (masked) PNP_CUDA_OK(set_dynamic_smem((const void*)k_solve_thread<T, METHOD, true>, thread_smem));
+        }
+        if (!masked) PNP_CUDA_OK(set_dynamic_smem((const void*)k_solve_thread<T, METHOD>, thread_smem));
         SolveArgs<T> at = a;
         at.row_pitch = g.row_pitch;
         at.use_tma = g.use_tma;
@@ -1227,17 +1528,29 @@ static int launch_solve(const SolveArgs<T>& a, int mapping, cudaStream_t stream)
         const long long grid = n_tiles < 0x7fffffffLL ? n_tiles : 0x7fffffffLL;
         const int slot = a.profile ? g_prof.begin() : -1;
         g_prof.mark(slot, stream);
-        k_solve_thread<T, METHOD><<<(unsigned)grid, 32, thread_smem, stream>>>(at); count_kernel_launches(1);
+        if constexpr (can_mask) {
+            if (masked) k_solve_thread<T, METHOD, true><<<(unsigned)grid, 32, thread_smem, stream>>>(at);
+        }
+        if (!masked) k_solve_thread<T, METHOD><<<(unsigned)grid, 32, thread_smem, stream>>>(at);
+        count_kernel_launches(1);
         g_prof.mark(slot, stream);
     } else if (mapping == PNPB200_MAP_WARP) {
         if (warp_smem > (size_t)dp.max_smem_optin) return PNPB200_ETOOLARGE;
-        PNP_CUDA_OK(set_dynamic_smem((const void*)k_solve_warp<T, METHOD>, warp_smem));
+        const void* kfn = (const void*)k_solve_warp<T, METHOD>;
+        if constexpr (can_mask) {
+            if (masked) kfn = (const void*)k_solve_warp<T, METHOD, true>;
+        }
+        PNP_CUDA_OK(set_dynamic_smem(kfn, warp_smem));
         int per_sm = 1;
-        PNP_CUDA_OK(blocks_per_sm(&per_sm, (const void*)k_solve_warp<T, METHOD>, kWarpsPerBlock * 32, warp_smem));
+        PNP_CUDA_OK(blocks_per_sm(&per_sm, kfn, kWarpsPerBlock * 32, warp_smem));
         const long long grid = persistent_grid((a.B + kWarpsPerBlock - 1) / kWarpsPerBlock, dp.sm_count, per_sm);
         const int slot = a.profile ? g_prof.begin() : -1;
         g_prof.mark(slot, stream);
-        k_solve_warp<T, METHOD><<<(unsigned)grid, kWarpsPerBlock * 32, warp_smem, stream>>>(a); count_kernel_launches(1);
+        if constexpr (can_mask) {
+            if (masked) k_solve_warp<T, METHOD, true><<<(unsigned)grid, kWarpsPerBlock * 32, warp_smem, stream>>>(a);
+        }
+        if (!masked) k_solve_warp<T, METHOD><<<(unsigned)grid, kWarpsPerBlock * 32, warp_smem, stream>>>(a);
+        count_kernel_launches(1);
         g_prof.mark(slot, stream);
     } else {
         return PNPB200_EINVAL;
@@ -1249,7 +1562,8 @@ static int launch_solve(const SolveArgs<T>& a, int mapping, cudaStream_t stream)
 template <typename T>
 static int solve_typed(int method, long long B, int n_total, int n, const void* uv, const void* pattern,
                        int n_patterns, const int32_t* idx_host, const int32_t* idx_dev, const double* K, const pnpb200_params& prm,
-                       void* R, void* t, void* euler, void* res, int32_t* iters, int32_t* best, cudaStream_t stream)
+                       void* R, void* t, void* euler, void* res, int32_t* iters, int32_t* best, cudaStream_t stream,
+                       const uint32_t* vis)
 {
     SolveArgs<T> a;
     a.uv = (const T*)uv; a.pattern = (const T*)pattern; a.idx = idx_dev;
@@ -1268,6 +1582,7 @@ static int solve_typed(int method, long long B, int n_total, int n, const void* 
     a.skip_residual = (prm.flags & PNP_FLAG_INTERNAL_NO_RESIDUAL) ? 1 : 0;
     a.tune = (prm.flags >> 8) & 0xff;                     // undocumented tuning knob (register budget of k_iterate, slice size)
     a.ws = prm.workspace; a.ws_bytes = (prm.workspace && prm.workspace_bytes > 0) ? (size_t)prm.workspace_bytes : 0;
+    a.vis = vis; a.vis_words = (n_total + 31) / 32;
     switch (method) {
 #if PNP_GROUP == 0
     case PNPB200_METHOD_QEIF:
@@ -1282,7 +1597,7 @@ static int solve_typed(int method, long long B, int n_total, int n, const void* 
         }
         return launch_solve<T, PNPB200_METHOD_LM>(a, prm.mapping, stream);
     case PNPB200_METHOD_LM_PLUS: {
-        // non-parity extra: exists in the moment mapping only, one pattern
+        // non-parity extra: exists in the moment mapping only
         if (prm.mapping != PNPB200_MAP_AUTO && prm.mapping != PNPB200_MAP_MOMENT) return PNPB200_EINVAL;
         DeviceProps dp;
         int rc = get_device_props(&dp);
@@ -1312,7 +1627,7 @@ typedef float part_scalar;
 int PNP_PART_NAME(PNP_SOLVE_PART_ARGS)
 {
     return solve_typed<part_scalar>(method, B, n_total, n, uv, pattern, n_patterns, idx_host, idx_dev, K, prm, R, t, euler, res,
-                                    iters, best, stream);
+                                    iters, best, stream, vis);
 }
 
 }  // namespace pnpb200

@@ -183,6 +183,7 @@ PNP_DEV void accumulate_moments(const Pts& pts, const T* __restrict__ sP, int n,
     mom.zero();
 #pragma unroll (LPP == 32 ? 8 : 4)
     for (int i = sub; i < n; i += LPP) {
+        if (!pts.vis(i)) continue;
         const T th[3] = { sP[3 * i], sP[3 * i + 1], sP[3 * i + 2] };
         T bx, by;
         pts.get(i, bx, by);
@@ -290,7 +291,7 @@ PNP_DEV void qeif_loop(const Pts& pts, const T* __restrict__ sP, const T* __rest
     bool done = false;
     int iters = 0;
     const T w = prm.meas_w;                               // 1 / (9 / f^2) (:2844-2852)
-    const T nT = T(n);
+    const T nT = T(pts.count(n));                        // landmarks taking part (the visible ones under a mask)
 
     for (int it = 0; it < prm.max_it; ++it) {
         if (LPP == 1) { if (__all_sync(0xffffffffu, done)) break; }
@@ -317,6 +318,7 @@ PNP_DEV void qeif_loop(const Pts& pts, const T* __restrict__ sP, const T* __rest
 #pragma unroll
             for (int e = 0; e < 6; ++e) hv[e] = T(0);
             for (int i = sub; i < n; i += LPP) {
+                if (!pts.vis(i)) continue;
                 const T th0 = sP[3 * i], th1 = sP[3 * i + 1], th2 = sP[3 * i + 2];
                 T bx, by;
                 pts.get(i, bx, by);
@@ -357,6 +359,7 @@ PNP_DEV void qeif_loop(const Pts& pts, const T* __restrict__ sP, const T* __rest
                 // ---- residual, point by point (:2905-2907)
 #pragma unroll 4
                 for (int i = sub; i < n; i += LPP) {
+                    if (!pts.vis(i)) continue;
                     const T th0 = sP[3 * i], th1 = sP[3 * i + 1], th2 = sP[3 * i + 2];
                     T bx, by;
                     pts.get(i, bx, by);
@@ -481,6 +484,8 @@ PNP_DEV void solve_qeif_with_tail(const Pts& pts, const T* __restrict__ sP, cons
 // No points inside the loop (moment mapping)
 struct NoPts {
     template <typename T> PNP_DEV void get(int, T& bx, T& by) const { bx = T(0); by = T(0); }
+    PNP_DEV bool vis(int) const { return true; }
+    PNP_DEV int count(int n) const { return n; }
 };
 
 template <typename T>
@@ -797,6 +802,7 @@ PNP_DEV T lm_residual_direct(const Pts& pts, const T* __restrict__ sP, int n, in
     T rr = T(0);
 #pragma unroll 4
     for (int i = sub; i < n; i += LPP) {
+        if (!pts.vis(i)) continue;
         const T th[3] = { sP[3 * i], sP[3 * i + 1], sP[3 * i + 2] };
         T bx, by;
         pts.get(i, bx, by);
@@ -836,6 +842,7 @@ PNP_DEV void solve_lm(const Pts& pts, const T* __restrict__ sP, const T* __restr
         r.q1 = r.q2 = r.qg = T(0);
         T rr = T(0);
         for (int i = sub; i < n; i += LPP) {
+            if (!pts.vis(i)) continue;
             const T th[3] = { sP[3 * i], sP[3 * i + 1], sP[3 * i + 2] };
             T bx, by;
             pts.get(i, bx, by);
@@ -1005,6 +1012,7 @@ PNP_DEV void eif2_loop(const Pts& pts, const T* __restrict__ sP, const T* __rest
         if (!RES_MOM) {
 #pragma unroll 4
             for (int i = sub; i < n; i += LPP) {
+                if (!pts.vis(i)) continue;
                 const T th0 = sP[3 * i], th1 = sP[3 * i + 1], th2 = sP[3 * i + 2];
                 T bx, by;
                 pts.get(i, bx, by);
@@ -1161,6 +1169,7 @@ PNP_DEV T f2_residual_direct(const Pts& pts, const T* __restrict__ sP, int n, in
     T rx2 = T(0), ry2 = T(0);
 #pragma unroll 4
     for (int i = sub; i < n; i += LPP) {
+        if (!pts.vis(i)) continue;
         const T th0 = sP[3 * i], th1 = sP[3 * i + 1], th2 = sP[3 * i + 2];
         T bx, by;
         pts.get(i, bx, by);
@@ -1296,6 +1305,7 @@ PNP_DEV void solve_linear_f1(const Pts& pts, const T* __restrict__ sP, int n, in
 #pragma unroll
         for (int e = 0; e < 4; ++e) { bxv[e] = T(0); byv[e] = T(0); }
         for (int i = sub; i < n; i += LPP) {
+            if (!pts.vis(i)) continue;
             const T th0 = sP[3 * i], th1 = sP[3 * i + 1], th2 = sP[3 * i + 2];
             T bx, by;
             pts.get(i, bx, by);
@@ -1325,6 +1335,7 @@ PNP_DEV void solve_linear_f1(const Pts& pts, const T* __restrict__ sP, int n, in
             pn[6] = out.t[0] / t3; pn[7] = out.t[1] / t3;
             T r2 = T(0);
             for (int i = sub; i < n; i += LPP) {
+                if (!pts.vis(i)) continue;
                 const T th0 = sP[3 * i], th1 = sP[3 * i + 1], th2 = sP[3 * i + 2];
                 T bx, by;
                 pts.get(i, bx, by);

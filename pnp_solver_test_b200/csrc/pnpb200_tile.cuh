@@ -29,7 +29,40 @@ struct PtsRow {
         bx = p.x;
         by = p.y;
     }
+    // every selected landmark takes part (the masked accessor below overrides these two)
+    PNP_DEV bool vis(int) const { return true; }
+    PNP_DEV int count(int n) const { return n; }
 };
+
+// bit j % 32 of word j / 32: landmark j of the caller's 0..n_total-1 numbering is visible (per-problem mask)
+PNP_DEV bool mask_bit(const uint32_t* words, int j) { return (__ldg(words + (j >> 5)) >> (j & 31)) & 1u; }
+
+// A point accessor restricted to the visible landmarks of one problem: the solvers skip i where vis(i) is false, so
+// hidden pixels are never read, and count() is the number of visible selected landmarks.
+template <typename Base>
+struct PtsMasked : Base {
+    const uint32_t* words;   // this problem's visibility words
+    int nvis;
+    PNP_DEV bool vis(int i) const { return mask_bit(words, this->idx ? this->idx[i] : i); }
+    PNP_DEV int count(int) const { return nvis; }
+};
+
+// fewer visible landmarks than this: a problem is not solved (NaN pose), its report and check statistics are NaN
+constexpr int kMinVisible = 4;
+
+// visible landmarks among the n selected ones (idx = nullptr: landmarks 0..n-1)
+PNP_DEV int count_visible(const uint32_t* words, const int32_t* idx, int n)
+{
+    if (idx) {
+        int c = 0;
+        for (int i = 0; i < n; ++i) c += mask_bit(words, idx[i]) ? 1 : 0;
+        return c;
+    }
+    int c = 0;
+    for (int w = 0; w < (n >> 5); ++w) c += __popc(__ldg(words + w));
+    if (n & 31) c += __popc(__ldg(words + (n >> 5)) & ((1u << (n & 31)) - 1u));
+    return c;
+}
 
 // ---- TMA bulk copy + mbarrier (sm_90+ PTX; SASS: UBLKCP / SYNCS)
 PNP_DEV uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }

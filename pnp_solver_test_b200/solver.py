@@ -47,12 +47,61 @@ def _copy_params(p):
     return q
 
 
-def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R", "t", "euler", "res_norm", "iters", "best_pattern")):
+def _check_visible(visible, B, n_total):
+    """visible must be a bool [B, n_total] torch tensor or NumPy array"""
+    if torch.is_tensor(visible):
+        ok = visible.dtype == torch.bool
+    elif isinstance(visible, np.ndarray):
+        ok = visible.dtype == np.bool_
+    else:
+        raise ValueError("visible must be a bool torch tensor or NumPy array, not %s" % type(visible).__name__)
+    if not ok:
+        raise ValueError("visible must have dtype bool, not %s" % (visible.dtype,))
+    if tuple(visible.shape) != (B, n_total):
+        raise ValueError("visible must be [B, n_total] = [%d, %d], not %s" % (B, n_total, tuple(visible.shape)))
+
+
+def visible_words(visible, device):
+    """bool [B, n_total] visibility -> the [B, ceil(n_total / 32)] words of the masked entries (bit i % 32 of word i / 32 =
+    landmark i, least significant bit first), packed with torch ops on `device`: eight landmarks per byte, four bytes per word
+    (little-endian), one byte per landmark of temporary memory.  The int32 tensor holds the uint32 bits."""
+    if isinstance(visible, np.ndarray):
+        visible = torch.from_numpy(np.ascontiguousarray(visible))
+    B, n_total = int(visible.shape[0]), int(visible.shape[1])
+    W = (n_total + 31) // 32
+    u8 = visible.to(device).contiguous().view(torch.uint8)
+    if W * 32 != n_total:
+        u8 = torch.nn.functional.pad(u8, (0, W * 32 - n_total))
+    shifts = torch.arange(8, dtype=torch.uint8, device=device)
+    byte = (u8.reshape(B, W * 4, 8) << shifts).sum(-1, dtype=torch.uint8)
+    return byte.contiguous().view(torch.int32)
+
+
+def visible_words_host(visible):
+    """the same words on the host, np.packbits(..., bitorder="little"): a [B, ceil(n_total / 32)] uint32 NumPy array"""
+    if torch.is_tensor(visible):
+        visible = visible.cpu().numpy()
+    B, n_total = int(visible.shape[0]), int(visible.shape[1])
+    W = (n_total + 31) // 32
+    v = np.zeros((B, W * 32), dtype=np.bool_)
+    v[:, :n_total] = visible
+    return np.ascontiguousarray(np.packbits(v, axis=1, bitorder="little").view("<u4"))
+
+
+def _u32(t):
+    return C.cast(ptr(t), C.POINTER(C.c_uint32))
+
+
+def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R", "t", "euler", "res_norm", "iters", "best_pattern"),
+                visible=None):
     """pnpb200_solve_batch on device tensors.
 
     uv [B, n_total, 2] and patterns [P, n_total, 3] are CUDA tensors of the same float dtype;
     K is a host 3x3.  Returns a dict of CUDA tensors: R [B,3,3], t [B,3], euler [B,3] =
-    (roll, yaw, pitch) in degrees, res_norm [B], iters [B] int32, best_pattern [B] int32."""
+    (roll, yaw, pitch) in degrees, res_norm [B], iters [B] int32, best_pattern [B] int32.
+    visible: bool [B, n_total] (torch tensor or NumPy array) -> pnpb200_solve_batch_masked: each problem is solved on its
+    visible landmarks alone (those of point_index, in its order); hidden pixels are never read, and a problem with fewer
+    than 4 of them comes back NaN with iters 0 (include/pnpb200.h)."""
     m = _lib.METHODS[method] if isinstance(method, str) else int(method)
     if not (uv.is_cuda and patterns.is_cuda):
         raise ValueError("uv and patterns must be CUDA tensors (no CPU fallback)")
@@ -66,6 +115,8 @@ def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R
     B, n_total = int(uv.shape[0]), int(uv.shape[1])
     if uv.dim() != 3 or uv.shape[2] != 2 or patterns.shape[1] != n_total or patterns.shape[2] != 3:
         raise ValueError("shape mismatch: uv [B,n,2], patterns [P,n,3]")
+    if visible is not None:
+        _check_visible(visible, B, n_total)
     if point_index is None:
         n, idx_p, idx = n_total, None, None
     else:
@@ -84,14 +135,26 @@ def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R
         return o
     # scratch for the moment mapping from torch's caching allocator (stream-ordered, no driver call)
     prm = _lib.default_params() if params is None else params
-    ws_bytes = int(lib.pnpb200_workspace_bytes(C.c_int(m), C.c_int(dt), C.c_int64(B), C.c_int(int(patterns.shape[0])),
-                                               C.c_int(int(prm.mapping))))
+    ws_query = lib.pnpb200_workspace_bytes if visible is None else lib.pnpb200_workspace_bytes_masked
+    ws_bytes = int(ws_query(C.c_int(m), C.c_int(dt), C.c_int64(B), C.c_int(int(patterns.shape[0])), C.c_int(int(prm.mapping))))
     ws = None
     if ws_bytes > 0 and not prm.workspace:
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
         prm = _copy_params(prm)
         prm.workspace, prm.workspace_bytes = ws.data_ptr(), ws_bytes
     params = prm
+    if visible is not None:
+        words = visible_words(visible, dev)
+        with torch.cuda.device(dev):
+            rc = lib.pnpb200_solve_batch_masked(
+                m, dt, B, n_total, n, ptr(uv), ptr(patterns), int(patterns.shape[0]), idx_p, Kp, C.byref(params),
+                ptr(o.get("R")), ptr(o.get("t")), ptr(o.get("euler")), ptr(o.get("res_norm")),
+                None if o.get("iters") is None else C.cast(ptr(o["iters"]), C.POINTER(C.c_int32)),
+                None if o.get("best_pattern") is None else C.cast(ptr(o["best_pattern"]), C.POINTER(C.c_int32)),
+                _u32(words), _stream_ptr(dev))
+        check(rc, "pnpb200_solve_batch_masked")
+        _lib.count_launch(1)
+        return o
     with torch.cuda.device(dev):
         rc = lib.pnpb200_solve_batch(
             C.c_int(m), C.c_int(dt), C.c_int64(B), C.c_int(n_total), C.c_int(n), ptr(uv), ptr(patterns),
@@ -103,14 +166,15 @@ def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R
     return o
 
 
-def check_batch(uv, patterns, K, R, t, res_norm=None, best_pattern=None, reproj_limit_px=1.0):
+def check_batch(uv, patterns, K, R, t, res_norm=None, best_pattern=None, reproj_limit_px=1.0, visible=None):
     """pnpb200_check_batch on device tensors: the solution check of any pose, without ground truth.
 
     uv [B, n_total, 2], patterns [P, n_total, 3] (or [n_total, 3]), R [B,3,3], t [B,3] and res_norm [B] are CUDA
     tensors of one float dtype; best_pattern [B] int32 picks each problem's pattern (None: pattern 0); K is a host
     3x3.  Returns dict(status [B] int32 of CHECK_* bits, reproj [B,2] = (mean, max) prediction-vs-landmark distance in
     pixels over all n_total landmarks).  REPROJ is set where the mean exceeds reproj_limit_px (<= 0 turns it off).
-    What the bits find, and what they miss (EIF2), is in include/pnpb200.h."""
+    What the bits find, and what they miss (EIF2), is in include/pnpb200.h.
+    visible: bool [B, n_total] -> pnpb200_check_batch_masked: reproj and BEHIND over each problem's visible landmarks."""
     if not all(x.is_cuda for x in (uv, patterns, R, t)):
         raise ValueError("uv, patterns, R and t must be CUDA tensors (no CPU fallback)")
     if len({x.dtype for x in (uv, patterns, R, t) + (() if res_norm is None else (res_norm,))}) != 1:
@@ -124,6 +188,8 @@ def check_batch(uv, patterns, K, R, t, res_norm=None, best_pattern=None, reproj_
         raise ValueError("R [B,3,3], t [B,3] and res_norm [B] must hold B = %d problems" % B)
     if best_pattern is not None and (best_pattern.dtype != torch.int32 or best_pattern.numel() != B or not best_pattern.is_cuda):
         raise ValueError("best_pattern must be a CUDA int32 tensor of B = %d entries" % B)
+    if visible is not None:
+        _check_visible(visible, B, n_total)
     dev = uv.device
     uv, patterns, R, t = uv.contiguous(), patterns.contiguous(), R.contiguous(), t.contiguous()
     res_norm = None if res_norm is None else res_norm.contiguous()
@@ -134,11 +200,18 @@ def check_batch(uv, patterns, K, R, t, res_norm=None, best_pattern=None, reproj_
         return dict(status=status, reproj=reproj)
     Kh, Kp = _k_host(K)
     PI = C.POINTER(C.c_int32)
+    bp = None if best_pattern is None else C.cast(ptr(best_pattern), PI)
     with torch.cuda.device(dev):
-        rc = lib.pnpb200_check_batch(_dtype_code(uv.dtype), B, n_total, ptr(patterns), int(patterns.shape[0]), ptr(uv), Kp, ptr(R),
-                                     ptr(t), ptr(res_norm), None if best_pattern is None else C.cast(ptr(best_pattern), PI),
-                                     float(reproj_limit_px), C.cast(ptr(status), PI), ptr(reproj), _stream_ptr(dev))
-    check(rc, "pnpb200_check_batch")
+        if visible is None:
+            rc = lib.pnpb200_check_batch(_dtype_code(uv.dtype), B, n_total, ptr(patterns), int(patterns.shape[0]), ptr(uv), Kp, ptr(R),
+                                         ptr(t), ptr(res_norm), bp, float(reproj_limit_px), C.cast(ptr(status), PI), ptr(reproj),
+                                         _stream_ptr(dev))
+        else:
+            words = visible_words(visible, dev)
+            rc = lib.pnpb200_check_batch_masked(_dtype_code(uv.dtype), B, n_total, ptr(patterns), int(patterns.shape[0]), ptr(uv), Kp,
+                                                ptr(R), ptr(t), ptr(res_norm), bp, float(reproj_limit_px), C.cast(ptr(status), PI),
+                                                ptr(reproj), _u32(words), _stream_ptr(dev))
+    check(rc, "pnpb200_check_batch" if visible is None else "pnpb200_check_batch_masked")
     _lib.count_launch()
     return dict(status=status, reproj=reproj)
 
@@ -188,7 +261,7 @@ class HostPipeline(object):
     _OUT_SHAPES = {"R": (9, None), "t": (3, None), "euler": (3, None), "res_norm": (1, None), "iters": (1, torch.int32),
                    "best_pattern": (1, torch.int32), "status": (1, torch.int32), "reproj": (2, None)}
 
-    def solve(self, method, uv_host, patterns_host, K, out, point_index=None, params=None, check=None):
+    def solve(self, method, uv_host, patterns_host, K, out, point_index=None, params=None, check=None, visible=None):
         """uv_host [B,n_total,2], patterns_host [P,n_total,3]: contiguous CPU torch tensors (pinned for overlap).
         uv_host may also be int16, uint16 or float32 whatever the pipeline's dtype (detections as a detector
         delivers them: pnpb200_solve_batch_host_px ships them as they are and widens them on the device).
@@ -196,7 +269,9 @@ class HostPipeline(object):
         (pipeline dtype), iters [B], best_pattern [B] (int32).  check = a limit in px: each chunk's solve is followed
         by the solution check (pnpb200_solve_check_batch_host), whose status [B] (int32, required then) and
         reproj [B,2] (pipeline dtype) go to out as well.  Everything is checked here: the C side reads and
-        writes B * (row size) elements through the raw pointers."""
+        writes B * (row size) elements through the raw pointers.
+        visible: bool [B, n_total] (NumPy array or torch tensor) -> pnpb200_solve_batch_host_masked: every chunk's mask words
+        travel with its pixels, and the solve (and check) of each problem use its visible landmarks alone."""
         m = _lib.METHODS[method] if isinstance(method, str) else int(method)
         tdt = _TORCH_DTYPE[self.dt]
         if not (torch.is_tensor(uv_host) and torch.is_tensor(patterns_host)):
@@ -227,28 +302,40 @@ class HostPipeline(object):
             raise ValueError("check= needs out['status']")
         if params is not None and params.workspace:
             raise ValueError("params.workspace is not used by the host pipeline (it owns one scratch per stream)")
+        words = None
+        if visible is not None:
+            _check_visible(visible, B, self.n_total)
+            words = visible_words_host(visible)
         if point_index is None:
             n, idx_p = self.n_total, None
         else:
             idx = np.ascontiguousarray(np.asarray(point_index, dtype=np.int32))
             n, idx_p = int(idx.shape[0]), idx.ctypes.data_as(C.POINTER(C.c_int32))
         Kh, Kp = _k_host(K)
+        PI = C.POINTER(C.c_int32)
+        pi = (lambda k: None if out.get(k) is None else C.cast(ptr(out[k]), PI))
         with torch.cuda.device(self.device):
-            if check is None:
+            if words is not None:
+                rc = lib.pnpb200_solve_batch_host_masked(
+                    self._h, m, B, n, px, ptr(uv_host), ptr(patterns_host), idx_p, Kp,
+                    C.byref(params) if params is not None else None,
+                    ptr(out.get("R")), ptr(out.get("t")), ptr(out.get("euler")), ptr(out.get("res_norm")),
+                    pi("iters"), pi("best_pattern"), words.ctypes.data_as(C.POINTER(C.c_uint32)),
+                    float(check) if check is not None else 0.0, pi("status"), ptr(out.get("reproj")))
+            elif check is None:
                 rc = lib.pnpb200_solve_batch_host_px(
                     self._h, C.c_int(m), C.c_int64(B), C.c_int(n), C.c_int(px), ptr(uv_host), ptr(patterns_host), idx_p, Kp,
                     C.byref(params) if params is not None else None,
                     ptr(out.get("R")), ptr(out.get("t")), ptr(out.get("euler")), ptr(out.get("res_norm")),
                     ptr(out.get("iters")), ptr(out.get("best_pattern")))
             else:
-                PI = C.POINTER(C.c_int32)
-                pi = (lambda k: None if out.get(k) is None else C.cast(ptr(out[k]), PI))
                 rc = lib.pnpb200_solve_check_batch_host(
                     self._h, m, B, n, px, ptr(uv_host), ptr(patterns_host), idx_p, Kp,
                     C.byref(params) if params is not None else None,
                     ptr(out.get("R")), ptr(out.get("t")), ptr(out.get("euler")), ptr(out.get("res_norm")),
                     pi("iters"), pi("best_pattern"), float(check), pi("status"), ptr(out.get("reproj")))
-        _check_rc(rc, "pnpb200_solve_batch_host_px" if check is None else "pnpb200_solve_check_batch_host")
+        _check_rc(rc, "pnpb200_solve_batch_host_masked" if words is not None else
+                  ("pnpb200_solve_batch_host_px" if check is None else "pnpb200_solve_check_batch_host"))
         _lib.count_launch((B + self.chunk - 1) // self.chunk)
         return out
 
@@ -483,7 +570,7 @@ class PNP_SOLVER(object):
         """PNP_SOLVER_LIB.py:205-430 (rows follow the image dict's key order, :3069)"""
         return self._solve_single("linear_f1", np_point_image_dict, np_point_3d_pretransfer_dict, list(np_point_image_dict.keys()))
 
-    def solve_pnp_batch(self, uv, method=None, key_list="default", params=None, check=None):
+    def solve_pnp_batch(self, uv, method=None, key_list="default", params=None, check=None, visible=None):
         """The per-problem script loop as one launch.
 
         uv: [B, n_total, 2] pixels (or [B, n_total, 3] homogeneous image points, third entry as the reference's
@@ -492,7 +579,9 @@ class PNP_SOLVER(object):
         the 6 keys of solve_pnp() for 'qeif', all points otherwise.  Returns a dict of CUDA
         tensors (see solve_batch) and, like solve_pnp, works over every stored pattern.
         check: a limit in px -> the dict also holds status [B] int32 and reproj [B,2] of check_batch on the
-        returned poses, over all n_total landmarks and each problem's winning pattern (0: no REPROJ bit)."""
+        returned poses, over all n_total landmarks and each problem's winning pattern (0: no REPROJ bit).
+        visible: bool [B, n_total] (a detector's per-frame visibility, e.g. isfinite(uv).all(-1)) -> each problem is solved
+        and checked on its visible landmarks alone (of key_list, in its order); hidden pixels may hold anything, NaN too."""
         method = method or self.method
         all_keys = list(self.np_point_3d_pretransfer_dict_list[0].keys())
         if isinstance(key_list, str) and key_list == "default":
@@ -500,19 +589,21 @@ class PNP_SOLVER(object):
         idx = None if key_list is None else [all_keys.index(k) for k in key_list]
         if not torch.is_tensor(uv):
             uv = torch.from_numpy(np.ascontiguousarray(uv))
+        if visible is not None:
+            _check_visible(visible, int(uv.shape[0]), len(all_keys))
         uv, K = self._uv_and_K(uv.to(device=self.device, dtype=self._tdtype()))
         ck = ("all", self.dtype_code)
         if ck not in self._dev_cache:
             self._dev_cache[ck] = self._pack_patterns(self.np_point_3d_pretransfer_dict_list, all_keys)
         out = solve_batch(method, uv, self._dev_cache[ck], K, point_index=idx,
-                          params=params if params is not None else self.params)
+                          params=params if params is not None else self.params, visible=visible)
         if check is not None:
             out.update(check_batch(uv, self._dev_cache[ck], K, out["R"], out["t"], res_norm=out["res_norm"],
-                                   best_pattern=out["best_pattern"], reproj_limit_px=check))
+                                   best_pattern=out["best_pattern"], reproj_limit_px=check, visible=visible))
         return out
 
     def solve_pnp_batch_host(self, uv, method=None, key_list="default", params=None, chunk_problems=1 << 16, pack_threads=None,
-                             check=None):
+                             check=None, visible=None):
         """solve_pnp_batch for data that lives on the HOST (what a script that loops over NumPy samples
         has): uv [B, n_total, 2] NumPy array or CPU tensor in; dict of NumPy arrays R [B,3,3], t [B,3],
         euler [B,3] (roll, yaw, pitch, deg.), res_norm [B], iters [B], best_pattern [B] out.  uv may be int16,
@@ -521,7 +612,9 @@ class PNP_SOLVER(object):
         pack_threads host threads (default: half the visible cores, at most 8) let chunks of whole-pixel
         landmarks cross PCIe as int16 (lossless, checked per chunk; other chunks travel as they are).
         check: a limit in px -> each chunk's solve is followed by the solution check on the device, and the dict also
-        holds status [B] int32 and reproj [B,2] (see solve_pnp_batch); every other output is unchanged."""
+        holds status [B] int32 and reproj [B,2] (see solve_pnp_batch); every other output is unchanged.
+        visible: bool [B, n_total] -> the masked pipeline (see solve_pnp_batch); a chunk whose hidden pixels are NaN travels
+        unpacked."""
         method = method or self.method
         all_keys = list(self.np_point_3d_pretransfer_dict_list[0].keys())
         if isinstance(key_list, str) and key_list == "default":
@@ -537,6 +630,8 @@ class PNP_SOLVER(object):
         B, n_total = int(uv_h.shape[0]), int(uv_h.shape[1])
         if n_total != len(all_keys):
             raise ValueError("uv holds %d landmarks per problem, the stored patterns %d" % (n_total, len(all_keys)))
+        if visible is not None:
+            _check_visible(visible, B, n_total)
         pats = np.stack([np.stack([np.asarray(d[k], dtype=np.float64).reshape(3) for k in all_keys])
                          for d in self.np_point_3d_pretransfer_dict_list])
         pat_h = torch.from_numpy(pats).to(dtype=tdt).contiguous()
@@ -571,7 +666,7 @@ class PNP_SOLVER(object):
             sel["status"], sel["reproj"] = outs["status"], outs["reproj"]
         if B > 0:
             pipe.solve(method, uv_h, pat_h, self.np_K_camera_est, sel, point_index=idx,
-                       params=params if params is not None else self.params, check=check)
+                       params=params if params is not None else self.params, check=check, visible=visible)
         return {k: v.numpy().copy() for k, v in sel.items()}
 
     # ---------------------------------------------------------------- Euler <-> R (:4442-4517)

@@ -12,7 +12,7 @@ import torch
 
 from . import _lib
 from ._lib import lib, check, ptr
-from .solver import _copy_params, _dtype_code, _k_host, _stream_ptr
+from .solver import _check_visible, _copy_params, _dtype_code, _k_host, _stream_ptr, _u32, visible_words
 
 # TEST_TOOLBOX.get_classification_parameters("drpy_expand") (TEST_TOOLBOX.py:133-162)
 CLASS_BINS = {
@@ -64,15 +64,18 @@ def synth_batch(b0, B, pattern, K, cfg=None, dtype=torch.float64, device=None, w
     return out
 
 
-def report_batch(pattern, uv, K, R, t, euler, gt, bounds=(10.0, 10.0, 10.0, 10.0), layout="columns"):
+def report_batch(pattern, uv, K, R, t, euler, gt, bounds=(10.0, 10.0, 10.0, 10.0), layout="columns", visible=None):
     """Per-problem error report (pnpb200_report_batch_strided): dict(report [B,16] f64, flags [B,4]
     int32, max_idx [B,3] int32).  Column meaning: include/pnpb200.h.  pattern [n,3], uv [B,n,2]: every
     landmark of the pattern, as in compare_result_and_generate_result_dict (TEST_TOOLBOX.py:291).
     layout="columns" (default): report is the transposed view of a [16,B] array, so report[:, k] is
-    contiguous (what the statistics read); layout="rows": a contiguous [B,16] array."""
+    contiguous (what the statistics read); layout="rows": a contiguous [B,16] array.
+    visible: bool [B, n] -> pnpb200_report_batch_strided_masked: columns 4-9 and max_idx over the visible landmarks."""
     dev = uv.device
     pattern = torch.as_tensor(pattern, device=dev).to(uv.dtype).contiguous()
     B, n = int(uv.shape[0]), int(uv.shape[1])
+    if visible is not None:
+        _check_visible(visible, B, n)
     if layout == "columns":
         rep = torch.empty((_lib.REPORT_WIDTH, B), dtype=torch.float64, device=dev).t()
     else:
@@ -84,6 +87,19 @@ def report_batch(pattern, uv, K, R, t, euler, gt, bounds=(10.0, 10.0, 10.0, 10.0
     Kh, Kp = _k_host(K)
     bd = (C.c_double * 4)(*[float(b) for b in bounds])
     gt = gt.to(torch.float64).contiguous()
+    if visible is not None:
+        if B == 0:
+            return dict(report=rep, flags=flags, max_idx=midx)
+        PD, PI = C.POINTER(C.c_double), C.POINTER(C.c_int32)
+        words = visible_words(visible, dev)
+        with torch.cuda.device(dev):
+            check(lib.pnpb200_report_batch_strided_masked(_dtype_code(uv.dtype), B, n, ptr(pattern), ptr(uv.contiguous()), Kp,
+                                                          ptr(R.contiguous()), ptr(t.contiguous()), ptr(euler.contiguous()),
+                                                          C.cast(ptr(gt), PD), bd, C.cast(ptr(rep), PD), rs_b, rs_k,
+                                                          C.cast(ptr(flags), PI), C.cast(ptr(midx), PI), _u32(words),
+                                                          _stream_ptr(dev)), "pnpb200_report_batch_strided_masked")
+        _lib.count_launch()
+        return dict(report=rep, flags=flags, max_idx=midx)
     with torch.cuda.device(dev):
         check(lib.pnpb200_report_batch_strided(C.c_int(_dtype_code(uv.dtype)), C.c_int64(B), C.c_int(n), ptr(pattern),
                                                ptr(uv.contiguous()), Kp, ptr(R.contiguous()), ptr(t.contiguous()),
@@ -95,12 +111,13 @@ def report_batch(pattern, uv, K, R, t, euler, gt, bounds=(10.0, 10.0, 10.0, 10.0
     return dict(report=rep, flags=flags, max_idx=midx)
 
 
-def solve_report_batch(method, uv, pattern, K, gt, params=None, bounds=(10.0, 10.0, 10.0, 10.0), point_index=None):
+def solve_report_batch(method, uv, pattern, K, gt, params=None, bounds=(10.0, 10.0, 10.0, 10.0), point_index=None, visible=None):
     """pnpb200_solve_report_batch: solve_batch (one pattern) and report_batch (column layout) of the same problems in
     one call -- the body of the loop of random_stress_test.py:322-377.  With LM / linear F2 over all landmarks the
     residual pass of the solve rides in the report kernel (the pixel rows are read twice instead of three times);
     the results are those of the two separate calls.  uv [B,n,2], pattern [n,3] (or [1,n,3]) CUDA tensors of one
-    dtype, gt [B,4] FP64.  Returns the union of both dicts."""
+    dtype, gt [B,4] FP64.  Returns the union of both dicts.
+    visible: bool [B, n] -> pnpb200_solve_report_batch_masked: the masked solve, then the masked report."""
     m = _lib.METHODS[method] if isinstance(method, str) else int(method)
     dev = uv.device
     uv = uv.contiguous()
@@ -108,6 +125,8 @@ def solve_report_batch(method, uv, pattern, K, gt, params=None, bounds=(10.0, 10
     B, n_total = int(uv.shape[0]), int(uv.shape[1])
     if uv.dim() != 3 or uv.shape[2] != 2 or pattern.shape[0] != n_total:
         raise ValueError("shape mismatch: uv [B,n,2], pattern [n,3]")
+    if visible is not None:
+        _check_visible(visible, B, n_total)
     dt = _dtype_code(uv.dtype)
     if point_index is None:
         n, idx_p = n_total, None
@@ -122,7 +141,8 @@ def solve_report_batch(method, uv, pattern, K, gt, params=None, bounds=(10.0, 10
     if B == 0:
         return o
     prm = _lib.default_params() if params is None else params
-    ws_bytes = int(lib.pnpb200_workspace_bytes(C.c_int(m), C.c_int(dt), C.c_int64(B), C.c_int(1), C.c_int(int(prm.mapping))))
+    ws_query = lib.pnpb200_workspace_bytes if visible is None else lib.pnpb200_workspace_bytes_masked
+    ws_bytes = int(ws_query(C.c_int(m), C.c_int(dt), C.c_int64(B), C.c_int(1), C.c_int(int(prm.mapping))))
     ws = None
     if ws_bytes > 0 and not prm.workspace:                 # scratch from torch's caching allocator (stream-ordered, no driver call)
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
@@ -133,6 +153,17 @@ def solve_report_batch(method, uv, pattern, K, gt, params=None, bounds=(10.0, 10
     gt = gt.to(torch.float64).contiguous()
     PD, PI = C.POINTER(C.c_double), C.POINTER(C.c_int32)
     rep = o["report"]
+    if visible is not None:
+        words = visible_words(visible, dev)
+        with torch.cuda.device(dev):
+            check(lib.pnpb200_solve_report_batch_masked(m, dt, B, n_total, n, ptr(uv), ptr(pattern), idx_p, Kp, C.byref(prm), ptr(o["R"]),
+                                                        ptr(o["t"]), ptr(o["euler"]), ptr(o["res_norm"]), C.cast(ptr(o["iters"]), PI),
+                                                        C.cast(ptr(gt), PD), bd, C.cast(ptr(rep), PD), max(int(rep.stride(0)), 1),
+                                                        max(int(rep.stride(1)), 1), C.cast(ptr(o["flags"]), PI),
+                                                        C.cast(ptr(o["max_idx"]), PI), _u32(words), _stream_ptr(dev)),
+                  "pnpb200_solve_report_batch_masked")
+        _lib.count_launch(2)
+        return o
     with torch.cuda.device(dev):
         check(lib.pnpb200_solve_report_batch(C.c_int(m), C.c_int(dt), C.c_int64(B), C.c_int(n_total), C.c_int(n), ptr(uv), ptr(pattern),
                                              idx_p, Kp, C.byref(prm), ptr(o["R"]), ptr(o["t"]), ptr(o["euler"]), ptr(o["res_norm"]),
