@@ -22,6 +22,8 @@ _LAZY = {
     "euler_from_R_batch": (".solver", "euler_from_R_batch"), "project_batch": (".solver", "project_batch"),
     "check_batch": (".solver", "check_batch"), "CHECK_NONFINITE": ("._lib", "CHECK_NONFINITE"),
     "CHECK_DEPTH": ("._lib", "CHECK_DEPTH"), "CHECK_BEHIND": ("._lib", "CHECK_BEHIND"), "CHECK_REPROJ": ("._lib", "CHECK_REPROJ"),
+    "solve_robust_batch": (".solver", "solve_robust_batch"), "ROBUST_TOO_FEW": ("._lib", "ROBUST_TOO_FEW"),
+    "ROBUST_NOT_CONVERGED": ("._lib", "ROBUST_NOT_CONVERGED"),
 }
 
 

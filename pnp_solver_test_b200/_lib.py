@@ -24,6 +24,8 @@ MAX_PATTERNS = 8
 PIXEL_NATIVE, PIXEL_I16, PIXEL_U16, PIXEL_F32 = 0, 1, 2, 3
 # bits of the status word of the solution check (pnpb200_check_batch)
 CHECK_NONFINITE, CHECK_DEPTH, CHECK_BEHIND, CHECK_REPROJ = 1, 2, 4, 8
+# bits of robust_status of the outlier-robust solve (pnpb200_solve_robust_batch)
+ROBUST_TOO_FEW, ROBUST_NOT_CONVERGED = 1, 2
 
 EXPORTS = [
     "pnpb200_version", "pnpb200_launch_count", "pnpb200_last_error", "pnpb200_default_params", "pnpb200_default_synth",
@@ -36,6 +38,7 @@ EXPORTS = [
     "pnpb200_check_batch", "pnpb200_solve_check_batch_host",
     "pnpb200_solve_batch_masked", "pnpb200_solve_report_batch_masked", "pnpb200_report_batch_strided_masked",
     "pnpb200_check_batch_masked", "pnpb200_workspace_bytes_masked", "pnpb200_solve_batch_host_masked",
+    "pnpb200_default_robust_params", "pnpb200_robust_workspace_bytes", "pnpb200_solve_robust_batch",
 ]
 
 
@@ -46,6 +49,11 @@ class Params(C.Structure):
                 ("proc_q", C.c_double), ("proc_d", C.c_double), ("omega0", C.c_double),
                 ("res_old0", C.c_double), ("mapping", C.c_int32), ("flags", C.c_int32),
                 ("workspace", C.c_void_p), ("workspace_bytes", C.c_int64)]
+
+
+class RobustParams(C.Structure):
+    """struct pnpb200_robust_params"""
+    _fields_ = [("max_rounds", C.c_int32), ("k_median", C.c_double), ("floor_px", C.c_double), ("min_inliers", C.c_int32)]
 
 
 class Synth(C.Structure):
@@ -93,6 +101,11 @@ lib.pnpb200_check_batch_masked.argtypes = [C.c_int, C.c_int64, C.c_int, _VP, C.c
                                            _PI, _VP, _U32P, _VP]
 lib.pnpb200_solve_batch_host_masked.argtypes = [_VP, C.c_int, C.c_int64, C.c_int, C.c_int, _VP, _VP, _PI, _PD, _VP, _VP, _VP,
                                                 _VP, _VP, _PI, _PI, _U32P, C.c_double, _PI, _VP]
+lib.pnpb200_robust_workspace_bytes.restype = C.c_int64
+lib.pnpb200_robust_workspace_bytes.argtypes = [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int]
+# pnpb200_solve_batch_masked's arguments, then the robust parameters and the three outputs
+lib.pnpb200_solve_robust_batch.argtypes = [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, _VP, _VP, C.c_int, _PI, _PD, _VP,
+                                           _VP, _VP, _VP, _VP, _PI, _PI, _U32P, _VP, _U32P, _PI, _PI, _VP]
 
 _ERR = {-1: "EINVAL (bad argument)", -2: "ECUDA (CUDA runtime error)", -3: "ENODEVICE (no usable CUDA device)",
         -4: "ETOOLARGE (n too large for the selected mapping)"}

@@ -217,11 +217,14 @@ int64_t pnpb200_workspace_bytes_masked(int method, int dtype, int64_t B, int n_p
     return plain > 0 ? plain + (int64_t)PNP_NPMOM * B * ((dtype == PNPB200_DTYPE_F32) ? 4 : 8) : 0;
 }
 
+}  // extern "C"
+
+namespace pnpb200 {
 // vis: [B, ceil(n_total / 32)] per-problem visibility bits (device), or nullptr for every landmark
-static int solve_batch_impl(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
-                            int n_patterns, const int32_t* point_index, const double* K, const pnpb200_params& prm,
-                            void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters, int32_t* best_pattern,
-                            cudaStream_t st, const uint32_t* vis = nullptr)
+int solve_batch_impl(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
+                     int n_patterns, const int32_t* point_index, const double* K, const pnpb200_params& prm,
+                     void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters, int32_t* best_pattern,
+                     cudaStream_t st, const uint32_t* vis)
 {
     if (B < 0 || n_total < 1 || n < 1 || (!point_index && n != n_total) || !uv || !pattern || !K) return PNPB200_EINVAL;
     if (vis && !vis_aligned(vis)) return PNPB200_EINVAL;
@@ -249,6 +252,9 @@ static int solve_batch_impl(int method, int dtype, int64_t B, int n_total, int n
     if (idx_dev) cudaFreeAsync(idx_dev, st);
     return rc;
 }
+}  // namespace pnpb200
+
+extern "C" {
 
 int pnpb200_solve_batch(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
                         int n_patterns, const int32_t* point_index, const double* K, const pnpb200_params* params,

@@ -73,6 +73,10 @@ inline bool vis_aligned(const uint32_t* vis) { return ((uintptr_t)vis & 3u) == 0
 int check_launch(int dtype, int64_t B, int n, const void* pattern, int n_patterns, const void* uv, const double* K,
                  const void* R, const void* t, const void* res_norm, const int32_t* best_pattern, double limit,
                  int32_t* status, void* reproj, cudaStream_t st, const uint32_t* vis = nullptr);
+// pnpb200_solve_batch(_masked) without the entry's parameter copy (pnpb200_api.cu); vis = nullptr: every landmark
+int solve_batch_impl(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern, int n_patterns,
+                     const int32_t* point_index, const double* K, const pnpb200_params& prm, void* R, void* t, void* euler_deg,
+                     void* res_norm, int32_t* iters, int32_t* best_pattern, cudaStream_t st, const uint32_t* vis = nullptr);
 cudaError_t set_dynamic_smem(const void* kernel, size_t bytes);                                   // defined in pnpb200_api.cu
 cudaError_t blocks_per_sm(int* out, const void* kernel, int block_threads, size_t smem_bytes);   // defined in pnpb200_api.cu
 

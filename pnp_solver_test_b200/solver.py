@@ -92,16 +92,8 @@ def _u32(t):
     return C.cast(ptr(t), C.POINTER(C.c_uint32))
 
 
-def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R", "t", "euler", "res_norm", "iters", "best_pattern"),
-                visible=None):
-    """pnpb200_solve_batch on device tensors.
-
-    uv [B, n_total, 2] and patterns [P, n_total, 3] are CUDA tensors of the same float dtype;
-    K is a host 3x3.  Returns a dict of CUDA tensors: R [B,3,3], t [B,3], euler [B,3] =
-    (roll, yaw, pitch) in degrees, res_norm [B], iters [B] int32, best_pattern [B] int32.
-    visible: bool [B, n_total] (torch tensor or NumPy array) -> pnpb200_solve_batch_masked: each problem is solved on its
-    visible landmarks alone (those of point_index, in its order); hidden pixels are never read, and a problem with fewer
-    than 4 of them comes back NaN with iters 0 (include/pnpb200.h)."""
+def _batch_args(method, uv, patterns, point_index, visible):
+    """the argument checks and conversions of solve_batch and solve_robust_batch (ValueError before any launch)"""
     m = _lib.METHODS[method] if isinstance(method, str) else int(method)
     if not (uv.is_cuda and patterns.is_cuda):
         raise ValueError("uv and patterns must be CUDA tensors (no CPU fallback)")
@@ -117,11 +109,22 @@ def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R
         raise ValueError("shape mismatch: uv [B,n,2], patterns [P,n,3]")
     if visible is not None:
         _check_visible(visible, B, n_total)
-    if point_index is None:
-        n, idx_p, idx = n_total, None, None
-    else:
-        idx = np.ascontiguousarray(np.asarray(point_index, dtype=np.int32))
-        n, idx_p = int(idx.shape[0]), idx.ctypes.data_as(C.POINTER(C.c_int32))
+    idx = None if point_index is None else np.ascontiguousarray(np.asarray(point_index, dtype=np.int32))
+    return m, dt, uv, patterns, B, n_total, idx
+
+
+def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R", "t", "euler", "res_norm", "iters", "best_pattern"),
+                visible=None):
+    """pnpb200_solve_batch on device tensors.
+
+    uv [B, n_total, 2] and patterns [P, n_total, 3] are CUDA tensors of the same float dtype;
+    K is a host 3x3.  Returns a dict of CUDA tensors: R [B,3,3], t [B,3], euler [B,3] =
+    (roll, yaw, pitch) in degrees, res_norm [B], iters [B] int32, best_pattern [B] int32.
+    visible: bool [B, n_total] (torch tensor or NumPy array) -> pnpb200_solve_batch_masked: each problem is solved on its
+    visible landmarks alone (those of point_index, in its order); hidden pixels are never read, and a problem with fewer
+    than 4 of them comes back NaN with iters 0 (include/pnpb200.h)."""
+    m, dt, uv, patterns, B, n_total, idx = _batch_args(method, uv, patterns, point_index, visible)
+    n, idx_p = (n_total, None) if idx is None else (int(idx.shape[0]), idx.ctypes.data_as(C.POINTER(C.c_int32)))
     dev = uv.device
     o = {}
     if "R" in want: o["R"] = torch.empty((B, 3, 3), dtype=uv.dtype, device=dev)
@@ -163,6 +166,72 @@ def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R
             ptr(o.get("iters")), ptr(o.get("best_pattern")), _stream_ptr(dev))
     check(rc, "pnpb200_solve_batch")
     _lib.count_launch(1 if B > 0 else 0)
+    return o
+
+
+def robust_params(max_rounds=4, k=3.0, floor_px=2.0, min_inliers=6):
+    """struct pnpb200_robust_params; ValueError for what pnpb200_solve_robust_batch refuses with EINVAL"""
+    max_rounds, min_inliers, k, floor_px = int(max_rounds), int(min_inliers), float(k), float(floor_px)
+    if max_rounds < 1:
+        raise ValueError("max_rounds must be >= 1, not %d" % max_rounds)
+    if min_inliers < 4:
+        raise ValueError("min_inliers must be >= 4, not %d" % min_inliers)
+    if not (np.isfinite(k) and k >= 0.0):
+        raise ValueError("k must be finite and >= 0, not %r" % k)
+    if not floor_px >= 0.0:
+        raise ValueError("floor_px must be >= 0 (inf allowed), not %r" % floor_px)
+    return _lib.RobustParams(max_rounds=max_rounds, k_median=k, floor_px=floor_px, min_inliers=min_inliers)
+
+
+def unpack_words(words, n_total):
+    """the inverse of visible_words: [B, W] int32 words -> bool [B, n_total] on the words' device"""
+    B, W = int(words.shape[0]), int(words.shape[1])
+    shifts = torch.arange(8, dtype=torch.uint8, device=words.device)
+    bits = (words.contiguous().view(torch.uint8).reshape(B, W * 4, 1) >> shifts) & 1
+    return bits.reshape(B, W * 32)[:, :n_total].bool()
+
+
+def solve_robust_batch(method, uv, patterns, K, point_index=None, params=None, visible=None, max_rounds=4, k=3.0, floor_px=2.0,
+                       min_inliers=6):
+    """pnpb200_solve_robust_batch on device tensors: each problem is solved on its candidates (the landmarks of point_index
+    that are visible), the landmarks whose reprojection distance exceeds max(floor_px, k * median) are dropped, and the
+    problem is solved again on the rest, until the inlier set stops changing or after max_rounds solves.  Returns the dict of
+    solve_batch plus inliers (bool [B, n_total]: the landmarks the returned pose was solved on), rounds [B] int32 (solves)
+    and robust_status [B] int32 (ROBUST_TOO_FEW, ROBUST_NOT_CONVERGED bits; 0 = converged).  Every output of a problem is
+    bit for bit that of solve_batch(..., visible=inliers).  The rule, its defaults and what it rescues are in
+    include/pnpb200.h.  The call synchronises the stream once per round."""
+    rp = robust_params(max_rounds, k, floor_px, min_inliers)
+    m, dt, uv, patterns, B, n_total, idx = _batch_args(method, uv, patterns, point_index, visible)
+    n, idx_p = (n_total, None) if idx is None else (int(idx.shape[0]), idx.ctypes.data_as(C.POINTER(C.c_int32)))
+    dev = uv.device
+    P = int(patterns.shape[0])
+    o = dict(R=torch.empty((B, 3, 3), dtype=uv.dtype, device=dev), t=torch.empty((B, 3), dtype=uv.dtype, device=dev),
+             euler=torch.empty((B, 3), dtype=uv.dtype, device=dev), res_norm=torch.empty((B,), dtype=uv.dtype, device=dev),
+             iters=torch.empty((B,), dtype=torch.int32, device=dev), best_pattern=torch.empty((B,), dtype=torch.int32, device=dev))
+    words = torch.empty((B, (n_total + 31) // 32), dtype=torch.int32, device=dev)
+    o["rounds"] = torch.empty((B,), dtype=torch.int32, device=dev)
+    o["robust_status"] = torch.empty((B,), dtype=torch.int32, device=dev)
+    if B == 0:
+        o["inliers"] = torch.empty((0, n_total), dtype=torch.bool, device=dev)
+        return o
+    Kh, Kp = _k_host(K)
+    prm = _lib.default_params() if params is None else params
+    ws_bytes = int(lib.pnpb200_robust_workspace_bytes(m, dt, B, n_total, P, int(prm.mapping)))
+    ws = None
+    if ws_bytes > 0 and not prm.workspace:
+        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+        prm = _copy_params(prm)
+        prm.workspace, prm.workspace_bytes = ws.data_ptr(), ws_bytes
+    vw = None if visible is None else visible_words(visible, dev)
+    PI = C.POINTER(C.c_int32)
+    with torch.cuda.device(dev):
+        rc = lib.pnpb200_solve_robust_batch(
+            m, dt, B, n_total, n, ptr(uv), ptr(patterns), P, idx_p, Kp, C.byref(prm), ptr(o["R"]), ptr(o["t"]), ptr(o["euler"]),
+            ptr(o["res_norm"]), C.cast(ptr(o["iters"]), PI), C.cast(ptr(o["best_pattern"]), PI), None if vw is None else _u32(vw),
+            C.byref(rp), _u32(words), C.cast(ptr(o["rounds"]), PI), C.cast(ptr(o["robust_status"]), PI), _stream_ptr(dev))
+    check(rc, "pnpb200_solve_robust_batch")
+    _lib.count_launch(1)
+    o["inliers"] = unpack_words(words, n_total)
     return o
 
 
@@ -570,7 +639,7 @@ class PNP_SOLVER(object):
         """PNP_SOLVER_LIB.py:205-430 (rows follow the image dict's key order, :3069)"""
         return self._solve_single("linear_f1", np_point_image_dict, np_point_3d_pretransfer_dict, list(np_point_image_dict.keys()))
 
-    def solve_pnp_batch(self, uv, method=None, key_list="default", params=None, check=None, visible=None):
+    def solve_pnp_batch(self, uv, method=None, key_list="default", params=None, check=None, visible=None, robust=None):
         """The per-problem script loop as one launch.
 
         uv: [B, n_total, 2] pixels (or [B, n_total, 3] homogeneous image points, third entry as the reference's
@@ -581,8 +650,16 @@ class PNP_SOLVER(object):
         check: a limit in px -> the dict also holds status [B] int32 and reproj [B,2] of check_batch on the
         returned poses, over all n_total landmarks and each problem's winning pattern (0: no REPROJ bit).
         visible: bool [B, n_total] (a detector's per-frame visibility, e.g. isfinite(uv).all(-1)) -> each problem is solved
-        and checked on its visible landmarks alone (of key_list, in its order); hidden pixels may hold anything, NaN too."""
+        and checked on its visible landmarks alone (of key_list, in its order); hidden pixels may hold anything, NaN too.
+        robust: None, or a dict of any of max_rounds, k, floor_px, min_inliers -> solve_robust_batch: misplaced landmarks are
+        rejected by their reprojection distance and each problem re-solved on its inliers; the dict then also holds inliers,
+        rounds and robust_status, and the check (if asked for) runs on the inliers."""
         method = method or self.method
+        if robust is not None:
+            unknown = set(robust) - {"max_rounds", "k", "floor_px", "min_inliers"}
+            if unknown:
+                raise ValueError("robust takes max_rounds, k, floor_px, min_inliers; not %s" % sorted(unknown))
+            robust_params(**robust)
         all_keys = list(self.np_point_3d_pretransfer_dict_list[0].keys())
         if isinstance(key_list, str) and key_list == "default":
             key_list = self.LM_key_list if method == "qeif" else None
@@ -595,8 +672,12 @@ class PNP_SOLVER(object):
         ck = ("all", self.dtype_code)
         if ck not in self._dev_cache:
             self._dev_cache[ck] = self._pack_patterns(self.np_point_3d_pretransfer_dict_list, all_keys)
-        out = solve_batch(method, uv, self._dev_cache[ck], K, point_index=idx,
-                          params=params if params is not None else self.params, visible=visible)
+        prm = params if params is not None else self.params
+        if robust is None:
+            out = solve_batch(method, uv, self._dev_cache[ck], K, point_index=idx, params=prm, visible=visible)
+        else:
+            out = solve_robust_batch(method, uv, self._dev_cache[ck], K, point_index=idx, params=prm, visible=visible, **robust)
+            visible = out["inliers"]
         if check is not None:
             out.update(check_batch(uv, self._dev_cache[ck], K, out["R"], out["t"], res_norm=out["res_norm"],
                                    best_pattern=out["best_pattern"], reproj_limit_px=check, visible=visible))
