@@ -484,7 +484,7 @@ int pnpb200_solve_batch_host_masked(pnpb200_pipeline* p, int method, int64_t B, 
  * 30 % far outliers, LM+.
  * EIF2's pose under outliers is too far off for its distances to single the outliers out: the rule does not rescue it (as
  * the check does not find EIF2's failures).  Neither does it rescue LM+ at 30 % far outliers: that needs minimal-sample
- * hypotheses (RANSAC), which this entry does not draw.
+ * hypotheses (RANSAC), which pnpb200_solve_ransac_batch below draws before it runs this loop.
  */
 #define PNPB200_ROBUST_TOO_FEW       1   /* M_{r+1} held fewer than min_inliers landmarks: pose_r on M_r kept               */
 #define PNPB200_ROBUST_NOT_CONVERGED 2   /* max_rounds solves without a fixed point: the last pose and its mask kept         */
@@ -504,6 +504,89 @@ int pnpb200_solve_robust_batch(int method, int dtype, int64_t B, int n_total, in
                                int32_t* iters, int32_t* best_pattern, const uint32_t* visible,
                                const pnpb200_robust_params* robust, uint32_t* inliers, int32_t* rounds,
                                int32_t* robust_status, void* stream);
+
+/*
+ * Minimal-sample hypotheses (RANSAC, Fischler & Bolles 1981).  Not a reference function.  The robust solve above starts from
+ * the pose solved on all candidates, so a contaminated first pose decides which landmarks it rejects.  This stage finds each
+ * problem's largest consensus set from minimal samples instead.  Per problem b, with C = its candidates (the landmarks of
+ * point_index, in solver order, that are visible) and c = |C|:
+ *  - Sample s (s = 0, 1, ...): u = Philox4x32-10 with counter (g lo, g hi, s, 4) and key seed, g = idx0 + b;
+ *    j_k = u_k mod (c - k), k = 0..3; the k-th sample landmark is the j_k-th candidate not yet chosen, in candidate order.
+ *  - Hypothesis: a P3P pose (Lambda Twist, FP64) of the first three sample landmarks, for every pattern; bearings are
+ *    K^-1 [u, v, 1] normalised.  Among its 0..4 roots the one whose distance d (below) at the 4th landmark is smallest wins
+ *    (strict <, the first root wins ties; a NaN distance never wins); the pattern's hypothesis survives where that distance
+ *    is <= consensus_px.  A sample none of whose patterns survives is not scored.
+ *  - Consensus of a surviving hypothesis: the number of candidates i with d_i <= consensus_px, d_i the check's
+ *    prediction-vs-landmark distance (pnpb200_check_batch's arithmetic, FP64 for both dtypes; NaN is an outlier).  A sample's
+ *    consensus is the maximum over its patterns (ties to the lower pattern); the winner has the largest consensus (ties to
+ *    the lower s).
+ *  - Stop after sample s when (1 - w^4)^(s + 1) <= 1 - confidence, w = best consensus / c (evaluated as
+ *    ((c^4 - best^4) / c^4)^(s + 1), one division and binary powering), and after max_samples samples in any case.  On clean
+ *    data the first good sample ends the search.
+ *   arguments   as pnpb200_solve_batch_masked (visible may be NULL: every landmark visible); n <= 1024 and n_total <= 65536,
+ *               else PNPB200_ETOOLARGE
+ *   hyp         [host] or NULL for pnpb200_default_hypothesis_params; PNPB200_EINVAL, before any launch, unless
+ *               max_samples >= 0, consensus_px >= 0 (not NaN) and 0 < confidence <= 1
+ *   R, t        [device] [B,3,3], [B,3] (dtype): the winner's pose; best_pattern [device] [B] int32 (may be NULL for one pattern)
+ *   consensus_mask [device] [B, W] uint32 (the format of `visible`): the winner's consensus set, a subset of C
+ *   consensus   [device] [B] int32: its size;  drawn [device] [B] int32 or NULL: the number of samples taken
+ * Speed (1 Mi x 68, B200 at 1000 W, tools/time_ransac.py): 9.6 ms on clean data, 17.8 ms with 30 % far outliers (DESIGN.md 6).
+ * c < 4, or no sample survives: consensus 0, mask 0, NaN pose, best_pattern 0.  The candidates' pixels sit in shared memory
+ * (one warp per problem, 18 bytes per candidate), so every n up to 1024 fits.  The result of problem b depends on idx0 + b
+ * and its own row only: a shard called with idx0 = its first global index returns, bit for bit, its slice of the
+ * unsharded call.  The entry does not synchronise and allocates nothing, so it can be captured into a CUDA graph.
+ */
+typedef struct pnpb200_hypothesis_params {
+    int32_t  max_samples;   /* 128                                                                                    */
+    double   consensus_px;  /* 4.0  px: the 4th-landmark test and the consensus threshold                             */
+    double   confidence;    /* 0.999                                                                                  */
+    uint64_t seed;          /* 0                                                                                      */
+    int64_t  idx0;          /* 0    global index of problem 0 of the call                                             */
+} pnpb200_hypothesis_params;
+int pnpb200_default_hypothesis_params(pnpb200_hypothesis_params* p);
+int pnpb200_hypothesize_batch(int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern, int n_patterns,
+                              const int32_t* point_index, const double* K, const uint32_t* visible,
+                              const pnpb200_hypothesis_params* hyp, void* R, void* t, int32_t* best_pattern,
+                              uint32_t* consensus_mask, int32_t* consensus, int32_t* drawn, void* stream);
+
+/*
+ * RANSAC solve: the hypothesis stage above, then the robust loop of pnpb200_solve_robust_batch started from its consensus set.
+ * M0 = the winner's consensus set where consensus >= min_inliers, else C; then exactly the loop of the robust entry from M0
+ * instead of C (solve on M_r, the median rule on C, compacted re-solves, the same rounds and robust_status).
+ * Contract: that of the robust entry, unchanged.  Every output of problem b (R, t, euler_deg, res_norm, iters, best_pattern)
+ * is bit for bit pnpb200_solve_batch_masked's on the returned inlier mask, with the same QEIF / EIF2 FP64 fix-up exception.
+ * With max_samples = 0 every output, mask, round count and status word is bit-identical to pnpb200_solve_robust_batch.
+ *   arguments   those of pnpb200_solve_robust_batch, plus hyp (as pnpb200_hypothesize_batch), consensus [device] [B] int32
+ *               (the hypothesis stage's) and drawn [device] [B] int32 or NULL
+ *   params->workspace: NULL, or pnpb200_ransac_workspace_bytes of scratch (the robust entry's plus the hypothesis stage's)
+ * The call synchronises `stream` once per round, as the robust entry does.
+ * Pass rate on the 10 cm / 10 deg test, on the problems of the robust entry's table plus a 50 % row (C oracle,
+ * tests/ransac_accuracy.py), plain -> robust -> RANSAC, defaults:
+ *   moved by    f      LM+                QEIF               EIF2
+ *   -           0 %    99.0  99.1  99.1  100.0 100.0 100.0   99.2  99.2  99.2
+ *   5-30 px    10 %    48.8  98.3  99.2   50.1 100.0 100.0    9.8  21.9  99.0
+ *   5-30 px    30 %    26.8  97.5  99.0   28.1 100.0 100.0    3.4   4.3  98.7
+ *   30-150 px  10 %     2.3  87.2  99.0    3.2 100.0 100.0    0.1   3.0  99.1
+ *   30-150 px  30 %     0.1  43.8  99.0    0.4  99.5 100.0    0.0   0.0  98.7
+ *   30-150 px  50 %     0.0   0.1  98.6    0.1   2.9  99.9    0.0   0.0  98.2
+ * The minimal samples rescue every method, EIF2 included: its pose is as good on the consensus set as on clean data.
+ * consensus_px: the RANSAC pass rate per method on clean data, 30 % and 50 % moved by 30-150 px:
+ *     2 px           99.1  99.0  98.5   100.0 100.0  99.8    99.2  98.7  98.1
+ *     4 px           99.1  99.0  98.6   100.0 100.0  99.9    99.2  98.7  98.2
+ *     8 px           99.1  99.0  98.6   100.0 100.0  99.9    99.2  98.7  98.2
+ * 4 px is the default: the smallest threshold within 0.1 point of the best everywhere (a tighter one keeps near outliers,
+ * the 5-30 px rows, out of the consensus set; 2 px loses samples to the whole-pixel rounding of the detections).
+ */
+int64_t pnpb200_ransac_workspace_bytes(int method, int dtype, int64_t B, int n_total, int n_patterns, int mapping);
+int pnpb200_solve_ransac_batch(int method, int dtype, int64_t B, int n_total, int n,
+                               const void* uv, const void* pattern, int n_patterns,
+                               const int32_t* point_index, const double* K,
+                               const pnpb200_params* params,
+                               void* R, void* t, void* euler_deg, void* res_norm,
+                               int32_t* iters, int32_t* best_pattern, const uint32_t* visible,
+                               const pnpb200_robust_params* robust, uint32_t* inliers, int32_t* rounds,
+                               int32_t* robust_status, const pnpb200_hypothesis_params* hyp, int32_t* consensus,
+                               int32_t* drawn, void* stream);
 
 /*
  * Error statistics, two passes so that shards can be combined with two small all-reduce phases
@@ -614,6 +697,12 @@ int pnpb200_selftest_math(int64_t n, const double* in, double* rcp, double* rsqr
  * kernels build the ground-truth rotation with (csrc/pnpb200_math.cuh, sincos_bounded).
  */
 int pnpb200_selftest_sincos(int64_t n, const double* in, double* sin_out, double* cos_out, void* stream);
+
+/*
+ * Test hook: the P3P solver of the hypothesis stage (csrc/pnpb200_p3p.cuh), on m device triples: pattern points X [m,3,3]
+ * (metres) and unit bearings f [m,3,3].  R [m,4,9], t [m,4,3]: the valid roots first, NaN after; n_sol [m]: their number.
+ */
+int pnpb200_selftest_p3p(int64_t m, const double* X, const double* f, double* R, double* t, int32_t* n_sol, void* stream);
 
 #ifdef __cplusplus
 }

@@ -23,7 +23,7 @@ _LAZY = {
     "check_batch": (".solver", "check_batch"), "CHECK_NONFINITE": ("._lib", "CHECK_NONFINITE"),
     "CHECK_DEPTH": ("._lib", "CHECK_DEPTH"), "CHECK_BEHIND": ("._lib", "CHECK_BEHIND"), "CHECK_REPROJ": ("._lib", "CHECK_REPROJ"),
     "solve_robust_batch": (".solver", "solve_robust_batch"), "ROBUST_TOO_FEW": ("._lib", "ROBUST_TOO_FEW"),
-    "ROBUST_NOT_CONVERGED": ("._lib", "ROBUST_NOT_CONVERGED"),
+    "ROBUST_NOT_CONVERGED": ("._lib", "ROBUST_NOT_CONVERGED"), "hypothesize_batch": (".solver", "hypothesize_batch"),
 }
 
 

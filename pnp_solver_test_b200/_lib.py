@@ -39,6 +39,8 @@ EXPORTS = [
     "pnpb200_solve_batch_masked", "pnpb200_solve_report_batch_masked", "pnpb200_report_batch_strided_masked",
     "pnpb200_check_batch_masked", "pnpb200_workspace_bytes_masked", "pnpb200_solve_batch_host_masked",
     "pnpb200_default_robust_params", "pnpb200_robust_workspace_bytes", "pnpb200_solve_robust_batch",
+    "pnpb200_default_hypothesis_params", "pnpb200_hypothesize_batch", "pnpb200_ransac_workspace_bytes", "pnpb200_solve_ransac_batch",
+    "pnpb200_selftest_p3p",
 ]
 
 
@@ -54,6 +56,12 @@ class Params(C.Structure):
 class RobustParams(C.Structure):
     """struct pnpb200_robust_params"""
     _fields_ = [("max_rounds", C.c_int32), ("k_median", C.c_double), ("floor_px", C.c_double), ("min_inliers", C.c_int32)]
+
+
+class HypothesisParams(C.Structure):
+    """struct pnpb200_hypothesis_params"""
+    _fields_ = [("max_samples", C.c_int32), ("consensus_px", C.c_double), ("confidence", C.c_double), ("seed", C.c_uint64),
+                ("idx0", C.c_int64)]
 
 
 class Synth(C.Structure):
@@ -106,6 +114,13 @@ lib.pnpb200_robust_workspace_bytes.argtypes = [C.c_int, C.c_int, C.c_int64, C.c_
 # pnpb200_solve_batch_masked's arguments, then the robust parameters and the three outputs
 lib.pnpb200_solve_robust_batch.argtypes = [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, _VP, _VP, C.c_int, _PI, _PD, _VP,
                                            _VP, _VP, _VP, _VP, _PI, _PI, _U32P, _VP, _U32P, _PI, _PI, _VP]
+# the hypothesis stage and the RANSAC solve: the robust entry's arguments, then the hypothesis parameters, consensus and drawn
+lib.pnpb200_hypothesize_batch.argtypes = [C.c_int, C.c_int64, C.c_int, C.c_int, _VP, _VP, C.c_int, _PI, _PD, _U32P, _VP, _VP, _VP,
+                                          _PI, _U32P, _PI, _PI, _VP]
+lib.pnpb200_ransac_workspace_bytes.restype = C.c_int64
+lib.pnpb200_ransac_workspace_bytes.argtypes = [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int]
+lib.pnpb200_solve_ransac_batch.argtypes = lib.pnpb200_solve_robust_batch.argtypes[:-1] + [_VP, _PI, _PI, _VP]
+lib.pnpb200_selftest_p3p.argtypes = [C.c_int64, _VP, _VP, _VP, _VP, _VP, _VP]
 
 _ERR = {-1: "EINVAL (bad argument)", -2: "ECUDA (CUDA runtime error)", -3: "ENODEVICE (no usable CUDA device)",
         -4: "ETOOLARGE (n too large for the selected mapping)"}

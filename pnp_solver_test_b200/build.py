@@ -15,10 +15,10 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 OBJ = os.path.join(CSRC, "_obj")
 LIB_PATH = os.path.join(_HERE, "libpnpb200.so")
-HEADERS = ["pnpb200_common.cuh", "pnpb200_math.cuh", "pnpb200_reproject.cuh", "pnpb200_solvers.cuh", "pnpb200_tile.cuh",
+HEADERS = ["pnpb200_common.cuh", "pnpb200_math.cuh", "pnpb200_p3p.cuh", "pnpb200_reproject.cuh", "pnpb200_solvers.cuh", "pnpb200_tile.cuh",
            os.path.join("..", "..", "include", "pnpb200.h")]
 # (object name, source, extra defines)
-UNITS = [("api", "pnpb200_api.cu", []), ("aux", "pnpb200_aux.cu", []), ("robust", "pnpb200_robust.cu", []), ("analysis", "pnpb200_analysis.cu", []),
+UNITS = [("api", "pnpb200_api.cu", []), ("aux", "pnpb200_aux.cu", []), ("robust", "pnpb200_robust.cu", []), ("ransac", "pnpb200_ransac.cu", []), ("analysis", "pnpb200_analysis.cu", []),
          ("writers", "pnpb200_writers.cpp", []), ("pack", "pnpb200_pack.cpp", [])]
 UNITS += [("kernels_%s_g%d" % ("f64" if f64 else "f32", g), "pnpb200_kernels.cu", ["-DPNP_F64=%d" % f64, "-DPNP_GROUP=%d" % g])
           for f64 in (1, 0) for g in (3, 1, 0, 2)]

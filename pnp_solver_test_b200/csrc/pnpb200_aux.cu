@@ -106,21 +106,8 @@ __global__ void k_project(long long B, int n, const void* pattern, KMat K, const
 // ------------------------------------------------------------------------------------------
 // synthetic workload  (random_stress_test.py:246-290, LM_noise_test.py noise model)
 // Philox4x32-10 keyed by seed, counter = (global problem index, stream id).  Bit-identical to
-// the integer part of oracle/pnp_oracle.c; the trigonometry may differ in the last ulp.
+// the integer part of oracle/pnp_oracle.c; the trigonometry may differ in the last ulp.  (philox4x32_10: pnpb200_math.cuh)
 // ------------------------------------------------------------------------------------------
-PNP_DEV void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1, uint32_t (&out)[4])
-{
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-        const uint32_t n0 = hi1 ^ c1 ^ k0, n1 = lo1, n2 = hi0 ^ c3 ^ k1, n3 = lo0;
-        c0 = n0; c1 = n1; c2 = n2; c3 = n3;
-        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-    }
-    out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
-}
-
 PNP_DEV double u01(uint32_t hi, uint32_t lo)
 {
     const unsigned long long v = (((unsigned long long)hi << 32) | lo) >> 11;

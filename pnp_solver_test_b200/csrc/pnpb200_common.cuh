@@ -77,6 +77,13 @@ int check_launch(int dtype, int64_t B, int n, const void* pattern, int n_pattern
 int solve_batch_impl(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern, int n_patterns,
                      const int32_t* point_index, const double* K, const pnpb200_params& prm, void* R, void* t, void* euler_deg,
                      void* res_norm, int32_t* iters, int32_t* best_pattern, cudaStream_t st, const uint32_t* vis = nullptr);
+// the hypothesis stage (pnpb200_hypothesize_batch) with its parameters given, and their checks; pnpb200_ransac.cu
+bool hypothesis_params_ok(const pnpb200_hypothesis_params& h);
+void fill_default_hypothesis(pnpb200_hypothesis_params* h);
+int hypothesize_impl(int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern, int n_patterns,
+                     const int32_t* point_index, const double* K, const uint32_t* visible, const pnpb200_hypothesis_params& hp,
+                     void* R, void* t, int32_t* best_pattern, uint32_t* consensus_mask, int32_t* consensus, int32_t* drawn,
+                     cudaStream_t st);
 cudaError_t set_dynamic_smem(const void* kernel, size_t bytes);                                   // defined in pnpb200_api.cu
 cudaError_t blocks_per_sm(int* out, const void* kernel, int block_threads, size_t smem_bytes);   // defined in pnpb200_api.cu
 

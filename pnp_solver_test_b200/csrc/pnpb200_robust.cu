@@ -264,6 +264,16 @@ __global__ void __launch_bounds__(256) k_robust_init(long long B, int W, const u
     status[b] = 0;
 }
 
+// the RANSAC solve's M0: the hypothesis stage's consensus set where it holds at least min_inliers landmarks (else C, as set
+// by k_robust_init)
+__global__ void __launch_bounds__(256) k_ransac_seed(long long B, int W, int min_inliers, const int32_t* __restrict__ consensus,
+                                                     const uint32_t* __restrict__ cmask, uint32_t* inliers)
+{
+    const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B || consensus[b] < min_inliers) return;
+    for (int w = 0; w < W; ++w) inliers[b * W + w] = cmask[b * W + w];
+}
+
 // compact entry k <- problem idx[k]: its pixel row and its mask (16-byte rows; the mask as words)
 template <typename T>
 __global__ void __launch_bounds__(256) k_robust_gather(long long m, int n_total, const int32_t* __restrict__ idx, const T* __restrict__ uv,
@@ -337,12 +347,13 @@ unsigned blocks_for(long long n) { return (unsigned)((n + 255) / 256 < 1 ? 1 : (
 
 size_t up256(size_t x) { return (x + 255) & ~(size_t)255; }
 
-// the robust scratch behind the masked solve's: index lists, flags, count, cub's storage, the compacted batch
+// the robust scratch behind the masked solve's: index lists, flags, count, cub's storage, the compacted batch; for the
+// RANSAC solve (ransac) then the hypothesis stage's pose, pattern, consensus mask and sample count
 struct RobustLayout {
-    size_t solve, idx_a, idx_b, flag, count, sel, cub, cub_bytes, uv, mask, R, t, e, res, it, best, total;
+    size_t solve, idx_a, idx_b, flag, count, sel, cub, cub_bytes, uv, mask, R, t, e, res, it, best, hR, ht, hbest, hmask, hdrawn, total;
 };
 
-RobustLayout robust_layout(int method, int dtype, int64_t B, int n_total, int n_patterns, int mapping)
+RobustLayout robust_layout(int method, int dtype, int64_t B, int n_total, int n_patterns, int mapping, bool ransac = false)
 {
     RobustLayout L;
     const size_t esz = (dtype == PNPB200_DTYPE_F32) ? 4 : 8, b = (size_t)B, W = ((size_t)n_total + 31) / 32;
@@ -365,6 +376,15 @@ RobustLayout robust_layout(int method, int dtype, int64_t B, int n_total, int n_
     L.res = o; o += up256(esz * b);
     L.it = o; o += up256(4 * b);
     L.best = o; o += up256(4 * b);
+    if (ransac) {
+        L.hR = o; o += up256(esz * 9 * b);
+        L.ht = o; o += up256(esz * 3 * b);
+        L.hbest = o; o += up256(4 * b);
+        L.hmask = o; o += up256(4 * W * b);
+        L.hdrawn = o; o += up256(4 * b);
+    } else {
+        L.hR = L.ht = L.hbest = L.hmask = L.hdrawn = o;
+    }
     L.total = o;
     return L;
 }
@@ -405,35 +425,18 @@ void launch_scatter(long long m, const int32_t* idx, void* const* c, void* const
     count_kernel_launches(1);
 }
 
-}  // namespace
-}  // namespace pnpb200
-
-using namespace pnpb200;
-
-extern "C" {
-
-int pnpb200_default_robust_params(pnpb200_robust_params* p)
-{
-    if (!p) return PNPB200_EINVAL;
-    fill_default_robust(p);
-    return PNPB200_OK;
-}
-
-int64_t pnpb200_robust_workspace_bytes(int method, int dtype, int64_t B, int n_total, int n_patterns, int mapping)
-{
-    if (B <= 0 || B > 0x7fffffffLL || n_total < 1) return 0;
-    return (int64_t)robust_layout(method, dtype, B, n_total, n_patterns, mapping).total;
-}
-
-int pnpb200_solve_robust_batch(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
-                               int n_patterns, const int32_t* point_index, const double* K, const pnpb200_params* params,
-                               void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters, int32_t* best_pattern,
-                               const uint32_t* visible, const pnpb200_robust_params* robust, uint32_t* inliers, int32_t* rounds,
-                               int32_t* robust_status, void* stream)
+// The loop of the robust entry.  hp = NULL: the robust solve, from M0 = C.  Otherwise the RANSAC solve: the hypothesis stage
+// first, and M0 = its consensus set where that holds at least min_inliers landmarks.
+int robust_run(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern, int n_patterns,
+               const int32_t* point_index, const double* K, const pnpb200_params* params, void* R, void* t, void* euler_deg,
+               void* res_norm, int32_t* iters, int32_t* best_pattern, const uint32_t* visible, const pnpb200_robust_params* robust,
+               uint32_t* inliers, int32_t* rounds, int32_t* robust_status, const pnpb200_hypothesis_params* hp, int32_t* consensus,
+               int32_t* drawn, cudaStream_t st)
 {
     pnpb200_robust_params rp;
     if (robust) rp = *robust; else fill_default_robust(&rp);
     if (!robust_params_ok(rp)) return PNPB200_EINVAL;
+    if (hp && (!hypothesis_params_ok(*hp) || !consensus)) return PNPB200_EINVAL;
     if (B < 0 || n_total < 1 || n < 1 || (!point_index && n != n_total) || !uv || !pattern || !K) return PNPB200_EINVAL;
     if (!R || !t || !inliers || !rounds || !robust_status || (n_patterns > 1 && !best_pattern)) return PNPB200_EINVAL;
     if (n_patterns < 1 || n_patterns > PNPB200_MAX_PATTERNS) return PNPB200_EINVAL;
@@ -448,11 +451,10 @@ int pnpb200_solve_robust_batch(int method, int dtype, int64_t B, int n_total, in
         sel[(size_t)(j >> 5)] |= 1u << (j & 31);
     }
     if (B == 0) return PNPB200_OK;
-    cudaStream_t st = (cudaStream_t)stream;
     pnpb200_params prm;
     if (params) prm = *params; else fill_default_params(&prm);
     prm.flags &= ~PNP_FLAG_INTERNAL_NO_RESIDUAL;
-    const RobustLayout L = robust_layout(method, dtype, B, n_total, n_patterns, prm.mapping);
+    const RobustLayout L = robust_layout(method, dtype, B, n_total, n_patterns, prm.mapping, hp != nullptr);
     char* ws = nullptr;
     const bool own_ws = !(prm.workspace && prm.workspace_bytes >= (int64_t)L.total);
     if (own_ws) PNP_CUDA_OK(cudaMallocAsync((void**)&ws, L.total, st));
@@ -473,10 +475,21 @@ int pnpb200_solve_robust_batch(int method, int dtype, int64_t B, int n_total, in
     if (!h_count) return PNPB200_ECUDA;
 
     PNP_CUDA_OK(cudaMemcpyAsync(d_sel, sel.data(), sizeof(uint32_t) * (size_t)W, cudaMemcpyHostToDevice, st));
+    int rc;
+    if (hp) {
+        rc = hypothesize_impl(dtype, B, n_total, n, uv, pattern, n_patterns, point_index, K, visible, *hp, ws + L.hR, ws + L.ht,
+                              (int32_t*)(ws + L.hbest), (uint32_t*)(ws + L.hmask), consensus, drawn ? drawn : (int32_t*)(ws + L.hdrawn), st);
+        if (rc != PNPB200_OK) return rc;
+    }
     k_robust_init<<<blocks_for(B), 256, 0, st>>>(B, W, d_sel, visible, inliers, idx_cur, rounds, robust_status);
     count_kernel_launches(1);
     PNP_CUDA_OK(cudaGetLastError());
-    int rc = solve_batch_impl(method, dtype, B, n_total, n, uv, pattern, n_patterns, point_index, K, prm, R, t, euler_deg, res_norm,
+    if (hp) {
+        k_ransac_seed<<<blocks_for(B), 256, 0, st>>>(B, W, rp.min_inliers, consensus, (const uint32_t*)(ws + L.hmask), inliers);
+        count_kernel_launches(1);
+        PNP_CUDA_OK(cudaGetLastError());
+    }
+    rc = solve_batch_impl(method, dtype, B, n_total, n, uv, pattern, n_patterns, point_index, K, prm, R, t, euler_deg, res_norm,
                               iters, best_pattern, st, inliers);
     if (rc != PNPB200_OK) return rc;
     // the batch the next classification reads: the whole call first, then each round's compacted problems
@@ -522,6 +535,55 @@ int pnpb200_solve_robust_batch(int method, int dtype, int64_t B, int n_total, in
         int32_t* sw = idx_cur; idx_cur = idx_next; idx_next = sw;
     }
     return PNPB200_OK;
+}
+
+}  // namespace
+}  // namespace pnpb200
+
+using namespace pnpb200;
+
+extern "C" {
+
+int pnpb200_default_robust_params(pnpb200_robust_params* p)
+{
+    if (!p) return PNPB200_EINVAL;
+    fill_default_robust(p);
+    return PNPB200_OK;
+}
+
+int64_t pnpb200_robust_workspace_bytes(int method, int dtype, int64_t B, int n_total, int n_patterns, int mapping)
+{
+    if (B <= 0 || B > 0x7fffffffLL || n_total < 1) return 0;
+    return (int64_t)robust_layout(method, dtype, B, n_total, n_patterns, mapping).total;
+}
+
+int64_t pnpb200_ransac_workspace_bytes(int method, int dtype, int64_t B, int n_total, int n_patterns, int mapping)
+{
+    if (B <= 0 || B > 0x7fffffffLL || n_total < 1) return 0;
+    return (int64_t)robust_layout(method, dtype, B, n_total, n_patterns, mapping, true).total;
+}
+
+int pnpb200_solve_robust_batch(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
+                               int n_patterns, const int32_t* point_index, const double* K, const pnpb200_params* params,
+                               void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters, int32_t* best_pattern,
+                               const uint32_t* visible, const pnpb200_robust_params* robust, uint32_t* inliers, int32_t* rounds,
+                               int32_t* robust_status, void* stream)
+{
+    return robust_run(method, dtype, B, n_total, n, uv, pattern, n_patterns, point_index, K, params, R, t, euler_deg, res_norm, iters,
+                      best_pattern, visible, robust, inliers, rounds, robust_status, nullptr, nullptr, nullptr, (cudaStream_t)stream);
+}
+
+int pnpb200_solve_ransac_batch(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
+                               int n_patterns, const int32_t* point_index, const double* K, const pnpb200_params* params,
+                               void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters, int32_t* best_pattern,
+                               const uint32_t* visible, const pnpb200_robust_params* robust, uint32_t* inliers, int32_t* rounds,
+                               int32_t* robust_status, const pnpb200_hypothesis_params* hyp, int32_t* consensus, int32_t* drawn,
+                               void* stream)
+{
+    pnpb200_hypothesis_params hp;
+    if (hyp) hp = *hyp; else fill_default_hypothesis(&hp);
+    return robust_run(method, dtype, B, n_total, n, uv, pattern, n_patterns, point_index, K, params, R, t, euler_deg, res_norm, iters,
+                      best_pattern, visible, robust, inliers, rounds, robust_status, &hp, consensus, drawn, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -183,6 +183,55 @@ def robust_params(max_rounds=4, k=3.0, floor_px=2.0, min_inliers=6):
     return _lib.RobustParams(max_rounds=max_rounds, k_median=k, floor_px=floor_px, min_inliers=min_inliers)
 
 
+def hypothesis_params(samples=128, consensus_px=4.0, confidence=0.999, seed=0, idx0=0):
+    """struct pnpb200_hypothesis_params; ValueError for what pnpb200_hypothesize_batch refuses with EINVAL"""
+    samples, consensus_px, confidence, seed, idx0 = int(samples), float(consensus_px), float(confidence), int(seed), int(idx0)
+    if samples < 0:
+        raise ValueError("samples must be >= 0, not %d" % samples)
+    if not consensus_px >= 0.0:
+        raise ValueError("consensus_px must be >= 0 (inf allowed), not %r" % consensus_px)
+    if not 0.0 < confidence <= 1.0:
+        raise ValueError("confidence must lie in (0, 1], not %r" % confidence)
+    if not 0 <= seed < 1 << 64:
+        raise ValueError("seed must be a 64-bit unsigned integer, not %d" % seed)
+    if idx0 < 0:
+        raise ValueError("idx0 must be >= 0, not %d" % idx0)
+    return _lib.HypothesisParams(max_samples=samples, consensus_px=consensus_px, confidence=confidence, seed=seed, idx0=idx0)
+
+
+def hypothesize_batch(uv, patterns, K, point_index=None, visible=None, samples=128, consensus_px=4.0, confidence=0.999, seed=0, idx0=0):
+    """pnpb200_hypothesize_batch on device tensors: per problem, minimal samples of 4 candidates (the landmarks of point_index
+    that are visible), a P3P pose per sample and pattern tested on the 4th landmark, and the largest consensus set under the
+    check's reprojection distance (<= consensus_px).  Returns dict(R [B,3,3], t [B,3] (the winner's pose; NaN where no sample
+    survived), best_pattern [B] int32, consensus_mask bool [B, n_total], consensus [B] int32 (its size), drawn [B] int32 (the
+    samples taken)).  The rule is in include/pnpb200.h; idx0 = the global index of problem 0 (shards draw what the unsharded
+    call draws)."""
+    hp = hypothesis_params(samples, consensus_px, confidence, seed, idx0)
+    _, dt, uv, patterns, B, n_total, idx = _batch_args(0, uv, patterns, point_index, visible)
+    n, idx_p = (n_total, None) if idx is None else (int(idx.shape[0]), idx.ctypes.data_as(C.POINTER(C.c_int32)))
+    dev = uv.device
+    P = int(patterns.shape[0])
+    o = dict(R=torch.empty((B, 3, 3), dtype=uv.dtype, device=dev), t=torch.empty((B, 3), dtype=uv.dtype, device=dev),
+             best_pattern=torch.empty((B,), dtype=torch.int32, device=dev), consensus=torch.empty((B,), dtype=torch.int32, device=dev),
+             drawn=torch.empty((B,), dtype=torch.int32, device=dev))
+    words = torch.empty((B, (n_total + 31) // 32), dtype=torch.int32, device=dev)
+    if B == 0:
+        o["consensus_mask"] = torch.empty((0, n_total), dtype=torch.bool, device=dev)
+        return o
+    Kh, Kp = _k_host(K)
+    vw = None if visible is None else visible_words(visible, dev)
+    PI = C.POINTER(C.c_int32)
+    with torch.cuda.device(dev):
+        rc = lib.pnpb200_hypothesize_batch(
+            dt, B, n_total, n, ptr(uv), ptr(patterns), P, idx_p, Kp, None if vw is None else _u32(vw), C.byref(hp), ptr(o["R"]),
+            ptr(o["t"]), C.cast(ptr(o["best_pattern"]), PI), _u32(words), C.cast(ptr(o["consensus"]), PI),
+            C.cast(ptr(o["drawn"]), PI), _stream_ptr(dev))
+    check(rc, "pnpb200_hypothesize_batch")
+    _lib.count_launch(1)
+    o["consensus_mask"] = unpack_words(words, n_total)
+    return o
+
+
 def unpack_words(words, n_total):
     """the inverse of visible_words: [B, W] int32 words -> bool [B, n_total] on the words' device"""
     B, W = int(words.shape[0]), int(words.shape[1])
@@ -192,15 +241,19 @@ def unpack_words(words, n_total):
 
 
 def solve_robust_batch(method, uv, patterns, K, point_index=None, params=None, visible=None, max_rounds=4, k=3.0, floor_px=2.0,
-                       min_inliers=6):
+                       min_inliers=6, samples=None, consensus_px=4.0, confidence=0.999, seed=0, idx0=0):
     """pnpb200_solve_robust_batch on device tensors: each problem is solved on its candidates (the landmarks of point_index
     that are visible), the landmarks whose reprojection distance exceeds max(floor_px, k * median) are dropped, and the
     problem is solved again on the rest, until the inlier set stops changing or after max_rounds solves.  Returns the dict of
     solve_batch plus inliers (bool [B, n_total]: the landmarks the returned pose was solved on), rounds [B] int32 (solves)
     and robust_status [B] int32 (ROBUST_TOO_FEW, ROBUST_NOT_CONVERGED bits; 0 = converged).  Every output of a problem is
     bit for bit that of solve_batch(..., visible=inliers).  The rule, its defaults and what it rescues are in
-    include/pnpb200.h.  The call synchronises the stream once per round."""
+    include/pnpb200.h.  The call synchronises the stream once per round.
+    samples: None -> the loop starts from all candidates (pnpb200_solve_robust_batch).  An int >= 0 -> pnpb200_solve_ransac_batch:
+    the hypothesis stage of hypothesize_batch (samples, consensus_px, confidence, seed, idx0) runs first and the loop starts
+    from its consensus set where that holds at least min_inliers landmarks; the dict then also holds consensus and drawn."""
     rp = robust_params(max_rounds, k, floor_px, min_inliers)
+    hp = None if samples is None else hypothesis_params(samples, consensus_px, confidence, seed, idx0)
     m, dt, uv, patterns, B, n_total, idx = _batch_args(method, uv, patterns, point_index, visible)
     n, idx_p = (n_total, None) if idx is None else (int(idx.shape[0]), idx.ctypes.data_as(C.POINTER(C.c_int32)))
     dev = uv.device
@@ -211,12 +264,16 @@ def solve_robust_batch(method, uv, patterns, K, point_index=None, params=None, v
     words = torch.empty((B, (n_total + 31) // 32), dtype=torch.int32, device=dev)
     o["rounds"] = torch.empty((B,), dtype=torch.int32, device=dev)
     o["robust_status"] = torch.empty((B,), dtype=torch.int32, device=dev)
+    if hp is not None:
+        o["consensus"] = torch.empty((B,), dtype=torch.int32, device=dev)
+        o["drawn"] = torch.empty((B,), dtype=torch.int32, device=dev)
     if B == 0:
         o["inliers"] = torch.empty((0, n_total), dtype=torch.bool, device=dev)
         return o
     Kh, Kp = _k_host(K)
     prm = _lib.default_params() if params is None else params
-    ws_bytes = int(lib.pnpb200_robust_workspace_bytes(m, dt, B, n_total, P, int(prm.mapping)))
+    ws_query = lib.pnpb200_robust_workspace_bytes if hp is None else lib.pnpb200_ransac_workspace_bytes
+    ws_bytes = int(ws_query(m, dt, B, n_total, P, int(prm.mapping)))
     ws = None
     if ws_bytes > 0 and not prm.workspace:
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
@@ -224,12 +281,16 @@ def solve_robust_batch(method, uv, patterns, K, point_index=None, params=None, v
         prm.workspace, prm.workspace_bytes = ws.data_ptr(), ws_bytes
     vw = None if visible is None else visible_words(visible, dev)
     PI = C.POINTER(C.c_int32)
-    with torch.cuda.device(dev):
-        rc = lib.pnpb200_solve_robust_batch(
-            m, dt, B, n_total, n, ptr(uv), ptr(patterns), P, idx_p, Kp, C.byref(prm), ptr(o["R"]), ptr(o["t"]), ptr(o["euler"]),
+    args = (m, dt, B, n_total, n, ptr(uv), ptr(patterns), P, idx_p, Kp, C.byref(prm), ptr(o["R"]), ptr(o["t"]), ptr(o["euler"]),
             ptr(o["res_norm"]), C.cast(ptr(o["iters"]), PI), C.cast(ptr(o["best_pattern"]), PI), None if vw is None else _u32(vw),
-            C.byref(rp), _u32(words), C.cast(ptr(o["rounds"]), PI), C.cast(ptr(o["robust_status"]), PI), _stream_ptr(dev))
-    check(rc, "pnpb200_solve_robust_batch")
+            C.byref(rp), _u32(words), C.cast(ptr(o["rounds"]), PI), C.cast(ptr(o["robust_status"]), PI))
+    with torch.cuda.device(dev):
+        if hp is None:
+            rc, name = lib.pnpb200_solve_robust_batch(*args, _stream_ptr(dev)), "pnpb200_solve_robust_batch"
+        else:
+            rc, name = lib.pnpb200_solve_ransac_batch(*args, C.byref(hp), C.cast(ptr(o["consensus"]), PI), C.cast(ptr(o["drawn"]), PI),
+                                                      _stream_ptr(dev)), "pnpb200_solve_ransac_batch"
+    check(rc, name)
     _lib.count_launch(1)
     o["inliers"] = unpack_words(words, n_total)
     return o
@@ -653,13 +714,19 @@ class PNP_SOLVER(object):
         and checked on its visible landmarks alone (of key_list, in its order); hidden pixels may hold anything, NaN too.
         robust: None, or a dict of any of max_rounds, k, floor_px, min_inliers -> solve_robust_batch: misplaced landmarks are
         rejected by their reprojection distance and each problem re-solved on its inliers; the dict then also holds inliers,
-        rounds and robust_status, and the check (if asked for) runs on the inliers."""
+        rounds and robust_status, and the check (if asked for) runs on the inliers.  With samples (and any of consensus_px,
+        confidence, seed, idx0) the loop starts from the hypothesis stage's consensus set (RANSAC), and the dict also holds
+        consensus and drawn."""
         method = method or self.method
         if robust is not None:
-            unknown = set(robust) - {"max_rounds", "k", "floor_px", "min_inliers"}
+            hyp_keys = {"samples", "consensus_px", "confidence", "seed", "idx0"}
+            unknown = set(robust) - {"max_rounds", "k", "floor_px", "min_inliers"} - hyp_keys
             if unknown:
-                raise ValueError("robust takes max_rounds, k, floor_px, min_inliers; not %s" % sorted(unknown))
-            robust_params(**robust)
+                raise ValueError("robust takes max_rounds, k, floor_px, min_inliers, samples, consensus_px, confidence, seed, idx0; "
+                                 "not %s" % sorted(unknown))
+            robust_params(**{k: v for k, v in robust.items() if k not in hyp_keys})
+            if robust.get("samples") is not None:
+                hypothesis_params(**{k: v for k, v in robust.items() if k in hyp_keys})
         all_keys = list(self.np_point_3d_pretransfer_dict_list[0].keys())
         if isinstance(key_list, str) and key_list == "default":
             key_list = self.LM_key_list if method == "qeif" else None
