@@ -447,7 +447,9 @@ int pnpb200_solve_batch_host_masked(pnpb200_pipeline* p, int method, int64_t B, 
  *  - Round 0 solves on M0 = C.  After the solve on M_r, d_i (i in C) is the check's prediction-vs-landmark distance of landmark
  *    i (pnpb200_check_batch: pose_r, pattern best_pattern_r, FP64, the same arithmetic); med = the lower median of {d_i}, the
  *    element of rank floor((|C| - 1) / 2) in ascending order with NaN last; tau = max(floor_px, k_median * med), floor_px
- *    where k_median * med is not finite; M_{r+1} = {i in C : d_i <= tau} (a NaN distance is an outlier).
+ *    where k_median * med is not finite; M_{r+1} = {i in C : d_i <= tau} (a NaN distance is an outlier).  d_i is never
+ *    infinite: where its square is not finite (depth exactly 0, a non-finite pixel, an overflow) it is NaN, so even
+ *    floor_px = +Inf drops such a landmark.
  *  - M_{r+1} = M_r: converged, the result is pose_r on M_r.  Else |M_{r+1}| < min_inliers: pose_r and M_r are kept with
  *    PNPB200_ROBUST_TOO_FEW.  Else, if r + 1 < max_rounds, the problem is solved on M_{r+1} and classified again; if
  *    r + 1 = max_rounds, pose_r and M_r are kept with PNPB200_ROBUST_NOT_CONVERGED.
@@ -703,6 +705,26 @@ int pnpb200_selftest_sincos(int64_t n, const double* in, double* sin_out, double
  * (metres) and unit bearings f [m,3,3].  R [m,4,9], t [m,4,3]: the valid roots first, NaN after; n_sol [m]: their number.
  */
 int pnpb200_selftest_p3p(int64_t m, const double* X, const double* f, double* R, double* t, int32_t* n_sol, void* stream);
+
+/*
+ * Test hook: one inlier classification pass of the robust loop (pnpb200_solve_robust_batch above: d_i over C, the lower median
+ * with NaN last, tau, M' and the decision) on poses the caller supplies, in one of its two kernel shapes.
+ *   dtype, B, n_total, n, uv, pattern, n_patterns, point_index, K, visible, robust: as in pnpb200_solve_robust_batch
+ *   R, t        [device] [B,3,3], [B,3] (dtype); best_pattern [device] [B] int32 or NULL (pattern 0)
+ *   idx         [device] [B] int32 or NULL (the identity): batch entry k reads row k of uv, R, t and best_pattern, and problem
+ *               idx[k]'s rows of visible, inliers, rounds and robust_status (the compacted batch of rounds >= 1)
+ *   last_round  nonzero: a mask that would change is kept with NOT_CONVERGED
+ *   inliers, rounds, robust_status [device], in / out: M and its problem's state, updated as the robust loop updates them
+ *   flag        [device] [B] uint8: 1 where batch entry k is to be solved again;  tau [device] [B] double or NULL: its threshold
+ *   shape       0 the kernel the robust loop picks, 1 the streaming kernel (PNPB200_EINVAL where it cannot run), 2 one warp
+ *               per problem (PNPB200_ETOOLARGE where its shared memory does not fit)
+ * Argument errors return PNPB200_EINVAL before any CUDA call.
+ */
+int pnpb200_selftest_inliers(int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern, int n_patterns,
+                             const int32_t* point_index, const double* K, const uint32_t* visible,
+                             const pnpb200_robust_params* robust, const void* R, const void* t, const int32_t* best_pattern,
+                             const int32_t* idx, int last_round, uint32_t* inliers, int32_t* rounds, int32_t* robust_status,
+                             uint8_t* flag, double* tau, int shape, void* stream);
 
 #ifdef __cplusplus
 }

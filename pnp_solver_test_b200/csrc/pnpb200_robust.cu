@@ -18,14 +18,15 @@ namespace {
 // lower median med of {d_i} (rank floor((|C| - 1) / 2), NaN last), tau = max(floor_px, k med) (floor_px where k med is not
 // finite) and M' = {i in C : d_i <= tau}.  M' = M (the mask the pose was solved on): converged; |M'| < min_inliers:
 // TOO_FEW, M kept; last round: NOT_CONVERGED, M kept; otherwise M' replaces M, the round count grows and the problem is
-// flagged for the next solve.  Batch entry k is problem idx[k] of the call (inliers, vis, rounds, status are indexed by it).
+// flagged for the next solve.  Batch entry k is problem idx[k] of the call (inliers, vis, rounds, status are indexed by it);
+// flag and tau (where non-null: the threshold of the entry) by k.
 // ------------------------------------------------------------------------------------------
 constexpr int kInlierUnroll = 4;                          // landmarks in flight per thread, as k_check_chunk
 template <typename T>
 struct InlierArgs {
     const T* pattern; const T* uv; const T* R; const T* t; const int32_t* best;
     const int32_t* idx; const uint32_t* sel; const uint32_t* vis;
-    uint32_t* inliers; int32_t* rounds; int32_t* status; uint8_t* flag;
+    uint32_t* inliers; int32_t* rounds; int32_t* status; uint8_t* flag; double* tau;
     long long B;
     int n, n_patterns, row_pitch, chunk, vis_words, last_round, min_inliers;
     double K[9], k_median, floor_px;
@@ -168,7 +169,10 @@ __global__ void __launch_bounds__(32) k_inlier_chunk(const __grid_constant__ Inl
                 sNw[(i >> 5) * kTileProblems + lane] |= 1u << (i & 31);
             }
         }
-        if (ok) a.flag[b] = decide_inliers(a, o, sNw + lane, kTileProblems);
+        if (ok) {
+            if (a.tau) a.tau[b] = tau;
+            a.flag[b] = decide_inliers(a, o, sNw + lane, kTileProblems);
+        }
         tile += gridDim.x;
         if (tile < n_tiles) {
             fence_proxy_async();
@@ -249,7 +253,10 @@ __global__ void __launch_bounds__(kInlierWarps * 32) k_inlier_warp(const __grid_
         if (lane == 0) sNw[w] = word;
     }
     __syncwarp();
-    if (lane == 0) a.flag[b] = decide_inliers(a, o, sNw, 1);
+    if (lane == 0) {
+        if (a.tau) a.tau[b] = tau;
+        a.flag[b] = decide_inliers(a, o, sNw, 1);
+    }
 }
 
 
@@ -313,9 +320,10 @@ __global__ void __launch_bounds__(256) k_robust_scatter(long long m, const int32
     if (best) best[o] = cbest[k];
 }
 
-// the execution shapes of the check (check_launch): k_inlier_chunk where the check streams, k_inlier_warp otherwise
+// the execution shapes of the check (check_launch): k_inlier_chunk where the check streams, k_inlier_warp otherwise.
+// shape (pnpb200_selftest_inliers): 0 that choice, 1 k_inlier_chunk (EINVAL where it cannot run), 2 k_inlier_warp.
 template <typename T>
-int inlier_launch(InlierArgs<T> a, cudaStream_t st)
+int inlier_launch(InlierArgs<T> a, cudaStream_t st, int shape)
 {
     if (a.B == 0) return PNPB200_OK;
     DeviceProps dp;
@@ -326,7 +334,9 @@ int inlier_launch(InlierArgs<T> a, cudaStream_t st)
     const size_t smem = (size_t)a.n * kTileProblems * (sizeof(unsigned long long) + sizeof(uint16_t)) + 2 * words + 128 +
                         2 * sg.buf_bytes + sizeof(T) * (size_t)a.n_patterns * a.n * 3 + 32;
     a.use_tmap = 0;
-    if (report_can_fuse(sizeof(T) == 8 ? PNPB200_DTYPE_F64 : PNPB200_DTYPE_F32, a.n) && smem <= (size_t)dp.max_smem_optin) {
+    const bool chunk = report_can_fuse(sizeof(T) == 8 ? PNPB200_DTYPE_F64 : PNPB200_DTYPE_F32, a.n) && smem <= (size_t)dp.max_smem_optin;
+    if (shape == 1 && !chunk) return PNPB200_EINVAL;
+    if (chunk && shape != 2) {
         a.row_pitch = sg.pitch; a.chunk = sg.chunk;
         a.use_tmap = (sg.pitch == sg.chunk * 2) ? make_row_tensor_map(&a.tmap, a.uv, (int)sizeof(T), a.B, a.n, sg.chunk) : 0;
         PNP_CUDA_OK(set_dynamic_smem((const void*)k_inlier_chunk<T>, smem));
@@ -389,6 +399,18 @@ RobustLayout robust_layout(int method, int dtype, int64_t B, int n_total, int n_
     return L;
 }
 
+// the candidate words of point_index (all n_total landmarks where NULL); false for an index outside [0, n_total)
+bool candidate_words(int n, int n_total, const int32_t* point_index, std::vector<uint32_t>& sel)
+{
+    sel.assign((size_t)(n_total + 31) / 32, 0u);
+    for (int i = 0; i < n; ++i) {
+        const int j = point_index ? point_index[i] : i;
+        if (j < 0 || j >= n_total) return false;
+        sel[(size_t)(j >> 5)] |= 1u << (j & 31);
+    }
+    return true;
+}
+
 bool robust_params_ok(const pnpb200_robust_params& r)
 {
     return r.max_rounds >= 1 && r.min_inliers >= 4 && r.k_median >= 0.0 && r.k_median - r.k_median == 0.0 && r.floor_px >= 0.0;
@@ -444,12 +466,8 @@ int robust_run(int method, int dtype, int64_t B, int n_total, int n, const void*
     if ((visible && !vis_aligned(visible)) || !vis_aligned(inliers) || ((uintptr_t)uv & 15u)) return PNPB200_EINVAL;
     if (B > 0x7fffffffLL) return PNPB200_ETOOLARGE;       // int32 problem indices in the selection
     const int W = (n_total + 31) / 32;
-    std::vector<uint32_t> sel((size_t)W, 0u);
-    for (int i = 0; i < n; ++i) {
-        const int j = point_index ? point_index[i] : i;
-        if (j < 0 || j >= n_total) return PNPB200_EINVAL;
-        sel[(size_t)(j >> 5)] |= 1u << (j & 31);
-    }
+    std::vector<uint32_t> sel;
+    if (!candidate_words(n, n_total, point_index, sel)) return PNPB200_EINVAL;
     if (B == 0) return PNPB200_OK;
     pnpb200_params prm;
     if (params) prm = *params; else fill_default_params(&prm);
@@ -499,7 +517,7 @@ int robust_run(int method, int dtype, int64_t B, int n_total, int n, const void*
     ad.pattern = (const double*)pattern; af.pattern = (const float*)pattern;
     ad.idx = af.idx = idx_cur;
     ad.sel = af.sel = d_sel; ad.vis = af.vis = visible; ad.inliers = af.inliers = inliers; ad.rounds = af.rounds = rounds;
-    ad.status = af.status = robust_status; ad.flag = af.flag = flag; ad.B = af.B = B; ad.n = af.n = n_total;
+    ad.status = af.status = robust_status; ad.flag = af.flag = flag; ad.tau = af.tau = nullptr; ad.B = af.B = B; ad.n = af.n = n_total;
     ad.n_patterns = af.n_patterns = n_patterns; ad.vis_words = af.vis_words = W; ad.min_inliers = af.min_inliers = rp.min_inliers;
     for (int e = 0; e < 9; ++e) ad.K[e] = af.K[e] = K[e];
     ad.k_median = af.k_median = rp.k_median; ad.floor_px = af.floor_px = rp.floor_px;
@@ -510,7 +528,7 @@ int robust_run(int method, int dtype, int64_t B, int n_total, int n, const void*
         af.uv = (const float*)b_uv; af.R = (const float*)b_R; af.t = (const float*)b_t;
         ad.best = af.best = b_best;
         ad.last_round = af.last_round = (r + 1 >= rp.max_rounds) ? 1 : 0;
-        rc = f64 ? inlier_launch<double>(ad, st) : inlier_launch<float>(af, st);
+        rc = f64 ? inlier_launch<double>(ad, st, 0) : inlier_launch<float>(af, st, 0);
         if (rc != PNPB200_OK) return rc;
         if (ad.last_round) break;
         size_t cub_bytes = L.cub_bytes;
@@ -535,6 +553,23 @@ int robust_run(int method, int dtype, int64_t B, int n_total, int n, const void*
         int32_t* sw = idx_cur; idx_cur = idx_next; idx_next = sw;
     }
     return PNPB200_OK;
+}
+
+// one classification pass of the robust loop over the caller's poses (pnpb200_selftest_inliers)
+template <typename T>
+int inlier_pass(int64_t B, int n_total, const void* uv, const void* pattern, int n_patterns, const double* K, const uint32_t* visible,
+                const pnpb200_robust_params& rp, const void* R, const void* t, const int32_t* best, const int32_t* idx,
+                const uint32_t* sel, int last_round, uint32_t* inliers, int32_t* rounds, int32_t* status, uint8_t* flag, double* tau,
+                int shape, cudaStream_t st)
+{
+    InlierArgs<T> a;
+    a.pattern = (const T*)pattern; a.uv = (const T*)uv; a.R = (const T*)R; a.t = (const T*)t; a.best = best;
+    a.idx = idx; a.sel = sel; a.vis = visible; a.inliers = inliers; a.rounds = rounds; a.status = status; a.flag = flag; a.tau = tau;
+    a.B = B; a.n = n_total; a.n_patterns = n_patterns; a.vis_words = (n_total + 31) / 32;
+    a.last_round = last_round ? 1 : 0; a.min_inliers = rp.min_inliers;
+    for (int e = 0; e < 9; ++e) a.K[e] = K[e];
+    a.k_median = rp.k_median; a.floor_px = rp.floor_px;
+    return inlier_launch<T>(a, st, shape);
 }
 
 }  // namespace
@@ -584,6 +619,43 @@ int pnpb200_solve_ransac_batch(int method, int dtype, int64_t B, int n_total, in
     if (hyp) hp = *hyp; else fill_default_hypothesis(&hp);
     return robust_run(method, dtype, B, n_total, n, uv, pattern, n_patterns, point_index, K, params, R, t, euler_deg, res_norm, iters,
                       best_pattern, visible, robust, inliers, rounds, robust_status, &hp, consensus, drawn, (cudaStream_t)stream);
+}
+
+int pnpb200_selftest_inliers(int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern, int n_patterns,
+                             const int32_t* point_index, const double* K, const uint32_t* visible,
+                             const pnpb200_robust_params* robust, const void* R, const void* t, const int32_t* best_pattern,
+                             const int32_t* idx, int last_round, uint32_t* inliers, int32_t* rounds, int32_t* robust_status,
+                             uint8_t* flag, double* tau, int shape, void* stream)
+{
+    pnpb200_robust_params rp;
+    if (robust) rp = *robust; else fill_default_robust(&rp);
+    if (!robust_params_ok(rp) || shape < 0 || shape > 2) return PNPB200_EINVAL;
+    if (dtype != PNPB200_DTYPE_F64 && dtype != PNPB200_DTYPE_F32) return PNPB200_EINVAL;
+    if (B < 0 || n_total < 1 || n < 1 || (!point_index && n != n_total) || !uv || !pattern || !K || !R || !t) return PNPB200_EINVAL;
+    if (!inliers || !rounds || !robust_status || !flag || n_patterns < 1 || n_patterns > PNPB200_MAX_PATTERNS) return PNPB200_EINVAL;
+    if ((visible && !vis_aligned(visible)) || !vis_aligned(inliers) || ((uintptr_t)uv & 15u)) return PNPB200_EINVAL;
+    if (B > 0x7fffffffLL) return PNPB200_ETOOLARGE;
+    std::vector<uint32_t> sel;
+    if (!candidate_words(n, n_total, point_index, sel)) return PNPB200_EINVAL;
+    if (B == 0) return PNPB200_OK;
+    const cudaStream_t st = (cudaStream_t)stream;
+    const size_t W = sel.size(), sel_bytes = up256(4 * W);
+    char* buf = nullptr;
+    PNP_CUDA_OK(cudaMallocAsync((void**)&buf, sel_bytes + (idx ? 0 : 4 * (size_t)B), st));
+    struct Guard { void* p; cudaStream_t st; ~Guard() { cudaFreeAsync(p, st); } } guard = { buf, st };
+    uint32_t* d_sel = (uint32_t*)buf;
+    PNP_CUDA_OK(cudaMemcpyAsync(d_sel, sel.data(), 4 * W, cudaMemcpyHostToDevice, st));
+    if (!idx) {                                           // the identity: batch entry k is problem k
+        std::vector<int32_t> id((size_t)B);
+        for (int64_t k = 0; k < B; ++k) id[(size_t)k] = (int32_t)k;
+        PNP_CUDA_OK(cudaMemcpyAsync(buf + sel_bytes, id.data(), 4 * (size_t)B, cudaMemcpyHostToDevice, st));   // (pageable: staged)
+        idx = (const int32_t*)(buf + sel_bytes);
+    }
+    return dtype == PNPB200_DTYPE_F64
+        ? inlier_pass<double>(B, n_total, uv, pattern, n_patterns, K, visible, rp, R, t, best_pattern, idx, d_sel, last_round, inliers,
+                              rounds, robust_status, flag, tau, shape, st)
+        : inlier_pass<float>(B, n_total, uv, pattern, n_patterns, K, visible, rp, R, t, best_pattern, idx, d_sel, last_round, inliers,
+                             rounds, robust_status, flag, tau, shape, st);
 }
 
 }  // extern "C"
