@@ -293,7 +293,13 @@ int pnpb200_synth_face_variation(int dtype, int64_t b0, int64_t B, int n, const 
  *                  4,5 LM_GT avg,max  6,7 predict_LM avg,max  8,9 predict_GT avg,max (x distance_GT)
  *                  10 t3_est 11 distance_GT 12 roll_est 13 pitch_est 14 yaw_est 15 reserved
  *   flags [B,4] = depth, roll, pitch, yaw passed;  max_idx [B,3] = landmark index of each max
- *   bounds [host] 4 doubles (10 cm, 10, 10, 10 deg in the reference)
+ *   bounds [host] 4 doubles (10 cm, 10, 10, 10 deg in the reference; NULL = 10 each)
+ * The depth flag is |t3 * 100 - distance_GT * 100| < bounds[0] with both products rounded to FP64 before the difference,
+ * as the reference evaluates it; the angle flags are |est - GT| < bound; a NaN fails.  A landmark distance whose square is
+ * not finite (a projection at depth exactly 0, a non-finite pixel) is NaN, as in the solution check: the mean is then NaN
+ * and that landmark is never the maximum (strict >, the first landmark wins ties, -1 when no distance is > 0).  The
+ * prediction-vs-GT difference is taken through the pixel, (prediction - pixel) + (pixel - GT), so a non-finite visible
+ * pixel makes all three distances of its landmark NaN; hide such pixels with the masked entry.
  */
 int pnpb200_report_batch(int dtype, int64_t B, int n, const void* pattern, const void* uv,
                          const double* K, const void* R, const void* t, const void* euler_deg,

@@ -217,6 +217,14 @@ PNP_DEV void too_few_for_report(double& s0, double& s1, double& s2, double& m0, 
     i0 = i1 = i2 = -1;
 }
 
+// check_if_the_sample_passed on depth (TEST_TOOLBOX.py:55-62 with random_stress_test.py:374-377's t3 * 100 and dist_cm):
+// both products in centimetres are rounded before their difference, as the reference rounds them (contracting one of
+// them into an FMA flips the flag on some pairs within a few ulp of the bound)
+PNP_DEV int32_t depth_passed(double t3, double dist, double bound)
+{
+    return fabs(__dmul_rn(t3, 100.0) - __dmul_rn(dist, 100.0)) < bound;
+}
+
 PNP_DEV void warp_sum_max(double& s, double& m, int& im)
 {
 #pragma unroll
@@ -254,6 +262,9 @@ __global__ void k_report(long long B, int n, const void* pattern, const void* uv
     int i0 = -1, i1 = -1, i2 = -1;
     const uint32_t* vw = MASKED ? vis + (size_t)b * vis_words : nullptr;
     const int nv = MASKED ? count_visible(vw, nullptr, n) : 0;
+    // sqrt_nonneg, as homogeneous_distance: a distance whose square is not finite (depth 0, where the projection is +-inf;
+    // a non-finite pixel) is NaN, as in the streaming kernels, and so never the maximum.  The prediction-vs-GT difference is
+    // the sum of the two pixel differences, as in landmark_errors, so a non-finite pixel makes all three distances NaN.
     for (int i = lane; i < n; i += 32) {
         if constexpr (MASKED) { if (!mask_bit(vw, i)) continue; }
         const double x = ld<T>(pattern, 3 * i), y = ld<T>(pattern, 3 * i + 1), z = ld<T>(pattern, 3 * i + 2);
@@ -262,12 +273,12 @@ __global__ void k_report(long long B, int n, const void* pattern, const void* uv
         project_point_fast(K.k, Rg, tg, x, y, z, pg);          // :314
         const double mu = ld<T>(uv, ((size_t)b * n + i) * 2), mv = ld<T>(uv, ((size_t)b * n + i) * 2 + 1), mw = 1.0;
         double d0, d1, d2, e;
-        d0 = mu - pg[0]; d1 = mv - pg[1]; d2 = mw - pg[2];     // LM vs GT (:321)
-        e = sqrt(d0 * d0 + d1 * d1 + d2 * d2); s0 += e; if (e > m0) { m0 = e; i0 = i; }
+        const double g0 = mu - pg[0], g1 = mv - pg[1], g2 = mw - pg[2];   // LM vs GT (:321)
+        e = sqrt_nonneg(g0 * g0 + g1 * g1 + g2 * g2); s0 += e; if (e > m0) { m0 = e; i0 = i; }
         d0 = pe[0] - mu; d1 = pe[1] - mv; d2 = pe[2] - mw;     // prediction vs LM (:326)
-        e = sqrt(d0 * d0 + d1 * d1 + d2 * d2); s1 += e; if (e > m1) { m1 = e; i1 = i; }
-        d0 = pe[0] - pg[0]; d1 = pe[1] - pg[1]; d2 = pe[2] - pg[2];   // prediction vs GT (:331)
-        e = sqrt(d0 * d0 + d1 * d1 + d2 * d2); s2 += e; if (e > m2) { m2 = e; i2 = i; }
+        e = sqrt_nonneg(d0 * d0 + d1 * d1 + d2 * d2); s1 += e; if (e > m1) { m1 = e; i1 = i; }
+        d0 += g0; d1 += g1; d2 = pe[2] - pg[2];                 // prediction vs GT (:331) through the pixel, as landmark_errors
+        e = sqrt_nonneg(d0 * d0 + d1 * d1 + d2 * d2); s2 += e; if (e > m2) { m2 = e; i2 = i; }
     }
     warp_sum_max(s0, m0, i0); warp_sum_max(s1, m1, i1); warp_sum_max(s2, m2, i2);
     if constexpr (MASKED) { if (nv < kMinVisible) too_few_for_report(s0, s1, s2, m0, m1, m2, i0, i1, i2); }
@@ -280,7 +291,7 @@ __global__ void k_report(long long B, int n, const void* pattern, const void* uv
         rp[8 * sk] = (s2 / (MASKED ? nv : n)) * dist; rp[9 * sk] = m2 * dist;
         rp[10 * sk] = t3; rp[11 * sk] = dist; rp[12 * sk] = roll_e; rp[13 * sk] = pitch_e; rp[14 * sk] = yaw_e; rp[15 * sk] = 0.0;
         if (flags) {                                           // check_if_the_sample_passed (:55-62), depth in cm
-            flags[b * 4] = fabs(t3 * 100.0 - dist * 100.0) < bounds.b[0];
+            flags[b * 4] = depth_passed(t3, dist, bounds.b[0]);
             flags[b * 4 + 1] = fabs(roll_e - roll_g) < bounds.b[1];
             flags[b * 4 + 2] = fabs(pitch_e - pitch_g) < bounds.b[2];
             flags[b * 4 + 3] = fabs(yaw_e - yaw_g) < bounds.b[3];
@@ -392,7 +403,7 @@ __global__ void __launch_bounds__(32) k_report_thread(const __grid_constant__ Re
             rp[8 * sk] = (s2 / a.n) * dist; rp[9 * sk] = m2 * dist;
             rp[10 * sk] = t3; rp[11 * sk] = dist; rp[12 * sk] = roll_e; rp[13 * sk] = pitch_e; rp[14 * sk] = yaw_e; rp[15 * sk] = 0.0;
             if (a.flags) {
-                a.flags[b * 4] = fabs(t3 * 100.0 - dist * 100.0) < a.bounds[0];
+                a.flags[b * 4] = depth_passed(t3, dist, a.bounds[0]);
                 a.flags[b * 4 + 1] = fabs(roll_e - roll_g) < a.bounds[1];
                 a.flags[b * 4 + 2] = fabs(pitch_e - pitch_g) < a.bounds[2];
                 a.flags[b * 4 + 3] = fabs(yaw_e - yaw_g) < a.bounds[3];
@@ -515,7 +526,7 @@ __global__ void __launch_bounds__(32, PNP_REPORT_MINBLOCKS) k_report_chunk(const
             rp[8 * sk] = (s2 / (MASKED ? nv : a.n)) * dist; rp[9 * sk] = m2 * dist;
             rp[10 * sk] = t3; rp[11 * sk] = dist; rp[12 * sk] = roll_e; rp[13 * sk] = pitch_e; rp[14 * sk] = yaw_e; rp[15 * sk] = 0.0;
             if (a.flags) {
-                a.flags[b * 4] = fabs(t3 * 100.0 - dist * 100.0) < a.bounds[0];
+                a.flags[b * 4] = depth_passed(t3, dist, a.bounds[0]);
                 a.flags[b * 4 + 1] = fabs(roll_e - roll_g) < a.bounds[1];
                 a.flags[b * 4 + 2] = fabs(pitch_e - pitch_g) < a.bounds[2];
                 a.flags[b * 4 + 3] = fabs(yaw_e - yaw_g) < a.bounds[3];

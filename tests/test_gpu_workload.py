@@ -255,11 +255,16 @@ def test_face_variation_workload_and_fragility_analysis_match_reference():
 @pytest.mark.parametrize("method,n,dtype,subset", [("lm", 68, torch.float64, False), ("linear_f2", 68, torch.float64, False),
                                                  ("lm", 15, torch.float64, False), ("lm", 68, torch.float32, False),
                                                  ("lm_plus", 68, torch.float64, False), ("qeif", 15, torch.float64, True),
-                                                 ("lm", 1024, torch.float64, False), ("eif2", 15, torch.float64, False)])
+                                                 ("lm", 1024, torch.float64, False), ("eif2", 15, torch.float64, False),
+                                                 ("lm", 68, torch.float64, "skew"), ("linear_f2", 68, torch.float64, "skew"),
+                                                 ("lm", 68, torch.float32, "skew"), ("lm", 95, torch.float64, False),
+                                                 ("linear_f2", 190, torch.float32, False)])
 def test_fused_solve_report_equals_the_two_calls(method, n, dtype, subset):
     """pnpb200_solve_report_batch (the residual pass of the moment mapping folded into the report kernel, the pixel rows
     read twice instead of three times) returns what pnpb200_solve_batch followed by pnpb200_report_batch_strided return --
-    bit for bit, for a ragged batch, for every method and shape (those that cannot fuse run the two calls inside)."""
+    bit for bit, for a ragged batch, for every method and shape (those that cannot fuse run the two calls inside).
+    subset = "skew": all landmarks, K with a nonzero skew, so the fused kernel normalises the pixels with both FMAs
+    (k_report_chunk<T, RES, SKEW = true>); n = 95 (FP64) and 190 (FP32) are the largest n that fuse."""
     import pnp_solver_test_b200 as pnp
     from pnp_solver_test_b200 import workload as wl
     pat = pt.get_golden_pattern() if n == 15 else pt.synthetic_pattern(n)
@@ -276,8 +281,11 @@ def _fused_case(method, n, dtype, subset, B):
     from pnp_solver_test_b200 import workload as wl
     pat = pt.get_golden_pattern() if n == 15 else pt.synthetic_pattern(n)
     P, K = pt.pattern_array(pat), pt.default_camera_matrix()
+    if subset == "skew":
+        K = K.copy()
+        K[0, 1] = 1.75
     w = wl.synth_batch(7, B, P, K, dtype=dtype)
-    idx = [list(pat).index(k) for k in pt.LM_KEY_LIST_6] if subset else None
+    idx = [list(pat).index(k) for k in pt.LM_KEY_LIST_6] if subset is True else None
     patd = dev(P, dtype)[None]
     a = pnp.solve_batch(method, w["uv"], patd, K, point_index=idx)
     r = wl.report_batch(P, w["uv"], K, a["R"], a["t"], a["euler"], w["gt"])
