@@ -707,6 +707,13 @@ int pnpb200_selftest_math(int64_t n, const double* in, double* rcp, double* rsqr
 int pnpb200_selftest_sincos(int64_t n, const double* in, double* sin_out, double* cos_out, void* stream);
 
 /*
+ * Test hook: the projection the LM and EIF2 solves end with (csrc/pnpb200_math.cuh, so3_project), on n device 3x3
+ * matrices G [n,9] (row-major, dtype PNPB200_DTYPE_F64 or _F32): R [n,9] = U diag(1, 1, det(U V^T)) V^T, the rotation
+ * that maximises tr(R^T G), and sigma_max [n] = ||G||_2, in the same dtype.
+ */
+int pnpb200_selftest_project(int dtype, int64_t n, const void* G, void* R, void* sigma_max, void* stream);
+
+/*
  * Test hook: the P3P solver of the hypothesis stage (csrc/pnpb200_p3p.cuh), on m device triples: pattern points X [m,3,3]
  * (metres) and unit bearings f [m,3,3].  R [m,4,9], t [m,4,3]: the valid roots first, NaN after; n_sol [m]: their number.
  */

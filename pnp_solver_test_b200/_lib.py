@@ -40,7 +40,7 @@ EXPORTS = [
     "pnpb200_check_batch_masked", "pnpb200_workspace_bytes_masked", "pnpb200_solve_batch_host_masked",
     "pnpb200_default_robust_params", "pnpb200_robust_workspace_bytes", "pnpb200_solve_robust_batch",
     "pnpb200_default_hypothesis_params", "pnpb200_hypothesize_batch", "pnpb200_ransac_workspace_bytes", "pnpb200_solve_ransac_batch",
-    "pnpb200_selftest_p3p", "pnpb200_selftest_inliers",
+    "pnpb200_selftest_p3p", "pnpb200_selftest_inliers", "pnpb200_selftest_project",
 ]
 
 
@@ -121,6 +121,7 @@ lib.pnpb200_ransac_workspace_bytes.restype = C.c_int64
 lib.pnpb200_ransac_workspace_bytes.argtypes = [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int]
 lib.pnpb200_solve_ransac_batch.argtypes = lib.pnpb200_solve_robust_batch.argtypes[:-1] + [_VP, _PI, _PI, _VP]
 lib.pnpb200_selftest_p3p.argtypes = [C.c_int64, _VP, _VP, _VP, _VP, _VP, _VP]
+lib.pnpb200_selftest_project.argtypes = [C.c_int, C.c_int64, _VP, _VP, _VP, _VP]
 lib.pnpb200_selftest_inliers.argtypes = [C.c_int, C.c_int64, C.c_int, C.c_int, _VP, _VP, C.c_int, _PI, _PD, _U32P, _VP, _VP, _VP,
                                          _PI, _PI, C.c_int, _U32P, _PI, _PI, _VP, _PD, C.c_int, _VP]
 

@@ -1180,6 +1180,19 @@ __global__ void k_selftest_sincos(long long n, const double* __restrict__ in, do
     sincos_bounded(in[i], s[i], c[i]);
 }
 
+template <typename T>
+__global__ void k_selftest_project(long long n, const T* __restrict__ G, T* __restrict__ R, T* __restrict__ smax)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    T g[9], r[9];
+#pragma unroll
+    for (int e = 0; e < 9; ++e) g[e] = G[9 * i + e];
+    so3_project<T>(g, r, smax[i]);
+#pragma unroll
+    for (int e = 0; e < 9; ++e) R[9 * i + e] = r[e];
+}
+
 }  // namespace pnpb200
 
 namespace pnpb200 {
@@ -1627,6 +1640,19 @@ int pnpb200_selftest_sincos(int64_t n, const double* in, double* sin_out, double
     if (n < 0 || !in || !sin_out || !cos_out) return PNPB200_EINVAL;
     if (n == 0) return PNPB200_OK;
     k_selftest_sincos<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(n, in, sin_out, cos_out); count_kernel_launches(1);
+    PNP_CUDA_OK(cudaGetLastError());
+    return PNPB200_OK;
+}
+
+int pnpb200_selftest_project(int dtype, int64_t n, const void* G, void* R, void* sigma_max, void* stream)
+{
+    if (n < 0 || !G || !R || !sigma_max || (dtype != PNPB200_DTYPE_F64 && dtype != PNPB200_DTYPE_F32)) return PNPB200_EINVAL;
+    if (n == 0) return PNPB200_OK;
+    if (dtype == PNPB200_DTYPE_F64)
+        k_selftest_project<double><<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(n, (const double*)G, (double*)R, (double*)sigma_max);
+    else
+        k_selftest_project<float><<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(n, (const float*)G, (float*)R, (float*)sigma_max);
+    count_kernel_launches(1);
     PNP_CUDA_OK(cudaGetLastError());
     return PNPB200_OK;
 }

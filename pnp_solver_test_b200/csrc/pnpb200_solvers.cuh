@@ -818,7 +818,7 @@ PNP_DEV void lm_reconstruct(const T (&x)[12], Result<T>& out)
     T G[9], smax;
 #pragma unroll
     for (int e = 0; e < 9; ++e) G[e] = x[e];
-    svd3_project<T>(G, out.R, smax);
+    so3_project<T>(G, out.R, smax);
     const T t3 = T(1) / (smax * x[11]);                   // :3530-3533
     out.t[0] = x[9] * t3; out.t[1] = x[10] * t3; out.t[2] = t3;
 }
