@@ -446,6 +446,64 @@ int pnpb200_solve_batch_host_masked(pnpb200_pipeline* p, int method, int64_t B, 
                                     double reproj_limit_px, int32_t* status, void* reproj);
 
 /*
+ * Per-landmark weights.  Most face-landmark detectors emit a confidence per landmark, and the pixel noise of a jaw-line or
+ * half-occluded point is several times that of an eye corner.  pnpb200_solve_batch_weighted is pnpb200_solve_batch plus
+ *   weights  [device] [B, n_total] float32 (for both dtypes), row-major and contiguous, 4-byte aligned, in the caller's
+ *            0..n_total-1 numbering as `visible`: with point_index, selected landmark i has weight
+ *            weights[b, point_index[i]], and every repeat of an index gets that weight.  NULL or a misaligned pointer is
+ *            PNPB200_EINVAL, returned before any CUDA call.
+ * Which landmarks take part: a selected landmark takes part iff 0 < w < +Inf, compared as the stored float32.  Every other
+ * value (0, -0, negatives, NaN, +-Inf) hides it: its pixels are never read, as under the masked rule.  With fewer than 4
+ * selected landmarks taking part the problem is not solved, with the masked rule's outputs (NaN pose and res_norm, 0
+ * iterations, pattern 0); its neighbours in the batch are unaffected.
+ * The weighted problem is the reference's problem on the landmarks that take part, each landmark's information times w_i:
+ *  - LM, PNPB200_FLAG_LM_TRUE_JACOBIAN and the LM stage of LM+: the landmark's two measurement rows of the (2n + 9)-row
+ *    residual and Jacobian are multiplied by sqrt(w_i).  The 9 constraint rows, lambda and the iteration rule are unchanged.
+ *  - QEIF, EIF2: the landmark's two diagonal entries of Q^-1 are multiplied by w_i, i.e. its sigma is meas_sigma_px /
+ *    sqrt(w_i).  Priors, process noise and the exit rule are unchanged.
+ *  - Linear F1, F2 and LM+'s start: the least-squares systems with the landmark's rows multiplied by sqrt(w_i).
+ *  - res_norm = sqrt(sum w_i (r_x,i^2 + r_y,i^2)) at the state where the reference evaluates it, so the QEIF / EIF2 exit
+ *    tests and the arg-min over several patterns use the weighted residual.
+ * In exact arithmetic integer weights are the problem with landmark i repeated w_i times (point_index may repeat indices),
+ * and weights in {0, 1} are the masked solve with visible = (w > 0) -- bit for bit on the device: the weight multiplies a
+ * landmark's scalar factors (w bx, w by, w (bx^2 + by^2), w r), never an already rounded product, so w = 1 rounds as the
+ * unweighted sums do.  Scaling all weights is not neutral: lambda, Omega_0 and the process noise are absolute.  w = 1 is the
+ * reference's own per-landmark weight, and w = (meas_sigma_px / sigma_i)^2 is the natural choice for a landmark whose noise
+ * is sigma_i px.
+ * A weighted solve takes the mapping the call without weights takes, every method and flag included; explicit mappings are
+ * accepted wherever pnpb200_solve_batch_masked accepts them, and rows of 256 landmarks and more take the per-warp streaming
+ * shape (no weighted TMA ring).  A weighted solve's result does not depend on the batch around a problem, with the masked
+ * solve's one exception: the QEIF / EIF2 FP64 fix-up picks its per-warp or per-thread kernel by the number of marked tiles.
+ * The filters' exit test in the moment mapping certifies each decision against res2_error_bound, which counts the landmarks
+ * summed and weighs the offset term with sum w (pnpb200_solvers.cuh).  pnpb200_workspace_bytes_weighted is the scratch of a
+ * weighted solve: that of pnpb200_workspace_bytes plus 11 values per problem where that is not 0.  Weighted report and
+ * check entries do not exist: pass visible = (w > 0) to the masked ones.
+ * What weighting buys (weighted C oracle, tests/weights_accuracy.py: random_stress_test.py pose distribution, seed 42,
+ * 8 192 problems, 68 landmarks; hetero: sigma_i log-uniform on [0.5, 8] px per landmark, N(0, sigma_i^2) noise then whole
+ * pixels, w = float32((3 px / sigma_i)^2); homo: sigma = 2 px, every w = 2.25).  Pass rate of the 10 cm / 10 deg test,
+ * median and 95th percentile of max |d roll, d pitch, d yaw| in deg and of |d depth| in cm, unweighted -> weighted:
+ *   hetero LM     33.9 % ->  69.8 % |   9.60  149.36 ->   3.83   99.31 |   9.98   71.66 ->   4.53   53.38
+ *   hetero LM+    59.7 % ->  92.0 % |   6.07   28.24 ->   2.25    8.84 |   3.63   28.52 ->   1.33   10.64
+ *   hetero QEIF   60.9 % ->  92.9 % |   5.95   23.92 ->   2.21    8.27 |   3.47   25.78 ->   1.28    9.96
+ *   hetero EIF2   13.6 % ->  25.4 % |  34.74  108.59 ->  15.90   71.31 |  75.95  193.02 ->  40.24  130.34
+ *   homo   LM     51.4 % ->  54.6 % |   6.15  147.19 ->   5.74  139.70 |   7.20   67.75 ->   6.53   64.69
+ *   homo   LM+    80.3 % ->  80.6 % |   3.50   14.27 ->   3.47   13.79 |   2.07   16.99 ->   2.06   16.71
+ *   homo   QEIF   81.5 % ->  81.5 % |   3.43   12.79 ->   3.42   12.78 |   2.02   15.18 ->   2.02   15.18
+ *   homo   EIF2   27.1 % ->  21.1 % |  14.41   80.64 ->  24.55   87.12 |  32.86  149.36 ->  55.66  156.29
+ * On heteroscedastic noise weighting roughly doubles LM's and EIF2's pass rates and lifts LM+ and QEIF from ~60 % to
+ * ~92 %.  The homoscedastic row shows the absolute scale alone: w = 2.25 everywhere is a smaller measurement sigma, which
+ * leaves LM+ and QEIF where they were, helps LM's damped steps a little and hurts EIF2, whose process noise and prior are
+ * absolute -- a uniform weight other than 1 does not help a filter.
+ */
+int pnpb200_solve_batch_weighted(int method, int dtype, int64_t B, int n_total, int n,
+                                 const void* uv, const void* pattern, int n_patterns,
+                                 const int32_t* point_index, const double* K,
+                                 const pnpb200_params* params,
+                                 void* R, void* t, void* euler_deg, void* res_norm,
+                                 int32_t* iters, int32_t* best_pattern, const float* weights, void* stream);
+int64_t pnpb200_workspace_bytes_weighted(int method, int dtype, int64_t B, int n_patterns, int mapping);
+
+/*
  * Outlier-robust solve.  Not a reference function.  A detector also misplaces landmarks (a mouth corner on the lip, an eye
  * corner on the brow), and one such landmark ruins the pose of every method.  This entry rejects landmarks by their
  * reprojection distance and re-solves each problem on its inliers, with the masked solve above.  Per problem b:

@@ -41,6 +41,7 @@ EXPORTS = [
     "pnpb200_default_robust_params", "pnpb200_robust_workspace_bytes", "pnpb200_solve_robust_batch",
     "pnpb200_default_hypothesis_params", "pnpb200_hypothesize_batch", "pnpb200_ransac_workspace_bytes", "pnpb200_solve_ransac_batch",
     "pnpb200_selftest_p3p", "pnpb200_selftest_inliers", "pnpb200_selftest_project",
+    "pnpb200_solve_batch_weighted", "pnpb200_workspace_bytes_weighted",
 ]
 
 
@@ -109,6 +110,10 @@ lib.pnpb200_check_batch_masked.argtypes = [C.c_int, C.c_int64, C.c_int, _VP, C.c
                                            _PI, _VP, _U32P, _VP]
 lib.pnpb200_solve_batch_host_masked.argtypes = [_VP, C.c_int, C.c_int64, C.c_int, C.c_int, _VP, _VP, _PI, _PD, _VP, _VP, _VP,
                                                 _VP, _VP, _PI, _PI, _U32P, C.c_double, _PI, _VP]
+# the weighted entry: the unmasked one plus `const float* weights` (before the stream)
+lib.pnpb200_workspace_bytes_weighted.restype = C.c_int64
+lib.pnpb200_workspace_bytes_weighted.argtypes = [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int]
+lib.pnpb200_solve_batch_weighted.argtypes = lib.pnpb200_solve_batch_masked.argtypes[:-2] + [C.POINTER(C.c_float), _VP]
 lib.pnpb200_robust_workspace_bytes.restype = C.c_int64
 lib.pnpb200_robust_workspace_bytes.argtypes = [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int]
 # pnpb200_solve_batch_masked's arguments, then the robust parameters and the three outputs

@@ -217,17 +217,26 @@ int64_t pnpb200_workspace_bytes_masked(int method, int dtype, int64_t B, int n_p
     return plain > 0 ? plain + (int64_t)PNP_NPMOM * B * ((dtype == PNPB200_DTYPE_F32) ? 4 : 8) : 0;
 }
 
+int64_t pnpb200_workspace_bytes_weighted(int method, int dtype, int64_t B, int n_patterns, int mapping)
+{
+    // the weighted pattern moments (sum w theta theta^T, sum w theta, sum w) and the count of landmarks taking part
+    const int64_t plain = pnpb200_workspace_bytes(method, dtype, B, n_patterns, mapping);
+    return plain > 0 ? plain + (int64_t)PNP_NPMOM_W * B * ((dtype == PNPB200_DTYPE_F32) ? 4 : 8) : 0;
+}
+
 }  // extern "C"
 
 namespace pnpb200 {
 // vis: [B, ceil(n_total / 32)] per-problem visibility bits (device), or nullptr for every landmark
+// wts: [B, n_total] float32 per-landmark weights (device), or nullptr for weight 1 (at most one of vis, wts)
 int solve_batch_impl(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
                      int n_patterns, const int32_t* point_index, const double* K, const pnpb200_params& prm,
                      void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters, int32_t* best_pattern,
-                     cudaStream_t st, const uint32_t* vis)
+                     cudaStream_t st, const uint32_t* vis, const float* wts)
 {
     if (B < 0 || n_total < 1 || n < 1 || (!point_index && n != n_total) || !uv || !pattern || !K) return PNPB200_EINVAL;
     if (vis && !vis_aligned(vis)) return PNPB200_EINVAL;
+    if ((wts && ((uintptr_t)wts & 3u) != 0) || (vis && wts)) return PNPB200_EINVAL;
     if (((uintptr_t)uv & 15u) != 0) return PNPB200_EINVAL;   // rows are staged with 16-byte bulk copies / vector loads
     if (n_patterns < 1 || n_patterns > PNPB200_MAX_PATTERNS) return PNPB200_EINVAL;
     if (method < 0 || method > 5 || (dtype != PNPB200_DTYPE_F64 && dtype != PNPB200_DTYPE_F32)) return PNPB200_EINVAL;
@@ -248,7 +257,7 @@ int solve_batch_impl(int method, int dtype, int64_t B, int n_total, int n, const
                                          { solve_part_f32_g0, solve_part_f32_g1, solve_part_f32_g2, solve_part_f32_g3 } };
     const int rc = parts[dtype == PNPB200_DTYPE_F64 ? 0 : 1][group](method, B, n_total, n, uv, pattern, n_patterns, point_index,
                                                                    idx_dev, K, prm, R, t, euler_deg, res_norm, iters,
-                                                                   best_pattern, st, vis);
+                                                                   best_pattern, st, vis, wts);
     if (idx_dev) cudaFreeAsync(idx_dev, st);
     return rc;
 }
@@ -279,6 +288,19 @@ int pnpb200_solve_batch_masked(int method, int dtype, int64_t B, int n_total, in
     prm.flags &= ~PNP_FLAG_INTERNAL_NO_RESIDUAL;
     return solve_batch_impl(method, dtype, B, n_total, n, uv, pattern, n_patterns, point_index, K, prm, R, t, euler_deg, res_norm,
                             iters, best_pattern, (cudaStream_t)stream, visible);
+}
+
+int pnpb200_solve_batch_weighted(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,
+                                 int n_patterns, const int32_t* point_index, const double* K, const pnpb200_params* params,
+                                 void* R, void* t, void* euler_deg, void* res_norm, int32_t* iters, int32_t* best_pattern,
+                                 const float* weights, void* stream)
+{
+    if (!weights || ((uintptr_t)weights & 3u) != 0) return PNPB200_EINVAL;
+    pnpb200_params prm;
+    if (params) prm = *params; else fill_default_params(&prm);
+    prm.flags &= ~PNP_FLAG_INTERNAL_NO_RESIDUAL;
+    return solve_batch_impl(method, dtype, B, n_total, n, uv, pattern, n_patterns, point_index, K, prm, R, t, euler_deg, res_norm,
+                            iters, best_pattern, (cudaStream_t)stream, nullptr, weights);
 }
 
 static int solve_report_impl(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern,

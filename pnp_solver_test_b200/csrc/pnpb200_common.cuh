@@ -14,6 +14,7 @@
 #define PNP_NTAIL 12
 #define PNP_PATC 20
 #define PNP_NPMOM 10       // masked moment mapping: per-problem pattern moments (sum theta theta^T 6, sum theta 3, count) behind the moments
+#define PNP_NPMOM_W 11     // weighted moment mapping: the same with weights (the count is sum w) and the count of landmarks taking part
 // landmark selections up to this size travel inside the kernel arguments; larger ones through device memory
 #define PNP_MAX_INLINE_IDX 96
 // QEIF takes H^T H, H^T v (and, in the moment mapping, the residual of its exit test) from the moments from this many landmarks on
@@ -73,10 +74,12 @@ inline bool vis_aligned(const uint32_t* vis) { return ((uintptr_t)vis & 3u) == 0
 int check_launch(int dtype, int64_t B, int n, const void* pattern, int n_patterns, const void* uv, const double* K,
                  const void* R, const void* t, const void* res_norm, const int32_t* best_pattern, double limit,
                  int32_t* status, void* reproj, cudaStream_t st, const uint32_t* vis = nullptr);
-// pnpb200_solve_batch(_masked) without the entry's parameter copy (pnpb200_api.cu); vis = nullptr: every landmark
+// pnpb200_solve_batch(_masked / _weighted) without the entry's parameter copy (pnpb200_api.cu); vis = wts = nullptr: every
+// landmark with weight 1
 int solve_batch_impl(int method, int dtype, int64_t B, int n_total, int n, const void* uv, const void* pattern, int n_patterns,
                      const int32_t* point_index, const double* K, const pnpb200_params& prm, void* R, void* t, void* euler_deg,
-                     void* res_norm, int32_t* iters, int32_t* best_pattern, cudaStream_t st, const uint32_t* vis = nullptr);
+                     void* res_norm, int32_t* iters, int32_t* best_pattern, cudaStream_t st, const uint32_t* vis = nullptr,
+                     const float* wts = nullptr);
 // the hypothesis stage (pnpb200_hypothesize_batch) with its parameters given, and their checks; pnpb200_ransac.cu
 bool hypothesis_params_ok(const pnpb200_hypothesis_params& h);
 void fill_default_hypothesis(pnpb200_hypothesis_params* h);
@@ -133,7 +136,7 @@ extern thread_local ProfileRing g_prof;            // defined in pnpb200_api.cu
 #define PNP_SOLVE_PART_ARGS                                                                                          \
     int method, long long B, int n_total, int n, const void *uv, const void *pattern, int n_patterns,                 \
         const int32_t *idx_host, const int32_t *idx_dev, const double *K, const pnpb200_params &prm, void *R, void *t, \
-        void *euler, void *res, int32_t *iters, int32_t *best, cudaStream_t stream, const uint32_t *vis
+        void *euler, void *res, int32_t *iters, int32_t *best, cudaStream_t stream, const uint32_t *vis, const float *wts
 int solve_part_f64_g0(PNP_SOLVE_PART_ARGS);
 int solve_part_f64_g1(PNP_SOLVE_PART_ARGS);
 int solve_part_f64_g2(PNP_SOLVE_PART_ARGS);

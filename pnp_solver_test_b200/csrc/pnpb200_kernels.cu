@@ -19,6 +19,7 @@
 //
 // No tensor cores on purpose: the per-problem systems are 6x6 / 12x12.
 #include <string.h>
+#include <type_traits>
 
 #include "pnpb200_common.cuh"
 #include "pnpb200_solvers.cuh"
@@ -69,6 +70,7 @@ struct SolveArgs {
     int skip_residual;           // moment mapping: leave res_norm to the caller's fused report pass (pnpb200_solve_report_batch)
     const uint32_t* vis;         // [B, vis_words] per-problem visibility bits (masked kernels only)
     int vis_words;
+    const float* wts;            // [B, n_total] per-landmark weights (weighted kernels only)
 };
 
 // raw pixels of one problem in global memory, normalised on the fly (warp mapping)
@@ -85,7 +87,42 @@ struct PtsGlobal {
     }
     PNP_DEV bool vis(int) const { return true; }
     PNP_DEV int count(int n) const { return n; }
+    PNP_DEV float weight(int) const { return 1.0f; }
+    template <typename U> PNP_DEV U total(int n) const { return U(count(n)); }
+    static constexpr bool kWeighted = false;
 };
+
+// The MASKED template parameter of the kernels: which landmarks of a problem take part, and with what weight
+constexpr int kAllLandmarks = 0;   // every selected landmark, weight 1
+constexpr int kMaskBits = 1;       // the visible ones (a.vis), weight 1
+constexpr int kWeights = 2;        // those whose weight takes part (a.wts), with that weight
+template <int MASKED, typename Base>
+using PtsOf = typename std::conditional<MASKED == kWeights, PtsWeighted<Base>, PtsMasked<Base> >::type;
+
+template <typename T> struct MomArgs;
+
+// point accessor of problem b under a mask / weights (the base accessor's fields are set by the caller)
+template <typename Base, typename A>
+PNP_DEV void bind_problem(PtsMasked<Base>& p, const A& a, long long b)
+{
+    p.words = a.vis + (size_t)b * a.vis_words;
+    p.nvis = count_visible(p.words, p.idx, a.n);
+}
+template <typename Base, typename A>
+PNP_DEV void bind_problem(PtsWeighted<Base>& p, const A& a, long long b)
+{
+    p.wrow = a.wts + (size_t)b * a.n_total;
+    p.nvis = count_weights(p.wrow, p.idx, a.n, p.wsum);
+}
+// the residual pass of the weighted moment mapping: the count of landmarks taking part is the moments pass's count row
+// (weighted_count_row), not a second scan of the weights; the sum of the weights is not needed there
+template <typename Base, typename T>
+PNP_DEV void bind_problem_counted(PtsWeighted<Base>& p, const MomArgs<T>& a, long long b)
+{
+    p.wrow = a.wts + (size_t)b * a.n_total;
+    p.nvis = (int)a.pmom[(size_t)PNP_NPMOM * a.ld + b];
+    p.wsum = 0.0;
+}
 
 // Pattern constants (PNP_PATC per pattern) by one warp: M0, m0, n and G = (D^T D)^-1.
 // Accumulated in double whatever T is (they are shared by every problem of the launch).
@@ -126,12 +163,42 @@ PNP_DEV void pattern_constants(const T* __restrict__ sP, int n, T* __restrict__ 
 
 // Sum theta theta^T (6), sum theta (3) and the count (pm[9]) over the visible landmarks of ONE problem (masked kernels; LPP = 1:
 // one thread, 32: one warp, every lane ends with the sums).  The moment mapping keeps them per problem in the workspace.
+// Weighted (PtsWeighted): sum w theta theta^T, sum w theta and sum w in the same slots, and *crow = weighted_count_row().
 constexpr int kPatternMoments = PNP_NPMOM;
+
+// The workspace row behind the weighted pattern moments: the number of landmarks taking part, plus 1/2 when one of their
+// weights is not 1 (res2_error_bound then adds the roundings of the weight products).  Exact in FP32 as in FP64.
+PNP_DEV double weighted_count_row(int count, bool nonunit) { return (double)count + (nonunit ? 0.5 : 0.0); }
+
 template <typename T, int LPP, typename Pts>
-PNP_DEV void pattern_moments_masked(const Pts& pts, const T* __restrict__ sP, int n, int sub, double (&pm)[kPatternMoments])
+PNP_DEV void pattern_moments_masked(const Pts& pts, const T* __restrict__ sP, int n, int sub, double (&pm)[kPatternMoments],
+                                    double* crow = nullptr)
 {
 #pragma unroll
     for (int e = 0; e < 9; ++e) pm[e] = 0.0;
+    if constexpr (Pts::kWeighted) {
+        double ws = 0.0;
+        bool nonunit = false;
+        for (int i = sub; i < n; i += LPP) {
+            if (!pts.vis(i)) continue;
+            const double w = (double)pts.weight(i);
+            const double th[3] = { (double)sP[3 * i], (double)sP[3 * i + 1], (double)sP[3 * i + 2] };
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+#pragma unroll
+                for (int b = a; b < 3; ++b) pm[s3(a, b)] = fma(w * th[a], th[b], pm[s3(a, b)]);
+                pm[6 + a] += w * th[a];
+            }
+            ws += w;
+            nonunit |= (w != 1.0);
+        }
+#pragma unroll
+        for (int e = 0; e < 9; ++e) pm[e] = group_sum<LPP, double>(pm[e]);
+        pm[9] = group_sum<LPP, double>(ws);
+        if (LPP > 1) nonunit = __any_sync(0xffffffffu, nonunit);
+        if (crow) *crow = weighted_count_row(pts.count(n), nonunit);
+        return;
+    }
     for (int i = sub; i < n; i += LPP) {
         if (!pts.vis(i)) continue;
         const double th[3] = { (double)sP[3 * i], (double)sP[3 * i + 1], (double)sP[3 * i + 2] };
@@ -277,7 +344,7 @@ PNP_DEV void load_pattern(const T* __restrict__ pattern, const int32_t* __restri
 // direct mapping, one problem per thread; CTA = 1 warp = 32 consecutive problems
 // ------------------------------------------------------------------------------------------
 // MASKED: problem b sees only its visible landmarks (a.vis); every lane keeps its own constants, computed per tile
-template <typename T, int METHOD, bool MASKED = false>
+template <typename T, int METHOD, int MASKED = kAllLandmarks>
 __global__ void __launch_bounds__(32) k_solve_thread(const __grid_constant__ SolveArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -306,15 +373,14 @@ __global__ void __launch_bounds__(32) k_solve_thread(const __grid_constant__ Sol
         int best_p;
         if constexpr (MASKED) {
             // spare lanes of a ragged tile shadow the last problem, as their rows do (RowTile::acquire)
-            PtsMasked<PtsRow<T> > pts;
+            PtsOf<MASKED, PtsRow<T> > pts;
             pts.row = tile_buf.acquire(lane, valid);
             pts.idx = sel ? sIdx : nullptr;
-            pts.words = a.vis + (size_t)(b0 + (lane < valid ? lane : valid - 1)) * a.vis_words;
-            pts.nvis = count_visible(pts.words, pts.idx, a.n);
+            bind_problem(pts, a, b0 + (lane < valid ? lane : valid - 1));
             T* myC = sC + (size_t)lane * a.n_patterns * PNP_PATC;
             if (method_uses_patc(METHOD))
                 for (int p = 0; p < a.n_patterns; ++p) pattern_constants_masked<T, 1>(pts, sP + (size_t)p * a.n * 3, a.n, myC + p * PNP_PATC, 0);
-            solve_all_patterns<T, METHOD, 1, PtsMasked<PtsRow<T> > >(pts, sP, myC, a.n, a.n_patterns, 0, a.prm, best, best_p);
+            solve_all_patterns<T, METHOD, 1, PtsOf<MASKED, PtsRow<T> > >(pts, sP, myC, a.n, a.n_patterns, 0, a.prm, best, best_p);
             if (pts.nvis < kMinVisible) too_few_landmarks<T>(best, best_p);
         } else {
             PtsRow<T> pts;
@@ -361,6 +427,7 @@ struct MomArgs {
     // masked kernels: [B, vis_words] visibility bits, and the per-problem pattern moments [kPatternMoments][ld] in the workspace
     const uint32_t* vis; int vis_words;
     T* pmom;
+    const float* wts;       // weighted kernels: [B, n_total] per-landmark weights; pmom then has PNP_NPMOM_W rows
 };
 
 template <typename T>
@@ -407,7 +474,7 @@ __global__ void __launch_bounds__(32) k_pattern_constants(const __grid_constant_
 
 // PASS 0: moments.  PASS 1: residual at the stored state (LM: x before the last update; F2: tail).
 // MASKED: over each problem's visible landmarks; PASS 0 also stores the problem's pattern moments (a.pmom).
-template <typename T, int METHOD, int PASS, bool MASKED = false>
+template <typename T, int METHOD, int PASS, int MASKED = kAllLandmarks>
 __global__ void __launch_bounds__(32) k_stream_thread(const __grid_constant__ MomArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -436,20 +503,21 @@ __global__ void __launch_bounds__(32) k_stream_thread(const __grid_constant__ Mo
         pts.row = tile_buf.acquire(lane, valid);
         pts.idx = sel ? sIdx : nullptr;
         if constexpr (MASKED) {
-            PtsMasked<PtsRow<T> > pm;
+            PtsOf<MASKED, PtsRow<T> > pm;
             static_cast<PtsRow<T>&>(pm) = pts;
-            pm.words = a.vis + (size_t)b * a.vis_words;
-            pm.nvis = count_visible(pm.words, pm.idx, a.n);
+            if constexpr (MASKED == kWeights && PASS == 1) bind_problem_counted(pm, a, b);
+            else bind_problem(pm, a, b);
             if (PASS == 0) {
                 Moments<T> mom;
-                accumulate_moments<T, 1, PtsMasked<PtsRow<T> >, method_with_w(METHOD), method_with_s(METHOD)>(pm, sP, a.n, 0, mom);
-                double pmo[kPatternMoments];
-                pattern_moments_masked<T, 1>(pm, sP, a.n, 0, pmo);
+                accumulate_moments<T, 1, PtsOf<MASKED, PtsRow<T> >, method_with_w(METHOD), method_with_s(METHOD)>(pm, sP, a.n, 0, mom);
+                double pmo[kPatternMoments], crow = 0.0;
+                pattern_moments_masked<T, 1>(pm, sP, a.n, 0, pmo, &crow);
                 if (ok) {
 #pragma unroll
                     for (int k = 0; k < method_nmom(METHOD); ++k) a.mom[(size_t)k * a.ld + b] = mom.at(k);
 #pragma unroll
                     for (int k = 0; k < kPatternMoments; ++k) a.pmom[(size_t)k * a.ld + b] = (T)pmo[k];
+                    if constexpr (MASKED == kWeights) a.pmom[(size_t)kPatternMoments * a.ld + b] = (T)crow;
                 }
             } else {
                 T res;
@@ -457,14 +525,14 @@ __global__ void __launch_bounds__(32) k_stream_thread(const __grid_constant__ Mo
                     T x[12];
 #pragma unroll
                     for (int k = 0; k < 12; ++k) x[k] = st[k];
-                    res = lm_residual_direct<T, 1, PtsMasked<PtsRow<T> > >(pm, sP, a.n, 0, x);
+                    res = lm_residual_direct<T, 1, PtsOf<MASKED, PtsRow<T> > >(pm, sP, a.n, 0, x);
                 } else {
                     F2Tail<T> f;
 #pragma unroll
                     for (int k = 0; k < 3; ++k) f.phi3[k] = st[k];
 #pragma unroll
                     for (int k = 0; k < 4; ++k) { f.pxn[k] = st[3 + k]; f.pyn[k] = st[7 + k]; }
-                    res = f2_residual_direct<T, 1, PtsMasked<PtsRow<T> > >(pm, sP, a.n, 0, f);
+                    res = f2_residual_direct<T, 1, PtsOf<MASKED, PtsRow<T> > >(pm, sP, a.n, 0, f);
                 }
                 if (pm.nvis < kMinVisible) res = nan_of<T>();     // not solved (a sum over no landmark would read 0)
                 if (ok && a.res) a.res[b] = res;
@@ -508,7 +576,7 @@ __global__ void __launch_bounds__(32) k_stream_thread(const __grid_constant__ Mo
 #endif
 constexpr int kStreamUnroll = PNP_STREAM_UNROLL;
 // MASKED: over each problem's visible landmarks (a running mask word per chunk); PASS 0 also stores the pattern moments
-template <typename T, int METHOD, int PASS, bool MASKED = false>
+template <typename T, int METHOD, int PASS, int MASKED = kAllLandmarks>
 __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ MomArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -548,8 +616,11 @@ __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ Mom
                 for (int k = 0; k < 4; ++k) { f.pxn[k] = st[3 + k]; f.pyn[k] = st[7 + k]; }
             }
         }
-        const uint32_t* vw = MASKED ? a.vis + (size_t)b * a.vis_words : nullptr;
+        const uint32_t* vw = MASKED == kMaskBits ? a.vis + (size_t)b * a.vis_words : nullptr;
+        const float* wr = MASKED == kWeights ? a.wts + (size_t)b * a.n_total : nullptr;   // one __ldg per lane and landmark
         double pmo[kPatternMoments];
+        int n_part = 0;                                       // weighted: landmarks taking part, and whether a weight is not 1
+        bool nonunit = false;
         if constexpr (MASKED && PASS == 0) {
 #pragma unroll
             for (int e = 0; e < kPatternMoments; ++e) pmo[e] = 0.0;
@@ -558,38 +629,45 @@ __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ Mom
             const V2* row = rs.wait(c, lane);
             const int cnt = rs.count(c), i0 = c * rs.chunk;
             uint32_t word = 0;                                // MASKED: bit 0 = landmark i0 + k
-            if constexpr (MASKED) word = __ldg(vw + (i0 >> 5)) >> (i0 & 31);
+            if constexpr (MASKED == kMaskBits) word = __ldg(vw + (i0 >> 5)) >> (i0 & 31);
 #pragma unroll kStreamUnroll
             for (int k = 0; k < cnt; ++k) {
-                if constexpr (MASKED) {
+                float wf = 1.0f;                              // the landmark's weight
+                if constexpr (MASKED == kMaskBits) {
                     const int i = i0 + k;
                     const bool v = word & 1u;
                     word = ((i + 1) & 31) ? (word >> 1) : ((i + 1 < a.n) ? __ldg(vw + ((i + 1) >> 5)) : 0u);
                     if (!v) continue;
+                } else if constexpr (MASKED == kWeights) {
+                    wf = __ldg(wr + i0 + k);
+                    if (!weight_takes_part(wf)) continue;
+                    if (PASS == 0) { ++n_part; nonunit |= (wf != 1.0f); }
                 }
+                const T w = (T)wf;
                 const V2 px = row[k];
                 T bx, by;                                     // nu = K^-1 [u, v, 1]^T (:3305)
                 normalise_px<T>(px.x, px.y, k00, k01, k02, k10, k11, k12, bx, by);
                 const T th[3] = { sP[3 * (i0 + k)], sP[3 * (i0 + k) + 1], sP[3 * (i0 + k) + 2] };
                 if constexpr (MASKED && PASS == 0) {
+                    const double dw = (double)wf;
 #pragma unroll
                     for (int p = 0; p < 3; ++p) {
 #pragma unroll
-                        for (int q = p; q < 3; ++q) pmo[s3(p, q)] = fma((double)th[p], (double)th[q], pmo[s3(p, q)]);
-                        pmo[6 + p] += (double)th[p];
+                        for (int q = p; q < 3; ++q) pmo[s3(p, q)] = fma(dw * (double)th[p], (double)th[q], pmo[s3(p, q)]);
+                        pmo[6 + p] += dw * (double)th[p];
                     }
-                    pmo[9] += 1.0;
+                    pmo[9] += dw;
                 }
                 if (PASS == 0) {
-                    mom.template add<method_with_w(METHOD), method_with_s(METHOD)>(th, bx, by);
+                    mom.template add<method_with_w(METHOD), method_with_s(METHOD)>(th, bx, by, w);
                 } else if (method_lm_residual(METHOD)) {
-                    lr.add(th, bx, by, acc0);                 // z - hx (:3750, :2679)
+                    lr.add(th, bx, by, acc0, w);              // z - hx (:3750, :2679)
                 } else {
                     const T db = T(1) + (th[0] * f.phi3[0] + th[1] * f.phi3[1] + th[2] * f.phi3[2]);
                     const T dx = th[0] * f.pxn[0] + th[1] * f.pxn[1] + th[2] * f.pxn[2] + f.pxn[3];
                     const T dy = th[0] * f.pyn[0] + th[1] * f.pyn[1] + th[2] * f.pyn[2] + f.pyn[3];
                     const T ex = bx * db - dx, ey = by * db - dy;
-                    acc0 = t_fma(ex, ex, acc0); acc1 = t_fma(ey, ey, acc1);
+                    acc0 = t_fma(w * ex, ex, acc0); acc1 = t_fma(w * ey, ey, acc1);
                 }
             }
             rs.done(c, lane);
@@ -602,11 +680,14 @@ __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ Mom
 #pragma unroll
                     for (int k = 0; k < kPatternMoments; ++k) a.pmom[(size_t)k * a.ld + b] = (T)pmo[k];
                 }
+                if constexpr (MASKED == kWeights) a.pmom[(size_t)kPatternMoments * a.ld + b] = (T)weighted_count_row(n_part, nonunit);
             } else if (a.res) {
                 if (method_lm_residual(METHOD)) a.res[b] = t_sqrt(acc0);   // :2681
                 else { const T nx = t_sqrt(acc0), ny = t_sqrt(acc1); a.res[b] = t_sqrt(nx * nx + ny * ny); }   // :3374
-                if constexpr (MASKED) {
+                if constexpr (MASKED == kMaskBits) {
                     if (count_visible(vw, nullptr, a.n) < kMinVisible) a.res[b] = nan_of<T>();   // not solved
+                } else if constexpr (MASKED == kWeights) {   // the moments pass's count row (weighted_count_row)
+                    if ((int)a.pmom[(size_t)kPatternMoments * a.ld + b] < kMinVisible) a.res[b] = nan_of<T>();
                 }
             }
         }
@@ -619,7 +700,7 @@ __global__ void __launch_bounds__(32) k_stream_chunk(const __grid_constant__ Mom
 }
 
 // MASKED: over each problem's visible landmarks; PASS 0 also stores the pattern moments
-template <typename T, int METHOD, int PASS, bool MASKED = false>
+template <typename T, int METHOD, int PASS, int MASKED = kAllLandmarks>
 __global__ void __launch_bounds__(256) k_stream_warp(const __grid_constant__ MomArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -635,15 +716,15 @@ __global__ void __launch_bounds__(256) k_stream_warp(const __grid_constant__ Mom
     for (long long b = (long long)blockIdx.x * nwarps + warp; b < a.B; b += (long long)gridDim.x * nwarps) {
         pts.row = a.uv + (size_t)b * a.n_total * 2;
         if constexpr (MASKED) {
-            PtsMasked<PtsGlobal<T> > pm;
+            PtsOf<MASKED, PtsGlobal<T> > pm;
             static_cast<PtsGlobal<T>&>(pm) = pts;
-            pm.words = a.vis + (size_t)b * a.vis_words;
-            pm.nvis = count_visible(pm.words, pm.idx, a.n);
+            if constexpr (MASKED == kWeights && PASS == 1) bind_problem_counted(pm, a, b);
+            else bind_problem(pm, a, b);
             if (PASS == 0) {
                 Moments<T> mom;
-                accumulate_moments<T, 32, PtsMasked<PtsGlobal<T> >, method_with_w(METHOD), method_with_s(METHOD)>(pm, sP, a.n, lane, mom);
-                double pmo[kPatternMoments];
-                pattern_moments_masked<T, 32>(pm, sP, a.n, lane, pmo);
+                accumulate_moments<T, 32, PtsOf<MASKED, PtsGlobal<T> >, method_with_w(METHOD), method_with_s(METHOD)>(pm, sP, a.n, lane, mom);
+                double pmo[kPatternMoments], crow = 0.0;
+                pattern_moments_masked<T, 32>(pm, sP, a.n, lane, pmo, &crow);
                 T mine = T(0);
 #pragma unroll
                 for (int k = 0; k < method_nmom(METHOD); ++k) if (lane == k) mine = mom.at(k);
@@ -652,20 +733,23 @@ __global__ void __launch_bounds__(256) k_stream_warp(const __grid_constant__ Mom
 #pragma unroll
                 for (int k = 0; k < kPatternMoments; ++k) if (lane == k) pmine = pmo[k];
                 if (lane < kPatternMoments) a.pmom[(size_t)lane * a.ld + b] = (T)pmine;
+                if constexpr (MASKED == kWeights) {
+                    if (lane == kPatternMoments) a.pmom[(size_t)lane * a.ld + b] = (T)crow;
+                }
             } else {
                 T res;
                 if (method_lm_residual(METHOD)) {
                     T x[12];
 #pragma unroll
                     for (int k = 0; k < 12; ++k) x[k] = a.tail[(size_t)k * a.ld + b];
-                    res = lm_residual_direct<T, 32, PtsMasked<PtsGlobal<T> > >(pm, sP, a.n, lane, x);
+                    res = lm_residual_direct<T, 32, PtsOf<MASKED, PtsGlobal<T> > >(pm, sP, a.n, lane, x);
                 } else {
                     F2Tail<T> f;
 #pragma unroll
                     for (int k = 0; k < 3; ++k) f.phi3[k] = a.tail[(size_t)k * a.ld + b];
 #pragma unroll
                     for (int k = 0; k < 4; ++k) { f.pxn[k] = a.tail[(size_t)(3 + k) * a.ld + b]; f.pyn[k] = a.tail[(size_t)(7 + k) * a.ld + b]; }
-                    res = f2_residual_direct<T, 32, PtsMasked<PtsGlobal<T> > >(pm, sP, a.n, lane, f);
+                    res = f2_residual_direct<T, 32, PtsOf<MASKED, PtsGlobal<T> > >(pm, sP, a.n, lane, f);
                 }
                 if (pm.nvis < kMinVisible) res = nan_of<T>();     // not solved (a sum over no landmark would read 0)
                 if (lane == 0 && a.res) a.res[b] = res;
@@ -874,7 +958,7 @@ PNP_DEV void run_filter_with_tail(const Pts& pts, const T* sP, const T* sC, int 
 }
 
 // MASKED: each lane solves on its problem's visible landmarks with its own constants
-template <typename T, int METHOD, bool MASKED = false>
+template <typename T, int METHOD, int MASKED = kAllLandmarks>
 __global__ void __launch_bounds__(32) k_fixup_thread(const __grid_constant__ MomArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -908,13 +992,12 @@ __global__ void __launch_bounds__(32) k_fixup_thread(const __grid_constant__ Mom
         Result<T> out;
         T xt[12];
         if constexpr (MASKED) {
-            PtsMasked<PtsRow<T> > pm;
+            PtsOf<MASKED, PtsRow<T> > pm;
             static_cast<PtsRow<T>&>(pm) = pts;
-            pm.words = a.vis + (size_t)(tile * kTileProblems + (lane < valid ? lane : valid - 1)) * a.vis_words;
-            pm.nvis = count_visible(pm.words, pm.idx, a.n);
+            bind_problem(pm, a, tile * kTileProblems + (lane < valid ? lane : valid - 1));
             T* myC = sC + (size_t)lane * PNP_PATC;
             pattern_constants_masked<T, 1>(pm, sP, a.n, myC, 0);
-            run_filter_with_tail<T, METHOD, 1, PtsMasked<PtsRow<T> > >(pm, sP, myC, a.n, 0, a.prm, xt, out);
+            run_filter_with_tail<T, METHOD, 1, PtsOf<MASKED, PtsRow<T> > >(pm, sP, myC, a.n, 0, a.prm, xt, out);
         } else {
             run_filter_with_tail<T, METHOD, 1, PtsRow<T> >(pts, sP, sC, a.n, 0, a.prm, xt, out);
         }
@@ -927,7 +1010,7 @@ __global__ void __launch_bounds__(32) k_fixup_thread(const __grid_constant__ Mom
 }
 
 // MASKED: each warp solves on its problem's visible landmarks with the problem's constants
-template <typename T, int METHOD, bool MASKED = false>
+template <typename T, int METHOD, int MASKED = kAllLandmarks>
 __global__ void __launch_bounds__(256) k_fixup_warp(const __grid_constant__ MomArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -954,14 +1037,13 @@ __global__ void __launch_bounds__(256) k_fixup_warp(const __grid_constant__ MomA
         Result<T> out;
         T xt[12];
         if constexpr (MASKED) {
-            PtsMasked<PtsGlobal<T> > pm;
+            PtsOf<MASKED, PtsGlobal<T> > pm;
             static_cast<PtsGlobal<T>&>(pm) = pts;
-            pm.words = a.vis + (size_t)b * a.vis_words;
-            pm.nvis = count_visible(pm.words, pm.idx, a.n);
+            bind_problem(pm, a, b);
             T* myC = sC + (size_t)warp * PNP_PATC;
             pattern_constants_masked<T, 32>(pm, sP, a.n, myC, lane);
             __syncwarp();
-            run_filter_with_tail<T, METHOD, 32, PtsMasked<PtsGlobal<T> > >(pm, sP, myC, a.n, lane, a.prm, xt, out);
+            run_filter_with_tail<T, METHOD, 32, PtsOf<MASKED, PtsGlobal<T> > >(pm, sP, myC, a.n, lane, a.prm, xt, out);
             __syncwarp();                                     // the next problem's constants replace these
         } else {
             run_filter_with_tail<T, METHOD, 32, PtsGlobal<T> >(pts, sP, sC, a.n, lane, a.prm, xt, out);
@@ -977,9 +1059,10 @@ __global__ void __launch_bounds__(256) k_fixup_warp(const __grid_constant__ MomA
 // The O(1)-per-iteration part of the moment mapping for one problem per thread: moments parked in shared
 // memory ([PNP_NMOM][stride] columns, this thread's column at sMomCol) -> pose `out` and the 12 numbers the
 // residual pass needs (LM: the state before the last update; F2: its tail).
-template <typename T, int METHOD>
+// NP: NoPts, or NoPtsWeighted (the filters' exit test under weights)
+template <typename T, int METHOD, typename NP = NoPts>
 __device__ __forceinline__ void iterate_core(T* sMomCol, int stride, const T* sC, const SolverPrm<T>& prm,
-                                             T (&st)[PNP_NTAIL], Result<T>& out)
+                                             T (&st)[PNP_NTAIL], Result<T>& out, const NP& np = NP())
 {
     MomentsRef<T> mom;
     mom.base = sMomCol;
@@ -1000,12 +1083,12 @@ __device__ __forceinline__ void iterate_core(T* sMomCol, int stride, const T* sC
 #pragma unroll
         for (int k = 0; k < PNP_NMOM; ++k) mr.at(k) = sMomCol[k * stride];
         T xt[12];
-        solve_qeif_from_moments<T>(mr, sC, prm, xt, out);
+        solve_qeif_from_moments<T, NP>(mr, sC, prm, xt, out, np);
 #pragma unroll
         for (int k = 0; k < 12; ++k) st[k] = xt[k];
     } else if (METHOD == PNPB200_METHOD_EIF2) {
         T xt[12];
-        solve_eif2_from_moments<T, MomentsRef<T> >(mom, sC, prm, xt, out);   // 12 x 12 system: moments stay in shared memory
+        solve_eif2_from_moments<T, MomentsRef<T>, NP>(mom, sC, prm, xt, out, np);   // 12 x 12 system: moments stay in shared memory
 #pragma unroll
         for (int k = 0; k < 12; ++k) st[k] = xt[k];
     } else if (METHOD == PNPB200_METHOD_LM_PLUS) {
@@ -1056,7 +1139,7 @@ __device__ __forceinline__ void write_pose(const MomArgs<T>& a, long long b, con
 }
 
 // MASKED: every thread builds its problem's constants from the pattern moments of the workspace (a.pmom)
-template <typename T, int METHOD, int BLOCK, bool MASKED = false>
+template <typename T, int METHOD, int BLOCK, int MASKED = kAllLandmarks>
 __device__ __forceinline__ void iterate_body(const MomArgs<T>& a)
 {
     constexpr int kIterBlock = BLOCK;
@@ -1083,7 +1166,18 @@ __device__ __forceinline__ void iterate_body(const MomArgs<T>& a)
     __syncthreads();
     Result<T> out;
     T st[PNP_NTAIL];
-    iterate_core<T, METHOD>(sMom + threadIdx.x, kIterBlock, myC, a.prm, st, out);
+    if constexpr (MASKED == kWeights) {
+        // sum w is the constants' count; the row behind the pattern moments holds the landmarks taking part (weighted_count_row)
+        const double crow = (double)a.pmom[(size_t)kPatternMoments * a.ld + b];
+        nvis = (int)crow;
+        NoPtsWeighted<T> np;
+        np.wsum = myC[9];
+        np.nland = (T)nvis;
+        np.extra = (crow != (double)nvis) ? T(4) : T(0);
+        iterate_core<T, METHOD, NoPtsWeighted<T> >(sMom + threadIdx.x, kIterBlock, myC, a.prm, st, out, np);
+    } else {
+        iterate_core<T, METHOD>(sMom + threadIdx.x, kIterBlock, myC, a.prm, st, out);
+    }
     if constexpr (MASKED) {
         if (nvis < kMinVisible) {                             // not solved: NaN pose, NaN state (so NaN res_norm), 0 iterations, unmarked
             int unused;
@@ -1106,13 +1200,13 @@ __device__ __forceinline__ void iterate_body(const MomArgs<T>& a)
 // 16 Ki registers: 2 warps per sub-partition from 169 to 255 registers, 3 at <= 168 (FP64 LM wants ~214 and spills
 // ~26 doubles at 168).  Measured for 1 Mi x 68 LM FP64 on B200 (final step): 0.886 ms at 224, 0.904 at 255 (240 used),
 // 0.912 at 184, 0.905 at 168, 0.931 at 160 -- the third warp does not pay for its spills.
-template <typename T, int METHOD, int BLOCK, int MAXREG, bool MASKED = false>
+template <typename T, int METHOD, int BLOCK, int MAXREG, int MASKED = kAllLandmarks>
 __global__ void __launch_bounds__(BLOCK) __maxnreg__(MAXREG) k_iterate(const __grid_constant__ MomArgs<T> a)
 {
     iterate_body<T, METHOD, BLOCK, MASKED>(a);
 }
 
-template <typename T, int METHOD, int BLOCK, int MAXREG, bool MASKED = false>
+template <typename T, int METHOD, int BLOCK, int MAXREG, int MASKED = kAllLandmarks>
 static void launch_iterate_as(const MomArgs<T>& m, cudaStream_t stream)
 {
     k_iterate<T, METHOD, BLOCK, MAXREG, MASKED><<<(unsigned)((m.B + BLOCK - 1) / BLOCK), BLOCK, 0, stream>>>(m); count_kernel_launches(1);
@@ -1121,6 +1215,10 @@ static void launch_iterate_as(const MomArgs<T>& m, cudaStream_t stream)
 template <typename T, int METHOD>
 static void launch_iterate(const MomArgs<T>& m, int tune, cudaStream_t stream)
 {
+    if (m.wts) {
+        launch_iterate_as<T, METHOD, 32, (METHOD == PNPB200_METHOD_EIF2 || METHOD == PNP_METHOD_QEIF_HYBRID) ? 255 : 224, kWeights>(m, stream);
+        return;
+    }
     if (m.vis) {
         launch_iterate_as<T, METHOD, 32, (METHOD == PNPB200_METHOD_EIF2 || METHOD == PNP_METHOD_QEIF_HYBRID) ? 255 : 224, true>(m, stream);
         return;
@@ -1147,7 +1245,7 @@ static void launch_iterate(const MomArgs<T>& m, int tune, cudaStream_t stream)
 constexpr int kWarpsPerBlock = 8;
 
 // MASKED: problem b sees only its visible landmarks (a.vis); every warp computes its problem's constants
-template <typename T, int METHOD, bool MASKED = false>
+template <typename T, int METHOD, int MASKED = kAllLandmarks>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32) k_solve_warp(const __grid_constant__ SolveArgs<T> a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -1172,17 +1270,16 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) k_solve_warp(const __grid
         Result<T> best;
         int best_p;
         if constexpr (MASKED) {
-            PtsMasked<PtsGlobal<T> > pm;
+            PtsOf<MASKED, PtsGlobal<T> > pm;
             static_cast<PtsGlobal<T>&>(pm) = pts;
-            pm.words = a.vis + (size_t)b * a.vis_words;
-            pm.nvis = count_visible(pm.words, pm.idx, a.n);
+            bind_problem(pm, a, b);
             T* myC = sC + (size_t)warp * a.n_patterns * PNP_PATC;
             if (method_uses_patc(METHOD)) {
                 for (int p = 0; p < a.n_patterns; ++p)
                     pattern_constants_masked<T, 32>(pm, sP + (size_t)p * a.n * 3, a.n, myC + p * PNP_PATC, lane);
                 __syncwarp();
             }
-            solve_all_patterns<T, METHOD, 32, PtsMasked<PtsGlobal<T> > >(pm, sP, myC, a.n, a.n_patterns, lane, a.prm, best, best_p);
+            solve_all_patterns<T, METHOD, 32, PtsOf<MASKED, PtsGlobal<T> > >(pm, sP, myC, a.n, a.n_patterns, lane, a.prm, best, best_p);
             if (pm.nvis < kMinVisible) too_few_landmarks<T>(best, best_p);
             __syncwarp();                                     // the next problem's constants replace these
         } else {
@@ -1212,6 +1309,12 @@ static SolverPrm<T> make_prm(const pnpb200_params& p)
     return s;
 }
 
+// the instantiation of a kernel for a launch's MASKED mode
+static const void* mode_kernel(int mode, const void* all, const void* mask_bits, const void* weights)
+{
+    return mode == kWeights ? weights : (mode == kMaskBits ? mask_bits : all);
+}
+
 static long long persistent_grid(long long work_items, int sm_count, int per_sm)
 {
     if (per_sm < 1) per_sm = 1;
@@ -1230,6 +1333,7 @@ static int launch_moment_pass(int pass, const MomArgs<T>& full, long long b0, lo
     m.mom = full.mom + b0; m.tail = full.tail + b0;
     if (full.pmom) m.pmom = full.pmom + b0;
     if (full.vis) m.vis = full.vis + (size_t)b0 * full.vis_words;
+    if (full.wts) m.wts = full.wts + (size_t)b0 * full.n_total;
     if (full.R) m.R = full.R + b0 * 9;
     if (full.t) m.t = full.t + b0 * 3;
     if (full.euler) m.euler = full.euler + b0 * 3;
@@ -1239,19 +1343,25 @@ static int launch_moment_pass(int pass, const MomArgs<T>& full, long long b0, lo
     if (pass == 1) { launch_iterate<T, METHOD>(m, tune, stream); return PNPB200_OK; }
     const long long n_tiles = (nb + kTileProblems - 1) / kTileProblems;
     const unsigned tile_grid = (unsigned)(n_tiles < 0x7fffffffLL ? n_tiles : 0x7fffffffLL);
-    const bool masked = m.vis != nullptr;
+    const bool masked = m.vis != nullptr;                    // (m.wts: the weighted kernels)
     if (shape == 0) {                                         // chunked row streaming
         m.row_pitch = sg.pitch;
         m.use_tma = sg.chunk;                                 // RowStream: points per chunk
         m.use_tmap = (sg.pitch == sg.chunk * 2) ? make_row_tensor_map(&m.tmap, m.uv, (int)sizeof(T), nb, m.n_total, sg.chunk) : 0;
-        if (masked) {
+        if (m.wts) {
+            if (pass == 0) k_stream_chunk<T, METHOD, 0, kWeights><<<tile_grid, 32, smem, stream>>>(m);
+            else           k_stream_chunk<T, METHOD, 1, kWeights><<<tile_grid, 32, smem, stream>>>(m);
+        } else if (masked) {
             if (pass == 0) k_stream_chunk<T, METHOD, 0, true><<<tile_grid, 32, smem, stream>>>(m);
             else           k_stream_chunk<T, METHOD, 1, true><<<tile_grid, 32, smem, stream>>>(m);
         } else if (pass == 0) k_stream_chunk<T, METHOD, 0><<<tile_grid, 32, smem, stream>>>(m);
         else           k_stream_chunk<T, METHOD, 1><<<tile_grid, 32, smem, stream>>>(m);
         count_kernel_launches(1);
     } else if (shape == 1) {                                  // whole-row tiles
-        if (masked) {
+        if (m.wts) {
+            if (pass == 0) k_stream_thread<T, METHOD, 0, kWeights><<<tile_grid, 32, smem, stream>>>(m);
+            else           k_stream_thread<T, METHOD, 1, kWeights><<<tile_grid, 32, smem, stream>>>(m);
+        } else if (masked) {
             if (pass == 0) k_stream_thread<T, METHOD, 0, true><<<tile_grid, 32, smem, stream>>>(m);
             else           k_stream_thread<T, METHOD, 1, true><<<tile_grid, 32, smem, stream>>>(m);
         } else if (pass == 0) k_stream_thread<T, METHOD, 0><<<tile_grid, 32, smem, stream>>>(m);
@@ -1264,7 +1374,10 @@ static int launch_moment_pass(int pass, const MomArgs<T>& full, long long b0, lo
         count_kernel_launches(1);
     } else {                                                  // one problem per warp, coalesced loads
         const unsigned grid = (unsigned)persistent_grid((nb + 7) / 8, dp.sm_count, per_sm);
-        if (masked) {
+        if (m.wts) {
+            if (pass == 0) k_stream_warp<T, METHOD, 0, kWeights><<<grid, 256, smem, stream>>>(m);
+            else           k_stream_warp<T, METHOD, 1, kWeights><<<grid, 256, smem, stream>>>(m);
+        } else if (masked) {
             if (pass == 0) k_stream_warp<T, METHOD, 0, true><<<grid, 256, smem, stream>>>(m);
             else           k_stream_warp<T, METHOD, 1, true><<<grid, 256, smem, stream>>>(m);
         } else if (pass == 0) k_stream_warp<T, METHOD, 0><<<grid, 256, smem, stream>>>(m);
@@ -1277,7 +1390,7 @@ static int launch_moment_pass(int pass, const MomArgs<T>& full, long long b0, lo
 // A handful of marked tiles (the normal case on detected pixels) is latency: one problem per warp finishes them in a few
 // microseconds; thousands of them (noise-free pixels) is throughput: one problem per thread.  Both kernels read the count and
 // exactly one of them acts (rows too long for a tile: always per warp).
-template <typename T, int METHOD, bool MASKED>
+template <typename T, int METHOD, int MASKED>
 static int launch_filter_fixup_as(const MomArgs<T>& m, const RowGeom& g, bool by_thread, size_t thread_smem, size_t warp_smem,
                                   const DeviceProps& dp, cudaStream_t stream)
 {
@@ -1310,8 +1423,9 @@ template <typename T, int METHOD>
 static int launch_filter_fixup(const MomArgs<T>& m, const RowGeom& g, bool by_thread, size_t thread_smem, size_t warp_smem,
                                const DeviceProps& dp, cudaStream_t stream)
 {
-    if (m.vis) return launch_filter_fixup_as<T, METHOD, true>(m, g, by_thread, thread_smem, warp_smem, dp, stream);
-    return launch_filter_fixup_as<T, METHOD, false>(m, g, by_thread, thread_smem, warp_smem, dp, stream);
+    if (m.wts) return launch_filter_fixup_as<T, METHOD, kWeights>(m, g, by_thread, thread_smem, warp_smem, dp, stream);
+    if (m.vis) return launch_filter_fixup_as<T, METHOD, kMaskBits>(m, g, by_thread, thread_smem, warp_smem, dp, stream);
+    return launch_filter_fixup_as<T, METHOD, kAllLandmarks>(m, g, by_thread, thread_smem, warp_smem, dp, stream);
 }
 
 // LM / linear F2 with one pattern: moments -> iterate -> residual (see the kernels' header).
@@ -1333,10 +1447,12 @@ static int launch_moment(const SolveArgs<T>& a, const DeviceProps& dp, cudaStrea
     const bool by_thread = g.tile_bytes <= 48 * 1024 && thread_smem <= (size_t)dp.max_smem_optin;
     if (!by_thread && warp_smem > (size_t)dp.max_smem_optin) return PNPB200_ETOOLARGE;
 
-    const bool masked = a.vis != nullptr;
+    const bool weighted = a.wts != nullptr;
+    const bool masked = a.vis != nullptr || weighted;        // per-problem pattern constants
     T* ws = nullptr;
-    // masked: the per-problem pattern moments ride behind the moments ([kPatternMoments][B])
-    const size_t ws_elems = (size_t)(PNP_NMOM + (masked ? kPatternMoments : 0) + PNP_NTAIL) * (size_t)a.B + PNP_PATC;
+    // masked: the per-problem pattern moments ride behind the moments ([kPatternMoments][B]; weighted: PNP_NPMOM_W rows)
+    const int pm_rows = weighted ? PNP_NPMOM_W : (masked ? kPatternMoments : 0);
+    const size_t ws_elems = (size_t)(PNP_NMOM + pm_rows + PNP_NTAIL) * (size_t)a.B + PNP_PATC;
     const bool own_ws = !(a.ws && a.ws_bytes >= ws_elems * sizeof(T));
     if (own_ws) PNP_CUDA_OK(cudaMallocAsync((void**)&ws, ws_elems * sizeof(T), stream));
     else ws = (T*)a.ws;
@@ -1352,8 +1468,8 @@ static int launch_moment(const SolveArgs<T>& a, const DeviceProps& dp, cudaStrea
     for (int e = 0; e < 6; ++e) m.kinv[e] = a.kinv[e];
     m.prm = a.prm;
     m.mom = ws; m.tail = ws + (size_t)PNP_NMOM * a.B; m.patc = m.tail + (size_t)PNP_NTAIL * a.B;
-    m.vis = a.vis; m.vis_words = a.vis_words; m.pmom = nullptr;
-    if (masked) { m.pmom = ws + (size_t)PNP_NMOM * a.B; m.tail = m.pmom + (size_t)kPatternMoments * a.B; m.patc = m.tail + (size_t)PNP_NTAIL * a.B; }
+    m.vis = a.vis; m.vis_words = a.vis_words; m.pmom = nullptr; m.wts = a.wts;
+    if (masked) { m.pmom = ws + (size_t)PNP_NMOM * a.B; m.tail = m.pmom + (size_t)pm_rows * a.B; m.patc = m.tail + (size_t)PNP_NTAIL * a.B; }
     m.R = a.R; m.t = a.t; m.euler = a.euler; m.res = a.res; m.iters = a.iters; m.best = a.best;
     m.use_tmap = 0;
     struct ItersGuard { void* p; cudaStream_t st; ~ItersGuard() { if (p) cudaFreeAsync(p, st); } } iters_guard = { nullptr, stream }, list_guard = { nullptr, stream };
@@ -1373,14 +1489,19 @@ static int launch_moment(const SolveArgs<T>& a, const DeviceProps& dp, cudaStrea
     const StreamGeom sg = stream_geometry<T>(a.n_total);
     int shape, per_sm = 1;
     size_t smem;
+    const int mode = weighted ? kWeights : (masked ? kMaskBits : kAllLandmarks);
     if (by_thread && !a.idx_mode && sg.use_stream && a.tune != 9) {
         shape = 0; smem = 2 * sg.buf_bytes + pat_bytes + 32;
-        PNP_CUDA_OK(set_dynamic_smem(masked ? (const void*)k_stream_chunk<T, METHOD, 0, true> : (const void*)k_stream_chunk<T, METHOD, 0>, smem));
-        PNP_CUDA_OK(set_dynamic_smem(masked ? (const void*)k_stream_chunk<T, METHOD, 1, true> : (const void*)k_stream_chunk<T, METHOD, 1>, smem));
+        PNP_CUDA_OK(set_dynamic_smem(mode_kernel(mode, (const void*)k_stream_chunk<T, METHOD, 0>, (const void*)k_stream_chunk<T, METHOD, 0, kMaskBits>,
+                                                 (const void*)k_stream_chunk<T, METHOD, 0, kWeights>), smem));
+        PNP_CUDA_OK(set_dynamic_smem(mode_kernel(mode, (const void*)k_stream_chunk<T, METHOD, 1>, (const void*)k_stream_chunk<T, METHOD, 1, kMaskBits>,
+                                                 (const void*)k_stream_chunk<T, METHOD, 1, kWeights>), smem));
     } else if (by_thread) {
         shape = 1; smem = thread_smem;
-        PNP_CUDA_OK(set_dynamic_smem(masked ? (const void*)k_stream_thread<T, METHOD, 0, true> : (const void*)k_stream_thread<T, METHOD, 0>, smem));
-        PNP_CUDA_OK(set_dynamic_smem(masked ? (const void*)k_stream_thread<T, METHOD, 1, true> : (const void*)k_stream_thread<T, METHOD, 1>, smem));
+        PNP_CUDA_OK(set_dynamic_smem(mode_kernel(mode, (const void*)k_stream_thread<T, METHOD, 0>, (const void*)k_stream_thread<T, METHOD, 0, kMaskBits>,
+                                                 (const void*)k_stream_thread<T, METHOD, 0, kWeights>), smem));
+        PNP_CUDA_OK(set_dynamic_smem(mode_kernel(mode, (const void*)k_stream_thread<T, METHOD, 1>, (const void*)k_stream_thread<T, METHOD, 1, kMaskBits>,
+                                                 (const void*)k_stream_thread<T, METHOD, 1, kWeights>), smem));
     } else if (!masked && !a.idx_mode && ((size_t)a.n_total * 2 * sizeof(T)) % 16 == 0 && a.tune != 9 &&
                a.n_total >= kRingPoints) {                // (no masked ring kernel: masked rows take the per-warp shape below)
         shape = 3;
@@ -1390,9 +1511,11 @@ static int launch_moment(const SolveArgs<T>& a, const DeviceProps& dp, cudaStrea
         PNP_CUDA_OK(blocks_per_sm(&per_sm, (const void*)k_stream_warp_tma<T, METHOD, 0>, kRingWarps * 32, smem));
     } else {
         shape = 2; smem = warp_smem;
-        const void* k0 = masked ? (const void*)k_stream_warp<T, METHOD, 0, true> : (const void*)k_stream_warp<T, METHOD, 0>;
+        const void* k0 = mode_kernel(mode, (const void*)k_stream_warp<T, METHOD, 0>, (const void*)k_stream_warp<T, METHOD, 0, kMaskBits>,
+                                     (const void*)k_stream_warp<T, METHOD, 0, kWeights>);
         PNP_CUDA_OK(set_dynamic_smem(k0, smem));
-        PNP_CUDA_OK(set_dynamic_smem(masked ? (const void*)k_stream_warp<T, METHOD, 1, true> : (const void*)k_stream_warp<T, METHOD, 1>, smem));
+        PNP_CUDA_OK(set_dynamic_smem(mode_kernel(mode, (const void*)k_stream_warp<T, METHOD, 1>, (const void*)k_stream_warp<T, METHOD, 1, kMaskBits>,
+                                                 (const void*)k_stream_warp<T, METHOD, 1, kWeights>), smem));
         PNP_CUDA_OK(blocks_per_sm(&per_sm, k0, 256, smem));
     }
 
@@ -1500,7 +1623,8 @@ static int launch_solve(const SolveArgs<T>& a, int mapping, cudaStream_t stream)
     // a visibility mask (a.vis) takes the same mapping as the call without it; its kernels keep the pattern constants per
     // problem.  (LM_TRUEJAC exists in the moment mapping only: no direct kernels, masked or not, are launched for it.)
     constexpr bool can_mask = METHOD != PNP_METHOD_LM_TRUEJAC;
-    const bool masked = a.vis != nullptr;
+    const bool weighted = a.wts != nullptr;
+    const bool masked = a.vis != nullptr || weighted;     // per-problem pattern constants
     const RowGeom g = row_geometry<T>(a.n_total);
     const size_t pat_bytes = ((size_t)a.n_patterns * a.n * 3 + (size_t)a.n_patterns * PNP_PATC) * sizeof(T);
     const size_t idx_bytes = a.idx_mode ? (size_t)a.n * sizeof(int32_t) : 0;
@@ -1518,7 +1642,8 @@ static int launch_solve(const SolveArgs<T>& a, int mapping, cudaStream_t stream)
     if (mapping == PNPB200_MAP_THREAD) {
         if (thread_smem > (size_t)dp.max_smem_optin) return PNPB200_ETOOLARGE;
         if constexpr (can_mask) {
-            if (masked) PNP_CUDA_OK(set_dynamic_smem((const void*)k_solve_thread<T, METHOD, true>, thread_smem));
+            if (masked) PNP_CUDA_OK(set_dynamic_smem(weighted ? (const void*)k_solve_thread<T, METHOD, kWeights>
+                                                              : (const void*)k_solve_thread<T, METHOD, kMaskBits>, thread_smem));
         }
         if (!masked) PNP_CUDA_OK(set_dynamic_smem((const void*)k_solve_thread<T, METHOD>, thread_smem));
         SolveArgs<T> at = a;
@@ -1529,7 +1654,8 @@ static int launch_solve(const SolveArgs<T>& a, int mapping, cudaStream_t stream)
         const int slot = a.profile ? g_prof.begin() : -1;
         g_prof.mark(slot, stream);
         if constexpr (can_mask) {
-            if (masked) k_solve_thread<T, METHOD, true><<<(unsigned)grid, 32, thread_smem, stream>>>(at);
+            if (weighted) k_solve_thread<T, METHOD, kWeights><<<(unsigned)grid, 32, thread_smem, stream>>>(at);
+            else if (masked) k_solve_thread<T, METHOD, true><<<(unsigned)grid, 32, thread_smem, stream>>>(at);
         }
         if (!masked) k_solve_thread<T, METHOD><<<(unsigned)grid, 32, thread_smem, stream>>>(at);
         count_kernel_launches(1);
@@ -1538,7 +1664,7 @@ static int launch_solve(const SolveArgs<T>& a, int mapping, cudaStream_t stream)
         if (warp_smem > (size_t)dp.max_smem_optin) return PNPB200_ETOOLARGE;
         const void* kfn = (const void*)k_solve_warp<T, METHOD>;
         if constexpr (can_mask) {
-            if (masked) kfn = (const void*)k_solve_warp<T, METHOD, true>;
+            if (masked) kfn = weighted ? (const void*)k_solve_warp<T, METHOD, kWeights> : (const void*)k_solve_warp<T, METHOD, true>;
         }
         PNP_CUDA_OK(set_dynamic_smem(kfn, warp_smem));
         int per_sm = 1;
@@ -1547,7 +1673,8 @@ static int launch_solve(const SolveArgs<T>& a, int mapping, cudaStream_t stream)
         const int slot = a.profile ? g_prof.begin() : -1;
         g_prof.mark(slot, stream);
         if constexpr (can_mask) {
-            if (masked) k_solve_warp<T, METHOD, true><<<(unsigned)grid, kWarpsPerBlock * 32, warp_smem, stream>>>(a);
+            if (weighted) k_solve_warp<T, METHOD, kWeights><<<(unsigned)grid, kWarpsPerBlock * 32, warp_smem, stream>>>(a);
+            else if (masked) k_solve_warp<T, METHOD, true><<<(unsigned)grid, kWarpsPerBlock * 32, warp_smem, stream>>>(a);
         }
         if (!masked) k_solve_warp<T, METHOD><<<(unsigned)grid, kWarpsPerBlock * 32, warp_smem, stream>>>(a);
         count_kernel_launches(1);
@@ -1563,7 +1690,7 @@ template <typename T>
 static int solve_typed(int method, long long B, int n_total, int n, const void* uv, const void* pattern,
                        int n_patterns, const int32_t* idx_host, const int32_t* idx_dev, const double* K, const pnpb200_params& prm,
                        void* R, void* t, void* euler, void* res, int32_t* iters, int32_t* best, cudaStream_t stream,
-                       const uint32_t* vis)
+                       const uint32_t* vis, const float* wts)
 {
     SolveArgs<T> a;
     a.uv = (const T*)uv; a.pattern = (const T*)pattern; a.idx = idx_dev;
@@ -1583,6 +1710,7 @@ static int solve_typed(int method, long long B, int n_total, int n, const void* 
     a.tune = (prm.flags >> 8) & 0xff;                     // undocumented tuning knob (register budget of k_iterate, slice size)
     a.ws = prm.workspace; a.ws_bytes = (prm.workspace && prm.workspace_bytes > 0) ? (size_t)prm.workspace_bytes : 0;
     a.vis = vis; a.vis_words = (n_total + 31) / 32;
+    a.wts = wts;
     switch (method) {
 #if PNP_GROUP == 0
     case PNPB200_METHOD_QEIF:
@@ -1627,7 +1755,7 @@ typedef float part_scalar;
 int PNP_PART_NAME(PNP_SOLVE_PART_ARGS)
 {
     return solve_typed<part_scalar>(method, B, n_total, n, uv, pattern, n_patterns, idx_host, idx_dev, K, prm, R, t, euler, res,
-                                    iters, best, stream, vis);
+                                    iters, best, stream, vis, wts);
 }
 
 }  // namespace pnpb200

@@ -104,26 +104,30 @@ struct Moments {
         sx0 = T(0); sy0 = T(0); sw0 = T(0);
     }
     // WITH_W = false skips the (bx^2 + by^2)-weighted moments, which the linear stage F2 never reads;
-    // WITH_S adds sum (bx^2 + by^2) itself (QEIF / EIF2 in the moment mapping)
+    // WITH_S adds sum (bx^2 + by^2) itself (QEIF / EIF2 in the moment mapping).
+    // w: the landmark's weight, multiplied into its scalar factors bx, by and bx^2 + by^2 (not into rounded products with
+    // theta), so that w = 1 rounds exactly as the unweighted sums do.
     template <bool WITH_W = true, bool WITH_S = false>
-    PNP_DEV void add(const T (&th)[3], T bx, T by)
+    PNP_DEV void add(const T (&th)[3], T bx, T by, T w = T(1))
     {
-        const T ww = WITH_W ? (bx * bx + by * by) : T(0);
+        const T wx = w * bx, wy = w * by;
+        // (bx^2 + by^2 with the contraction the unweighted sums compile to, written out)
+        const T ww = WITH_W ? w * t_fma(bx, bx, by * by) : T(0);
         if (WITH_S) sw0 += ww;
 #pragma unroll
         for (int a = 0; a < 3; ++a) {
 #pragma unroll
             for (int b = a; b < 3; ++b) {
                 const T m = th[a] * th[b];
-                Mx[s3(a, b)] = t_fma(bx, m, Mx[s3(a, b)]);
-                My[s3(a, b)] = t_fma(by, m, My[s3(a, b)]);
+                Mx[s3(a, b)] = t_fma(wx, m, Mx[s3(a, b)]);
+                My[s3(a, b)] = t_fma(wy, m, My[s3(a, b)]);
                 if (WITH_W) Mw[s3(a, b)] = t_fma(ww, m, Mw[s3(a, b)]);
             }
-            mx[a] = t_fma(bx, th[a], mx[a]);
-            my[a] = t_fma(by, th[a], my[a]);
+            mx[a] = t_fma(wx, th[a], mx[a]);
+            my[a] = t_fma(wy, th[a], my[a]);
             if (WITH_W) mw[a] = t_fma(ww, th[a], mw[a]);
         }
-        sx0 += bx; sy0 += by;
+        sx0 += wx; sy0 += wy;
     }
     template <int LPP, bool WITH_W = true, bool WITH_S = false>
     PNP_DEV void reduce()
@@ -187,7 +191,7 @@ PNP_DEV void accumulate_moments(const Pts& pts, const T* __restrict__ sP, int n,
         const T th[3] = { sP[3 * i], sP[3 * i + 1], sP[3 * i + 2] };
         T bx, by;
         pts.get(i, bx, by);
-        mom.template add<WITH_W, WITH_S>(th, bx, by);
+        mom.template add<WITH_W, WITH_S>(th, bx, by, (T)pts.weight(i));
     }
     mom.template reduce<LPP, WITH_W, WITH_S>();
 }
@@ -216,12 +220,26 @@ PNP_DEV T dot3(const T (&a)[3], const T (&b)[3]) { return a[0] * b[0] + a[1] * b
 // (iters = -1), and the fix-up pass of the moment mapping re-solves the marked problems point by point with the direct
 // kernel's arithmetic.  On detected pixels a few problems per million are marked; on noise-free pixels, where the
 // residual falls to rounding noise, most are -- the result is the direct mapping's either way.
+//
+// n: the number of landmarks summed into the moments; extra: roundings per summand beyond those of the unweighted sums;
+// wsum: the weight of n (d1^2 + d2^2) in the scale, i.e. the moment sum (w_i) (= n without weights).
+// Weighted moments (sum w_i f_i instead of sum f_i, f_i a landmark's product of pixels and pattern): the bound is a sum
+// over the moments of |coefficient| x (absolute error of that moment), and a moment of n summands accumulated one after
+// the other carries at most (n - 1 + k) eps sum |w_i f_i| with k the roundings inside one summand.  So
+//  - the factor in front of eps counts SUMMANDS: it stays 2n + 16 with n the landmark count, whatever the weights are.
+//    Taking sum w_i there instead understates the bound by 2 (n - sum w_i) eps scale, which is most of it when the
+//    weights are small -- exactly where the residual, and so the margin of the exit test, shrinks with them;
+//  - the magnitudes are the weighted ones: scale = sum w (bx^2 + by^2) + gamma^2 (...) + sum(w) (d1^2 + d2^2), each
+//    term the weighted moment the unweighted bound has there;
+//  - the product w_i * bx_i (Moments::add) is one more rounding per summand wherever w_i is not 1: extra = 4 covers it,
+//    the rounding of sum w_i in the count term and their products with the rounded moments, twice over.  Where every
+//    weight that takes part is 1 the products are exact and extra = 0: the bound is then the masked solve's, bit for bit.
 template <typename T>
-PNP_DEV T res2_error_bound(T n, T sw0, T gam, T d1, T d2, T tr_m0, T tr_mw, T u11_plus_u22, T u33)
+PNP_DEV T res2_error_bound(T n, T extra, T wsum, T sw0, T gam, T d1, T d2, T tr_m0, T tr_mw, T u11_plus_u22, T u33)
 {
-    const T scale = sw0 + (gam * gam) * t_fma(tr_m0, u11_plus_u22, tr_mw * u33) + n * t_fma(d1, d1, d2 * d2);
+    const T scale = sw0 + (gam * gam) * t_fma(tr_m0, u11_plus_u22, tr_mw * u33) + wsum * t_fma(d1, d1, d2 * d2);
     const T eps = (sizeof(T) == 8) ? T(1.1102230246251565e-16) : T(5.9604645e-8);
-    return (T(2) * n + T(16)) * eps * scale;
+    return (T(2) * n + (T(16) + extra)) * eps * scale;
 }
 
 template <typename T>
@@ -291,7 +309,7 @@ PNP_DEV void qeif_loop(const Pts& pts, const T* __restrict__ sP, const T* __rest
     bool done = false;
     int iters = 0;
     const T w = prm.meas_w;                               // 1 / (9 / f^2) (:2844-2852)
-    const T nT = T(pts.count(n));                        // landmarks taking part (the visible ones under a mask)
+    const T nT = pts.template total<T>(n);               // landmarks taking part (the visible ones under a mask), or the sum of their weights
 
     for (int it = 0; it < prm.max_it; ++it) {
         if (LPP == 1) { if (__all_sync(0xffffffffu, done)) break; }
@@ -322,6 +340,7 @@ PNP_DEV void qeif_loop(const Pts& pts, const T* __restrict__ sP, const T* __rest
                 const T th0 = sP[3 * i], th1 = sP[3 * i + 1], th2 = sP[3 * i + 2];
                 T bx, by;
                 pts.get(i, bx, by);
+                const T wi = (T)pts.weight(i);                // Q^-1 rows of the landmark times its weight
                 const T P1 = th0 * p1[0] + th1 * p1[1] + th2 * p1[2];
                 const T P2 = th0 * p2[0] + th1 * p2[1] + th2 * p2[2];
                 const T P3 = th0 * p3[0] + th1 * p3[1] + th2 * p3[2];
@@ -342,15 +361,16 @@ PNP_DEV void qeif_loop(const Pts& pts, const T* __restrict__ sP, const T* __rest
                 const T vx = dzx + hxq, vy = dzy + hyq;       // z - hx + H x (:2898)
 #pragma unroll
                 for (int a = 0; a < 4; ++a) {
+                    const T wHx = wi * Hx[a], wHy = wi * Hy[a];
 #pragma unroll
                     for (int b = a; b < 4; ++b)
-                        qq[sidx<4>(a, b)] = t_fma(Hx[a], Hx[b], t_fma(Hy[a], Hy[b], qq[sidx<4>(a, b)]));
-                    qd1[a] += Hx[a];
-                    qd2[a] += Hy[a];
-                    hv[a] = t_fma(Hx[a], vx, t_fma(Hy[a], vy, hv[a]));
+                        qq[sidx<4>(a, b)] = t_fma(wHx, Hx[b], t_fma(wHy, Hy[b], qq[sidx<4>(a, b)]));
+                    qd1[a] += wHx;
+                    qd2[a] += wHy;
+                    hv[a] = t_fma(wHx, vx, t_fma(wHy, vy, hv[a]));
                 }
-                hv[4] += vx; hv[5] += vy;
-                res2 = t_fma(dzx, dzx, t_fma(dzy, dzy, res2));
+                hv[4] += wi * vx; hv[5] += wi * vy;
+                res2 = t_fma(wi * dzx, dzx, t_fma(wi * dzy, dzy, res2));
             }
             group_sum_arr<LPP>(qq); group_sum_arr<LPP>(qd1); group_sum_arr<LPP>(qd2); group_sum_arr<LPP>(hv);
             res2 = group_sum<LPP>(res2);
@@ -368,7 +388,8 @@ PNP_DEV void qeif_loop(const Pts& pts, const T* __restrict__ sP, const T* __rest
                     const T P3 = th0 * p3[0] + th1 * p3[1] + th2 * p3[2];
                     const T dzx = bx - (P1 - bx * P3 + x[4]);
                     const T dzy = by - (P2 - by * P3 + x[5]);
-                    res2 = t_fma(dzx, dzx, t_fma(dzy, dzy, res2));
+                    const T wi = (T)pts.weight(i);
+                    res2 = t_fma(wi * dzx, dzx, t_fma(wi * dzy, dzy, res2));
                 }
                 res2 = group_sum<LPP>(res2);
             }
@@ -407,11 +428,12 @@ PNP_DEV void qeif_loop(const Pts& pts, const T* __restrict__ sP, const T* __rest
             const T s1 = dot3<T>(m0, p1) - dot3<T>(mom.mx, p3), s2 = dot3<T>(m0, p2) - dot3<T>(mom.my, p3);
             hv[4] = mom.sx0 + s1;
             hv[5] = mom.sy0 + s2;
-            if (RES_MOM) {                                    // ||z - hx||^2 from the moments (:2905-2907)
+            if constexpr (RES_MOM) {                          // ||z - hx||^2 from the moments (:2905-2907)
                 const T qa = dot3<T>(mom.mx, p1) + dot3<T>(mom.my, p2) - dot3<T>(mom.mw, p3);
                 const T sgg = dot3<T>(p1, t1) - T(2) * dot3<T>(p1, t2) + dot3<T>(p2, t3v) - T(2) * dot3<T>(p2, t4) + dot3<T>(p3, t7);
                 res2 = res2_combine<T>(mom.sw0, mom.sx0, mom.sy0, nT, x[4], x[5], T(1), qa, s1, s2, sgg);
-                res2_err = res2_error_bound<T>(nT, mom.sw0, T(1), x[4], x[5], M0[0] + M0[3] + M0[5], mom.Mw[0] + mom.Mw[3] + mom.Mw[5],
+                res2_err = res2_error_bound<T>(pts.landmarks(nT), pts.template extra_roundings<T>(), nT, mom.sw0, T(1), x[4], x[5],
+                                               M0[0] + M0[3] + M0[5], mom.Mw[0] + mom.Mw[3] + mom.Mw[5],
                                                dot3<T>(p1, p1) + dot3<T>(p2, p2), dot3<T>(p3, p3));
             }
         }
@@ -481,19 +503,34 @@ PNP_DEV void solve_qeif_with_tail(const Pts& pts, const T* __restrict__ sP, cons
     qeif_loop<T, LPP, Pts, true, false, true>(pts, sP, sC, n, sub, prm, mom, x_tail, out);
 }
 
-// No points inside the loop (moment mapping)
+// No points inside the loop (moment mapping).  landmarks() and extra_roundings() feed res2_error_bound: without weights the
+// count in the pattern constants is the number of landmarks and no summand carries a weight's rounding.
 struct NoPts {
     template <typename T> PNP_DEV void get(int, T& bx, T& by) const { bx = T(0); by = T(0); }
     PNP_DEV bool vis(int) const { return true; }
     PNP_DEV int count(int n) const { return n; }
+    PNP_DEV float weight(int) const { return 1.0f; }
+    template <typename U> PNP_DEV U total(int n) const { return U(n); }
+    template <typename U> PNP_DEV U landmarks(U from_constants) const { return from_constants; }
+    template <typename U> PNP_DEV U extra_roundings() const { return U(0); }
+    static constexpr bool kWeighted = false;
 };
 
+// ... with per-landmark weights: the sum of the weights (the pattern constants' count), the number of landmarks taking part
+// and whether a weight other than 1 takes part come from the moments pass
 template <typename T>
+struct NoPtsWeighted : NoPts {
+    T wsum, nland, extra;
+    template <typename U> PNP_DEV U total(int) const { return wsum; }
+    template <typename U> PNP_DEV U landmarks(U) const { return nland; }
+    template <typename U> PNP_DEV U extra_roundings() const { return extra; }
+};
+
+template <typename T, typename NP = NoPts>
 PNP_DEV void solve_qeif_from_moments(const Moments<T>& mom, const T* __restrict__ sC, const SolverPrm<T>& prm, T (&x_tail)[12],
-                                     Result<T>& out)
+                                     Result<T>& out, const NP& none = NP())
 {
-    NoPts none;
-    qeif_loop<T, 1, NoPts, true, true>(none, nullptr, sC, (int)sC[9], 0, prm, mom, x_tail, out);
+    qeif_loop<T, 1, NP, true, true>(none, nullptr, sC, (int)sC[9], 0, prm, mom, x_tail, out);
 }
 
 // -------------------------------------------------------------------------------------------
@@ -806,7 +843,7 @@ PNP_DEV T lm_residual_direct(const Pts& pts, const T* __restrict__ sP, int n, in
         const T th[3] = { sP[3 * i], sP[3 * i + 1], sP[3 * i + 2] };
         T bx, by;
         pts.get(i, bx, by);
-        lr.add(th, bx, by, rr);
+        lr.add(th, bx, by, rr, (T)pts.weight(i));
     }
     return t_sqrt(group_sum<LPP>(rr));
 }
@@ -852,13 +889,15 @@ PNP_DEV void solve_lm(const Pts& pts, const T* __restrict__ sP, const T* __restr
             const T g1 = a - bx * c, g2 = b - by * c;     // hu1_bar, hu2_bar (:3738-3741)
             const T rx = bx - (gam * g1 + d1);            // z - hx (:3750, :2679)
             const T ry = by - (gam * g2 + d2);
-            const T v3 = bx * rx + by * ry;
+            const T wi = (T)pts.weight(i);                // rows times sqrt(w): J^T (z - hx) and the residual gain w
+            const T wrx = wi * rx, wry = wi * ry;
+            const T v3 = bx * wrx + by * wry;
 #pragma unroll
             for (int k = 0; k < 3; ++k) {
-                r.r1[k] = t_fma(th[k], rx, r.r1[k]); r.r2[k] = t_fma(th[k], ry, r.r2[k]); r.r3[k] = t_fma(th[k], v3, r.r3[k]);
+                r.r1[k] = t_fma(th[k], wrx, r.r1[k]); r.r2[k] = t_fma(th[k], wry, r.r2[k]); r.r3[k] = t_fma(th[k], v3, r.r3[k]);
             }
-            r.q1 += rx; r.q2 += ry; r.qg = t_fma(g1, rx, t_fma(g2, ry, r.qg));
-            rr = t_fma(rx, rx, t_fma(ry, ry, rr));
+            r.q1 += wrx; r.q2 += wry; r.qg = t_fma(g1, wrx, t_fma(g2, wry, r.qg));
+            rr = t_fma(wrx, rx, t_fma(wry, ry, rr));
         }
         group_sum_arr<LPP>(r.r1); group_sum_arr<LPP>(r.r2); group_sum_arr<LPP>(r.r3);
         r.q1 = group_sum<LPP>(r.q1); r.q2 = group_sum<LPP>(r.q2); r.qg = group_sum<LPP>(r.qg); rr = group_sum<LPP>(rr);
@@ -1021,7 +1060,8 @@ PNP_DEV void eif2_loop(const Pts& pts, const T* __restrict__ sP, const T* __rest
                 const T c = th0 * u3[0] + th1 * u3[1] + th2 * u3[2];
                 const T rx = bx - (gam * (a - bx * c) + d1);
                 const T ry = by - (gam * (b - by * c) + d2);
-                res2 = t_fma(rx, rx, t_fma(ry, ry, res2));
+                const T wi = (T)pts.weight(i);
+                res2 = t_fma(wi * rx, rx, t_fma(wi * ry, ry, res2));
             }
             res2 = group_sum<LPP>(res2);
         }
@@ -1066,11 +1106,11 @@ PNP_DEV void eif2_loop(const Pts& pts, const T* __restrict__ sP, const T* __rest
             zeta[D1] = t_fma(w, mom.gsx0() + gam * gc.s1, zeta[D1]);
             zeta[D2] = t_fma(w, mom.gsy0() + gam * gc.s2, zeta[D2]);
             zeta[GG] = t_fma(w, qa + gam * gc.sgg, zeta[GG]);
-            if (RES_MOM) {                                           // :2176-2178 from the moments
+            if constexpr (RES_MOM) {                                 // :2176-2178 from the moments
                 res2 = res2_from_moments<T, M>(mom, sC, gc, qa, gam, d1, d2);
                 r2_new = res2;
-                e_new = res2_error_bound<T>(sC[9], mom.gsw0(), gam, d1, d2, sC[0] + sC[3] + sC[5],
-                                            mom.gMw(0) + mom.gMw(3) + mom.gMw(5), u11 + u22, u33);
+                e_new = res2_error_bound<T>(pts.landmarks(sC[9]), pts.template extra_roundings<T>(), sC[9], mom.gsw0(), gam, d1, d2,
+                                            sC[0] + sC[3] + sC[5], mom.gMw(0) + mom.gMw(3) + mom.gMw(5), u11 + u22, u33);
             }
         }
         // ---- update, the nine constraint rows (:3753-3772, Jacobians :3787-3823), collected per 3 x 3 block.  Row k adds
@@ -1135,11 +1175,11 @@ PNP_DEV void solve_eif2_with_tail(const Pts& pts, const T* __restrict__ sP, cons
     eif2_loop<T, LPP, Pts, Moments<T>, false, true>(pts, sP, sC, n, sub, prm, mom, x_tail, out);
 }
 
-template <typename T, typename M>
-PNP_DEV void solve_eif2_from_moments(const M& mom, const T* __restrict__ sC, const SolverPrm<T>& prm, T (&x_tail)[12], Result<T>& out)
+template <typename T, typename M, typename NP = NoPts>
+PNP_DEV void solve_eif2_from_moments(const M& mom, const T* __restrict__ sC, const SolverPrm<T>& prm, T (&x_tail)[12], Result<T>& out,
+                                     const NP& none = NP())
 {
-    NoPts none;
-    eif2_loop<T, 1, NoPts, M, true>(none, nullptr, sC, (int)sC[9], 0, prm, mom, x_tail, out);
+    eif2_loop<T, 1, NP, M, true>(none, nullptr, sC, (int)sC[9], 0, prm, mom, x_tail, out);
 }
 
 // -------------------------------------------------------------------------------------------
@@ -1177,7 +1217,8 @@ PNP_DEV T f2_residual_direct(const Pts& pts, const T* __restrict__ sP, int n, in
         const T dx = th0 * f.pxn[0] + th1 * f.pxn[1] + th2 * f.pxn[2] + f.pxn[3];
         const T dy = th0 * f.pyn[0] + th1 * f.pyn[1] + th2 * f.pyn[2] + f.pyn[3];
         const T ex = bx * db - dx, ey = by * db - dy;
-        rx2 = t_fma(ex, ex, rx2); ry2 = t_fma(ey, ey, ry2);
+        const T wi = (T)pts.weight(i);
+        rx2 = t_fma(wi * ex, ex, rx2); ry2 = t_fma(wi * ey, ey, ry2);
     }
     rx2 = group_sum<LPP>(rx2); ry2 = group_sum<LPP>(ry2);
     const T nx = t_sqrt(rx2), ny = t_sqrt(ry2);
@@ -1313,12 +1354,14 @@ PNP_DEV void solve_linear_f1(const Pts& pts, const T* __restrict__ sP, int n, in
             if (t_abs(Delta) <= eps) Delta = (Delta < T(0)) ? -eps : eps;
             const T iD = t_rcp<T>(Delta);                 // |Delta| >= 1e-7 after the clamp: normal range
             const T a[4] = { th0 * iD, th1 * iD, th2 * iD, iD };                          // get_A_i :3048-3062
+            const T wi = (T)pts.weight(i);                // rows times sqrt(w)
 #pragma unroll
             for (int p = 0; p < 4; ++p) {
+                const T wa = wi * a[p];
 #pragma unroll
-                for (int q = p; q < 4; ++q) N[sidx<4>(p, q)] = t_fma(a[p], a[q], N[sidx<4>(p, q)]);
-                bxv[p] = t_fma(a[p], bx, bxv[p]);
-                byv[p] = t_fma(a[p], by, byv[p]);
+                for (int q = p; q < 4; ++q) N[sidx<4>(p, q)] = t_fma(wa, a[q], N[sidx<4>(p, q)]);
+                bxv[p] = t_fma(wa, bx, bxv[p]);
+                byv[p] = t_fma(wa, by, byv[p]);
             }
         }
         group_sum_arr<LPP>(N); group_sum_arr<LPP>(bxv); group_sum_arr<LPP>(byv);
@@ -1344,7 +1387,8 @@ PNP_DEV void solve_linear_f1(const Pts& pts, const T* __restrict__ sP, int n, in
                 const T a3 = t_rcp<T>(Delta), a0 = th0 * a3, a1 = th1 * a3, a2 = th2 * a3;
                 const T ex = bx - (a0 * pn[0] + a1 * pn[1] + a2 * pn[2] + a3 * pn[6]);
                 const T ey = by - (a0 * pn[3] + a1 * pn[4] + a2 * pn[5] + a3 * pn[7]);
-                r2 = t_fma(ex, ex, t_fma(ey, ey, r2));
+                const T wi = (T)pts.weight(i);
+                r2 = t_fma(wi * ex, ex, t_fma(wi * ey, ey, r2));
             }
             r2 = group_sum<LPP>(r2);
             res = t_sqrt(r2);

@@ -29,9 +29,12 @@ struct PtsRow {
         bx = p.x;
         by = p.y;
     }
-    // every selected landmark takes part (the masked accessor below overrides these two)
+    // every selected landmark takes part, with weight 1 (the masked and weighted accessors below override these)
     PNP_DEV bool vis(int) const { return true; }
     PNP_DEV int count(int n) const { return n; }
+    PNP_DEV float weight(int) const { return 1.0f; }
+    template <typename U> PNP_DEV U total(int n) const { return U(count(n)); }   // sum of the weights taking part
+    static constexpr bool kWeighted = false;
 };
 
 // bit j % 32 of word j / 32: landmark j of the caller's 0..n_total-1 numbering is visible (per-problem mask)
@@ -45,7 +48,39 @@ struct PtsMasked : Base {
     int nvis;
     PNP_DEV bool vis(int i) const { return mask_bit(words, this->idx ? this->idx[i] : i); }
     PNP_DEV int count(int) const { return nvis; }
+    template <typename U> PNP_DEV U total(int) const { return U(nvis); }
 };
+
+// a per-landmark weight takes part iff 0 < w < +Inf as stored (0, -0, negatives, NaN and +-Inf hide the landmark)
+PNP_DEV bool weight_takes_part(float w) { return w > 0.0f && w < __int_as_float(0x7f800000); }
+
+// A point accessor with a weight per landmark (float32 row of the caller's 0..n_total-1 numbering): landmarks whose weight
+// does not take part are skipped as hidden ones are, and every per-landmark sum of the solvers gains the factor weight(i).
+// count() is the number of landmarks taking part, total() the sum of their weights.
+template <typename Base>
+struct PtsWeighted : Base {
+    const float* wrow;       // this problem's weights [n_total]
+    int nvis;
+    double wsum;
+    PNP_DEV float weight(int i) const { return __ldg(wrow + (this->idx ? this->idx[i] : i)); }
+    PNP_DEV bool vis(int i) const { return weight_takes_part(weight(i)); }
+    PNP_DEV int count(int) const { return nvis; }
+    template <typename U> PNP_DEV U total(int) const { return U(wsum); }
+    static constexpr bool kWeighted = true;
+};
+
+// landmarks taking part among the n selected ones of a weight row, and the sum of their weights (in selection order)
+PNP_DEV int count_weights(const float* wrow, const int32_t* idx, int n, double& wsum)
+{
+    int c = 0;
+    double s = 0.0;
+    for (int i = 0; i < n; ++i) {
+        const float w = __ldg(wrow + (idx ? idx[i] : i));
+        if (weight_takes_part(w)) { ++c; s += (double)w; }
+    }
+    wsum = s;
+    return c;
+}
 
 // fewer visible landmarks than this: a problem is not solved (NaN pose), its report and check statistics are NaN
 constexpr int kMinVisible = 4;

@@ -92,6 +92,39 @@ def _u32(t):
     return C.cast(ptr(t), C.POINTER(C.c_uint32))
 
 
+def _check_weights(weights, B, n_total, visible=None):
+    """weights must be a real floating [B, n_total] torch tensor or NumPy array, and excludes visible (a hidden landmark is
+    weight 0)"""
+    if visible is not None:
+        raise ValueError("weights and visible exclude each other: give a hidden landmark weight 0")
+    if torch.is_tensor(weights):
+        ok = weights.dtype.is_floating_point and not weights.dtype.is_complex
+    elif isinstance(weights, np.ndarray):
+        ok = np.issubdtype(weights.dtype, np.floating)
+    else:
+        raise ValueError("weights must be a floating torch tensor or NumPy array, not %s" % type(weights).__name__)
+    if not ok:
+        raise ValueError("weights must have a real floating dtype, not %s" % (weights.dtype,))
+    if tuple(weights.shape) != (B, n_total):
+        raise ValueError("weights must be [B, n_total] = [%d, %d], not %s" % (B, n_total, tuple(weights.shape)))
+
+
+def weights_f32(weights, device):
+    """weights -> the contiguous float32 [B, n_total] device tensor of pnpb200_solve_batch_weighted"""
+    if isinstance(weights, np.ndarray):
+        weights = torch.from_numpy(np.ascontiguousarray(weights))
+    return weights.to(device=device, dtype=torch.float32).contiguous()
+
+
+def weights_take_part(weights):
+    """bool [B, n_total]: the landmarks a weighted solve uses (0 < w < +Inf as float32), e.g. the `visible` of the masked
+    report and check entries"""
+    if isinstance(weights, np.ndarray):
+        weights = torch.from_numpy(np.ascontiguousarray(weights))
+    w = weights.to(torch.float32)
+    return (w > 0) & (w < float("inf"))
+
+
 def _batch_args(method, uv, patterns, point_index, visible):
     """the argument checks and conversions of solve_batch and solve_robust_batch (ValueError before any launch)"""
     m = _lib.METHODS[method] if isinstance(method, str) else int(method)
@@ -114,7 +147,7 @@ def _batch_args(method, uv, patterns, point_index, visible):
 
 
 def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R", "t", "euler", "res_norm", "iters", "best_pattern"),
-                visible=None):
+                visible=None, weights=None):
     """pnpb200_solve_batch on device tensors.
 
     uv [B, n_total, 2] and patterns [P, n_total, 3] are CUDA tensors of the same float dtype;
@@ -122,8 +155,14 @@ def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R
     (roll, yaw, pitch) in degrees, res_norm [B], iters [B] int32, best_pattern [B] int32.
     visible: bool [B, n_total] (torch tensor or NumPy array) -> pnpb200_solve_batch_masked: each problem is solved on its
     visible landmarks alone (those of point_index, in its order); hidden pixels are never read, and a problem with fewer
-    than 4 of them comes back NaN with iters 0 (include/pnpb200.h)."""
+    than 4 of them comes back NaN with iters 0 (include/pnpb200.h).
+    weights: real floating [B, n_total] (torch tensor or NumPy array, e.g. a detector's confidences) ->
+    pnpb200_solve_batch_weighted: each problem is a weighted fit, landmark i's information times weights[b, i].  They are
+    converted to contiguous float32 on the device whatever the dtype of uv; a weight that is not 0 < w < +Inf hides its
+    landmark as visible does.  Excludes visible (ValueError)."""
     m, dt, uv, patterns, B, n_total, idx = _batch_args(method, uv, patterns, point_index, visible)
+    if weights is not None:
+        _check_weights(weights, B, n_total, visible)
     n, idx_p = (n_total, None) if idx is None else (int(idx.shape[0]), idx.ctypes.data_as(C.POINTER(C.c_int32)))
     dev = uv.device
     o = {}
@@ -138,7 +177,8 @@ def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R
         return o
     # scratch for the moment mapping from torch's caching allocator (stream-ordered, no driver call)
     prm = _lib.default_params() if params is None else params
-    ws_query = lib.pnpb200_workspace_bytes if visible is None else lib.pnpb200_workspace_bytes_masked
+    ws_query = (lib.pnpb200_workspace_bytes_weighted if weights is not None else
+                lib.pnpb200_workspace_bytes if visible is None else lib.pnpb200_workspace_bytes_masked)
     ws_bytes = int(ws_query(C.c_int(m), C.c_int(dt), C.c_int64(B), C.c_int(int(patterns.shape[0])), C.c_int(int(prm.mapping))))
     ws = None
     if ws_bytes > 0 and not prm.workspace:
@@ -146,6 +186,18 @@ def solve_batch(method, uv, patterns, K, point_index=None, params=None, want=("R
         prm = _copy_params(prm)
         prm.workspace, prm.workspace_bytes = ws.data_ptr(), ws_bytes
     params = prm
+    if weights is not None:
+        w32 = weights_f32(weights, dev)
+        with torch.cuda.device(dev):
+            rc = lib.pnpb200_solve_batch_weighted(
+                m, dt, B, n_total, n, ptr(uv), ptr(patterns), int(patterns.shape[0]), idx_p, Kp, C.byref(params),
+                ptr(o.get("R")), ptr(o.get("t")), ptr(o.get("euler")), ptr(o.get("res_norm")),
+                None if o.get("iters") is None else C.cast(ptr(o["iters"]), C.POINTER(C.c_int32)),
+                None if o.get("best_pattern") is None else C.cast(ptr(o["best_pattern"]), C.POINTER(C.c_int32)),
+                C.cast(ptr(w32), C.POINTER(C.c_float)), _stream_ptr(dev))
+        check(rc, "pnpb200_solve_batch_weighted")
+        _lib.count_launch(1)
+        return o
     if visible is not None:
         words = visible_words(visible, dev)
         with torch.cuda.device(dev):
@@ -700,7 +752,7 @@ class PNP_SOLVER(object):
         """PNP_SOLVER_LIB.py:205-430 (rows follow the image dict's key order, :3069)"""
         return self._solve_single("linear_f1", np_point_image_dict, np_point_3d_pretransfer_dict, list(np_point_image_dict.keys()))
 
-    def solve_pnp_batch(self, uv, method=None, key_list="default", params=None, check=None, visible=None, robust=None):
+    def solve_pnp_batch(self, uv, method=None, key_list="default", params=None, check=None, visible=None, robust=None, weights=None):
         """The per-problem script loop as one launch.
 
         uv: [B, n_total, 2] pixels (or [B, n_total, 3] homogeneous image points, third entry as the reference's
@@ -716,8 +768,14 @@ class PNP_SOLVER(object):
         rejected by their reprojection distance and each problem re-solved on its inliers; the dict then also holds inliers,
         rounds and robust_status, and the check (if asked for) runs on the inliers.  With samples (and any of consensus_px,
         confidence, seed, idx0) the loop starts from the hypothesis stage's consensus set (RANSAC), and the dict also holds
-        consensus and drawn."""
+        consensus and drawn.
+        weights: real floating [B, n_total] per-landmark weights (e.g. a detector's confidences, or (meas_sigma_px / sigma)^2
+        for a landmark of noise sigma px) -> each problem is a weighted fit of its landmarks (see solve_batch); converted to
+        contiguous float32 on the device.  Excludes visible (a hidden landmark is weight 0) and robust (ValueError).  The check
+        then runs on the landmarks that take part (0 < w < +Inf)."""
         method = method or self.method
+        if weights is not None and robust is not None:
+            raise ValueError("weights and robust exclude each other")
         if robust is not None:
             hyp_keys = {"samples", "consensus_px", "confidence", "seed", "idx0"}
             unknown = set(robust) - {"max_rounds", "k", "floor_px", "min_inliers"} - hyp_keys
@@ -735,12 +793,17 @@ class PNP_SOLVER(object):
             uv = torch.from_numpy(np.ascontiguousarray(uv))
         if visible is not None:
             _check_visible(visible, int(uv.shape[0]), len(all_keys))
+        if weights is not None:
+            _check_weights(weights, int(uv.shape[0]), len(all_keys), visible)
         uv, K = self._uv_and_K(uv.to(device=self.device, dtype=self._tdtype()))
         ck = ("all", self.dtype_code)
         if ck not in self._dev_cache:
             self._dev_cache[ck] = self._pack_patterns(self.np_point_3d_pretransfer_dict_list, all_keys)
         prm = params if params is not None else self.params
-        if robust is None:
+        if weights is not None:
+            out = solve_batch(method, uv, self._dev_cache[ck], K, point_index=idx, params=prm, weights=weights)
+            visible = weights_take_part(weights).to(self.device)
+        elif robust is None:
             out = solve_batch(method, uv, self._dev_cache[ck], K, point_index=idx, params=prm, visible=visible)
         else:
             out = solve_robust_batch(method, uv, self._dev_cache[ck], K, point_index=idx, params=prm, visible=visible, **robust)
